@@ -3,6 +3,7 @@
 trajectory, and ms per denoise step).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp32|fp16] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one denoise step (graph + Ponita forward + VE/VP/D3PM update) of one batch of synthetic crystals;
 the N=1 workload is BASELINE.json configs[1] (C2: 1024 crystals x 40 atoms, 5 A cutoff, max_neighbors 8 as in the
@@ -39,6 +40,33 @@ T_STEPS = 1000          # Makefile:7 num_timesteps -> 999 denoise steps per traj
 Z = 90
 RADIUS = 5.0
 O, C, D, L, MONO = 16, 128, 256, 5, 83
+DUMP_LIMIT = 64_000_000  # bytes of --dump-outputs in all, .npy headers included
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy, float32 and float64 arrays as they are, any other dtype as float64.  Above
+    DUMP_LIMIT bytes in all, the arrays of each row count that holds more than 1 MB keep one seeded sample of their rows
+    (per-atom arrays the same atoms, per-crystal arrays the same crystals), so the dumps of two builds run with the same
+    arguments compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        host[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes + 4096 for a in host.values())            # 4 KB per .npy header is ample
+    per_rows = {}
+    for a in host.values():
+        if a.ndim:
+            per_rows[a.shape[0]] = per_rows.get(a.shape[0], 0) + a.nbytes
+    big = {n: b for n, b in per_rows.items() if b > 1 << 20}
+    large = sum(big.values())
+    budget = DUMP_LIMIT - (total - large)                           # left for the rows of the sampled arrays
+    rows = ({n: np.sort(np.random.default_rng(n).choice(n, max(1, n * budget // large), replace=False)) for n in big}
+            if total > DUMP_LIMIT else {})
+    for name, a in host.items():
+        if a.ndim and a.shape[0] in rows:
+            a = a[rows[a.shape[0]]]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_weights(atoms_per_crystal: int):
@@ -278,6 +306,8 @@ def run_train(args):
     e1.record()
     torch.cuda.synchronize(dev)
     launches = _lib.launch_count() - l0
+    if args.dump_outputs and rank == 0:        # before the breakdown steps below train further
+        dump_outputs(args.dump_outputs, {"loss": te.loss, "grad": p.grad, "params": p.data})
     ms = e0.elapsed_time(e1) / args.steps
     if world > 1:
         tmax = torch.tensor([ms], device=dev)
@@ -311,7 +341,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workload", default="sample", choices=["sample", "train"])
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 10)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default=os.environ.get("ARREAU_PRECISION", "fp16"), choices=["fp32", "fp16"],
@@ -336,7 +366,19 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e-trajectory", action="store_true", help="skip the whole-trajectory e2e leg (~7 s at C2)")
     ap.add_argument("--no-other-precision", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0's "
+                         "batch): the sampler state and model outputs, or with --workload train the loss, gradient and "
+                         "updated parameters; a seeded sample of rows above 64 MB in all")
     args = ap.parse_args()
+    if args.trajectory and args.steps is not None:
+        ap.error("--trajectory times every step of one trajectory; it takes no --steps")
+    if args.steps is None:
+        args.steps = 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         return run_reference(args)
@@ -421,6 +463,10 @@ def main():
     epa_last = eng.num_edges() / N
     overflow = int(eng.overflow_flag.item())
     clk = clocks.summary()
+    if args.dump_outputs and rank == 0:        # before the legs below overwrite the engine's state
+        dump_outputs(args.dump_outputs, {"frac": eng.frac, "types": eng.types, "lengths": eng.lengths,
+                                         "lattice": eng.lattice, "score": eng.score, "logits": eng.logits,
+                                         "len0": eng.len0})
 
     # ---- end to end: state + noise from pinned host memory every step, result read back --------------
     pin = lambda a: torch.as_tensor(a).pin_memory()  # noqa: E731
