@@ -115,6 +115,8 @@ SIGNATURES = {
     "arreau_d3pm_q_sample": [vp, vp, vp, vp, vp, i32, i32, vp, vp],
     "arreau_training_loss": [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f64, f64, i32, i32, i32, i32, f64, vp, vp, vp,
                              vp, vp, vp],
+    "arreau_eval_noise": [C.c_uint64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp],
+    "arreau_eval_loss": [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f64, f64, i32, i32, i32, i32, vp, vp, vp],
     "arreau_train_layout": [i32, i32, i32, C.POINTER(TrainLayout)],
     "arreau_ponita_backward_workspace_bytes": [i32, i64, i32, i32],
     "arreau_ponita_backward": [vp, C.POINTER(TrainLayout), C.POINTER(Weights), C.POINTER(Workspace), vp, vp, vp, vp, vp,

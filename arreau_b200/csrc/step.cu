@@ -7,7 +7,7 @@ long long g_arreau_launches = 0;
 
 namespace {
 
-// ---- Philox4x32-10 counter-based generator (Salmon et al., SC'11) for throughput-run noise ----
+// ---- Philox4x32-10 counter-based generator (Salmon et al., SC'11) for throughput-run and evaluation noise ----
 __device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
   const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
   const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
@@ -31,6 +31,15 @@ __device__ __forceinline__ double u01(uint32_t a, uint32_t b) {   // 53-bit unif
   const uint64_t v = ((uint64_t)a << 21) ^ (uint64_t)(b >> 11);
   return (double)(v & ((1ull << 53) - 1)) * (1.0 / 9007199254740992.0);
 }
+// Box-Muller: two N(0,1) from one Philox output
+__device__ __forceinline__ void box_muller(const uint32_t (&r)[4], double& v0, double& v1) {
+  const double u1 = 1.0 - u01(r[0], r[1]), u2 = u01(r[2], r[3]);   // u1 in (0,1]
+  const double rad = sqrt(-2.0 * log(u1));
+  double s, c;
+  sincospi(2.0 * u2, &s, &c);
+  v0 = rad * c;
+  v1 = rad * s;
+}
 
 __global__ void step_noise_kernel(uint64_t seed, int step, long long n_normal, long long n_uniform,
                                   double* __restrict__ z_len, long long n_len, double* __restrict__ z_frac,
@@ -40,12 +49,9 @@ __global__ void step_noise_kernel(uint64_t seed, int step, long long n_normal, l
   uint32_t r[4];
   if (idx < (n_normal + 1) / 2) {   // Box-Muller: two normals per counter
     philox4x32_10(seed, (uint64_t)idx, (uint32_t)step, 0u, r);
-    const double u1 = 1.0 - u01(r[0], r[1]), u2 = u01(r[2], r[3]);   // u1 in (0,1]
-    const double rad = sqrt(-2.0 * log(u1));
-    double s, c;
-    sincospi(2.0 * u2, &s, &c);
     const long long k0 = 2 * idx, k1 = 2 * idx + 1;
-    const double v0 = rad * c, v1 = rad * s;
+    double v0, v1;
+    box_muller(r, v0, v1);
     if (k0 < n_len) z_len[k0] = v0; else z_frac[k0 - n_len] = v0;
     if (k1 < n_normal) {
       if (k1 < n_len) z_len[k1] = v1; else z_frac[k1 - n_len] = v1;
@@ -55,6 +61,53 @@ __global__ void step_noise_kernel(uint64_t seed, int step, long long n_normal, l
     philox4x32_10(seed, (uint64_t)idx, (uint32_t)step, 1u, r);
     u[2 * idx] = u01(r[0], r[1]);
     if (2 * idx + 1 < n_uniform) u[2 * idx + 1] = u01(r[2], r[3]);
+  }
+}
+
+// Per-crystal keyed draws of one evaluation batch (arreau_eval_noise).  Key = seed, counter = {crystal id (64 bits),
+// index within the crystal, stream tag}; tags 2..5 keep the counters apart from arreau_step_noise's tags 0 and 1.
+// Work items: [0, G) one per crystal (t, eps_l), [G, G + 2N) two per atom (eps_x), then ceil(Z/2) per atom (u).
+constexpr uint32_t kTagTimestep = 2, kTagLattice = 3, kTagFrac = 4, kTagType = 5;
+
+__global__ void eval_noise_kernel(uint64_t seed, int G, int N, int Z, int T, const int64_t* __restrict__ crystal_id,
+                                  const int32_t* __restrict__ atom_offset, const int32_t* __restrict__ crystal_of_atom,
+                                  int32_t* __restrict__ t_crystal, double* __restrict__ eps_x, double* __restrict__ u,
+                                  double* __restrict__ eps_l) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int H = (Z + 1) / 2;
+  uint32_t r[4];
+  if (idx < G) {
+    const int g = (int)idx;
+    const uint64_t id = (uint64_t)crystal_id[g];
+    philox4x32_10(seed, id, 0u, kTagTimestep, r);
+    t_crystal[g] = min(1 + (int)(u01(r[0], r[1]) * (double)T), T);      // U{1..T}
+    double v[4];
+    philox4x32_10(seed, id, 0u, kTagLattice, r);
+    box_muller(r, v[0], v[1]);
+    philox4x32_10(seed, id, 1u, kTagLattice, r);
+    box_muller(r, v[2], v[3]);
+#pragma unroll
+    for (int d = 0; d < 3; ++d) eps_l[3 * (size_t)g + d] = v[d];
+    return;
+  }
+  long long j = idx - G;
+  if (j < 2LL * N) {
+    const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
+    const uint32_t a = (uint32_t)(b - atom_offset[g]);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagFrac, r);
+    double v0, v1;
+    box_muller(r, v0, v1);
+    eps_x[3 * (size_t)b + 2 * k] = v0;
+    if (k == 0) eps_x[3 * (size_t)b + 1] = v1;
+    return;
+  }
+  j -= 2LL * N;
+  if (j < (long long)N * H) {
+    const int b = (int)(j / H), k = (int)(j % H), g = crystal_of_atom[b];
+    const uint32_t a = (uint32_t)(b - atom_offset[g]);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], a * (uint32_t)H + k, kTagType, r);
+    u[(size_t)b * Z + 2 * k] = u01(r[0], r[1]);
+    if (2 * k + 1 < Z) u[(size_t)b * Z + 2 * k + 1] = u01(r[2], r[3]);
   }
 }
 
@@ -124,6 +177,20 @@ extern "C" int arreau_step_noise(uint64_t seed, int32_t step, int32_t G, int32_t
   if (!z_len || !z_frac || !u) return ARREAU_ERR_NULL;
   step_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(seed, step, n_normal, n_uniform,
                                                                                      z_len, n_len, z_frac, u, nullptr);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+extern "C" int arreau_eval_noise(uint64_t seed, int32_t G, int32_t N, int32_t Z, int32_t num_steps,
+                                 const int64_t* crystal_id, const int32_t* atom_offset, const int32_t* crystal_of_atom,
+                                 int32_t* t_crystal, double* eps_x, double* u, double* eps_l, void* stream) {
+  if (G < 0 || N < 0 || Z <= 1 || Z > 128 || num_steps <= 0) return ARREAU_ERR_BAD_SHAPE;
+  if (G == 0) return ARREAU_OK;
+  if (!crystal_id || !atom_offset || !t_crystal || !eps_l || (N > 0 && (!crystal_of_atom || !eps_x || !u)))
+    return ARREAU_ERR_NULL;
+  const long long work = (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
+  eval_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      seed, G, N, Z, num_steps, crystal_id, atom_offset, crystal_of_atom, t_crystal, eps_x, u, eps_l);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

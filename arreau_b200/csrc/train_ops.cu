@@ -6,6 +6,8 @@
 //   VP_lattice.forward          diffusion/diffusion_helpers.py:156-163
 //   the three-term loss         diffusion/diffusion_loss.py:95-110,253-274, diffusion/d3pm.py:74-117,145-163
 //                               and its gradient with respect to the network outputs
+//   the same loss per crystal       for evaluation (no gradients): the per-atom terms of the training loss summed
+//                                   over each crystal's own atoms
 // The random draws are inputs (the reference's torch CPU stream is replayed by the host, or a device generator
 // fills them); nothing here draws numbers.
 #include "common.cuh"
@@ -149,6 +151,8 @@ __device__ __forceinline__ double post_logit(const Posterior& q, int d, double s
 
 constexpr int kPer = 4;   // Z <= 128
 
+// kGrad = false (evaluation): the same per-atom terms with every gradient store compiled out
+template <bool kGrad>
 __global__ void __launch_bounds__(256)
 atom_loss_kernel(const float* __restrict__ score, const float* __restrict__ logits, const double* __restrict__ target_eps,
                  const int64_t* __restrict__ types0, const int64_t* __restrict__ types_t,
@@ -168,9 +172,11 @@ atom_loss_kernel(const float* __restrict__ score, const float* __restrict__ logi
       double a = fmod(fabs(delta), 1.0);
       a = fmin(fmax(a, 0.0), 1.0);
       const double wdist = fmin(a, 1.0 - a);
-      const double sgn = (double)((delta > 0.0) - (delta < 0.0));
-      const double branch = (a < 1.0 - a) ? 1.0 : ((a > 1.0 - a) ? -1.0 : 0.0);
-      dscore[3 * (size_t)b + lane] = (float)(2.0 * wdist * branch * sgn * invN);
+      if constexpr (kGrad) {
+        const double sgn = (double)((delta > 0.0) - (delta < 0.0));
+        const double branch = (a < 1.0 - a) ? 1.0 : ((a > 1.0 - a) ? -1.0 : 0.0);
+        dscore[3 * (size_t)b + lane] = (float)(2.0 * wdist * branch * sgn * invN);
+      }
       w2 = wdist * wdist;
     }
     const double w0 = __shfl_sync(0xffffffffu, w2, 0), w1 = __shfl_sync(0xffffffffu, w2, 1),
@@ -190,12 +196,13 @@ atom_loss_kernel(const float* __restrict__ score, const float* __restrict__ logi
   const int x0 = (int)types0[b];
   // softmax of the predicted logits
   double lg[kPer], s[kPer];
-  double mx = -INFINITY;
+  double mx = -INFINITY, l_x0 = 0.0;
 #pragma unroll
   for (int r = 0; r < kPer; ++r) {
     const int d = lane + 32 * r;
     lg[r] = d < Z ? (double)logits[(size_t)b * Z + d] : -INFINITY;
     mx = fmax(mx, lg[r]);
+    if (d == x0) l_x0 = lg[r];
   }
   mx = warp_max(mx);
   double sum = 0.0;
@@ -206,18 +213,18 @@ atom_loss_kernel(const float* __restrict__ score, const float* __restrict__ logi
   }
   sum = warp_sum(sum);
   const double lse = mx + log(sum);
-  double s_nomask = 0.0, s_mask = 0.0, l_x0 = 0.0;
+  l_x0 = warp_sum(l_x0);
+  if (lane == 0) terms[2 * (size_t)N + b] = lse - l_x0;        // cross entropy (d3pm.py:161)
+  double s_nomask = 0.0, s_mask = 0.0;
 #pragma unroll
   for (int r = 0; r < kPer; ++r) {
     const int d = lane + 32 * r;
     s[r] /= sum;
     if (d < Z && d != q.mask) s_nomask += s[r];
     if (d == q.mask) s_mask = s[r];
-    if (d == x0) l_x0 = lg[r];
   }
   s_nomask = warp_sum(s_nomask);
   s_mask = warp_sum(s_mask);
-  l_x0 = warp_sum(l_x0);
   // "true" posterior from the integer x0 (d3pm.py:81-84): softmax(log(onehot + eps))
   const double tz = (1.0 + kEps) + (double)(Z - 1) * kEps;
   const double s0_hit = (1.0 + kEps) / tz, s0_miss = kEps / tz;
@@ -261,10 +268,8 @@ atom_loss_kernel(const float* __restrict__ score, const float* __restrict__ logi
     }
   }
   vb = warp_sum(vb);
-  if (lane == 0) {
-    terms[(size_t)N + b] = vb;
-    terms[2 * (size_t)N + b] = lse - l_x0;        // cross entropy (d3pm.py:161)
-  }
+  if (lane == 0) terms[(size_t)N + b] = vb;
+  if constexpr (!kGrad) return;
   // gradient w.r.t. the logits
   const double cv = hybrid_coeff * invN;
   double dl[kPer];
@@ -333,6 +338,33 @@ loss_finish_kernel(const double* __restrict__ terms, const float* __restrict__ l
     out[0] = e_frac + (vb * hybrid_coeff + ce) + e_lat;
     out[1] = e_frac; out[2] = vb; out[3] = ce; out[4] = e_lat;
   }
+}
+
+// one thread per crystal: sums over its own atoms in atom order, so a crystal's four numbers do not depend on which
+// other crystals share the batch.  out[G][4] = {frac, vb, ce, sum_d (len0 - lengths / n)^2}
+__global__ void crystal_loss_kernel(const double* __restrict__ terms, const float* __restrict__ len0,
+                                    const double* __restrict__ lengths, const int32_t* __restrict__ atom_offset, int N,
+                                    int G, double* __restrict__ out) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= G) return;
+  const int lo = atom_offset[g], hi = atom_offset[g + 1];
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0;
+  for (int b = lo; b < hi; ++b) {
+    s0 += terms[b];
+    s1 += terms[(size_t)N + b];
+    s2 += terms[2 * (size_t)N + b];
+  }
+  const double n = (double)(hi - lo);
+  double lat = 0.0;
+#pragma unroll
+  for (int d = 0; d < 3; ++d) {
+    const double diff = (double)len0[3 * g + d] - lengths[3 * g + d] / n;        // diffusion_loss.py:262-265
+    lat += diff * diff;
+  }
+  out[4 * (size_t)g] = s0;
+  out[4 * (size_t)g + 1] = s1;
+  out[4 * (size_t)g + 2] = s2;
+  out[4 * (size_t)g + 3] = lat;
 }
 
 // torch.optim.Adam step (diffusion.py:161-210: two weight-decay groups, L2 decay folded into the gradient) with the
@@ -435,12 +467,33 @@ extern "C" int arreau_training_loss(const float* score, const float* logits, con
     return ARREAU_ERR_NULL;
   if (N <= 0 || G <= 0 || Z <= 1 || Z > 128 || num_steps <= 0) return ARREAU_ERR_BAD_SHAPE;
   const long long threads = (long long)N * 32;
-  atom_loss_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+  atom_loss_kernel<true><<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       score, logits, target_eps, types0, types_t, t_of_atom, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps,
       N, Z, hybrid_coeff, terms_scratch, dscore, dlogits);
   CUDA_LAUNCH_CHECK();
   loss_finish_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(terms_scratch, len0, lengths, atom_offset, N, G, hybrid_coeff,
                                                           loss_out, dlen0);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+extern "C" int arreau_eval_loss(const float* score, const float* logits, const float* len0, const double* target_eps,
+                                const int64_t* types0, const int64_t* types_t, const int32_t* t_of_atom,
+                                const double* lengths, const int32_t* atom_offset, const double* q_keep,
+                                const double* q_to_mask, double onestep_keep, double onestep_to_mask, int32_t num_steps,
+                                int32_t N, int32_t G, int32_t Z, double* terms_scratch, double* per_crystal,
+                                void* stream) {
+  if (!score || !logits || !len0 || !target_eps || !types0 || !types_t || !t_of_atom || !lengths || !atom_offset ||
+      !q_keep || !q_to_mask || !terms_scratch || !per_crystal)
+    return ARREAU_ERR_NULL;
+  if (N <= 0 || G <= 0 || Z <= 1 || Z > 128 || num_steps <= 0) return ARREAU_ERR_BAD_SHAPE;
+  const long long threads = (long long)N * 32;
+  atom_loss_kernel<false><<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      score, logits, target_eps, types0, types_t, t_of_atom, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps,
+      N, Z, 0.0, terms_scratch, nullptr, nullptr);
+  CUDA_LAUNCH_CHECK();
+  crystal_loss_kernel<<<(G + 127) / 128, 128, 0, (cudaStream_t)stream>>>(terms_scratch, len0, lengths, atom_offset, N, G,
+                                                                         per_crystal);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

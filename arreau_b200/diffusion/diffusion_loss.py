@@ -88,28 +88,29 @@ class DiffusionLoss(torch.nn.Module):
         return (cur if have.index is None else have.index) == (cur if want.index is None else want.index)
 
     # -- engine cache: one per (model weights, topology) --------------------------------------------
+    def packed_weights(self, net, device):
+        """The kernel layouts of net's current weights.  Engines read a packed COPY of the weights: a training step /
+        load_state_dict / callibrate in between bumps the version of the flat parameter buffer, and the copy is rebuilt
+        (ADVICE r1: sample -> train -> sample must not sample from the pre-training weights)."""
+        version = (getattr(getattr(net, "flat", None), "version", 0), getattr(net, "_pack_epoch", 0))
+        if getattr(net, "_packed", None) is None or getattr(net, "_packed_version", None) != version \
+                or not self._same_device(net._packed.device, device):
+            net.pack(device)
+            net._packed_version = version
+        return net._packed
+
     def engine_for(self, model, t_emb_weights, num_atoms, device, debug=False) -> DenoiseEngine:
         net = getattr(model, "model", model)          # PONITA_DIFFUSION.model or a bare PonitaFiberBundle
         na = tuple(int(v) for v in torch.as_tensor(num_atoms).reshape(-1).tolist())
         key = (id(net), na, str(device), debug, self.precision)
-        # the engine reads a packed COPY of the weights: a training step / load_state_dict / callibrate in between
-        # bumps the version of the flat parameter buffer, and the copy is rebuilt (ADVICE r1: sample -> train ->
-        # sample must not sample from the pre-training weights)
-        version = (getattr(getattr(net, "flat", None), "version", 0), getattr(net, "_pack_epoch", 0))
-        stale = getattr(net, "_packed_version", None) != version
+        packed = self.packed_weights(net, device)
         if self._engine is None or self._engine_key != key:
-            packed = net._packed if getattr(net, "_packed", None) is not None and not stale \
-                and self._same_device(net._packed.device, device) else net.pack(device)
-            net._packed_version = version
             fw = t_emb_weights.gaussian_fourier_proj_w if hasattr(t_emb_weights, "gaussian_fourier_proj_w") else t_emb_weights
             self._engine = DenoiseEngine(packed, self.tables, fw, na, self.cutoff, self.max_neighbors,
                                          precision=self.precision, debug=debug, device=device)
             self._engine_key = key
-        elif stale or self._engine.w is not net._packed:
-            if stale or net._packed is None:
-                net.pack(device)
-                net._packed_version = version
-            self._engine.w = net._packed
+        elif self._engine.w is not packed:
+            self._engine.w = packed
         return self._engine
 
     # -- training step (diffusion_loss.py:95-110,199-274) ---------------------------------------------
@@ -137,6 +138,48 @@ class DiffusionLoss(torch.nn.Module):
         elif tuple(na) != te.eng.topology:
             te.set_topology(na)
         return te
+
+    # -- evaluation (validation / test loss, arreau_b200/evaluation.py) --------------------------------
+    def eval_engine_for(self, net, t_emb_weights, num_atoms, device, capacity=None, headroom: float = 1.25):
+        """ONE capacity-based EvalEngine (model precision, its own buffers: the training and sampling engines are not
+        touched), re-bound to every batch topology; rebuilt only when a batch exceeds the capacity.  capacity:
+        (atoms, crystals) to size it for up front."""
+        from ..evaluation import EvalEngine
+        na = [int(v) for v in np.asarray(num_atoms).reshape(-1)]
+        ee = getattr(self, "_eval_engine", None)
+        if ee is not None and (ee.eng.precision != self.precision or not self._same_device(ee.device, device)):
+            ee = None
+        if ee is None or not ee.fits(na):
+            n_cap, g_cap = capacity if capacity is not None else (int(sum(na) * headroom), int(len(na) * headroom))
+            if ee is not None:
+                n_cap, g_cap = max(n_cap, ee.eng.N_cap), max(g_cap, ee.eng.G_cap)
+            fw = t_emb_weights.gaussian_fourier_proj_w if hasattr(t_emb_weights, "gaussian_fourier_proj_w") else t_emb_weights
+            self._eval_engine = ee = None                       # free the old buffers before allocating the larger ones
+            ee = EvalEngine(self.packed_weights(net, device), self.tables, fw, na, self.cutoff, self.max_neighbors,
+                            precision=self.precision, device=device, node_capacity=n_cap, crystal_capacity=g_cap)
+            self._eval_engine = ee
+        elif tuple(na) != ee.eng.topology:
+            ee.set_topology(na)
+        return ee
+
+    @torch.no_grad()
+    def evaluate(self, model, batch, t_emb_weights, crystal_ids, seed: int = 0, timestep=None, noise=None,
+                 capacity=None):
+        """Forward-only loss of a batch, per crystal (no backward, no torch RNG, the training state untouched):
+        returns an EvalResult (t[G], num_atoms[G], terms[G,4]; see arreau_b200/evaluation.py).  The draws are keyed by
+        (seed, crystal_ids[g]) (arreau_eval_noise), so a crystal's terms do not depend on the batch it is in;
+        `timestep` / `noise` inject draws as in __call__.  Precision: self.precision."""
+        from ..evaluation import EvalResult
+        dev = batch.X0.device
+        if dev.type != "cuda":
+            raise RuntimeError("arreau_b200 runs on CUDA tensors only (no CPU fallback)")
+        net = getattr(model, "model", model)
+        na = getattr(batch, "num_atoms_cpu", None)
+        na = np.asarray(batch.num_atoms.cpu() if na is None else na, dtype=np.int64)
+        ee = self.eval_engine_for(net, t_emb_weights, na, dev, capacity=capacity)
+        ee.eng.w = self.packed_weights(net, dev)
+        t, terms = ee.run(batch.X0, batch.A0, batch.L0.view(-1, 3, 3), crystal_ids, seed, timestep, noise)
+        return EvalResult(t=t.clone(), num_atoms=torch.from_numpy(na.copy()), terms=terms.clone())
 
     def compute_frac_x_error(self, pred_frac_eps_x, target_frac_eps_x, batch=None):
         """diffusion_loss.py:95-110 (value only; gradients flow through __call__)."""

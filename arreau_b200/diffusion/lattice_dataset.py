@@ -109,6 +109,10 @@ class CrystalDataset(torch.utils.data.Dataset):
         pos = np.einsum("bi,bij->bj", X0, L0m[batch])
         return _to_namespace(dict(X0=X0, A0=A0, L0=L0m.reshape(-1, 3), num_atoms=na, batch=batch, pos=pos), device, pin)
 
+    def atom_counts(self) -> np.ndarray:
+        """Atoms per crystal, in dataset order."""
+        return self._na
+
     def __len__(self):
         return len(self.configs)
 
@@ -116,6 +120,42 @@ class CrystalDataset(torch.utils.data.Dataset):
         c = self.configs[idx]
         A0 = np.asarray([self._index[int(z)] for z in np.asarray(c.atomic_numbers).reshape(-1)], dtype=np.int64)
         return dict(X0=np.asarray(c.X0, dtype=np.float64), A0=A0, L0=np.asarray(c.L0, dtype=np.float64), num_atoms=len(A0))
+
+
+class CrystalSubset(torch.utils.data.Dataset):
+    """The crystals `indices` of a CrystalDataset (a train / valid / test split) with the parent's z_table and collation.
+    `crystal_ids` are the crystals' indices in the parent: the evaluation noise is keyed by them, so a crystal draws the
+    same numbers whichever split view, batch or rank it is evaluated in."""
+
+    def __init__(self, parent: CrystalDataset, indices):
+        self.parent = parent
+        self.crystal_ids = np.asarray(indices, dtype=np.int64).reshape(-1)
+        self.z_table = parent.z_table
+
+    def collate_indices(self, indices, device=None, pin: bool = True):
+        return self.parent.collate_indices(self.crystal_ids[np.asarray(indices, dtype=np.int64)], device=device, pin=pin)
+
+    def atom_counts(self) -> np.ndarray:
+        return self.parent.atom_counts()[self.crystal_ids]
+
+    def __len__(self):
+        return int(self.crystal_ids.shape[0])
+
+    def __getitem__(self, idx: int):
+        return self.parent[int(self.crystal_ids[idx])]
+
+
+def split_indices(n: int, fractions: Sequence[float], seed: int = 0) -> List[np.ndarray]:
+    """Seeded split of range(n) into len(fractions) disjoint parts that together cover it (fractions sum to 1): part k
+    takes the next round(n * (f_0 + .. + f_k)) - round(n * (f_0 + .. + f_{k-1})) entries of one seeded permutation.
+    Each part is returned in ascending order."""
+    f = np.asarray(fractions, dtype=np.float64).reshape(-1)
+    if f.size == 0 or np.any(f < 0) or abs(float(f.sum()) - 1.0) > 1e-9:
+        raise ValueError(f"fractions must be non-negative and sum to 1, got {list(f)}")
+    bounds = np.round(n * np.cumsum(f)).astype(np.int64)
+    bounds[-1] = n
+    order = np.random.default_rng(seed).permutation(n)
+    return [np.sort(p) for p in np.split(order, bounds[:-1])]
 
 
 def collate_crystals(items: Sequence[dict], device=None, pin: bool = True):

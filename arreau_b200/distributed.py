@@ -3,7 +3,7 @@ per rank, whole trajectories per GPU, and ONE collective at the end (gather of t
 no per-step communication: graph edges never cross crystals (diffusion_helpers.py:350-383)."""
 from __future__ import annotations
 
-from typing import List, Optional, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -19,35 +19,40 @@ def shard_range(num_crystals: int, rank: int, world: int) -> Tuple[int, int]:
     return lo, lo + base + (1 if rank < rem else 0)
 
 
-def gather_sample_results(local: SampleResult, group=None, device: Optional[torch.device] = None) -> SampleResult:
-    """All-gather the per-rank SampleResult (ragged in atoms) into the global one, rank-major = crystal order.
-    Uses the group's backend (NCCL on the GPUs, gloo in the CPU tests); counts first, then padded payloads."""
+def all_gather_rows(arrays: Sequence[np.ndarray], group=None, device: Optional[torch.device] = None) -> List[np.ndarray]:
+    """All-gather arrays that are ragged in their leading dimension (each array its own row count per rank) and
+    concatenate every array's parts in rank order.  Floating arrays travel as float64, integer arrays as int64.
+    Counts first (one collective), then one padded payload per array.  Uses the group's backend (NCCL on the GPUs,
+    gloo in the CPU tests); world size 1 returns the arrays unchanged."""
     if not dist.is_initialized() or dist.get_world_size(group) == 1:
-        return local
+        return list(arrays)
     world = dist.get_world_size(group)
     dev = device if device is not None else torch.device("cpu")
-    n_atoms = torch.tensor([local.frac_x.shape[0], local.num_atoms.shape[0]], dtype=torch.int64, device=dev)
-    counts = [torch.zeros_like(n_atoms) for _ in range(world)]
-    dist.all_gather(counts, n_atoms, group=group)
+    n_rows = torch.tensor([a.shape[0] for a in arrays], dtype=torch.int64, device=dev)
+    counts = [torch.zeros_like(n_rows) for _ in range(world)]
+    dist.all_gather(counts, n_rows, group=group)
     counts = torch.stack(counts).cpu().numpy()
-    max_n, max_g = int(counts[:, 0].max()), int(counts[:, 1].max())
-
-    def gather(arr: np.ndarray, rows: int, dtype) -> List[np.ndarray]:
-        t = torch.zeros((rows,) + arr.shape[1:], dtype=dtype, device=dev)
+    out = []
+    for i, arr in enumerate(arrays):
+        dtype = torch.float64 if np.asarray(arr).dtype.kind == "f" else torch.int64
+        t = torch.zeros((int(counts[:, i].max()),) + arr.shape[1:], dtype=dtype, device=dev)
         t[: arr.shape[0]] = torch.as_tensor(arr, dtype=dtype)
-        outs = [torch.empty_like(t) for _ in range(world)]
-        dist.all_gather(outs, t, group=group)
-        return [o.cpu().numpy() for o in outs]
+        parts = [torch.empty_like(t) for _ in range(world)]
+        dist.all_gather(parts, t, group=group)
+        out.append(np.concatenate([p[: int(counts[r, i])].cpu().numpy() for r, p in enumerate(parts)]))
+    return out
 
-    frac = gather(local.frac_x, max_n, torch.float64)
-    zs = gather(local.atomic_numbers, max_n, torch.int64)
-    lat = gather(local.lattice, max_g, torch.float64)
-    na = gather(local.num_atoms, max_g, torch.int64)
-    cat = lambda parts, col: np.concatenate([p[: int(counts[r, col])] for r, p in enumerate(parts)])  # noqa: E731
-    num_atoms = cat(na, 1)
+
+def gather_sample_results(local: SampleResult, group=None, device: Optional[torch.device] = None) -> SampleResult:
+    """All-gather the per-rank SampleResult (ragged in atoms) into the global one, rank-major = crystal order."""
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return local
+    frac, zs, lat, num_atoms = all_gather_rows([np.asarray(local.frac_x, dtype=np.float64),
+                                                np.asarray(local.atomic_numbers, dtype=np.int64),
+                                                np.asarray(local.lattice, dtype=np.float64),
+                                                np.asarray(local.num_atoms, dtype=np.int64)], group, device)
     idx_start = np.concatenate([[0], np.cumsum(num_atoms)[:-1]]) if num_atoms.size else num_atoms
-    return SampleResult(frac_x=cat(frac, 0), atomic_numbers=cat(zs, 0), lattice=cat(lat, 1), idx_start=idx_start,
-                        num_atoms=num_atoms)
+    return SampleResult(frac_x=frac, atomic_numbers=zs, lattice=lat, idx_start=idx_start, num_atoms=num_atoms)
 
 
 def allreduce_gradients(flat_grad: torch.Tensor, group=None) -> torch.Tensor:

@@ -55,6 +55,13 @@ class PONITA_DIFFUSION(nn.Module):
     def training_step(self, graph, timestep=None):
         return self.diffusion_loss(self, graph, self.t_emb, timestep)
 
+    def validation_step(self, graph, crystal_ids, seed: int = 0):
+        """Forward-only loss of a batch per crystal (DiffusionLoss.evaluate -> EvalResult); `evaluation.evaluate_dataset`
+        reduces a whole split to the reference's "valid loss"."""
+        return self.diffusion_loss.evaluate(self, graph, self.t_emb, crystal_ids, seed=seed)
+
+    test_step = validation_step
+
     def configure_optimizers(self, device="cuda"):
         """torch.optim.Adam with the two weight-decay groups of :161-207 as ONE fused kernel over the flat parameter
         buffer, plus the trainer's gradient_clip_val=0.5 (main_diffusion.py:297); the cosine-warmup factor of

@@ -129,7 +129,54 @@ class FusedAdam:
         return float(np.sqrt(self.moments[1].item()))
 
 
-class TrainEngine:
+def noising_buffers(N: int, G: int, Z: int, dev) -> Dict[str, tuple]:
+    """Capacity buffers of a clean batch, its random draws and the noising outputs: name -> (leading extent kind,
+    buffer), the layout `noise_into` reads."""
+    f64 = lambda *s: torch.zeros(*s, dtype=torch.float64, device=dev)  # noqa: E731
+    return {"frac0": ("N", f64(N, 3)), "types0": ("N", torch.zeros(N, dtype=torch.int64, device=dev)),
+            "lattice0": ("G", f64(G, 3, 3)), "lengths0": ("G", f64(G, 3)), "angles0": ("G", f64(G, 3)),
+            "target_eps": ("N", f64(N, 3)), "eps_x": ("N", f64(N, 3)), "u": ("N", f64(N, Z)), "eps_l": ("G", f64(G, 3)),
+            "t_crystal": ("G", torch.ones(G, dtype=torch.int32, device=dev)),
+            "t_atom": ("N", torch.ones(N, dtype=torch.int32, device=dev)), "terms": ("3N", f64(3 * N))}
+
+
+def noise_into(e: DenoiseEngine, b) -> None:
+    """VE_pbc.forward, D3PM.get_xt, matrix_to_params + VP_lattice.forward (diffusion_loss.py:218-237) of the clean
+    batch held by `b` (the `noising_buffers` of a training or evaluation engine, bound to e's topology) into the forward
+    engine's state."""
+    s = e.stream
+    _lib.call("arreau_matrix_to_params", b.lattice0.data_ptr(), e.G, b.lengths0.data_ptr(), b.angles0.data_ptr(), s)
+    _lib.call("arreau_ve_pbc_forward", b.frac0.data_ptr(), b.eps_x.data_ptr(), b.t_atom.data_ptr(),
+              e.d_ve_sigmas.data_ptr(), b.lattice0.data_ptr(), e.crystal_of_atom.data_ptr(), e.N,
+              e.frac.data_ptr(), b.target_eps.data_ptr(), s)
+    _lib.call("arreau_d3pm_q_sample", b.types0.data_ptr(), b.u.data_ptr(), b.t_atom.data_ptr(),
+              e.d_q_keep.data_ptr(), e.d_q_to_mask.data_ptr(), e.N, e.Z, e.types.data_ptr(), s)
+    _lib.call("arreau_vp_lattice_forward", b.lengths0.data_ptr(), b.eps_l.data_ptr(), b.t_crystal.data_ptr(),
+              b.d_alpha_bars.data_ptr(), e.G, e.lengths.data_ptr(), s)
+    e.angles.copy_(b.angles0)
+
+
+class BatchEngine:
+    """A DenoiseEngine plus per-batch buffers (`_bufs`: name -> (leading extent kind, capacity buffer)) sized for a
+    CAPACITY and re-bound in place to every batch topology."""
+
+    def _bind(self) -> None:
+        e = self.eng
+        ext = {"N": e.N, "G": e.G, "3N": 3 * e.N}
+        for name, (kind, buf) in self._bufs.items():
+            setattr(self, name, buf[: ext[kind]])
+
+    def fits(self, num_atoms) -> bool:
+        na = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
+        return int(na.sum()) <= self.eng.N_cap and int(na.shape[0]) <= self.eng.G_cap
+
+    def set_topology(self, num_atoms) -> None:
+        """Bind the next batch's atoms-per-crystal vector (no allocation)."""
+        self.eng.set_topology(num_atoms)
+        self._bind()
+
+
+class TrainEngine(BatchEngine):
     """The training step's buffers on one GPU, sized for a CAPACITY (atoms, crystals) and re-bound in place to every
     batch topology (`set_topology`): a shuffled epoch of variable-size batches (lattice_dataset.py:96-113,
     main_diffusion.py:221-230) runs through one engine without reallocating (SURVEY 8f-4)."""
@@ -154,33 +201,13 @@ class TrainEngine:
         N, G, Z = e.N_cap, e.G_cap, e.Z
         f64 = lambda *s: torch.zeros(*s, dtype=torch.float64, device=dev)  # noqa: E731
         f32 = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)  # noqa: E731
-        self._bufs = {   # name -> (leading extent kind, capacity buffer)
-            "frac0": ("N", f64(N, 3)), "types0": ("N", torch.zeros(N, dtype=torch.int64, device=dev)),
-            "lattice0": ("G", f64(G, 3, 3)), "lengths0": ("G", f64(G, 3)), "angles0": ("G", f64(G, 3)),
-            "target_eps": ("N", f64(N, 3)), "eps_x": ("N", f64(N, 3)), "u": ("N", f64(N, Z)), "eps_l": ("G", f64(G, 3)),
-            "t_crystal": ("G", torch.ones(G, dtype=torch.int32, device=dev)),
-            "t_atom": ("N", torch.ones(N, dtype=torch.int32, device=dev)), "terms": ("3N", f64(3 * N)),
-            "dscore": ("N", f32(N, 3)), "dlogits": ("N", f32(N, Z)), "dlen0": ("G", f32(G, 3))}
+        self._bufs = noising_buffers(N, G, Z, dev)
+        self._bufs.update({"dscore": ("N", f32(N, 3)), "dlogits": ("N", f32(N, Z)), "dlen0": ("G", f32(G, 3))})
         self.loss = f64(5)
         self.d_alpha_bars = tables.vp_alpha_bars.to(torch.float32).to(dev)
         self.fold = torch.as_tensor(monomial_fold_table(), dtype=torch.int32).to(dev)
         self.mom_scratch, self.mom_out = f64(512), f64(2)
         self._bwd_ws = None
-        self._bind()
-
-    def _bind(self) -> None:
-        e = self.eng
-        ext = {"N": e.N, "G": e.G, "3N": 3 * e.N}
-        for name, (kind, buf) in self._bufs.items():
-            setattr(self, name, buf[: ext[kind]])
-
-    def fits(self, num_atoms) -> bool:
-        na = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
-        return int(na.sum()) <= self.eng.N_cap and int(na.shape[0]) <= self.eng.G_cap
-
-    def set_topology(self, num_atoms) -> None:
-        """Bind the next batch's atoms-per-crystal vector (no allocation)."""
-        self.eng.set_topology(num_atoms)
         self._bind()
 
     # ------------------------------------------------------------------ pieces (each = the mirrored reference call)
@@ -204,17 +231,7 @@ class TrainEngine:
 
     def noise_batch(self) -> None:
         """VE_pbc.forward, D3PM.get_xt, matrix_to_params + VP_lattice.forward into the forward engine's state."""
-        e, s = self.eng, self.eng.stream
-        _lib.call("arreau_matrix_to_params", self.lattice0.data_ptr(), e.G, self.lengths0.data_ptr(),
-                  self.angles0.data_ptr(), s)
-        _lib.call("arreau_ve_pbc_forward", self.frac0.data_ptr(), self.eps_x.data_ptr(), self.t_atom.data_ptr(),
-                  e.d_ve_sigmas.data_ptr(), self.lattice0.data_ptr(), e.crystal_of_atom.data_ptr(), e.N,
-                  e.frac.data_ptr(), self.target_eps.data_ptr(), s)
-        _lib.call("arreau_d3pm_q_sample", self.types0.data_ptr(), self.u.data_ptr(), self.t_atom.data_ptr(),
-                  e.d_q_keep.data_ptr(), e.d_q_to_mask.data_ptr(), e.N, e.Z, e.types.data_ptr(), s)
-        _lib.call("arreau_vp_lattice_forward", self.lengths0.data_ptr(), self.eps_l.data_ptr(), self.t_crystal.data_ptr(),
-                  self.d_alpha_bars.data_ptr(), e.G, e.lengths.data_ptr(), s)
-        e.angles.copy_(self.angles0)
+        noise_into(self.eng, self)
 
     def _workspace(self) -> torch.Tensor:
         e = self.eng

@@ -457,6 +457,31 @@ int arreau_training_loss(const float* score, const float* logits, const float* l
                          int32_t num_states, double hybrid_coeff, double* terms_scratch, double* loss_out, float* dscore,
                          float* dlogits, float* dlen0, void* stream);
 
+/* ---- evaluation (validation / test loss) ---------------------------------------------------------------------- */
+
+/* The random draws of DiffusionLoss.__call__ (diffusion_loss.py:213-216 timestep t ~ U{1..T}; :228-237 eps_x[N,3] ~ N(0,1),
+ * u[N,Z] ~ U[0,1), eps_l[G,3] ~ N(0,1)), drawn PER CRYSTAL: Philox4x32-10 with key = seed and counter = {crystal_id[g]
+ * (64 bits), index within the crystal, stream tag}.  A crystal's draws depend on the seed and its own id only -- not on
+ * its position in the batch, the batch size or the rank -- so a loss evaluated with them does not depend on how a split
+ * is grouped into batches or spread over GPUs.  Same distributions as the reference's draws, but not the reference's
+ * torch CPU stream.  crystal_id[G] i64 (the crystal's index in its dataset), atom_offset[G+1], crystal_of_atom[N] of
+ * the batch; outputs t_crystal[G] i32, eps_x[N,3], u[N,Z], eps_l[G,3] f64.  2 <= num_states <= 128. */
+int arreau_eval_noise(uint64_t seed, int32_t num_crystals, int32_t num_atoms_total, int32_t num_states, int32_t num_steps,
+                      const int64_t* crystal_id, const int32_t* atom_offset, const int32_t* crystal_of_atom,
+                      int32_t* t_crystal, double* eps_x, double* u, double* eps_l, void* stream);
+
+/* The loss of arreau_training_loss per crystal, without gradients (forward-only evaluation of
+ * diffusion_loss.py:95-110,253-274; d3pm.py:74-117,145-163).  per_crystal[G][4] f64 = {sum of the wrapped squared frac
+ * error, sum of vb, sum of ce over the crystal's atoms (in atom order), sum_d (len0 - lengths / n)^2}.  The per-atom
+ * terms (terms_scratch, 3*N doubles: frac, vb, ce) come from the same device code as arreau_training_loss's.  A batch B's
+ * loss_out is rebuilt from these sums: frac, vb, ce divided by N_B, the lattice term by 3 G_B,
+ * loss = frac + (hybrid_coeff * vb + ce) + lattice.  2 <= num_states <= 128. */
+int arreau_eval_loss(const float* score, const float* logits, const float* len0, const double* target_eps,
+                     const int64_t* types0, const int64_t* types_t, const int32_t* t_of_atom, const double* lengths,
+                     const int32_t* atom_offset, const double* q_keep, const double* q_to_mask, double onestep_keep,
+                     double onestep_to_mask, int32_t num_steps, int32_t num_atoms_total, int32_t num_crystals,
+                     int32_t num_states, double* terms_scratch, double* per_crystal, void* stream);
+
 /* Flat parameter / gradient buffer: every trainable tensor of the reference's state_dict in its own layout
  * ([out, in] row-major), per-layer tensors stacked over the L layers, at these float offsets (SURVEY 8b names):
  * basis_fn.{1,3}.{weight,bias}, fiber_basis_fn.{1,3}.{weight,bias}, x_embedder.weight, then per layer
