@@ -126,7 +126,7 @@ SIGNATURES = {
     "arreau_sgemm": [i32, i32, vp, i64, vp, i64, vp, i64, i32, i32, i64, C.c_float, vp, i32, vp, i64, vp],
     "arreau_fold_basis_w1": [vp, vp, vp, vp, vp],
     "arreau_moments": [vp, vp, i64, vp, vp, vp],
-    "arreau_adam_step": [vp, vp, vp, vp, vp, i64, f64, f64, f64, f64, f64, i64, f64, vp, vp],
+    "arreau_adam_step": [vp, vp, vp, vp, vp, i64, f64, f64, f64, f64, f64, i64, f64, vp, vp, f64, vp],
 }
 RESTYPES = {"arreau_launch_count": i64, "arreau_ponita_backward_workspace_bytes": i64}
 

@@ -369,12 +369,15 @@ __global__ void crystal_loss_kernel(const double* __restrict__ terms, const floa
 
 // torch.optim.Adam step (diffusion.py:161-210: two weight-decay groups, L2 decay folded into the gradient) with the
 // trainer's global-norm clip (main_diffusion.py:297, clip_grad_norm_: coef = min(1, max_norm / (norm + 1e-6))) read
-// from the device so that the step never synchronises with the host.
+// from the device so that the step never synchronises with the host.  With `ema`, the exponential moving average of
+// the weights is updated from the new parameter in the same pass (the NeMo EMAOptimizer rule, applied after the inner
+// step): ema = decay * ema + (1 - decay) * p_new; the parameter arithmetic is the same with or without it.
 __global__ void __launch_bounds__(256)
 adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                  const uint8_t* __restrict__ decay_mask, long long n, float lr, float beta1, float beta2, float eps,
                  float weight_decay, float bias_c1, float bias_c2_sqrt, float max_grad_norm,
-                 const double* __restrict__ grad_moments) {
+                 const double* __restrict__ grad_moments, float* __restrict__ ema, float ema_decay,
+                 float ema_one_minus_decay) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float coef = 1.0f;
@@ -390,7 +393,9 @@ adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __re
   m[i] = mi;
   v[i] = vi;
   const float denom = sqrtf(vi) / bias_c2_sqrt + eps;
-  p[i] = pi - (lr / bias_c1) * (mi / denom);
+  const float p_new = pi - (lr / bias_c1) * (mi / denom);
+  p[i] = p_new;
+  if (ema) ema[i] = fmaf(ema_one_minus_decay, p_new, ema_decay * ema[i]);
 }
 
 }  // namespace
@@ -398,14 +403,16 @@ adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __re
 extern "C" int arreau_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
                                 const uint8_t* decay_mask, int64_t n, double lr, double beta1, double beta2, double eps,
                                 double weight_decay, int64_t step, double max_grad_norm, const double* grad_moments,
-                                void* stream) {
+                                float* ema, double ema_decay, void* stream) {
   if (n == 0) return ARREAU_OK;
   if (!params || !grads || !exp_avg || !exp_avg_sq) return ARREAU_ERR_NULL;
   if (n < 0 || step < 1) return ARREAU_ERR_BAD_SHAPE;
+  if (ema && !(ema_decay >= 0.0 && ema_decay <= 1.0)) return ARREAU_ERR_BAD_SHAPE;
   const double c1 = 1.0 - pow(beta1, (double)step), c2 = 1.0 - pow(beta2, (double)step);
   adam_step_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       params, grads, exp_avg, exp_avg_sq, decay_mask, n, (float)lr, (float)beta1, (float)beta2, (float)eps,
-      (float)weight_decay, (float)c1, (float)sqrt(c2), (float)max_grad_norm, grad_moments);
+      (float)weight_decay, (float)c1, (float)sqrt(c2), (float)max_grad_norm, grad_moments, ema, (float)ema_decay,
+      (float)(1.0 - ema_decay));
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

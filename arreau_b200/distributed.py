@@ -43,6 +43,22 @@ def all_gather_rows(arrays: Sequence[np.ndarray], group=None, device: Optional[t
     return out
 
 
+def gather_rng_states(state: torch.Tensor, group=None, device: Optional[torch.device] = None) -> List[torch.Tensor]:
+    """Every rank's generator state (a uint8 tensor such as torch.cuda.get_rng_state() returns) in rank order, on every
+    rank.  A collective (all_gather_rows): every rank must join it.  World size 1: [state]."""
+    rows = all_gather_rows([state.cpu().numpy().astype(np.int64).reshape(1, -1)], group, device)[0]
+    return [torch.as_tensor(r.astype(np.uint8)) for r in rows]
+
+
+def rank_rng_state(states: Sequence[torch.Tensor], group=None) -> torch.Tensor:
+    """This rank's entry of a `gather_rng_states` list written at the same world size."""
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    if len(states) != world:
+        raise ValueError(f"generator states of {len(states)} ranks cannot be restored at world size {world}")
+    return torch.as_tensor(states[rank], dtype=torch.uint8)
+
+
 def gather_sample_results(local: SampleResult, group=None, device: Optional[torch.device] = None) -> SampleResult:
     """All-gather the per-rank SampleResult (ragged in atoms) into the global one, rank-major = crystal order."""
     if not dist.is_initialized() or dist.get_world_size(group) == 1:

@@ -6,6 +6,7 @@ from __future__ import annotations
 
 import argparse
 import io
+import os
 import pickle
 from typing import Optional
 
@@ -62,13 +63,15 @@ class PONITA_DIFFUSION(nn.Module):
 
     test_step = validation_step
 
-    def configure_optimizers(self, device="cuda"):
+    def configure_optimizers(self, device="cuda", ema_decay=None):
         """torch.optim.Adam with the two weight-decay groups of :161-207 as ONE fused kernel over the flat parameter
         buffer, plus the trainer's gradient_clip_val=0.5 (main_diffusion.py:297); the cosine-warmup factor of
-        scheduler.py is applied per epoch with `optimizer.set_epoch(epoch, self.warmup, self.epochs)`."""
+        scheduler.py is applied per epoch with `optimizer.set_epoch(epoch, self.warmup, self.epochs)`.  ema_decay: the
+        optimizer also keeps an EMA of the weights (FusedAdam)."""
         from ..training import FusedAdam
         flat = self.model.flat if self.model.flat is not None else self.model.flatten_parameters(device)
-        self._optimizer = FusedAdam(flat, lr=self.lr, weight_decay=self.weight_decay, max_grad_norm=0.5)
+        self._optimizer = FusedAdam(flat, lr=self.lr, weight_decay=self.weight_decay, max_grad_norm=0.5,
+                                    ema_decay=ema_decay)
         return self._optimizer
 
     # ---- sampling (:220-253) ------------------------------------------------------------------------------------------
@@ -126,11 +129,16 @@ class PONITA_DIFFUSION(nn.Module):
         m.model._packed = None
         return m
 
-    def save_checkpoint(self, path) -> None:
-        """Lightning-shaped checkpoint (same keys) plus the orientation grid."""
+    def save_checkpoint(self, path, training_state: Optional[dict] = None) -> None:
+        """Lightning-shaped checkpoint (same keys) plus the orientation grid.  training_state: further top-level keys
+        that make the file a resume point (`train.fit` writes epoch, global_step, optimizer_states, ema and fit_state
+        into last.ckpt); `load_from_checkpoint` ignores them.  The file is written to a temporary name in the same
+        directory and renamed over `path`, so an interrupted write leaves the previous file intact."""
         sd = {k: v.detach().cpu() for k, v in self.state_dict().items()}
-        torch.save({"state_dict": sd, "hyper_parameters": {"args": self.hparams.args, "z_table": self.hparams.z_table},
-                    "ori_grid": self.model.ori_grid.detach().cpu()}, path)
+        ckpt = {"state_dict": sd, "hyper_parameters": {"args": self.hparams.args, "z_table": self.hparams.z_table},
+                "ori_grid": self.model.ori_grid.detach().cpu()}
+        ckpt.update(training_state or {})
+        save_atomic(ckpt, path)
 
 
 class _RefUnpickler(pickle.Unpickler):
@@ -148,6 +156,20 @@ class _PickleModule:
     Unpickler = _RefUnpickler
     load = staticmethod(lambda f, **kw: _RefUnpickler(f, **kw).load())
     loads = staticmethod(lambda b, **kw: _RefUnpickler(io.BytesIO(b), **kw).load())
+
+
+def save_atomic(obj, path) -> None:
+    """torch.save to a temporary file next to `path`, then os.replace: readers see the old file or the new one."""
+    path = os.fspath(path)
+    tmp = f"{path}.{os.getpid()}.tmp"
+    try:
+        with open(tmp, "wb") as f:
+            torch.save(obj, f)
+        os.replace(tmp, path)
+    except BaseException:
+        if os.path.exists(tmp):
+            os.unlink(tmp)
+        raise
 
 
 def load_checkpoint_file(path, map_location="cpu") -> dict:

@@ -95,19 +95,21 @@ class PonitaFiberBundle(nn.Module):
         self._packed = None
         return super().load_state_dict(sd, strict=False, **kw)
 
-    def flatten_parameters(self, device):
+    def flatten_parameters(self, device, into=None):
         """Re-home every trainable tensor into ONE flat fp32 CUDA buffer (arreau_train_layout_t order, see
         arreau_b200/training.py FlatParams): the nn.Parameters become views of it, keep their reference names, and an
-        optimizer / gradient all-reduce sees a single tensor.  Returns the FlatParams (also kept as `self.flat`)."""
+        optimizer / gradient all-reduce sees a single tensor.  into: an existing FlatParams of this layout whose contents
+        become the weights (nothing is copied into it).  Returns the FlatParams (also kept as `self.flat`)."""
         from ...training import FlatParams
         n_out = self.read_out_layers[0].out_features
-        flat = FlatParams(self.x_embedder.in_features - 4, 4, n_out - 4, device)
+        flat = into if into is not None else FlatParams(self.x_embedder.in_features - 4, 4, n_out - 4, device)
         views = flat.views()
         with torch.no_grad():
             for name, p in self.named_parameters():
                 if p.numel() == 0:
                     continue
-                views[name].copy_(p.detach().to(torch.float32))
+                if into is None:
+                    views[name].copy_(p.detach().to(torch.float32))
                 p.data = views[name]
                 p.grad = None
         self.flat = flat

@@ -11,7 +11,13 @@ forward.  The loss metric is reduced like DiffusionLossMetric (sum of losses / n
 With a validation split (--val_fraction) every epoch ends with a forward-only evaluation of it (arreau_b200/evaluation.py)
 logged as "valid loss"; --checkpoint_dir receives last.ckpt every epoch and best.ckpt whenever the valid loss improves
 (the reference keeps the top 3 by "valid loss"; here only the best).  A test split (--test_fraction) is evaluated once at
-the end with the best.ckpt weights (the final weights without a validation split)."""
+the end with the best.ckpt weights (the final weights without a validation split).
+
+last.ckpt also carries the training state (Adam moments and step, epoch, loss history, best valid loss, every rank's
+CUDA generator, the EMA), so `--resume out/ckpt/last.ckpt` with the same data, batch size, fractions and --epochs
+continues the run exactly where it stopped.  --ema_decay D keeps an exponential moving average of the weights (the NeMo
+EMA callback the reference carries): the EMA weights are the ones validated and tested, and last.ckpt, best.ckpt and
+--out each get a twin *-EMA.ckpt holding them (a plain model checkpoint, e.g. for `generate --model_path`)."""
 from __future__ import annotations
 
 import argparse
@@ -23,7 +29,8 @@ import torch
 import torch.distributed as dist
 
 from .diffusion.lattice_dataset import CrystalDataset, CrystalSubset, batches, split_indices
-from .distributed import allreduce_gradients, broadcast_parameters, reduce_loss_metric
+from .distributed import (allreduce_gradients, broadcast_parameters, gather_rng_states, rank_rng_state,
+                          reduce_loss_metric)
 from .evaluation import evaluate_dataset
 from .lightning_wrappers.diffusion import PONITA_DIFFUSION
 
@@ -38,25 +45,111 @@ def default_args(**over):
     return a
 
 
+def ema_path(path: str) -> str:
+    """The EMA twin of a checkpoint path: out/ckpt/last.ckpt -> out/ckpt/last-EMA.ckpt (NeMo's naming)."""
+    root, ext = os.path.splitext(path)
+    return f"{root}-EMA{ext}"
+
+
+def ema_model(model: PONITA_DIFFUSION, device) -> PONITA_DIFFUSION:
+    """A second model whose trainable tensors are views of the EMA buffer of `model`'s optimizer (FusedAdam with
+    ema_decay; the buffer is not written): evaluating or saving it reads the EMA, while the training weights, moments
+    and engines are not touched.  Its buffers (the `callibrated` flags) and time embedding are copies of `model`'s.
+    Every optimizer step bumps the EMA buffer's version, so its packed kernel weights are rebuilt when used.  The CPU
+    random generator is left as it was."""
+    opt = model._optimizer
+    if opt is None or opt.ema is None:
+        raise ValueError("the model's optimizer keeps no EMA: configure_optimizers(ema_decay=...) first")
+    with torch.random.fork_rng(devices=[]):
+        m = PONITA_DIFFUSION(model.hparams.args, model.hparams.z_table, ori_grid=model.model.ori_grid.detach().cpu(),
+                             precision=model.model.precision)
+    m.load_state_dict(model.state_dict(), strict=False)
+    m.to(device)
+    m.model.flatten_parameters(device, into=opt.ema)
+    return m
+
+
+def check_resume(ckpt, *, epochs: int, batch_size: int, world_size: int, backward_precision: str, num_train: int,
+                 num_valid: int, seed: int = 0, ema_decay: Optional[float] = None) -> dict:
+    """The checkpoint (a path or the loaded dict) if it is a resume point of the run these arguments describe; a
+    ValueError naming every mismatch otherwise.  Reads the file only (no device work)."""
+    from .lightning_wrappers.diffusion import load_checkpoint_file
+    name = ckpt if isinstance(ckpt, (str, os.PathLike)) else "checkpoint"
+    if not isinstance(ckpt, dict):
+        ckpt = load_checkpoint_file(ckpt)
+    fs = ckpt.get("fit_state")
+    if not isinstance(fs, dict) or "optimizer_states" not in ckpt or "epoch" not in ckpt:
+        raise ValueError(f"{name} holds no training state written by train.fit (a model-only checkpoint such as "
+                         "best.ckpt, or a Lightning checkpoint): resume from the last.ckpt of a fit run")
+    saved_ema = ckpt.get("ema")
+    have = {"batch_size": fs["batch_size"], "world size": fs["world_size"],
+            "backward_precision": fs["backward_precision"], "train split size": fs["num_train"],
+            "valid split size": fs["num_valid"], "seed": fs["seed"],
+            "ema_decay": None if saved_ema is None else float(saved_ema["decay"]),
+            "epochs": getattr(ckpt["hyper_parameters"]["args"], "epochs", None)}
+    want = {"batch_size": batch_size, "world size": world_size, "backward_precision": backward_precision,
+            "train split size": num_train, "valid split size": num_valid, "seed": seed,
+            "ema_decay": None if ema_decay is None else float(ema_decay), "epochs": epochs}
+    bad = [f"{k}: checkpoint {have[k]}, this run {want[k]}" for k in want if have[k] != want[k]]
+    if bad:
+        raise ValueError(f"{name} is not a resume point of this run: " + "; ".join(bad))
+    return ckpt
+
+
 def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_size: int, device, seed: int = 0,
         backward_precision: str = "tf32", calibrate: bool = True, log=print, val_dataset=None,
-        checkpoint_dir: Optional[str] = None, metrics: Optional[dict] = None):
+        checkpoint_dir: Optional[str] = None, metrics: Optional[dict] = None, resume_from: Optional[str] = None,
+        ema_decay: Optional[float] = None):
     """Trains `model` for `epochs` and returns the per-epoch train loss.  val_dataset: evaluated after every epoch
     (evaluate_dataset with the same batch_size and seed; logged as "valid loss").  checkpoint_dir: rank 0 writes
-    last.ckpt every epoch and, with a validation set, best.ckpt whenever the valid loss improves.  metrics (optional
-    dict): receives metrics["valid"], one evaluate_dataset result per epoch."""
+    last.ckpt every epoch -- the weights plus the training state a resume needs -- and, with a validation set, best.ckpt
+    whenever the valid loss improves.  metrics (optional dict): receives metrics["valid"], one evaluate_dataset result
+    per epoch of this call.
+
+    resume_from: a last.ckpt of a run with the same data splits, batch_size, world size, backward_precision, seed and
+    ema_decay, whose model was built with `epochs` epochs (checked before any device work, ValueError otherwise).  The
+    weights, the Adam state, the EMA, every rank's CUDA generator, the loss history and the best valid loss are
+    restored, calibration is skipped, and epochs epoch+1 .. epochs-1 run; the returned history starts at epoch 0, so
+    a resumed run returns what the uninterrupted run returns.
+
+    ema_decay: the optimizer keeps an EMA of the weights (FusedAdam).  The EMA weights are the ones validated (and
+    best.ckpt is chosen by their loss), and last.ckpt / best.ckpt each get a twin *-EMA.ckpt, a model checkpoint of
+    the EMA weights.  Training itself is the same as without EMA."""
     rank = dist.get_rank() if dist.is_initialized() else 0
     world = dist.get_world_size() if dist.is_initialized() else 1
+    ckpt = None
+    if resume_from is not None:
+        ckpt = check_resume(resume_from, epochs=epochs, batch_size=batch_size, world_size=world,
+                            backward_precision=backward_precision, num_train=len(dataset),
+                            num_valid=0 if val_dataset is None else len(val_dataset), seed=seed, ema_decay=ema_decay)
     model.to(device)
     model.diffusion_loss.backward_precision = backward_precision
-    opt = model.configure_optimizers(device)
+    opt = model.configure_optimizers(device, ema_decay=ema_decay)
     flat = model.model.flat
-    broadcast_parameters(flat.data)
-    history = []
+    history, valid_losses = [], []
     best = float("inf")
+    first = 0
+    if ckpt is not None:
+        sd = ckpt["state_dict"]
+        own = model.state_dict()
+        model.load_state_dict({k: v for k, v in sd.items() if k in own}, strict=False)   # parameters are views of flat
+        flat.version += 1
+        model.model._packed = None
+        opt.load_state_dict(ckpt["optimizer_states"][0])
+        fs = ckpt["fit_state"]
+        history, valid_losses, best = list(fs["train_losses"]), list(fs["valid_losses"]), float(fs["best_valid"])
+        first = int(ckpt["epoch"]) + 1
+        calibrate = False
+    broadcast_parameters(flat.data)
+    twin = ema_model(model, device) if ema_decay is not None else None
+    if ckpt is not None:
+        if twin is not None:
+            opt.ema.load_state_dict({k[len("model."):]: v for k, v in ckpt["ema"]["state_dict"].items()})
+        torch.cuda.set_rng_state(rank_rng_state(ckpt["fit_state"]["cuda_rng"]), device)
+    comm = device if dist.is_initialized() and dist.get_backend() == "nccl" else None
     if checkpoint_dir is not None and rank == 0:
         os.makedirs(checkpoint_dir, exist_ok=True)
-    for epoch in range(epochs):
+    for epoch in range(first, epochs):
         opt.set_epoch(epoch, model.warmup, max(model.epochs, 1))
         total_loss = torch.zeros((), dtype=torch.float64, device=device)
         total_samples = torch.zeros((), dtype=torch.float64, device=device)
@@ -73,28 +166,47 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
                 te = model.diffusion_loss.train_engine_for(model.model, model.t_emb, getattr(batch, "num_atoms_cpu", batch.num_atoms), device)
                 te.calibrate_from_last_forward()
                 broadcast_parameters(flat.data)
-                for layer in model.model.interaction_layers:
-                    layer.conv.callibrated.fill_(True)
+                for m in (model,) if twin is None else (model, twin):
+                    for layer in m.model.interaction_layers:
+                        layer.conv.callibrated.fill_(True)
                 calibrate = False
             allreduce_gradients(flat.grad)
-            opt.step()
+            opt.step()                                 # with ema_decay: the EMA is initialised at the first step
             total_loss += loss.detach().double()
             total_samples += batch.num_atoms.shape[0]
         metric = reduce_loss_metric(total_loss, total_samples)
         history.append(float(metric))
         valid = None
         if val_dataset is not None:
-            valid = evaluate_dataset(model, val_dataset, batch_size, device, seed=seed)
+            valid = evaluate_dataset(model if twin is None else twin, val_dataset, batch_size, device, seed=seed)
+            valid_losses.append(valid["loss"])
             if metrics is not None:
                 metrics.setdefault("valid", []).append(valid)
+        improved = valid is not None and valid["loss"] < best
+        if improved:
+            best = valid["loss"]
+        state = None
+        if checkpoint_dir is not None:                 # every rank's generator (a collective), then rank 0 writes
+            rng = gather_rng_states(torch.cuda.get_rng_state(device), device=comm)
+            if rank == 0:
+                state = {"epoch": epoch, "global_step": opt.step_count, "optimizer_states": [opt.state_dict()],
+                         "ema": None if twin is None else {
+                             "decay": opt.ema_decay,
+                             "state_dict": {"model." + k: v.detach().cpu() for k, v in opt.ema.views().items()}},
+                         "fit_state": {"seed": seed, "batch_size": batch_size, "world_size": world,
+                                       "backward_precision": backward_precision, "num_train": len(dataset),
+                                       "num_valid": 0 if val_dataset is None else len(val_dataset),
+                                       "train_losses": list(history), "valid_losses": list(valid_losses),
+                                       "best_valid": best, "cuda_rng": rng}}
         if rank == 0:
-            log(f"epoch {epoch}: train loss {history[-1]:.6f}" + (f", valid loss {valid['loss']:.6f}" if valid is not None else "")
-                + f" (lr {opt.lr:.3e})")
+            shown = "" if valid is None else f", valid loss {valid['loss']:.6f}" + (" (EMA weights)" if twin is not None else "")
+            log(f"epoch {epoch}: train loss {history[-1]:.6f}{shown} (lr {opt.lr:.3e})")
             if checkpoint_dir is not None:
-                model.save_checkpoint(os.path.join(checkpoint_dir, "last.ckpt"))
-                if valid is not None and valid["loss"] < best:
-                    best = valid["loss"]
-                    model.save_checkpoint(os.path.join(checkpoint_dir, "best.ckpt"))
+                saves = [("last.ckpt", state)] + ([("best.ckpt", None)] if improved else [])
+                for name, extra in saves:
+                    model.save_checkpoint(os.path.join(checkpoint_dir, name), training_state=extra)
+                    if twin is not None:
+                        twin.save_checkpoint(ema_path(os.path.join(checkpoint_dir, name)))
     return history
 
 
@@ -103,42 +215,69 @@ def main():
     ap.add_argument("--data", nargs="+", required=True, help="dataset files (.h5 as written by prep_datasets.py, or .npz)")
     ap.add_argument("--epochs", type=int, default=1)
     ap.add_argument("--batch_size", type=int, default=270)
-    ap.add_argument("--lr", type=float, default=3e-4)
-    ap.add_argument("--warmup", type=int, default=0)
+    ap.add_argument("--lr", type=float, default=None, help="default 3e-4 (on --resume: the checkpoint's)")
+    ap.add_argument("--warmup", type=int, default=None, help="default 0 (on --resume: the checkpoint's)")
     ap.add_argument("--backward_precision", default="tf32", choices=["fp32", "tf32"])
     ap.add_argument("--out", default="out/model.ckpt")
     ap.add_argument("--val_fraction", type=float, default=0.0, help="share of the data held out for the valid loss")
     ap.add_argument("--test_fraction", type=float, default=0.0, help="share of the data held out for the test loss")
     ap.add_argument("--checkpoint_dir", default=None, help="last.ckpt every epoch, best.ckpt by valid loss")
+    ap.add_argument("--resume", default=None, metavar="PATH",
+                    help="continue the run whose last.ckpt this is; --data, --batch_size, the fractions, --epochs, "
+                         "--backward_precision and --ema_decay must be the run's")
+    ap.add_argument("--ema_decay", type=float, default=None,
+                    help="keep an EMA of the weights (e.g. 0.999): it is validated and saved as *-EMA.ckpt twins")
     args = ap.parse_args()
     if args.val_fraction < 0 or args.test_fraction < 0 or args.val_fraction + args.test_fraction >= 1:
         ap.error("--val_fraction and --test_fraction must be >= 0 and leave a training split")
     if args.val_fraction > 0 and args.test_fraction > 0 and args.checkpoint_dir is None:
         ap.error("a test split with a validation split is evaluated with best.ckpt: give --checkpoint_dir")
-    local = int(os.environ.get("LOCAL_RANK", "0"))
-    torch.cuda.set_device(local)
-    device = torch.device("cuda", local)
-    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
-        dist.init_process_group("nccl", device_id=device)
+    if args.ema_decay is not None and not 0.0 <= args.ema_decay <= 1.0:
+        ap.error("--ema_decay must be in [0, 1]")
     ds = CrystalDataset(args.data)
-    rank0 = not dist.is_initialized() or dist.get_rank() == 0
     train_ds, val_ds, test_ds = ds, None, None
     if args.val_fraction > 0 or args.test_fraction > 0:
         parts = split_indices(len(ds), [1.0 - args.val_fraction - args.test_fraction, args.val_fraction,
                                         args.test_fraction], seed=0)
         train_ds, val_ds, test_ds = (CrystalSubset(ds, p) if len(p) else None for p in parts)
-    torch.manual_seed(0)
-    model = PONITA_DIFFUSION(default_args(lr=args.lr, epochs=args.epochs, warmup=args.warmup, batch_size=args.batch_size), ds.z_table)
+    if args.resume is not None:         # refused before any device work
+        try:
+            hp = check_resume(args.resume, epochs=args.epochs, batch_size=args.batch_size,
+                              world_size=int(os.environ.get("WORLD_SIZE", "1")),
+                              backward_precision=args.backward_precision, num_train=len(train_ds),
+                              num_valid=0 if val_ds is None else len(val_ds), ema_decay=args.ema_decay)["hyper_parameters"]["args"]
+        except ValueError as e:
+            ap.error(str(e))
+        for k in ("lr", "warmup"):
+            if getattr(args, k) is not None and getattr(args, k) != getattr(hp, k):
+                ap.error(f"--{k} {getattr(args, k)} differs from the resumed run's {getattr(hp, k)}")
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local)
+    device = torch.device("cuda", local)
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        dist.init_process_group("nccl", device_id=device)
+    rank0 = not dist.is_initialized() or dist.get_rank() == 0
+    if args.resume is not None:
+        model = PONITA_DIFFUSION.load_from_checkpoint(args.resume)
+    else:
+        torch.manual_seed(0)
+        model = PONITA_DIFFUSION(default_args(lr=3e-4 if args.lr is None else args.lr, epochs=args.epochs,
+                                              warmup=args.warmup or 0, batch_size=args.batch_size), ds.z_table)
     fit(model, train_ds, args.epochs, args.batch_size, device, backward_precision=args.backward_precision,
-        val_dataset=val_ds, checkpoint_dir=args.checkpoint_dir)
+        val_dataset=val_ds, checkpoint_dir=args.checkpoint_dir, resume_from=args.resume, ema_decay=args.ema_decay)
+    twin = ema_model(model, device) if args.ema_decay is not None else None
     if rank0:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)) or ".", exist_ok=True)
         model.save_checkpoint(args.out)
+        if twin is not None:
+            twin.save_checkpoint(ema_path(args.out))
     if test_ds is not None:
+        model = model if twin is None else twin
         if val_ds is not None:           # the weights of the best epoch, as every rank reads them from rank 0's file
             if dist.is_initialized():
                 dist.barrier()
-            model = PONITA_DIFFUSION.load_from_checkpoint(os.path.join(args.checkpoint_dir, "best.ckpt"))
+            best = os.path.join(args.checkpoint_dir, "best.ckpt")
+            model = PONITA_DIFFUSION.load_from_checkpoint(best if twin is None else ema_path(best))
         res = evaluate_dataset(model, test_ds, args.batch_size, device)
         if rank0:
             print(f"test loss {res['loss']:.6f} (e_frac {res['e_frac']:.6f}, vb {res['vb']:.6f}, ce {res['ce']:.6f}, "

@@ -99,10 +99,15 @@ def cosine_warmup_factor(epoch: int, warmup: int, max_iters: int) -> float:
 
 class FusedAdam:
     """torch.optim.Adam over the flat buffers as one kernel (arreau_adam_step) with the reference's two weight-decay
-    groups and the trainer's global-norm clip (gradient_clip_val=0.5, main_diffusion.py:297)."""
+    groups and the trainer's global-norm clip (gradient_clip_val=0.5, main_diffusion.py:297).
+
+    ema_decay: keep an exponential moving average of the weights in `self.ema` (a FlatParams of the same layout), the
+    rule of the NeMo EMA callback the reference carries (lightning_wrappers/callbacks.py): the EMA is set to the weights
+    as they are just before the first optimizer step (device copy), and every step updates it from the post-step weights,
+    ema = decay * ema + (1 - decay) * p, inside the Adam kernel."""
 
     def __init__(self, params: FlatParams, lr: float = 3e-4, betas=(0.9, 0.999), eps: float = 1e-8,
-                 weight_decay: float = 0.0, max_grad_norm: float = 0.5):
+                 weight_decay: float = 0.0, max_grad_norm: float = 0.5, ema_decay: Optional[float] = None):
         self.p, self.base_lr, self.lr = params, lr, lr
         self.betas, self.eps, self.weight_decay, self.max_grad_norm = betas, eps, weight_decay, max_grad_norm
         self.exp_avg, self.exp_avg_sq = torch.zeros_like(params.data), torch.zeros_like(params.data)
@@ -110,6 +115,12 @@ class FusedAdam:
         self.step_count = 0
         self.scratch = torch.zeros(512, dtype=torch.float64, device=params.device)
         self.moments = torch.zeros(2, dtype=torch.float64, device=params.device)
+        if ema_decay is not None and not 0.0 <= float(ema_decay) <= 1.0:
+            raise ValueError(f"ema_decay must be in [0, 1], got {ema_decay}")
+        self.ema_decay = None if ema_decay is None else float(ema_decay)
+        self.ema = None if ema_decay is None else FlatParams(params.num_scalar, params.num_vec, params.num_states,
+                                                              params.device)
+        self.ema_initialized = False
 
     def set_epoch(self, epoch: int, warmup: int, max_epochs: int) -> None:
         self.lr = self.base_lr * cosine_warmup_factor(epoch, warmup, max_epochs)
@@ -119,14 +130,86 @@ class FusedAdam:
         s = torch.cuda.current_stream(p.device).cuda_stream
         self.step_count += 1
         p.version += 1
+        if self.ema is not None:
+            if not self.ema_initialized:
+                self.ema.data.copy_(p.data)
+                self.ema_initialized = True
+            self.ema.version += 1
         _lib.call("arreau_moments", p.grad.data_ptr(), None, p.total, self.scratch.data_ptr(), self.moments.data_ptr(), s)
         _lib.call("arreau_adam_step", p.data.data_ptr(), p.grad.data_ptr(), self.exp_avg.data_ptr(),
                   self.exp_avg_sq.data_ptr(), self.mask.data_ptr(), p.total, self.lr, self.betas[0], self.betas[1],
-                  self.eps, self.weight_decay, self.step_count, self.max_grad_norm, self.moments.data_ptr(), s)
+                  self.eps, self.weight_decay, self.step_count, self.max_grad_norm, self.moments.data_ptr(),
+                  _lib.ptr(None if self.ema is None else self.ema.data), self.ema_decay or 0.0, s)
 
     def grad_norm(self) -> float:
         """Global L2 norm of the last step's (unclipped) gradient (host synchronisation)."""
         return float(np.sqrt(self.moments[1].item()))
+
+    # -- state (the layout of torch.optim.Adam.state_dict) ------------------------------------------------------------
+    def param_groups(self):
+        """The two groups of the reference's configure_optimizers as (weight_decay, [names]): the decayed Linear
+        weights, then everything else, each in FlatParams.specs order (the names of FlatParams.decay_mask)."""
+        decayed = [k for k in self.p.specs if k.endswith(".weight") and ".norm." not in k]
+        rest = [k for k in self.p.specs if not (k.endswith(".weight") and ".norm." not in k)]
+        return [(self.weight_decay, decayed), (0.0, rest)]
+
+    def state_dict(self) -> dict:
+        """torch.optim.Adam.state_dict() of the same named groups: state[i] = {step, exp_avg, exp_avg_sq} in each
+        parameter's shape (host copies), param_groups with the hyper-parameters, `params` and `param_names` -- it loads
+        into a torch.optim.Adam built from those groups.  `ema`: the EMA's bookkeeping {decay, initialized} (its
+        weights are saved with the model's names by the checkpoint)."""
+        m, v = self.p._views(self.exp_avg), self.p._views(self.exp_avg_sq)
+        state, groups, i = {}, [], 0
+        for wd, names in self.param_groups():
+            idx = list(range(i, i + len(names)))
+            for j, k in zip(idx, names):
+                state[j] = {"step": torch.tensor(float(self.step_count), dtype=torch.float32),
+                            "exp_avg": m[k].detach().cpu().clone(), "exp_avg_sq": v[k].detach().cpu().clone()}
+            groups.append({"param_names": list(names), "weight_decay": wd, "lr": self.lr, "initial_lr": self.base_lr,
+                           "betas": tuple(self.betas), "eps": self.eps, "amsgrad": False, "maximize": False,
+                           "foreach": None, "capturable": False, "differentiable": False, "fused": None,
+                           "decoupled_weight_decay": False, "params": idx})
+            i += len(names)
+        return {"state": state, "param_groups": groups,
+                "ema": {"decay": self.ema_decay, "initialized": bool(self.ema_initialized)}}
+
+    def load_state_dict(self, sd: Mapping) -> None:
+        """Restores the step count, both moments and the EMA bookkeeping from `state_dict()`'s layout, matched by
+        parameter NAME (not position).  The hyper-parameters stay this optimizer's.  Refuses a state without
+        `param_names` (e.g. a Lightning checkpoint of the reference), with other names or shapes, or with a different
+        EMA decay.  The EMA weights themselves are restored with `self.ema.load_state_dict`.  Bumps the flat buffers'
+        versions like every other in-place load."""
+        groups = sd.get("param_groups", [])
+        if not groups or any("param_names" not in g for g in groups):
+            raise ValueError("optimizer state has no param_names: it was not written by this project's FusedAdam "
+                             "state_dict (a Lightning optimizer state cannot be mapped onto the parameters)")
+        by_name = {}
+        for g in groups:
+            if len(g["param_names"]) != len(g["params"]):
+                raise ValueError("optimizer state: param_names and params differ in length")
+            for k, i in zip(g["param_names"], g["params"]):
+                by_name[k] = sd["state"][i]
+        if set(by_name) != set(self.p.specs):
+            diff = sorted(set(by_name) ^ set(self.p.specs))
+            raise ValueError(f"optimizer state does not name this model's parameters: {diff[:8]}")
+        steps = {int(float(st["step"])) for st in by_name.values()}
+        if len(steps) != 1:
+            raise ValueError(f"optimizer state: parameters are at different steps {sorted(steps)}")
+        ema = sd.get("ema") or {"decay": None, "initialized": False}
+        if (ema["decay"] is None) != (self.ema_decay is None) or (ema["decay"] is not None and float(ema["decay"]) != self.ema_decay):
+            raise ValueError(f"optimizer state has EMA decay {ema['decay']}, this optimizer {self.ema_decay}")
+        m, v = self.p._views(self.exp_avg), self.p._views(self.exp_avg_sq)
+        for k, st in by_name.items():
+            for dst, key in ((m[k], "exp_avg"), (v[k], "exp_avg_sq")):
+                src = torch.as_tensor(st[key])
+                if tuple(src.shape) != tuple(dst.shape):
+                    raise ValueError(f"optimizer state {key} of {k}: shape {tuple(src.shape)}, parameter {tuple(dst.shape)}")
+                dst.copy_(src.to(torch.float32))
+        self.step_count = steps.pop()
+        self.ema_initialized = bool(ema["initialized"])
+        self.p.version += 1
+        if self.ema is not None:
+            self.ema.version += 1
 
 
 def noising_buffers(N: int, G: int, Z: int, dev) -> Dict[str, tuple]:

@@ -553,10 +553,13 @@ int arreau_moments(const float* x, const float* sub_cols, int64_t n, double* scr
  * elements whose decay_mask byte is set, i.e. the Linear weights) after the trainer's global-norm clip
  * (main_diffusion.py:297, gradient_clip_val = 0.5): coef = min(1, max_grad_norm / (sqrt(grad_moments[1]) + 1e-6)),
  * grad_moments = the {sum, sum of squares} arreau_moments wrote for the gradient buffer (device memory, so the step
- * does not synchronise; NULL or max_grad_norm <= 0 disables clipping).  step counts from 1. */
+ * does not synchronise; NULL or max_grad_norm <= 0 disables clipping).  step counts from 1.  ema[n] (NULL: none, and
+ * the step's arithmetic is unchanged): the exponential moving average of the weights, updated in the same pass from the
+ * post-step parameters as ema = ema_decay * ema + (1 - ema_decay) * params (the NeMo EMAOptimizer rule; the caller
+ * initialises ema to the weights before the run's first step); 0 <= ema_decay <= 1. */
 int arreau_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, const uint8_t* decay_mask,
                      int64_t n, double lr, double beta1, double beta2, double eps, double weight_decay, int64_t step,
-                     double max_grad_norm, const double* grad_moments, void* stream);
+                     double max_grad_norm, const double* grad_moments, float* ema, double ema_decay, void* stream);
 
 #ifdef __cplusplus
 }
