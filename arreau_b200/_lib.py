@@ -127,6 +127,8 @@ SIGNATURES = {
     "arreau_fold_basis_w1": [vp, vp, vp, vp, vp],
     "arreau_moments": [vp, vp, i64, vp, vp, vp],
     "arreau_adam_step": [vp, vp, vp, vp, vp, i64, f64, f64, f64, f64, f64, i64, f64, vp, vp, f64, vp],
+    # crystal metrics
+    "arreau_crystal_metrics": [vp, vp, vp, vp, i32, i32, vp, i32, f64, f64, vp, vp, vp, vp, vp, vp],
 }
 RESTYPES = {"arreau_launch_count": i64, "arreau_ponita_backward_workspace_bytes": i64}
 

@@ -12,6 +12,21 @@ _SYMBOLS = ("H He Li Be B C N O F Ne Na Mg Al Si P S Cl Ar K Ca Sc Ti V Cr Mn Fe
             "Pt Au Hg Tl Pb Bi Po At Rn Fr Ra Ac Th Pa U Np Pu Am Cm Bk Cf Es Fm Md No Lr").split()
 ATOMIC_NUMBER = {s: i + 1 for i, s in enumerate(_SYMBOLS)}
 
+# standard atomic weights (IUPAC, amu) of Z = 1..103, in _SYMBOLS order; for elements without stable isotopes the mass
+# number of the longest-lived isotope, as periodic tables print it in brackets
+ATOMIC_MASS = (
+    1.008, 4.002602, 6.94, 9.0121831, 10.81, 12.011, 14.007, 15.999, 18.998403163, 20.1797,
+    22.98976928, 24.305, 26.9815385, 28.085, 30.973761998, 32.06, 35.45, 39.948, 39.0983, 40.078,
+    44.955908, 47.867, 50.9415, 51.9961, 54.938044, 55.845, 58.933194, 58.6934, 63.546, 65.38,
+    69.723, 72.630, 74.921595, 78.971, 79.904, 83.798, 85.4678, 87.62, 88.90584, 91.224,
+    92.90637, 95.95, 98.0, 101.07, 102.90550, 106.42, 107.8682, 112.414, 114.818, 118.710,
+    121.760, 127.60, 126.90447, 131.293, 132.90545196, 137.327, 138.90547, 140.116, 140.90766, 144.242,
+    145.0, 150.36, 151.964, 157.25, 158.92535, 162.500, 164.93033, 167.259, 168.93422, 173.045,
+    174.9668, 178.49, 180.94788, 183.84, 186.207, 190.23, 192.217, 195.084, 196.966569, 200.592,
+    204.38, 207.2, 208.98040, 209.0, 210.0, 222.0, 223.0, 226.0, 227.0, 232.0377,
+    231.03588, 238.02891, 237.0, 244.0, 243.0, 247.0, 247.0, 251.0, 252.0, 257.0,
+    258.0, 259.0, 262.0)
+
 
 class AtomicNumberTable:
     """tools/atomic_number_table.py:7-26."""

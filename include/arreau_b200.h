@@ -561,6 +561,38 @@ int arreau_adam_step(float* params, const float* grads, float* exp_avg, float* e
                      int64_t n, double lr, double beta1, double beta2, double eps, double weight_decay, int64_t step,
                      double max_grad_norm, const double* grad_moments, float* ema, double ema_decay, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Beyond the reference: quality metrics of generated crystals.  The reference post-processes its
+ * samples with pymatgen (CDVAE's structure validity); there are no reference lines to cite.
+ * ------------------------------------------------------------------------------------------- */
+
+#define ARREAU_METRICS_VALID 1           /* not degenerate and min_dist >= min_dist_threshold            */
+#define ARREAU_METRICS_UNKNOWN_ELEMENT 2 /* some Z outside 0..max_z or with atomic_mass[Z] <= 0           */
+#define ARREAU_METRICS_DEGENERATE 4      /* see arreau_crystal_metrics; min_dist is NaN                    */
+#define ARREAU_METRICS_EXTENDED_SEARCH 8 /* the 27 images of the reduced cell did not prove the minimum    */
+
+/* Per-crystal structure metrics.  frac[N,3] f64 and lattice[G,3,3] f64 rows a, b, c (pos = frac @ lattice, Angstrom),
+ * atomic_numbers[N] i64, atom_offset[G+1] i32 (prefix sum of the atom counts), atomic_mass[max_z+1] f64: mass of
+ * Z = 0..max_z in amu, <= 0 for an unknown element.  Outputs per crystal:
+ *   volume[G]       |det lattice|, A^3;
+ *   min_dist[G]     the exact minimum over distinct pairs i < j and every lattice translation of |pos_j - pos_i + t|
+ *                   (+inf below 2 atoms); the basis is size-reduced and the 27 images are extended to the box that
+ *                   provably holds the minimum when they cannot (metrics.cu derives the bound);
+ *   density[G]      sum of masses (atom order) * 1.66053906660 / volume, g/cm^3, NaN with an unknown element;
+ *   num_elements[G] number of distinct known Z;
+ *   flags[G]        ARREAU_METRICS_* bits.  VALID follows CDVAE: min_dist >= min_dist_threshold (0.5 A) and
+ *                   volume >= min_volume (0.1 A^3).
+ * A crystal is DEGENERATE (no search, min_dist NaN, not VALID) when a lattice entry or coordinate is not finite, its
+ * volume is below min_volume, its atom_offset entries are out of order or outside 0..N, or the exact search would need
+ * more than 16 images either way along an axis of the reduced cell (a cell height below 1/16 of the crystal's
+ * shortest 27-image distance).  Any atom count is supported; one warp per crystal.  A crystal's outputs depend only
+ * on that crystal, bit for bit, whatever batch it is in. */
+int arreau_crystal_metrics(const double* frac, const double* lattice, const int64_t* atomic_numbers,
+                           const int32_t* atom_offset, int32_t num_atoms_total, int32_t num_crystals,
+                           const double* atomic_mass, int32_t max_z, double min_dist_threshold, double min_volume,
+                           double* volume, double* min_dist, double* density, int32_t* num_elements, int32_t* flags,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif
