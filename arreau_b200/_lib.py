@@ -53,7 +53,7 @@ class StepArgs(C.Structure):
 
 class StepReplay(C.Structure):
     _fields_ = [("counter", vp), ("vp_table", vp), ("t_of_atom", vp), ("dyn", vp), ("step_out", vp),
-                ("seed", C.c_uint64), ("t_first", i32), ("reserved", i32)]
+                ("seed", C.c_uint64), ("t_first", i32), ("reserved", i32), ("crystal_id", vp)]
 
 
 class WorkspaceSizes(C.Structure):
@@ -106,6 +106,8 @@ SIGNATURES = {
     "arreau_ve_pbc_reverse": [vp, vp, vp, vp, i32, vp, i32, vp, vp],
     "arreau_d3pm_reverse": [vp, vp, vp, vp, i32, vp, vp, f64, f64, i32, i32, i32, vp, vp],
     "arreau_step_noise": [C.c_uint64, i32, i32, i32, i32, vp, vp, vp, vp],
+    "arreau_sample_init_keyed": [C.c_uint64, i32, i32, vp, vp, vp, f64, vp, vp, vp, vp],
+    "arreau_sample_noise_keyed": [C.c_uint64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp],
     "arreau_denoise_step": [C.POINTER(Weights), C.POINTER(Workspace), C.POINTER(StepArgs), vp],
     "arreau_denoise_step_replay": [C.POINTER(Weights), C.POINTER(Workspace), C.POINTER(StepArgs), C.POINTER(StepReplay), vp],
     # training step

@@ -111,6 +111,95 @@ __global__ void eval_noise_kernel(uint64_t seed, int G, int N, int Z, int T, con
   }
 }
 
+// Per-crystal keyed draws of the sampler (arreau_sample_init_keyed / arreau_sample_noise_keyed).  Same key and counter
+// words as eval_noise_kernel; the tag word of a step draw carries the step ordinal above its low 4 bits
+// (tag | step << 4, step < 2^28), so no draw of a trajectory meets another or arreau_step_noise's (0, 1) or
+// arreau_eval_noise's (2..5) tags.
+constexpr uint32_t kTagInitCell = 6, kTagInitFrac = 7, kTagStepLattice = 8, kTagStepFrac = 9, kTagStepType = 10;
+constexpr int kMaxKeyedStep = (1 << 28) - 1;
+
+// Work items: [0, G) one per crystal (beta, lengths), [G, G + 2N) two per atom (frac).
+__global__ void sample_init_keyed_kernel(uint64_t seed, int G, int N, const int64_t* __restrict__ crystal_id,
+                                         const int32_t* __restrict__ atom_offset,
+                                         const int32_t* __restrict__ crystal_of_atom, double pos_sigma_max,
+                                         double* __restrict__ angles, double* __restrict__ lengths,
+                                         double* __restrict__ frac) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  uint32_t r[4];
+  if (idx < G) {
+    const int g = (int)idx;
+    const uint64_t id = (uint64_t)crystal_id[g];
+    philox4x32_10(seed, id, 0u, kTagInitCell, r);
+    angles[3 * (size_t)g + 0] = 90.0;                          // monoclinic (90, U(90, 180), 90), degrees (quirk B5)
+    angles[3 * (size_t)g + 1] = 90.0 + 90.0 * u01(r[0], r[1]);
+    angles[3 * (size_t)g + 2] = 90.0;
+    double v[4];
+    philox4x32_10(seed, id, 1u, kTagInitCell, r);
+    box_muller(r, v[0], v[1]);
+    philox4x32_10(seed, id, 2u, kTagInitCell, r);
+    box_muller(r, v[2], v[3]);
+#pragma unroll
+    for (int d = 0; d < 3; ++d) lengths[3 * (size_t)g + d] = v[d];
+    return;
+  }
+  const long long j = idx - G;
+  if (j < 2LL * N) {
+    const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
+    const uint32_t a = (uint32_t)(b - atom_offset[g]);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagInitFrac, r);
+    double v0, v1;
+    box_muller(r, v0, v1);
+    frac[3 * (size_t)b + 2 * k] = v0 * pos_sigma_max;
+    if (k == 0) frac[3 * (size_t)b + 1] = v1 * pos_sigma_max;
+  }
+}
+
+// Work items as eval_noise_kernel: [0, G) per crystal (z_len), [G, G + 2N) two per atom (z_frac), then ceil(Z/2) per
+// atom (u).  step_ptr (replay): the step ordinal is read from the device.
+__global__ void sample_noise_keyed_kernel(uint64_t seed, int step, int G, int N, int Z,
+                                          const int64_t* __restrict__ crystal_id,
+                                          const int32_t* __restrict__ atom_offset,
+                                          const int32_t* __restrict__ crystal_of_atom, double* __restrict__ z_len,
+                                          double* __restrict__ z_frac, double* __restrict__ u,
+                                          const int32_t* __restrict__ step_ptr) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (step_ptr) step = *step_ptr;
+  const uint32_t hi = (uint32_t)step << 4;
+  const int H = (Z + 1) / 2;
+  uint32_t r[4];
+  if (idx < G) {
+    const int g = (int)idx;
+    const uint64_t id = (uint64_t)crystal_id[g];
+    double v[4];
+    philox4x32_10(seed, id, 0u, kTagStepLattice | hi, r);
+    box_muller(r, v[0], v[1]);
+    philox4x32_10(seed, id, 1u, kTagStepLattice | hi, r);
+    box_muller(r, v[2], v[3]);
+#pragma unroll
+    for (int d = 0; d < 3; ++d) z_len[3 * (size_t)g + d] = v[d];
+    return;
+  }
+  long long j = idx - G;
+  if (j < 2LL * N) {
+    const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
+    const uint32_t a = (uint32_t)(b - atom_offset[g]);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagStepFrac | hi, r);
+    double v0, v1;
+    box_muller(r, v0, v1);
+    z_frac[3 * (size_t)b + 2 * k] = v0;
+    if (k == 0) z_frac[3 * (size_t)b + 1] = v1;
+    return;
+  }
+  j -= 2LL * N;
+  if (j < (long long)N * H) {
+    const int b = (int)(j / H), k = (int)(j % H), g = crystal_of_atom[b];
+    const uint32_t a = (uint32_t)(b - atom_offset[g]);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], a * (uint32_t)H + k, kTagStepType | hi, r);
+    u[(size_t)b * Z + 2 * k] = u01(r[0], r[1]);
+    if (2 * k + 1 < Z) u[(size_t)b * Z + 2 * k + 1] = u01(r[2], r[3]);
+  }
+}
+
 // Replayable step (CUDA graph): the per-step scalars live in device memory and advance by themselves.  One block:
 // k = *counter; t = max(t_first - k, 1); dyn = {t, VP posterior coefficients of t}; t_of_atom[:] = t; step_out = k;
 // then *counter = k + 1.
@@ -191,6 +280,39 @@ extern "C" int arreau_eval_noise(uint64_t seed, int32_t G, int32_t N, int32_t Z,
   const long long work = (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
   eval_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       seed, G, N, Z, num_steps, crystal_id, atom_offset, crystal_of_atom, t_crystal, eps_x, u, eps_l);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+extern "C" int arreau_sample_init_keyed(uint64_t seed, int32_t G, int32_t N, const int64_t* crystal_id,
+                                        const int32_t* atom_offset, const int32_t* crystal_of_atom,
+                                        double pos_sigma_max, double* angles, double* lengths, double* frac,
+                                        void* stream) {
+  if (G < 0 || N < 0) return ARREAU_ERR_BAD_SHAPE;
+  if (G == 0) return ARREAU_OK;
+  if (!crystal_id || !atom_offset || !angles || !lengths || (N > 0 && (!crystal_of_atom || !frac)))
+    return ARREAU_ERR_NULL;
+  const long long work = (long long)G + 2LL * N;
+  sample_init_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      seed, G, N, crystal_id, atom_offset, crystal_of_atom, pos_sigma_max, angles, lengths, frac);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+static long long sample_noise_keyed_work(int G, int N, int Z) {
+  return (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
+}
+
+extern "C" int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t G, int32_t N, int32_t Z,
+                                         const int64_t* crystal_id, const int32_t* atom_offset,
+                                         const int32_t* crystal_of_atom, double* z_len, double* z_frac, double* u,
+                                         void* stream) {
+  if (G < 0 || N < 0 || Z <= 0 || step < 0 || step > kMaxKeyedStep) return ARREAU_ERR_BAD_SHAPE;
+  if (G == 0) return ARREAU_OK;
+  if (!crystal_id || !atom_offset || !z_len || (N > 0 && (!crystal_of_atom || !z_frac || !u))) return ARREAU_ERR_NULL;
+  const long long work = sample_noise_keyed_work(G, N, Z);
+  sample_noise_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      seed, step, G, N, Z, crystal_id, atom_offset, crystal_of_atom, z_len, z_frac, u, nullptr);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }
@@ -329,7 +451,8 @@ extern "C" int arreau_denoise_step(const arreau_weights* w, const arreau_workspa
 
 // The same step with every per-step scalar in device memory, so that ONE captured CUDA graph replays the whole
 // trajectory: replay k runs timestep t = max(t_first - k, 1) with Philox noise of step ordinal k (bit-identical to
-// arreau_step_noise(seed, k) + arreau_denoise_step(t)).  capped graphs only (no host read of the edge count).
+// arreau_step_noise(seed, k) + arreau_denoise_step(t), or with r->crystal_id to arreau_sample_noise_keyed(seed, k)).
+// capped graphs only (no host read of the edge count).
 extern "C" int arreau_denoise_step_replay(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
                                           const arreau_step_replay* r, void* stream) {
   if (!w || !ws || !a || !r) return ARREAU_ERR_NULL;
@@ -342,7 +465,13 @@ extern "C" int arreau_denoise_step_replay(const arreau_weights* w, const arreau_
   cudaStream_t s = (cudaStream_t)stream;
   step_advance_kernel<<<1, 1024, 0, s>>>(r->counter, r->t_first, r->vp_table, N, r->t_of_atom, r->dyn, r->step_out);
   CUDA_LAUNCH_CHECK();
-  {
+  if (r->crystal_id) {      // per-crystal keyed noise (arreau_sample_noise_keyed with the replay's step ordinal)
+    const long long work = sample_noise_keyed_work(G, N, Z);
+    sample_noise_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(
+        r->seed, 0, G, N, Z, r->crystal_id, a->atom_offset, a->crystal_of_atom, const_cast<double*>(a->z_len),
+        const_cast<double*>(a->z_frac), const_cast<double*>(a->u_type), r->step_out);
+    CUDA_LAUNCH_CHECK();
+  } else {
     const long long n_len = 3LL * G, n_normal = n_len + 3LL * N, n_uniform = (long long)N * Z;
     const long long work = ((n_normal > n_uniform ? n_normal : n_uniform) + 1) / 2;
     // (the step's noise buffers are inputs of arreau_denoise_step; here the call itself fills them)

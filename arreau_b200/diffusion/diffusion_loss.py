@@ -2,7 +2,9 @@
 signatures.  The sampler keeps the whole state on the GPU and runs each step as one C call
 (arreau_denoise_step); the reference's torch CPU RNG stream (angles via numpy, randn lengths, randn frac, then
 per step randn_like(lengths), randn_like(frac), rand((N,Z)) -- SURVEY 3.1) is drawn on the host exactly as the
-reference draws it unless `device_noise=True` asks for the in-kernel Philox generator."""
+reference draws it unless `device_noise=True` asks for the in-kernel Philox generator, or `crystal_ids` asks for draws
+keyed per crystal on the device (initial state and step noise), which make a crystal's trajectory independent of the
+batch it is sampled in."""
 from __future__ import annotations
 
 from typing import Optional
@@ -245,33 +247,50 @@ class DiffusionLoss(torch.nn.Module):
                vis_name: str = "", visualization_setting=None, show_bonds: bool = False,
                constant_atoms: Optional[torch.Tensor] = None, num_atoms: Optional[torch.Tensor] = None,
                device="cuda", device_noise: bool = False, seed: int = 0, step_callback=None,
-               cuda_graph: bool = False) -> SampleResult:
+               cuda_graph: bool = False, crystal_ids=None) -> SampleResult:
         """diffusion/diffusion_loss.py:277-377.  Extra keyword-only options (defaults reproduce the reference):
         `num_atoms` a per-crystal atom-count vector, `device_noise` Philox noise generated on the GPU,
-        `step_callback(timestep, engine)` called after each step (e.g. to log E/N), `cuda_graph` (needs device_noise and
-        max_neighbors > 0): the loop body is captured once and replayed T - 1 times, one launch per step -- bit-identical
-        results; it pays for small batches, whose steps are launch bound."""
+        `step_callback(timestep, engine)` called after each step (e.g. to log E/N), `cuda_graph` (needs device_noise or
+        crystal_ids, and max_neighbors > 0): the loop body is captured once and replayed T - 1 times, one launch per
+        step -- bit-identical results; it pays for small batches, whose steps are launch bound.
+        `crystal_ids` (G integers): the initial state and every step's noise are drawn on the device per crystal, keyed
+        by (seed, id) (arreau_sample_init_keyed / arreau_sample_noise_keyed), so a crystal's trajectory depends on the
+        weights, the precision, the seed, its id and its atom count only -- not on the batch it is sampled in.  The
+        host generators (numpy, torch) are not touched; device_noise is implied."""
         Z = len(z_table)
         G = num_samples_in_batch
         dd = torch.float64                                     # main_diffusion_generate.py:27
-        angles = torch.tensor([sample_bravais_angles("monoclinic") for _ in range(G)], dtype=dd)
-        lengths = torch.randn([G, 3], dtype=dd)
+        keyed = crystal_ids is not None
+        if keyed:
+            crystal_ids = torch.as_tensor(crystal_ids).reshape(-1)
+            if crystal_ids.shape[0] != G:
+                raise ValueError(f"{crystal_ids.shape[0]} crystal ids for {G} crystals")
+        else:
+            angles = torch.tensor([sample_bravais_angles("monoclinic") for _ in range(G)], dtype=dd)
+            lengths = torch.randn([G, 3], dtype=dd)
         na = torch.full((G,), num_atoms_per_sample) if num_atoms is None else torch.as_tensor(num_atoms).reshape(-1)
         N = int(na.sum())
-        frac_x = torch.randn([N, 3], dtype=dd) * pos_sigma_max
+        if not keyed:
+            frac_x = torch.randn([N, 3], dtype=dd) * pos_sigma_max
         atom_types = constant_atoms if constant_atoms is not None else torch.full((N,), Z - 1)
         eng = self.engine_for(model, t_emb_weights, na, torch.device(device))
-        eng.set_state(frac_x, atom_types, lengths, angles)
+        if keyed:
+            eng.set_crystal_ids(crystal_ids)
+            eng.init_state_keyed(seed, atom_types, pos_sigma_max)
+        else:
+            eng.set_state(frac_x, atom_types, lengths, angles)
+        if cuda_graph and (not (device_noise or keyed) or self.max_neighbors <= 0):
+            raise ValueError("cuda_graph=True needs device_noise=True (or crystal_ids) and max_neighbors > 0")
         if cuda_graph:
-            if not device_noise or self.max_neighbors <= 0:
-                raise ValueError("cuda_graph=True needs device_noise=True and max_neighbors > 0")
-            g = eng.capture_trajectory_graph(self.T - 1, seed, update_types=constant_atoms is None)
+            g = eng.capture_trajectory_graph(self.T - 1, seed, update_types=constant_atoms is None, keyed=keyed)
             for timestep in reversed(range(1, self.T)):
                 g.replay()
                 if step_callback is not None:
                     step_callback(timestep, eng)
         for step_idx, timestep in enumerate(reversed(range(1, self.T)) if not cuda_graph else ()):
-            if device_noise:
+            if keyed:
+                eng.draw_noise_keyed(seed, step_idx)
+            elif device_noise:
                 eng.draw_noise(seed, step_idx)
             else:   # the reference's draw order per step: lengths, frac, types
                 eng.set_noise(torch.randn(G, 3, dtype=dd), torch.randn(N, 3, dtype=dd), torch.rand(N, Z, dtype=dd))

@@ -43,6 +43,13 @@ def all_gather_rows(arrays: Sequence[np.ndarray], group=None, device: Optional[t
     return out
 
 
+def gather_crystal_metrics(local, group=None, device: Optional[torch.device] = None):
+    """All-gather every rank's per-crystal CrystalMetrics rows (inference/crystal_metrics.py) into the whole set, in
+    rank order -- one all_gather_rows.  A collective: every rank joins, also one with no crystals."""
+    from .inference.crystal_metrics import METRIC_FIELDS, metrics_from_rows
+    return metrics_from_rows(all_gather_rows([np.asarray(getattr(local, k)) for k in METRIC_FIELDS], group, device))
+
+
 def gather_rng_states(state: torch.Tensor, group=None, device: Optional[torch.device] = None) -> List[torch.Tensor]:
     """Every rank's generator state (a uint8 tensor such as torch.cuda.get_rng_state() returns) in rank order, on every
     rank.  A collective (all_gather_rows): every rank must join it.  World size 1: [state]."""

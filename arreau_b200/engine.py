@@ -51,7 +51,8 @@ class DenoiseEngine:
                   "z_frac": ((3,), torch.float64)}
     _CRYSTAL_BUFS = {"lengths": ((3,), torch.float64), "angles": ((3,), torch.float64), "lattice": ((3, 3), torch.float64),
                      "angle_trig": ((6,), torch.float64), "num_neighbors_image": ((), torch.int64),
-                     "len0": ((3,), torch.float32), "z_len": ((3,), torch.float64), "num_atoms": ((), torch.int64)}
+                     "len0": ((3,), torch.float32), "z_len": ((3,), torch.float64), "num_atoms": ((), torch.int64),
+                     "crystal_id": ((), torch.int64)}
 
     def __init__(self, weights: PonitaWeights, tables: DiffusionTables, fourier_w, num_atoms: Sequence[int],
                  radius: float, max_neighbors: int, precision: str = "fp32", edge_capacity: Optional[int] = None,
@@ -278,6 +279,34 @@ class DenoiseEngine:
         _lib.call("arreau_step_noise", C.c_uint64(seed), step, self.G, self.N, self.Z, self.z_len.data_ptr(),
                   self.z_frac.data_ptr(), self.u_type.data_ptr(), self.stream)
 
+    # ------------------------------------------------------------------ per-crystal keyed sampling noise
+    def set_crystal_ids(self, crystal_ids) -> None:
+        """Bind the ids of the bound batch's crystals (G, any integer dtype, host or device): the key of the
+        keyed draws below.  Kept on the device next to the topology."""
+        ids = torch.as_tensor(crystal_ids).reshape(-1)
+        if ids.shape[0] != self.G:
+            raise ValueError(f"{ids.shape[0]} crystal ids for a batch of {self.G} crystals")
+        ids = ids.to(torch.int64)
+        self.crystal_id.copy_(ids.pin_memory() if ids.device.type == "cpu" and self.device.type == "cuda" else ids,
+                              non_blocking=True)
+
+    def init_state_keyed(self, seed: int, types, pos_sigma_max: float) -> None:
+        """The sampler's initial state drawn per crystal on the device (arreau_sample_init_keyed, keyed by seed and the
+        bound crystal ids): angles (90, U(90,180), 90), lengths N(0,1), frac N(0,1) * pos_sigma_max; types are given.
+        The angle factors are formed on the host from the drawn angles, as set_state does (one device->host read of
+        G x 3 doubles)."""
+        _lib.call("arreau_sample_init_keyed", C.c_uint64(int(seed)), self.G, self.N, self.crystal_id.data_ptr(),
+                  self.atom_offset.data_ptr(), self.crystal_of_atom.data_ptr(), float(pos_sigma_max),
+                  self.angles.data_ptr(), self.lengths.data_ptr(), self.frac.data_ptr(), self.stream)
+        self.types.copy_(torch.as_tensor(types).reshape(self.N), non_blocking=True)
+        self.angle_trig.copy_(angle_factors(self.angles.to("cpu", torch.float64)), non_blocking=True)
+
+    def draw_noise_keyed(self, seed: int, step: int) -> None:
+        """One step's noise drawn per crystal on the device (arreau_sample_noise_keyed, step ordinal `step`)."""
+        _lib.call("arreau_sample_noise_keyed", C.c_uint64(int(seed)), int(step), self.G, self.N, self.Z,
+                  self.crystal_id.data_ptr(), self.atom_offset.data_ptr(), self.crystal_of_atom.data_ptr(),
+                  self.z_len.data_ptr(), self.z_frac.data_ptr(), self.u_type.data_ptr(), self.stream)
+
     # ------------------------------------------------------------------ graph
     def _count(self) -> None:
         s = self.stream
@@ -380,11 +409,13 @@ class DenoiseEngine:
             self.ws.onehot_types = None
 
     # ------------------------------------------------------------------ whole trajectory as one replayed CUDA graph
-    def capture_trajectory_graph(self, t_first: int, seed: int, update_types: bool = True) -> "torch.cuda.CUDAGraph":
+    def capture_trajectory_graph(self, t_first: int, seed: int, update_types: bool = True,
+                                 keyed: bool = False) -> "torch.cuda.CUDAGraph":
         """Capture ONE denoise step (arreau_denoise_step_replay: Philox noise + graph + network + update, every
         per-step scalar in device memory) as a CUDA graph; replay k runs timestep max(t_first - k, 1) with the noise of
         step ordinal k, so `for _ in range(steps): g.replay()` is the sampler loop of diffusion_loss.py:318-349 with one
-        launch per step instead of 26.  Bit-identical to `draw_noise(seed, k); step(t)`.  Capped graphs only.
+        launch per step instead of 26.  Bit-identical to `draw_noise(seed, k); step(t)`, or with `keyed` (the noise
+        keyed per crystal by the bound crystal ids) to `draw_noise_keyed(seed, k); step(t)`.  Capped graphs only.
         `reset_trajectory_graph()` rewinds the device-side step counter (a new trajectory on new state)."""
         if self.cap <= 0:
             raise ValueError("the replayable step needs max_neighbors > 0 (uncapped graphs size their buffers on the host)")
@@ -399,6 +430,7 @@ class DenoiseEngine:
         b, r = self._replay_bufs, self._replay
         r.counter, r.vp_table, r.t_of_atom = b["counter"].data_ptr(), b["table"].data_ptr(), b["t_of_atom"].data_ptr()
         r.dyn, r.step_out, r.seed, r.t_first = b["dyn"].data_ptr(), b["step_out"].data_ptr(), int(seed), int(t_first)
+        r.crystal_id = self.crystal_id.data_ptr() if keyed else None
         a = self.args
         a.update_types = 1 if update_types else 0
         self.ws.onehot_types = self.types.data_ptr()

@@ -2,6 +2,7 @@
 
     python -m arreau_b200.generate --model_path model.ckpt --num_crystals 1024 --num_atoms 40 [--batch 1024]
     python -m arreau_b200.generate --model_path model.ckpt --num_crystals 1024 --num_atoms_from data/train.h5
+    python -m arreau_b200.generate ... --keyed_noise      # the same crystals whatever --batch and the number of GPUs
     torchrun --nproc-per-node 8 -m arreau_b200.generate ...      # crystals sharded over the GPUs, one gather at the end
 
 The reference samples 10 crystals per batch on the CPU; here a batch is as large as fits (1024 by default), every
@@ -28,12 +29,15 @@ OUT_DIR = "out"
 def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional[int],
                         use_constant_atomic_symbols: Optional[list] = None, num_crystals_per_batch: int = 1024,
                         device="cuda", device_noise: bool = True, seed: int = 0, out_path: Optional[str] = None,
-                        group=None, timings: Optional[dict] = None, num_atoms=None) -> SampleResult:
+                        group=None, timings: Optional[dict] = None, num_atoms=None,
+                        keyed_noise: bool = False) -> SampleResult:
     """main_diffusion_generate.py:52-94.  With torch.distributed initialised the crystals are sharded over the ranks;
     every rank returns the full gathered result and rank 0 writes `out_path`.  `timings` (optional dict) receives this
     rank's wall-clock seconds per phase: `sample` (list, one per batch), `gather`, `write`.  `num_atoms` (optional,
     length num_crystals) gives every crystal its own atom count instead of `num_atoms_per_sample`; each rank samples
-    its shard of it (see `draw_num_atoms`)."""
+    its shard of it (see `draw_num_atoms`).  `keyed_noise`: crystal i of the run gets id i and every draw of its
+    trajectory is keyed by (seed, i) on the device (DiffusionLoss.sample's crystal_ids), so the result does not depend
+    on num_crystals_per_batch or on the number of ranks.  Without it, batch b0.. is sampled with seed + b0."""
     if num_atoms is not None:
         num_atoms = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
         if num_atoms.shape[0] != num_crystals or np.any(num_atoms < 1):
@@ -48,10 +52,12 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
     for b0 in range(lo, hi, num_crystals_per_batch):
         nb = min(num_crystals_per_batch, hi - b0)
         kw = {} if num_atoms is None else {"num_atoms": torch.from_numpy(num_atoms[b0:b0 + nb].copy())}
+        if keyed_noise:
+            kw["crystal_ids"] = torch.arange(b0, b0 + nb, dtype=torch.int64)
         t0 = time.perf_counter()
         parts.append(model.sample(num_atoms_per_sample=num_atoms_per_sample, num_samples_in_batch=nb,
                                   use_constant_atomic_symbols=use_constant_atomic_symbols, device=device,
-                                  device_noise=device_noise, seed=seed + b0, **kw))
+                                  device_noise=device_noise, seed=seed if keyed_noise else seed + b0, **kw))
         t_batches.append(time.perf_counter() - t0)      # sample() ends with the device->host copy of the result
     n_local = hi - lo
     if parts:
@@ -91,6 +97,9 @@ def main(argv=None):
     ap.add_argument("--num_atoms_from", nargs="+", default=None, metavar="DATA",
                     help="draw every crystal's atom count from these dataset files' counts (.h5 or .npz)")
     ap.add_argument("--seed", type=int, default=0, help="seed of the sampling noise and of the --num_atoms_from draw")
+    ap.add_argument("--keyed_noise", action="store_true",
+                    help="key every crystal's noise by (seed, its index in the run): the output then does not depend on "
+                         "--batch or the number of GPUs")
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--precision", default="fp16", choices=["fp32", "fp16"])
     ap.add_argument("--symbols", nargs="*", default=None, help="constant atomic symbols (use_constant_atomic_symbols)")
@@ -122,7 +131,7 @@ def main(argv=None):
     model = PONITA_DIFFUSION.load_from_checkpoint(args.model_path, ori_grid=grid, strict=not args.no_strict,
                                                   precision=args.precision)
     res = generate_n_crystals(model, args.num_crystals, args.num_atoms, args.symbols, args.batch, device=dev,
-                              seed=args.seed, out_path=args.out, num_atoms=counts)
+                              seed=args.seed, out_path=args.out, num_atoms=counts, keyed_noise=args.keyed_noise)
     if not dist.is_initialized() or dist.get_rank() == 0:
         print(f"wrote {res.num_atoms.shape[0]} crystals ({res.frac_x.shape[0]} atoms)")
     if dist.is_initialized():

@@ -7,7 +7,9 @@ minimum-image distance over distinct atom pairs, the density and the number of d
 crystal is structurally valid when every pair of distinct atoms is at least 0.5 A apart under periodic boundary
 conditions and the cell volume is at least 0.1 A^3 (CDVAE's `structure_validity`).  `summarize` turns the per-crystal
 values into the valid fractions and the Wasserstein-1 distances of density, element count and atom count against a
-reference set (the data the model was trained on, or its test split).  Compositional validity (oxidation states),
+reference set (the data the model was trained on, or its test split).  `quality_record` is the compact subset that
+train.fit's sample-quality monitoring logs per pass (the per-crystal rows of all ranks are gathered with
+distributed.gather_crystal_metrics first).  Compositional validity (oxidation states),
 coverage, novelty and uniqueness need pymatgen / SMACT / CrystalNN and are not computed here."""
 from __future__ import annotations
 
@@ -196,6 +198,33 @@ def summarize(generated: CrystalMetrics, reference: Optional[CrystalMetrics] = N
                    w1_num_elements=_w1(generated.num_elements[sel], reference.num_elements[rk]),
                    w1_num_atoms=_w1(generated.num_atoms, reference.num_atoms))
     return out
+
+
+METRIC_FIELDS = ("num_atoms", "volume", "min_dist", "density", "num_elements", "flags")
+_FIELD_DTYPES = (np.int64, np.float64, np.float64, np.float64, np.int32, np.int32)
+# the compact record of one sample-quality pass of train.fit (its `sample_quality` history): the epoch and these keys
+# of `summarize` against the reference split
+QUALITY_KEYS = ("frac_valid", "w1_density", "w1_num_elements", "min_dist_p1", "min_dist_p5", "min_dist_p25",
+                "min_dist_p50")
+
+
+def metrics_from_rows(rows) -> CrystalMetrics:
+    """CrystalMetrics from its METRIC_FIELDS arrays in that order (e.g. as all_gather_rows returns them, integers
+    widened to int64), each cast back to the field's dtype."""
+    return CrystalMetrics(**{k: np.asarray(v).astype(dt, copy=False).reshape(-1)
+                             for k, v, dt in zip(METRIC_FIELDS, rows, _FIELD_DTYPES)})
+
+
+def concat_metrics(parts) -> CrystalMetrics:
+    """The crystals of several CrystalMetrics, in order (no parts: an empty one)."""
+    return metrics_from_rows([np.concatenate([getattr(p, k) for p in parts]) if parts else np.zeros(0)
+                              for k in METRIC_FIELDS])
+
+
+def quality_record(summary: dict, epoch: int) -> dict:
+    """{epoch, frac_valid, w1_density, w1_num_elements, min_dist_p1 .. p50} of a `summarize` result (None where it has
+    none)."""
+    return {"epoch": int(epoch), **{k: summary.get(k) for k in QUALITY_KEYS}}
 
 
 def main(argv=None):

@@ -17,7 +17,14 @@ last.ckpt also carries the training state (Adam moments and step, epoch, loss hi
 CUDA generator, the EMA), so `--resume out/ckpt/last.ckpt` with the same data, batch size, fractions and --epochs
 continues the run exactly where it stopped.  --ema_decay D keeps an exponential moving average of the weights (the NeMo
 EMA callback the reference carries): the EMA weights are the ones validated and tested, and last.ckpt, best.ckpt and
---out each get a twin *-EMA.ckpt holding them (a plain model checkpoint, e.g. for `generate --model_path`)."""
+--out each get a twin *-EMA.ckpt holding them (a plain model checkpoint, e.g. for `generate --model_path`).
+
+--sample_every K --sample_count M tracks sample quality during training: after the validation of every K-th and of the
+last epoch, M crystals (atom counts drawn once from the training split, noise keyed per crystal, so every pass samples
+the same crystals) are generated at fp16 with the validated weights, each GPU its shard; their structural validity,
+density and element-count distances to the validation split (the training split without one) and min-distance
+percentiles are logged on the epoch line and kept in last.ckpt (SampleMonitor).  best.ckpt stays chosen by the valid
+loss, and the training itself is the same with and without monitoring."""
 from __future__ import annotations
 
 import argparse
@@ -30,7 +37,7 @@ import torch.distributed as dist
 
 from .diffusion.lattice_dataset import CrystalDataset, CrystalSubset, batches, split_indices
 from .distributed import (allreduce_gradients, broadcast_parameters, gather_rng_states, rank_rng_state,
-                          reduce_loss_metric)
+                          reduce_loss_metric, shard_range)
 from .evaluation import evaluate_dataset
 from .lightning_wrappers.diffusion import PONITA_DIFFUSION
 
@@ -69,10 +76,101 @@ def ema_model(model: PONITA_DIFFUSION, device) -> PONITA_DIFFUSION:
     return m
 
 
+def sampling_model(model: PONITA_DIFFUSION, device, flat=None) -> PONITA_DIFFUSION:
+    """A twin of `model` for sampling, built like `ema_model`'s: fp16 (generate's default precision), its trainable
+    tensors views of `flat` (a FlatParams; default the model's own weight buffer, or e.g. its optimizer's EMA buffer),
+    which is only read.  It has its own DiffusionLoss, so its sampling engine is neither the train nor the eval engine.
+    Its buffers and time embedding are copies of `model`'s.  The CPU random generator is left as it was."""
+    flat = model.model.flat if flat is None else flat
+    if flat is None:
+        raise ValueError("the model has no flat weight buffer: flatten_parameters / configure_optimizers first")
+    with torch.random.fork_rng(devices=[]):
+        m = PONITA_DIFFUSION(model.hparams.args, model.hparams.z_table, ori_grid=model.model.ori_grid.detach().cpu(),
+                             precision="fp16")
+    m.load_state_dict(model.state_dict(), strict=False)
+    m.to(device)
+    m.model.flatten_parameters(device, into=flat)
+    return m
+
+
+# crystals per sampling batch of a sample-quality pass (the batch bounds the device memory, not the result)
+SAMPLE_BATCH = 1024
+
+
+class SampleMonitor:
+    """Sample quality inside `fit`: `count` crystals with ids 0..count-1, their atom counts drawn once per run from the
+    training split (draw_num_atoms with the run's seed) and their noise keyed by (seed, id), so every pass samples the
+    same crystals with the same noise and a change between passes comes from the weights only.  Each rank samples its
+    shard_range of the ids with the fp16 sampling twin (the CUDA-graph trajectory when max_neighbors > 0), computes
+    crystal_metrics on the device, and the rows are all-gathered once; rank 0 summarizes them against a reference
+    computed once from `reference_dataset`.  No torch RNG, and neither the training weights nor the train / eval
+    engines are written."""
+
+    def __init__(self, model: PONITA_DIFFUSION, flat, train_dataset, reference_dataset, count: int, seed: int, device):
+        from .generate import draw_num_atoms
+        self.model, self.flat, self.device, self.seed = model, flat, torch.device(device), int(seed)
+        self.num_atoms = draw_num_atoms(train_dataset.atom_counts(), int(count), self.seed)
+        self.reference_dataset = reference_dataset
+        self.reference = None
+        self.twin = None
+
+    def local_metrics(self):
+        """crystal_metrics of this rank's shard of the crystals (its SampleResults never leave the rank)."""
+        from .inference.crystal_metrics import concat_metrics, crystal_metrics, sample_inputs
+        rank = dist.get_rank() if dist.is_initialized() else 0
+        world = dist.get_world_size() if dist.is_initialized() else 1
+        if self.twin is None:
+            self.twin = sampling_model(self.model, self.device, self.flat)
+        lo, hi = shard_range(len(self.num_atoms), rank, world)
+        graph = self.twin.diffusion_loss.max_neighbors > 0
+        parts = []
+        for b0 in range(lo, hi, SAMPLE_BATCH):
+            b1 = min(b0 + SAMPLE_BATCH, hi)
+            res = self.twin.sample(None, b1 - b0, num_atoms=torch.from_numpy(self.num_atoms[b0:b1].copy()),
+                                   crystal_ids=torch.arange(b0, b1, dtype=torch.int64), seed=self.seed,
+                                   device=self.device, cuda_graph=graph)
+            parts.append(crystal_metrics(*sample_inputs(res), device=self.device))
+        return concat_metrics(parts)
+
+    def run(self, epoch: int) -> Optional[dict]:
+        """One pass (a collective): the quality_record of `epoch` on rank 0, None on the other ranks."""
+        from .distributed import gather_crystal_metrics
+        from .inference.crystal_metrics import crystal_metrics, dataset_inputs, quality_record, summarize
+        local = self.local_metrics()
+        comm = self.device if dist.is_initialized() and dist.get_backend() == "nccl" else None
+        rows = gather_crystal_metrics(local, device=comm)
+        if dist.is_initialized() and dist.get_rank() != 0:
+            return None
+        if self.reference is None:
+            self.reference = crystal_metrics(*dataset_inputs(self.reference_dataset), device=self.device)
+        return quality_record(summarize(rows, self.reference), epoch)
+
+
+def _fmt(v) -> str:
+    return "n/a" if v is None else f"{v:.4g}"
+
+
+def format_quality(rec: dict) -> str:
+    """The sample-quality part of fit's epoch line."""
+    return (f"samples: valid {_fmt(rec['frac_valid'])}, w1 density {_fmt(rec['w1_density'])}, w1 elements "
+            f"{_fmt(rec['w1_num_elements'])}, min dist p1/p5/p25/p50 "
+            + "/".join(_fmt(rec[f"min_dist_p{p}"]) for p in (1, 5, 25, 50)))
+
+
+def check_monitoring(sample_every: int, sample_count: int) -> None:
+    """ValueError unless sample_every >= 0 (0: off) and sample_count >= 1."""
+    if int(sample_every) != sample_every or sample_every < 0:
+        raise ValueError(f"sample_every must be an integer >= 0 (0 turns sample monitoring off), got {sample_every}")
+    if int(sample_count) != sample_count or sample_count < 1:
+        raise ValueError(f"sample_count must be an integer >= 1, got {sample_count}")
+
+
 def check_resume(ckpt, *, epochs: int, batch_size: int, world_size: int, backward_precision: str, num_train: int,
-                 num_valid: int, seed: int = 0, ema_decay: Optional[float] = None) -> dict:
+                 num_valid: int, seed: int = 0, ema_decay: Optional[float] = None, sample_every: int = 0,
+                 sample_count: int = 1024) -> dict:
     """The checkpoint (a path or the loaded dict) if it is a resume point of the run these arguments describe; a
-    ValueError naming every mismatch otherwise.  Reads the file only (no device work)."""
+    ValueError naming every mismatch otherwise.  Reads the file only (no device work).  A checkpoint written before
+    sample monitoring existed is a run with sample_every 0; with monitoring off the sample count is not compared."""
     from .lightning_wrappers.diffusion import load_checkpoint_file
     name = ckpt if isinstance(ckpt, (str, os.PathLike)) else "checkpoint"
     if not isinstance(ckpt, dict):
@@ -87,9 +185,12 @@ def check_resume(ckpt, *, epochs: int, batch_size: int, world_size: int, backwar
             "valid split size": fs["num_valid"], "seed": fs["seed"],
             "ema_decay": None if saved_ema is None else float(saved_ema["decay"]),
             "epochs": getattr(ckpt["hyper_parameters"]["args"], "epochs", None)}
+    saved_every = int(fs.get("sample_every", 0))
+    have.update({"sample_every": saved_every, "sample_count": fs.get("sample_count") if saved_every else None})
     want = {"batch_size": batch_size, "world size": world_size, "backward_precision": backward_precision,
             "train split size": num_train, "valid split size": num_valid, "seed": seed,
-            "ema_decay": None if ema_decay is None else float(ema_decay), "epochs": epochs}
+            "ema_decay": None if ema_decay is None else float(ema_decay), "epochs": epochs,
+            "sample_every": int(sample_every), "sample_count": int(sample_count) if sample_every else None}
     bad = [f"{k}: checkpoint {have[k]}, this run {want[k]}" for k in want if have[k] != want[k]]
     if bad:
         raise ValueError(f"{name} is not a resume point of this run: " + "; ".join(bad))
@@ -99,12 +200,22 @@ def check_resume(ckpt, *, epochs: int, batch_size: int, world_size: int, backwar
 def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_size: int, device, seed: int = 0,
         backward_precision: str = "tf32", calibrate: bool = True, log=print, val_dataset=None,
         checkpoint_dir: Optional[str] = None, metrics: Optional[dict] = None, resume_from: Optional[str] = None,
-        ema_decay: Optional[float] = None):
+        ema_decay: Optional[float] = None, sample_every: int = 0, sample_count: int = 1024):
     """Trains `model` for `epochs` and returns the per-epoch train loss.  val_dataset: evaluated after every epoch
     (evaluate_dataset with the same batch_size and seed; logged as "valid loss").  checkpoint_dir: rank 0 writes
     last.ckpt every epoch -- the weights plus the training state a resume needs -- and, with a validation set, best.ckpt
     whenever the valid loss improves.  metrics (optional dict): receives metrics["valid"], one evaluate_dataset result
-    per epoch of this call.
+    per epoch of this call, and (rank 0, with sample monitoring) metrics["samples"], one record per pass of this call,
+    and metrics["sample_quality"], the run's whole history of them.
+
+    sample_every K > 0: after the validation of every K-th epoch and of the last epoch, `sample_count` crystals are
+    sampled with the weights that are validated (the EMA when there is one) and their quality is measured on the
+    device (SampleMonitor: keyed noise, so every pass samples the same crystals with the same noise).  Rank 0 appends a
+    compact record -- epoch, valid fraction, w1_density, w1_num_elements, min-distance percentiles (quality_record),
+    against the validation split, or the training split without one -- to the run's `sample_quality` history, which
+    last.ckpt carries and a resume restores; it is logged on the epoch line.  best.ckpt is still chosen by the valid
+    loss, and training is bit-identical with and without monitoring.  K < 0 or sample_count < 1 is a ValueError,
+    raised before any device work.
 
     resume_from: a last.ckpt of a run with the same data splits, batch_size, world size, backward_precision, seed and
     ema_decay, whose model was built with `epochs` epochs (checked before any device work, ValueError otherwise).  The
@@ -115,18 +226,20 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
     ema_decay: the optimizer keeps an EMA of the weights (FusedAdam).  The EMA weights are the ones validated (and
     best.ckpt is chosen by their loss), and last.ckpt / best.ckpt each get a twin *-EMA.ckpt, a model checkpoint of
     the EMA weights.  Training itself is the same as without EMA."""
+    check_monitoring(sample_every, sample_count)
     rank = dist.get_rank() if dist.is_initialized() else 0
     world = dist.get_world_size() if dist.is_initialized() else 1
     ckpt = None
     if resume_from is not None:
         ckpt = check_resume(resume_from, epochs=epochs, batch_size=batch_size, world_size=world,
                             backward_precision=backward_precision, num_train=len(dataset),
-                            num_valid=0 if val_dataset is None else len(val_dataset), seed=seed, ema_decay=ema_decay)
+                            num_valid=0 if val_dataset is None else len(val_dataset), seed=seed, ema_decay=ema_decay,
+                            sample_every=sample_every, sample_count=sample_count)
     model.to(device)
     model.diffusion_loss.backward_precision = backward_precision
     opt = model.configure_optimizers(device, ema_decay=ema_decay)
     flat = model.model.flat
-    history, valid_losses = [], []
+    history, valid_losses, quality = [], [], []
     best = float("inf")
     first = 0
     if ckpt is not None:
@@ -138,6 +251,7 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
         opt.load_state_dict(ckpt["optimizer_states"][0])
         fs = ckpt["fit_state"]
         history, valid_losses, best = list(fs["train_losses"]), list(fs["valid_losses"]), float(fs["best_valid"])
+        quality = [dict(r) for r in fs.get("sample_quality", [])]
         first = int(ckpt["epoch"]) + 1
         calibrate = False
     broadcast_parameters(flat.data)
@@ -146,6 +260,10 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
         if twin is not None:
             opt.ema.load_state_dict({k[len("model."):]: v for k, v in ckpt["ema"]["state_dict"].items()})
         torch.cuda.set_rng_state(rank_rng_state(ckpt["fit_state"]["cuda_rng"]), device)
+    monitor = None
+    if sample_every > 0:
+        monitor = SampleMonitor(model, opt.ema if twin is not None else flat, dataset,
+                                val_dataset if val_dataset is not None else dataset, sample_count, seed, device)
     comm = device if dist.is_initialized() and dist.get_backend() == "nccl" else None
     if checkpoint_dir is not None and rank == 0:
         os.makedirs(checkpoint_dir, exist_ok=True)
@@ -185,6 +303,13 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
         improved = valid is not None and valid["loss"] < best
         if improved:
             best = valid["loss"]
+        sampled = None
+        if monitor is not None and ((epoch + 1) % sample_every == 0 or epoch == epochs - 1):
+            sampled = monitor.run(epoch)              # a collective; the record on rank 0 only
+            if sampled is not None:
+                quality.append(sampled)
+                if metrics is not None:
+                    metrics.setdefault("samples", []).append(sampled)
         state = None
         if checkpoint_dir is not None:                 # every rank's generator (a collective), then rank 0 writes
             rng = gather_rng_states(torch.cuda.get_rng_state(device), device=comm)
@@ -197,9 +322,13 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
                                        "backward_precision": backward_precision, "num_train": len(dataset),
                                        "num_valid": 0 if val_dataset is None else len(val_dataset),
                                        "train_losses": list(history), "valid_losses": list(valid_losses),
-                                       "best_valid": best, "cuda_rng": rng}}
+                                       "best_valid": best, "cuda_rng": rng, "sample_every": int(sample_every),
+                                       "sample_count": int(sample_count),
+                                       "sample_quality": [dict(r) for r in quality]}}
         if rank == 0:
             shown = "" if valid is None else f", valid loss {valid['loss']:.6f}" + (" (EMA weights)" if twin is not None else "")
+            if sampled is not None:
+                shown += ", " + format_quality(sampled)
             log(f"epoch {epoch}: train loss {history[-1]:.6f}{shown} (lr {opt.lr:.3e})")
             if checkpoint_dir is not None:
                 saves = [("last.ckpt", state)] + ([("best.ckpt", None)] if improved else [])
@@ -207,10 +336,12 @@ def fit(model: PONITA_DIFFUSION, dataset: CrystalDataset, epochs: int, batch_siz
                     model.save_checkpoint(os.path.join(checkpoint_dir, name), training_state=extra)
                     if twin is not None:
                         twin.save_checkpoint(ema_path(os.path.join(checkpoint_dir, name)))
+    if metrics is not None and monitor is not None and rank == 0:
+        metrics["sample_quality"] = [dict(r) for r in quality]
     return history
 
 
-def main():
+def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--data", nargs="+", required=True, help="dataset files (.h5 as written by prep_datasets.py, or .npz)")
     ap.add_argument("--epochs", type=int, default=1)
@@ -227,7 +358,15 @@ def main():
                          "--backward_precision and --ema_decay must be the run's")
     ap.add_argument("--ema_decay", type=float, default=None,
                     help="keep an EMA of the weights (e.g. 0.999): it is validated and saved as *-EMA.ckpt twins")
-    args = ap.parse_args()
+    ap.add_argument("--sample_every", type=int, default=0, metavar="K",
+                    help="every K-th and the last epoch, sample --sample_count crystals with the validated weights and "
+                         "log their quality (0: off)")
+    ap.add_argument("--sample_count", type=int, default=1024, metavar="M", help="crystals per sample-quality pass")
+    args = ap.parse_args(argv)
+    try:
+        check_monitoring(args.sample_every, args.sample_count)
+    except ValueError as e:
+        ap.error(str(e))
     if args.val_fraction < 0 or args.test_fraction < 0 or args.val_fraction + args.test_fraction >= 1:
         ap.error("--val_fraction and --test_fraction must be >= 0 and leave a training split")
     if args.val_fraction > 0 and args.test_fraction > 0 and args.checkpoint_dir is None:
@@ -245,7 +384,9 @@ def main():
             hp = check_resume(args.resume, epochs=args.epochs, batch_size=args.batch_size,
                               world_size=int(os.environ.get("WORLD_SIZE", "1")),
                               backward_precision=args.backward_precision, num_train=len(train_ds),
-                              num_valid=0 if val_ds is None else len(val_ds), ema_decay=args.ema_decay)["hyper_parameters"]["args"]
+                              num_valid=0 if val_ds is None else len(val_ds), ema_decay=args.ema_decay,
+                              sample_every=args.sample_every,
+                              sample_count=args.sample_count)["hyper_parameters"]["args"]
         except ValueError as e:
             ap.error(str(e))
         for k in ("lr", "warmup"):
@@ -264,7 +405,8 @@ def main():
         model = PONITA_DIFFUSION(default_args(lr=3e-4 if args.lr is None else args.lr, epochs=args.epochs,
                                               warmup=args.warmup or 0, batch_size=args.batch_size), ds.z_table)
     fit(model, train_ds, args.epochs, args.batch_size, device, backward_precision=args.backward_precision,
-        val_dataset=val_ds, checkpoint_dir=args.checkpoint_dir, resume_from=args.resume, ema_decay=args.ema_decay)
+        val_dataset=val_ds, checkpoint_dir=args.checkpoint_dir, resume_from=args.resume, ema_decay=args.ema_decay,
+        sample_every=args.sample_every, sample_count=args.sample_count)
     twin = ema_model(model, device) if args.ema_decay is not None else None
     if rank0:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)) or ".", exist_ok=True)

@@ -346,6 +346,29 @@ int arreau_d3pm_reverse(const int64_t* types, const float* logits, const double*
 int arreau_step_noise(uint64_t seed, int32_t step, int32_t num_crystals, int32_t num_atoms_total,
                       int32_t num_states, double* z_len, double* z_frac, double* u, void* stream);
 
+/* Per-crystal keyed sampling noise: the draws of DiffusionLoss.sample (diffusion_loss.py:294-301 initial state, :319-337
+ * per-step noise) from Philox4x32-10 with key = seed and counter {c0, c1, c2, c3} = {crystal_id[g] (64 bits), index
+ * within the crystal, tag word}, like arreau_eval_noise.  A crystal's draws -- and so its whole trajectory -- depend on
+ * the seed, its id and its atom count only: not on its position in the batch, the batch's other crystals, the batch
+ * size or the rank.  Same distributions as the reference's host draws, not the reference's torch / numpy CPU stream.
+ * Tag words (disjoint from arreau_step_noise's 0, 1 and arreau_eval_noise's 2..5):
+ *   6              initial cell: index 0 -> beta = 90 + 90 U[0,1) (angles (90, beta, 90), degrees consumed as radians,
+ *                  quirk B5); indices 1, 2 -> lengths[3] N(0,1) (Box-Muller pairs, the 4th normal unused);
+ *   7              initial frac: index 2a + k (atom a of the crystal, k = 0, 1) -> N(0,1) * pos_sigma_max;
+ *   8 | step << 4  step noise z_len[3] (indices 0, 1, as tag 6's lengths);
+ *   9 | step << 4  step noise z_frac (index 2a + k, as tag 7);
+ *   10 | step << 4 step noise u[a, 2k .. 2k+1] (index a * ceil(Z/2) + k).
+ * So the step ordinal is bounded by 0 <= step < 2^28 (ARREAU_ERR_BAD_SHAPE otherwise), and a crystal holds fewer than
+ * 2^32 / ceil(Z/2) atoms.  crystal_id[G] i64, atom_offset[G+1], crystal_of_atom[N] of the batch.
+ * arreau_sample_init_keyed writes angles[G,3], lengths[G,3], frac[N,3] (f64; frac is NOT wrapped, as the reference's);
+ * arreau_sample_noise_keyed writes one step's z_len[G,3], z_frac[N,3] N(0,1) and u[N,Z] U[0,1) (f64). */
+int arreau_sample_init_keyed(uint64_t seed, int32_t num_crystals, int32_t num_atoms_total, const int64_t* crystal_id,
+                             const int32_t* atom_offset, const int32_t* crystal_of_atom, double pos_sigma_max,
+                             double* angles, double* lengths, double* frac, void* stream);
+int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t num_crystals, int32_t num_atoms_total,
+                              int32_t num_states, const int64_t* crystal_id, const int32_t* atom_offset,
+                              const int32_t* crystal_of_atom, double* z_len, double* z_frac, double* u, void* stream);
+
 /* One whole denoise step (the body of the sampler loop, diffusion_loss.py:319-349), every kernel
  * above on one stream with no host synchronisation.  State is updated in place. */
 typedef struct arreau_step_args {
@@ -406,7 +429,11 @@ int arreau_denoise_step(const arreau_weights* w, const arreau_workspace* ws, con
  * trajectory: replay k (k = *counter, incremented by the call) runs timestep t = max(t_first - k, 1) with Philox noise
  * of step ordinal k written into a->z_len / z_frac / u_type -- bit-identical to arreau_step_noise(seed, k, ...)
  * followed by arreau_denoise_step with a->t = t and the VP posterior coefficients of t.  a->t and a->vp_* are ignored.
- * Capped graphs only (max_neighbors > 0: no host read of the edge count); ARREAU_ERR_UNSUPPORTED otherwise. */
+ * With crystal_id set, the noise of replay k is arreau_sample_noise_keyed(seed, k, ..., crystal_id, ...) instead (the
+ * per-crystal keyed draws; k < 2^28); NULL keeps the per-batch noise above, bit for bit.
+ * Capped graphs only (max_neighbors > 0: no host read of the edge count); ARREAU_ERR_UNSUPPORTED otherwise.
+ * ABI note: crystal_id was appended after `reserved`, so the fields before it keep their offsets; a caller must
+ * zero-initialise it (or set it) -- a struct of the earlier size is read past its end. */
 typedef struct arreau_step_replay {
   int32_t* counter;        /* [1] device: replays done so far; reset it to restart a trajectory */
   const double* vp_table;  /* [T+1][4] device: {cx0, cxt, denom, var} of VP_lattice.reverse_given_x0 per timestep */
@@ -416,6 +443,7 @@ typedef struct arreau_step_replay {
   uint64_t seed;           /* Philox seed */
   int32_t t_first;         /* timestep of replay 0 (T - 1 for a whole trajectory) */
   int32_t reserved;
+  const int64_t* crystal_id; /* [G] device, or NULL: per-crystal keyed noise (see arreau_sample_noise_keyed) */
 } arreau_step_replay;
 
 int arreau_denoise_step_replay(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
