@@ -723,6 +723,7 @@ constexpr int kFusedWarps = 8;
 constexpr int kFusedRowBytes = kC * kO * 2 + (kC / 4) * 16 + 16;              // 4624
 constexpr int kFusedTileBytes = kFiberGroup * kFusedRowBytes;
 constexpr size_t kFusedSmem = (size_t)kFusedTileBytes + (size_t)kFusedWarps * 32 * 16 * sizeof(float) + 3 * kC * sizeof(float);
+constexpr int kPrefetchLead = 1;                 // gather iterations between a slab prefetch and its use
 
 __device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
   const __half2 v = __floats2half2_rn(lo, hi);
@@ -734,7 +735,7 @@ message_fiber_norm_fused_kernel(const __half* __restrict__ kern, const float* __
                                 const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ src,
                                 const uint4* __restrict__ fk_frag, const float* __restrict__ bias,
                                 const float* __restrict__ ln_w, const float* __restrict__ ln_b, int N,
-                                __half* __restrict__ y, float* __restrict__ x2_dbg, int prefetch) {
+                                __half* __restrict__ y, float* __restrict__ x2_dbg) {
   extern __shared__ __align__(128) uint8_t fsm[];
   uint8_t* s_a = fsm;                                                            // [16 atoms][kFusedRowBytes]
   float* s_stats = reinterpret_cast<float*>(s_a + (size_t)kFusedTileBytes);      // [warps][32 lanes][16]
@@ -765,13 +766,13 @@ message_fiber_norm_fused_kernel(const __half* __restrict__ kern, const float* __
       for (int op = 0; op < kO / 2; ++op) {
         // both orientations of the pair at once: 32 independent loads per lane in flight
         const int o0 = 2 * op;
-        if (prefetch) {
+        {
           // The slab is streamed from HBM exactly once, so each of these iterations would wait for 16 DRAM misses.  Pull
-          // the slab block of the iteration `prefetch` steps ahead into L2 now (a later orientation pair of this atom,
+          // the slab block of the iteration kPrefetchLead steps ahead into L2 now (a later orientation pair of this atom,
           // the warp's second atom -- its edges follow in CSR order --, or the warp's first atom of the CTA's next
           // tile): 8 edges x 512 B = one 128-byte line per lane, no registers held; the lead time turns the misses
-          // into L2 hits (445 -> 405 us per launch at C2 with one step of lead).
-          const int kk = rep * (kO / 2) + op + prefetch;            // iteration index within the tile (16 per warp)
+          // into L2 hits (445 -> 405 us per launch at C2 with one step of lead, profiles/r2_ab_message_prefetch.txt).
+          const int kk = rep * (kO / 2) + op + kPrefetchLead;       // iteration index within the tile (16 per warp)
           const int pe0 = kk >= kO ? next_e0 : ((kk >> 3) == rep ? e0 : e1);
           const int pe = min(pe0 + (lane >> 2), e_last);
           const char* pa = reinterpret_cast<const char*>(kern + ((size_t)pe * kO + 2 * (kk & 7)) * kC) + (lane & 3) * 128;
@@ -1540,12 +1541,6 @@ extern "C" int arreau_fiber_norm(const float* x1, int32_t x1_f16_transposed, con
   return ARREAU_OK;
 }
 
-int g_message_prefetch = 1;     // debug switch for same-process A/B (scratch/ab_message.py)
-extern "C" int arreau_debug_set_message_prefetch(int v) {
-  g_message_prefetch = v < 0 ? 0 : (v > 4 ? 4 : v);     // 0 = off, k = slab prefetch k iterations ahead
-  return ARREAU_OK;
-}
-
 extern "C" int arreau_message_fiber_norm_fused(const void* kernels_f16, const float* h, const int32_t* row_ptr,
                                                const int32_t* src, const void* fiber_frag, const float* conv_bias,
                                                const float* ln_w, const float* ln_b, int32_t N, void* y_f16,
@@ -1562,8 +1557,7 @@ extern "C" int arreau_message_fiber_norm_fused(const void* kernels_f16, const fl
   const int groups = (N + kFiberGroup - 1) / kFiberGroup;
   const int grid = groups < 2 * num_sms() ? groups : 2 * num_sms();
   message_fiber_norm_fused_kernel<<<grid, kFusedWarps * 32, kFusedSmem, (cudaStream_t)stream>>>(
-      (const __half*)kernels_f16, h, row_ptr, src, (const uint4*)fiber_frag, conv_bias, ln_w, ln_b, N, (__half*)y_f16, x2_debug,
-      g_message_prefetch);
+      (const __half*)kernels_f16, h, row_ptr, src, (const uint4*)fiber_frag, conv_bias, ln_w, ln_b, N, (__half*)y_f16, x2_debug);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

@@ -1,11 +1,9 @@
-// tcgen05 (fp16 operands, fp32 accumulation in TMEM) variants of the two GEMM-shaped kernels of the step.
+// tcgen05 (fp16 operands, fp32 accumulation in TMEM) kernels for the two GEMM-shaped stages of the step.
 //
-//   convnext_mlp_tc_kernel    K6     h += layer_scale * (W2 gelu(W1 y + b1) + b2)          convnext.py:26-32
-//   edge_kernels_tc3_kernel   K3+K4a invariants -> monomials -> basis MLP -> window -> 5 kernel projections
-//   (edge_kernels_tc2_kernel: the same pipeline with ONE epilogue group and run-time clock64 stamps, kept for A/B timing
-//    and for the timeline in profiles/)
+//   convnext_mlp_tc_kernel   K6     h += layer_scale * (W2 gelu(W1 y + b1) + b2)          convnext.py:26-32
+//   edge_kernels_tc_kernel   K3+K4a invariants -> monomials -> basis MLP -> window -> 5 kernel projections
 //
-// All are persistent (one CTA per SM, 128-row tiles) and warp specialised:
+// Both are persistent (one CTA per SM, 128-row tiles) and warp specialised:
 //   warp 0   producer: cp.async.bulk (TMA engine) of pre-swizzled weight / activation tiles into an mbarrier ring
 //   warp 1   MMA issuer: the warp runs the issue loop uniformly, one elected lane issues tcgen05.mma (M = 128, N = 128,
 //            K = 16) and tcgen05.commit; the hidden slice (MLP) and the kernel basis (edge) are TENSOR-MEMORY operands
@@ -29,7 +27,6 @@ constexpr int kTileM = 128;
 constexpr uint32_t kIdesc128 = umma_idesc_f16(128, 128);
 
 __device__ long long* g_tc_prof = nullptr;   // debug: per-phase clock64 stamps of CTA 0 (scratch/prof_tc.py)
-__device__ unsigned g_tc_prof_tile0 = 2;     // first of the 8 stamped tiles (ordinal within the CTA)
 #ifdef ARREAU_TC_PROFILE
 #define TC_STAMP(slot)                                                                     \
   do {                                                                                      \
@@ -38,63 +35,6 @@ __device__ unsigned g_tc_prof_tile0 = 2;     // first of the 8 stamped tiles (or
 #else
 #define TC_STAMP(slot) do { (void)prof; } while (0)
 #endif
-
-// issue the UMMA_K = 16 steps of one 64-wide K slab: D[128 x 128] (+)= A_slab[128 x 64] * B_slab[128 x 64]^T
-__device__ __forceinline__ void mma_slab(uint32_t tmem_d, uint32_t a_slab, uint32_t b_slab, int ksteps, bool accumulate_first) {
-  const uint64_t ad = umma_desc_sw128(a_slab), bd = umma_desc_sw128(b_slab);
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (k < ksteps) umma_f16(tmem_d, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), kIdesc128, (accumulate_first || k > 0) ? 1u : 0u);
-  }
-}
-
-// 32 accumulator columns -> (+ bias) -> GELU (* scale) -> fp16 -> the four 16-byte chunks chunk0..chunk0+3 of
-// operand row m (row base pointer `row`, chunk positions XOR-swizzled by the row index)
-template <bool kBias, bool kScale>
-__device__ __forceinline__ void gelu_store32(const float (&v)[32], const float* __restrict__ bias_s, float scale,
-                                             uint8_t* row, int chunk0, int m) {
-  const __half2 sc = __float2half2_rn(scale);
-#pragma unroll
-  for (int cc = 0; cc < 4; ++cc) {
-    float x[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) x[i] = v[cc * 8 + i];
-    if constexpr (kBias) {
-      const float4 b0 = *reinterpret_cast<const float4*>(bias_s + cc * 8);       // warp-uniform: smem broadcast
-      const float4 b1 = *reinterpret_cast<const float4*>(bias_s + cc * 8 + 4);
-      x[0] += b0.x; x[1] += b0.y; x[2] += b0.z; x[3] += b0.w;
-      x[4] += b1.x; x[5] += b1.y; x[6] += b1.z; x[7] += b1.w;
-    }
-    uint4 pk;
-    if constexpr (kScale) {
-      pk.x = gelu2_scaled_f16(x[0], x[1], sc);
-      pk.y = gelu2_scaled_f16(x[2], x[3], sc);
-      pk.z = gelu2_scaled_f16(x[4], x[5], sc);
-      pk.w = gelu2_scaled_f16(x[6], x[7], sc);
-    } else {
-      pk.x = gelu2_f16(x[0], x[1]);
-      pk.y = gelu2_f16(x[2], x[3]);
-      pk.z = gelu2_f16(x[4], x[5]);
-      pk.w = gelu2_f16(x[6], x[7]);
-    }
-    *reinterpret_cast<uint4*>(row + (((chunk0 + cc) ^ (m & 7)) << 4)) = pk;
-  }
-}
-
-// 32 accumulator columns -> + bias -> GELU * scale -> 16 packed fp16 registers
-__device__ __forceinline__ void gelu_scaled_pack32(const float (&v)[32], const float* __restrict__ bias_s, float scale,
-                                                   uint32_t (&pk)[16]) {
-  const __half2 sc = __float2half2_rn(scale);
-#pragma unroll
-  for (int cc = 0; cc < 4; ++cc) {
-    const float4 b0 = *reinterpret_cast<const float4*>(bias_s + cc * 8);
-    const float4 b1 = *reinterpret_cast<const float4*>(bias_s + cc * 8 + 4);
-    pk[cc * 4 + 0] = gelu2_scaled_f16(v[cc * 8 + 0] + b0.x, v[cc * 8 + 1] + b0.y, sc);
-    pk[cc * 4 + 1] = gelu2_scaled_f16(v[cc * 8 + 2] + b0.z, v[cc * 8 + 3] + b0.w, sc);
-    pk[cc * 4 + 2] = gelu2_scaled_f16(v[cc * 8 + 4] + b1.x, v[cc * 8 + 5] + b1.y, sc);
-    pk[cc * 4 + 3] = gelu2_scaled_f16(v[cc * 8 + 6] + b1.z, v[cc * 8 + 7] + b1.w, sc);
-  }
-}
 
 // 32 accumulator columns -> + bias -> GELU -> four packed fp16 chunks (registers only)
 __device__ __forceinline__ void gelu_pack32(const float (&v)[32], const float* __restrict__ bias_s, uint4 (&pk)[4]) {
@@ -474,9 +414,52 @@ convnext_mlp_tc_kernel(const uint8_t* __restrict__ y_img, const uint8_t* __restr
 // =================================================================================================
 // K3 + K4a  edge pipeline
 // =================================================================================================
+// Per 128-row tile (8 edges x 16 orientations) the tensor pipe runs
+//   G1     ACC = monomials [128 x 96] . W1m^T            -> GELU -> hidden tile A2 (shared memory, UMMA image)
+//   G2a/b  ACC = hidden [128 x 128] . W2[half]^T         -> + b2, GELU, * window -> kernel basis KB (tensor memory)
+//   L0..4  ACC = KB [128 x 256] . Wk_l^T                 -> fp16 -> kernels[l] in HBM (staging + bulk store)
+// The kernel basis is a TENSOR-MEMORY operand: the G2 epilogue writes it with tcgen05.st and the five projections (80
+// of a tile's 102 MMAs) read it as A from there (tcgen05.mma ... [a_tmem]).  An SS-mode 128 x 128 x 16 MMA reads 8 KB
+// of operands per 64 tensor cycles, the shared-memory port's whole 128 B/clk, so a basis in shared memory would leave
+// the port no room for the weight ring's writes and the output staging; out of shared memory, it also leaves the space
+// for a 5-stage weight ring.
+//   TMEM     ACC0 = [0,128): G jobs, ACC1 = [128,256): L jobs; KB0 = [256,384), KB1 = [384,512): kernel basis of the
+//            current / the next tile (packed fp16 pairs)
+//   jobs     MMA issue order per tile i: L0 G1' L1 G2a' L2 G2b' L3 L4 (' = tile i+1), so the head of the next tile runs
+//            under this tile's projections
+//   ring     Wk0 W1' Wk1 W2a' Wk2 W2b' Wk3 Wk4  (13 chunks of 32 KB per tile, 5 stages)
+// The jobs are drained by two epilogue groups with one accumulator slot each, working at the same time:
+//   G-group (warps 4..19)   gen' -> G1' (GELU -> hidden tile A2) -> G2a', G2b' (GELU * window -> kernel basis in TMEM)
+//   L-group (warps 20..27)  L0 .. L4: fp16 pack -> staging -> bulk store of kernels[l]  (64 columns per thread)
+// A group pulls a finished accumulator into registers and hands the slot back before its post-processing, so the
+// tensor pipe runs ahead of both.  Every producer/consumer chain of the tile head (monomials, hidden layer, kernel
+// basis) stays inside the G-group, so no cross-group hand-off is needed: completion of earlier MMAs is implied by the
+// in-order tensor pipe (a finished GEMM2 says that the previous tile's five projections have finished reading the
+// other kernel-basis buffer).  Warp 3 computes the per-edge geometry up to two tiles ahead.
+// 896 threads (a block holds at most 1024) -> at most 73 registers per thread.
+// The earlier version with a single epilogue group is at commit be8d4ea; profiles/r2_ab_edge_variants.txt has the A/B
+// of the two.
 namespace edge {
 constexpr int kEdgesPerTile = kTileM / kO;
 constexpr int kGeo = 12;                // floats per edge: dir (3), dist, cos(dir, a/b/c) (3), window, valid, pad
+constexpr int kChunkBytes = 32768;
+constexpr int kStages = 5;
+constexpr int kStageBytes = 32768;
+constexpr int kA2Bytes = 32768;
+constexpr int kTilesBytes = kA2Bytes + kStageBytes + kStages * kChunkBytes;
+constexpr int kSmemBytes = 232448;
+constexpr uint32_t kKbCol = 256;
+constexpr int kLWarps = 8;                 // L-group: 4 lane quarters x 2 column halves
+constexpr int kEdgeThreads = (kEpiWarp0 + kEpiWarps + kLWarps) * 32;   // 896: 4 service warps + G-group (16) + L-group (8)
+constexpr int kLWarp0 = kEpiWarp0 + kEpiWarps;
+
+struct Bars {
+  uint64_t w_full[kStages], w_empty[kStages];
+  uint64_t a1_full, a2_full;
+  uint64_t acc_full[2], acc_empty[2];      // [0] = G jobs (ACC0), [1] = L jobs (ACC1)
+  uint64_t kb_full[2];
+  uint64_t g_full[2], g_empty[2];
+};
 
 // monomial n of csrc/common.cuh monomials83 as compile-time index triples; 83 = constant 1 (bias), > 83 = 0
 struct MonoIdx { int deg, a, b, c; };
@@ -526,76 +509,15 @@ __device__ __forceinline__ void store_mono_part(const float (&v)[6], float one, 
   }
 }
 
-// fp32 edge invariants for the fp16 path (the monomials are rounded to fp16 right after; the fp32 path and the
-// graph keep fp64): [dir.ori, |dir - (dir.ori) ori|, dist, cos(dir,a), cos(dir,b), cos(dir,c)]
-__device__ __forceinline__ void edge_invariants_f32(const double* __restrict__ dir3, double dist, const double* __restrict__ lat9,
-                                                    const float* __restrict__ ori3, float (&attr)[6]) {
-  const float dx = (float)dir3[0], dy = (float)dir3[1], dz = (float)dir3[2];
-  const float ox = ori3[0], oy = ori3[1], oz = ori3[2];
-  const float i1 = dx * ox + dy * oy + dz * oz;
-  const float px = dx - i1 * ox, py = dy - i1 * oy, pz = dz - i1 * oz;
-  attr[0] = i1;
-  attr[1] = sqrtf(px * px + py * py + pz * pz);
-  attr[2] = (float)dist;
-  const float dd = dx * dx + dy * dy + dz * dz;
-#pragma unroll
-  for (int mm = 0; mm < 3; ++mm) {
-    const float ax = (float)lat9[3 * mm], ay = (float)lat9[3 * mm + 1], az = (float)lat9[3 * mm + 2];
-    const float w12 = dx * ax + dy * ay + dz * az, w2 = ax * ax + ay * ay + az * az;
-    attr[3 + mm] = w12 * rsqrtf(fmaxf(dd * w2, 1e-16f));     // CosineSimilarity, eps = 1e-8
-  }
-}
 }  // namespace edge
 
-// =================================================================================================
-// K3 + K4a  edge pipeline, version 2: the kernel basis is a TENSOR-MEMORY operand
-// =================================================================================================
-// Round 1's kernel kept the kernel basis in shared memory (tile A3) and was bound by the SM's shared-memory port
-// (profiles/README.md): an SS-mode 128 x 128 x 16 MMA
-// reads 8 KB of operands per 64 tensor cycles = the port's whole 128 B/clk, before the weight ring's writes, the
-// epilogue stores and the output staging.  Here the five kernel projections (80 of a tile's 102 MMAs) take their A
-// operand -- the kernel basis [128 rows x 256] fp16 -- from tensor memory (tcgen05.mma ... [a_tmem]), where the second
-// GELU epilogue writes it directly (tcgen05.st): the 64 KB shared-memory tile A3, its 64 KB of epilogue stores and its
-// 320 KB of operand reads per tile are gone (1.66 -> 1.28 MB through the port per 128-row tile), and the freed shared
-// memory deepens the weight ring from 3 to 5 stages.
-//   TMEM     ACC0 = [0,128), ACC1 = [128,256): ONE two-slot accumulator ring shared by every GEMM of the pipeline;
-//            KB0 = [256,384), KB1 = [384,512): kernel basis of the current / the next tile (packed fp16 pairs)
-//   jobs     per tile i, in this order on BOTH sides (MMA warp issues, epilogue warps drain):
-//              L0  G1'  L1  G2a'  L2  G2b'  L3  L4          (' = tile i+1: GEMM1, GEMM2 output halves 0 / 1)
-//            job number j uses slot j & 1; the epilogue pulls a finished slot into registers first (tcgen05.ld) and
-//            hands it back before its own post-processing, so the tensor pipe runs up to two GEMMs ahead
-//   post     L_l : fp16 pack -> staging -> bulk store of kernels[l] (as in version 1)
-//            G1' : GELU -> hidden tile A2 (shared memory, UMMA image)           -> a2_full
-//            G2x': + b2, GELU, * window -> packed fp16 -> KB[(i+1) & 1] (TMEM)  -> kb_full
-//   ring     Wk0 W1' Wk1 W2a' Wk2 W2b' Wk3 Wk4  (13 chunks of 32 KB per tile, 5 stages)
-namespace edge2 {
-constexpr int kChunkBytes = 32768;
-constexpr int kStages = 5;
-constexpr int kStageBytes = 32768;
-constexpr int kA2Bytes = 32768;
-constexpr int kTilesBytes = kA2Bytes + kStageBytes + kStages * kChunkBytes;
-constexpr int kSmemBytes = 232448;
-constexpr int kEdgesPerTile = kTileM / kO;
-constexpr int kGeo = edge::kGeo;
-constexpr uint32_t kKbCol = 256;
-
-struct Bars {
-  uint64_t w_full[kStages], w_empty[kStages];
-  uint64_t a1_full, a2_full;
-  uint64_t acc_full[2], acc_empty[2];
-  uint64_t kb_full[2];
-  uint64_t g_full[2], g_empty[2];
-};
-}  // namespace edge2
-
-__global__ void __launch_bounds__(kThreads, 1)
-edge_kernels_tc2_kernel(const double* __restrict__ dir, const double* __restrict__ dist, const double* __restrict__ lattice,
+__global__ void __launch_bounds__(edge::kEdgeThreads, 1)
+edge_kernels_tc_kernel(const double* __restrict__ dir, const double* __restrict__ dist, const double* __restrict__ lattice,
                         const int32_t* __restrict__ crystal_of_atom, const int32_t* __restrict__ src,
                         const int32_t* __restrict__ num_edges_ptr, long long edge_capacity, const float* __restrict__ ori,
                         const uint8_t* __restrict__ w1_img, const uint8_t* __restrict__ w_img, const float* __restrict__ b2,
                         double radius, __half* __restrict__ kernels) {
-  using namespace edge2;
-  using edge::store_mono_part;
+  using namespace edge;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
@@ -615,373 +537,7 @@ edge_kernels_tc2_kernel(const double* __restrict__ dir, const double* __restrict
   const long long tiles = (E + kEdgesPerTile - 1) / kEdgesPerTile;
   const long long first = blockIdx.x, stride = gridDim.x;
 
-  for (int i = threadIdx.x; i < kD; i += kThreads) s_b2[i] = b2[i];
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < kStages; ++i) { mbar_init(&bars.w_full[i], 1); mbar_init(&bars.w_empty[i], 1); }
-    mbar_init(&bars.a1_full, kEpiWarps); mbar_init(&bars.a2_full, kEpiWarps);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&bars.acc_full[i], 1); mbar_init(&bars.acc_empty[i], kEpiWarps);
-      mbar_init(&bars.kb_full[i], 2 * kEpiWarps);            // both output halves of GEMM2
-      mbar_init(&bars.g_full[i], 1); mbar_init(&bars.g_empty[i], kEpiWarps);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 2) tmem_alloc(&tmem_base_s, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = tmem_base_s;
-  const uint32_t t0p = g_tc_prof_tile0;
-
-  if (warp == 3) {
-    // ---------------- geometry: the per-edge part of the invariants, up to two tiles ahead (as in version 1) --------
-    uint32_t k = 0;
-    for (long long tile = first; tile < tiles; tile += stride, ++k) {
-      const int buf = k & 1;
-      mbar_wait(&bars.g_empty[buf], ((k >> 1) & 1) ^ 1);
-      if (lane < kEdgesPerTile) {
-        const long long e = tile * kEdgesPerTile + lane;
-        float* gp = s_geo + (buf * kEdgesPerTile + lane) * kGeo;
-        float vals[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        if (e < E) {
-          const double* lat9 = lattice + 9 * (size_t)crystal_of_atom[src[e]];
-          const float dx = (float)dir[3 * e], dy = (float)dir[3 * e + 1], dz = (float)dir[3 * e + 2];
-          const float dd = dx * dx + dy * dy + dz * dz;
-          vals[0] = dx; vals[1] = dy; vals[2] = dz;
-          vals[3] = (float)dist[e];
-#pragma unroll
-          for (int mm = 0; mm < 3; ++mm) {
-            const float ax = (float)lat9[3 * mm], ay = (float)lat9[3 * mm + 1], az = (float)lat9[3 * mm + 2];
-            const float w12 = dx * ax + dy * ay + dz * az, w2 = ax * ax + ay * ay + az * az;
-            vals[4 + mm] = w12 * rsqrtf(fmaxf(dd * w2, 1e-16f));     // CosineSimilarity, eps = 1e-8
-          }
-          vals[7] = cutoff_window(dist[e], radius);
-          vals[8] = 1.0f;
-        }
-#pragma unroll
-        for (int i = 0; i < 9; ++i) gp[i] = vals[i];
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.g_full[buf]);
-    }
-  } else if (warp == 0 && lane == 0) {
-    // ---------------- producer: 32 KB weight chunks in the order the MMA warp consumes them ----------------
-    if (first < tiles) {
-      uint32_t st = 0, par = 1;          // waits on w_empty start at parity 1 (a fresh barrier passes)
-      auto push = [&](const uint8_t* src_chunk) {
-        mbar_wait(&bars.w_empty[st], par);
-        mbar_expect_tx(&bars.w_full[st], kChunkBytes);
-        bulk_g2s(W + st * kChunkBytes, src_chunk, kChunkBytes, &bars.w_full[st]);
-        if (++st == kStages) { st = 0; par ^= 1; }
-      };
-      auto push_w = [&](int c0, int n) { for (int c = c0; c < c0 + n; ++c) push(w_img + (size_t)c * kChunkBytes); };
-      push(w1_img);
-      push_w(0, 2);                                   // first tile: W1, W2 (both output halves)
-      for (long long tile = first; tile < tiles; tile += stride) {
-        const bool has_next = tile + stride < tiles;
-        push_w(2, 2);                                 // Wk_0
-        if (has_next) push(w1_img);
-        push_w(4, 2);                                 // Wk_1
-        if (has_next) push_w(0, 1);                   // W2, output half 0
-        push_w(6, 2);                                 // Wk_2
-        if (has_next) push_w(1, 1);                   // W2, output half 1
-        push_w(8, 4);                                 // Wk_3, Wk_4
-      }
-    }
-  } else if (warp == 1) {
-    // ---------------- MMA issuer (warp-uniform, one elected lane; see version 1) ----------------
-    if (first < tiles) {
-      const uint32_t el = elect_one();
-      const uint32_t a2_lo = umma_desc_lo(smem_u32(A2)), w_lo = umma_desc_lo(smem_u32(W));
-      const uint32_t wfull = smem_u32(&bars.w_full[0]), wempty = smem_u32(&bars.w_empty[0]);
-      const uint32_t accfull = smem_u32(&bars.acc_full[0]), accempty = smem_u32(&bars.acc_empty[0]);
-      constexpr uint32_t kSlabLo = 16384 >> 4;
-      uint32_t st = 0, par = 0, j = 0;
-      // debug: clock64 stamps of CTA 0, tiles 2..9 of this CTA: [tile][role 0 = MMA][3 * job + {entry, waits done, issued}]
-      long long* const prof = (blockIdx.x == 0 && el) ? g_tc_prof : nullptr;
-      uint32_t pit = 0, pjob = 0;
-      auto stamp = [&](int what) { if (prof && pit >= t0p && pit < t0p + 8) prof[((pit - t0p) * 2 + 0) * 32 + 3 * pjob + what] = clock64(); };
-      auto advance = [&]() { if (++st == kStages) { st = 0; par ^= 1; } };
-      // accumulator slot of job j: wait until the epilogue has pulled the slot's previous content into registers
-      auto acc_begin = [&]() -> uint32_t {
-        const uint32_t slot = j & 1u;
-        mbar_wait_addr(accempty + 8 * slot, ((j >> 1) & 1u) ^ 1u);
-        tc_fence_after();
-        return tmem + slot * 128;
-      };
-      auto acc_end = [&]() { umma_commit_e(accfull + 8 * (j & 1u), el); ++j; };
-      // one ring chunk = two K slabs, A from shared memory (GEMM1 / GEMM2)
-      auto pair_ss = [&](uint32_t d, uint32_t a_lo, int ksteps1) {
-        mbar_wait_addr(wfull + 8 * st, par);
-        const uint32_t b_lo = w_lo + st * (2 * kSlabLo);
-        umma_slab_e<4>(d, a_lo, b_lo, kIdesc128, el, 0u);
-        if (ksteps1 == 4) umma_slab_e<4>(d, a_lo + kSlabLo, b_lo + kSlabLo, kIdesc128, el, 1u);
-        else umma_slab_e<2>(d, a_lo + kSlabLo, b_lo + kSlabLo, kIdesc128, el, 1u);
-        umma_commit_e(wempty + 8 * st, el);
-        advance();
-      };
-      // one ring chunk = two K slabs (128 K values = 64 TMEM columns of packed pairs), A from tensor memory (GEMM3)
-      auto pair_ts = [&](uint32_t d, uint32_t a_t, uint32_t accumulate) {
-        mbar_wait_addr(wfull + 8 * st, par);
-        const uint32_t b_lo = w_lo + st * (2 * kSlabLo);
-        umma_slab_ts_e<4>(d, a_t, b_lo, kIdesc128, el, accumulate);
-        umma_slab_ts_e<4>(d, a_t + 32, b_lo + kSlabLo, kIdesc128, el, 1u);
-        umma_commit_e(wempty + 8 * st, el);
-        advance();
-      };
-      auto gemm1 = [&](uint32_t k) {       // ACC = A1[128 x 96] . W1m^T   (tile ordinal k)
-        stamp(0);
-        mbar_wait(&bars.a1_full, k & 1);
-        const uint32_t d = acc_begin();
-        stamp(1);
-        pair_ss(d, a2_lo, 2);
-        acc_end();
-        stamp(2); ++pjob;
-      };
-      auto gemm2 = [&](uint32_t k, int nh) {   // ACC = hidden[128 x 128] . W2[nh]^T
-        stamp(0);
-        if (nh == 0) mbar_wait(&bars.a2_full, k & 1);
-        const uint32_t d = acc_begin();
-        stamp(1);
-        pair_ss(d, a2_lo, 4);
-        acc_end();
-        stamp(2); ++pjob;
-      };
-      gemm1(0);
-      gemm2(0, 0);
-      gemm2(0, 1);
-      uint32_t it = 0;
-      for (long long tile = first; tile < tiles; tile += stride, ++it) {
-        const bool has_next = tile + stride < tiles;
-        const uint32_t kb = tmem + kKbCol + (it & 1u) * 128;
-        pit = it; pjob = 0;
-        if (prof && (it == 0 || it == 256)) {       // SM clock during the kernel: cycles and nanoseconds at two distant tiles
-          unsigned long long ns;
-          asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-          prof[8 * 2 * 32 + (it ? 2 : 0)] = clock64();
-          prof[8 * 2 * 32 + (it ? 3 : 1)] = (long long)ns;
-        }
-#pragma unroll 1
-        for (int l = 0; l < kL; ++l) {
-          stamp(0);
-          const uint32_t d = acc_begin();
-          if (l == 0) {                        // kernel basis of this tile is in tensor memory
-            mbar_wait(&bars.kb_full[it & 1u], (it >> 1) & 1u);
-            tc_fence_after();
-          }
-          stamp(1);
-          pair_ts(d, kb, 0u);
-          pair_ts(d, kb + 64, 1u);
-          acc_end();
-          stamp(2); ++pjob;
-          if (has_next) {
-            if (l == 0) gemm1(it + 1);
-            else if (l == 1) gemm2(it + 1, 0);
-            else if (l == 2) gemm2(it + 1, 1);
-          }
-        }
-      }
-    }
-  } else if (warp >= kEpiWarp0) {
-    // ---------------- generator + epilogues: warp = (lane quarter q, column group cgi of 32 columns) ----------------
-    const int q = warp & 3, cgi = (warp - kEpiWarp0) >> 2;
-    const int m = q * 32 + lane;                     // tile row = (edge m / 16, orientation m % 16)
-    const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    const int hf = q >> 1;                           // staging half of this warp's rows
-    const bool is_issuer = cgi == 0 && (q & 1) == 0 && lane == 0;     // one bulk-store issuer per half tile
-    const float ox = ori[3 * (m & 15)], oy = ori[3 * (m & 15) + 1], oz = ori[3 * (m & 15) + 2];
-    float win_cur = 0.f;
-    uint32_t j = 0;
-    // debug stamps: [tile][role 1 = epilogue warp 4][3 * job + {entry, accumulator in registers, post-processing done}]
-    long long* const prof = (blockIdx.x == 0 && threadIdx.x == kEpiWarp0 * 32) ? g_tc_prof : nullptr;
-    uint32_t pit = 0, pjob = 0;
-    auto stamp = [&](int what) { if (prof && pit >= t0p && pit < t0p + 8) prof[((pit - t0p) * 2 + 1) * 32 + 3 * pjob + what] = clock64(); };
-    // pull the accumulator of job j (this thread: row m, columns cgi*32 .. +31) into registers and hand the slot back
-    auto acc_take = [&](float (&v)[32]) {
-      stamp(0);
-      const uint32_t slot = j & 1u;
-      mbar_wait(&bars.acc_full[slot], (j >> 1) & 1u);
-      tc_fence_after();
-      tmem_ld32(tmem + slot * 128 + lane_addr + cgi * 32, v);
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.acc_empty[slot]);
-      ++j;
-      stamp(1);
-    };
-    auto gen = [&](uint32_t k) {                     // monomials of tile ordinal k -> A2 (as A1), see version 1
-      const int buf = k & 1;
-      mbar_wait(&bars.g_full[buf], (k >> 1) & 1);
-      const float* gp = s_geo + (buf * kEdgesPerTile + (m >> 4)) * kGeo;
-      const float dx = gp[0], dy = gp[1], dz = gp[2];
-      float attr[6];
-      const float i1 = dx * ox + dy * oy + dz * oz;
-      const float px = dx - i1 * ox, py = dy - i1 * oy, pz = dz - i1 * oz;
-      attr[0] = i1;
-      attr[1] = sqrtf(px * px + py * py + pz * pz);
-      attr[2] = gp[3]; attr[3] = gp[4]; attr[4] = gp[5]; attr[5] = gp[6];
-      win_cur = gp[7];
-      const float one = gp[8];
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.g_empty[buf]);
-      switch (cgi) {
-        case 0: store_mono_part<0>(attr, one, A2, m); break;
-        case 1: store_mono_part<1>(attr, one, A2, m); break;
-        case 2: store_mono_part<2>(attr, one, A2, m); break;
-        default: store_mono_part<3>(attr, one, A2, m); break;
-      }
-      fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.a1_full);
-    };
-    auto job_g1 = [&]() {                            // hidden = GELU(GEMM1) -> A2 (unit cgi*32.. -> slab cgi>>1)
-      float v[32];
-      acc_take(v);
-      gelu_store32<false, false>(v, nullptr, 1.0f, A2 + (cgi >> 1) * 16384 + m * kRowBytes, (cgi & 1) * 4, m);
-      fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.a2_full);
-      stamp(2); ++pjob;
-    };
-    auto job_g2 = [&](uint32_t k, int nh) {          // kernel basis half nh of tile k -> KB[k & 1] (tensor memory)
-      float v[32];
-      acc_take(v);
-      uint32_t pk[16];
-      gelu_scaled_pack32(v, s_b2 + nh * 128 + cgi * 32, win_cur, pk);
-      tmem_st16(tmem + kKbCol + (k & 1u) * 128 + lane_addr + nh * 64 + cgi * 16, pk);
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars.kb_full[k & 1u]);
-      stamp(2); ++pjob;
-    };
-    auto job_layer = [&](int l, long long tile) {    // kernels[l][e][o][c] = ACC (fp16), staged + bulk store (version 1)
-      float v[32];
-      acc_take(v);
-      uint8_t* stage = S + hf * 16384;
-      if (is_issuer) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // this half's previous store has left smem
-      asm volatile("bar.sync %0, %1;" ::"r"(1 + hf), "n"(kEpiThreads / 2) : "memory");
-      uint8_t* orow = stage + (m & 63) * 256;
-#pragma unroll
-      for (int cc = 0; cc < 4; ++cc) {
-        uint4 pk;
-        pk.x = pack_f16(v[cc * 8 + 0], v[cc * 8 + 1]);
-        pk.y = pack_f16(v[cc * 8 + 2], v[cc * 8 + 3]);
-        pk.z = pack_f16(v[cc * 8 + 4], v[cc * 8 + 5]);
-        pk.w = pack_f16(v[cc * 8 + 6], v[cc * 8 + 7]);
-        *reinterpret_cast<uint4*>(orow + (((cgi * 4 + cc) ^ (m & 15)) << 4)) = pk;
-      }
-      fence_proxy_async();
-      asm volatile("bar.sync %0, %1;" ::"r"(1 + hf), "n"(kEpiThreads / 2) : "memory");
-      if (is_issuer) {
-        const long long left = E - tile * kEdgesPerTile - hf * (kEdgesPerTile / 2);   // edges of this half still valid
-        if (left > 0) {
-          const uint32_t bytes = (uint32_t)(left < kEdgesPerTile / 2 ? left : kEdgesPerTile / 2) * (kO * kC * 2);
-          __half* out = kernels + ((size_t)l * edge_capacity * kO + (size_t)tile * kTileM + hf * 64) * kC;
-          asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(out), "r"(smem_u32(stage)), "r"(bytes)
-                       : "memory");
-        }
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-      }
-      stamp(2); ++pjob;
-    };
-    if (first < tiles) {
-      gen(0);
-      job_g1();
-      job_g2(0, 0);
-      job_g2(0, 1);
-      uint32_t it = 0;
-      for (long long tile = first; tile < tiles; tile += stride, ++it) {
-        const bool has_next = tile + stride < tiles;
-        pit = it; pjob = 0;
-        if (prof && pit >= t0p && pit < t0p + 8) prof[((pit - t0p) * 2 + 1) * 32 + 30] = clock64();
-        if (has_next) gen(it + 1);                 // A2 is free: both halves of this tile's GEMM2 have been drained
-        if (prof && pit >= t0p && pit < t0p + 8) prof[((pit - t0p) * 2 + 1) * 32 + 31] = clock64();
-        job_layer(0, tile);
-        if (has_next) job_g1();
-        job_layer(1, tile);
-        if (has_next) job_g2(it + 1, 0);
-        job_layer(2, tile);
-        if (has_next) job_g2(it + 1, 1);
-        job_layer(3, tile);
-        job_layer(4, tile);
-      }
-      if (is_issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // all output tiles have landed
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem, 512);
-  }
-}
-
-// =================================================================================================
-// K3 + K4a  edge pipeline, version 3: version 2 with TWO epilogue groups working on different jobs at the same time
-// =================================================================================================
-// Version 2 is bound by its 16 epilogue warps (clock64 timeline, profiles/r2_edge_timeline.md): they take the tile's 8
-// jobs one after the other in lockstep -- every job pays the accumulator drain latency (~180 cycles), the block
-// barriers of the output staging and the XU-bound GELU chains back to back, 11.5 K cycles per tile against the tensor
-// pipe's 6.5 K.  Here 24 epilogue warps form two groups with one accumulator slot each:
-//   G-group (warps 4..19)   gen' -> G1' (GELU -> hidden tile A2) -> G2a', G2b' (GELU * window -> kernel basis in TMEM)
-//   L-group (warps 20..27)  L0 .. L4: fp16 pack -> staging -> bulk store of kernels[l]  (64 columns per thread)
-// Every producer/consumer chain of the tile head (monomials, hidden layer, kernel basis) stays inside the G-group, so
-// no cross-group hand-off is needed: completion of earlier MMAs is implied by the in-order tensor pipe (a finished
-// GEMM2 says that the previous tile's five projections have finished reading the other kernel-basis buffer).
-// MMA issue order per tile as in version 2 (L0 G1' L1 G2a' L2 G2b' L3 L4); L jobs use ACC1, G jobs ACC0.
-// 896 threads (a block holds at most 1024) -> 73 registers per thread.
-namespace edge3 {
-constexpr int kChunkBytes = 32768;
-constexpr int kStages = 5;
-constexpr int kStageBytes = 32768;
-constexpr int kA2Bytes = 32768;
-constexpr int kTilesBytes = kA2Bytes + kStageBytes + kStages * kChunkBytes;
-constexpr int kSmemBytes = 232448;
-constexpr int kEdgesPerTile = kTileM / kO;
-constexpr int kGeo = edge::kGeo;
-constexpr uint32_t kKbCol = 256;
-constexpr int kLWarps = 8;                 // L-group: 4 lane quarters x 2 column halves
-constexpr int kThreads3 = (kEpiWarp0 + kEpiWarps + kLWarps) * 32;   // 896: 4 service warps + G-group (16) + L-group (8)
-constexpr int kLWarp0 = kEpiWarp0 + kEpiWarps;
-
-struct Bars {
-  uint64_t w_full[kStages], w_empty[kStages];
-  uint64_t a1_full, a2_full;
-  uint64_t acc_full[2], acc_empty[2];      // [0] = G jobs (ACC0), [1] = L jobs (ACC1)
-  uint64_t kb_full[2];
-  uint64_t g_full[2], g_empty[2];
-};
-}  // namespace edge3
-
-__global__ void __launch_bounds__(edge3::kThreads3, 1)
-edge_kernels_tc3_kernel(const double* __restrict__ dir, const double* __restrict__ dist, const double* __restrict__ lattice,
-                        const int32_t* __restrict__ crystal_of_atom, const int32_t* __restrict__ src,
-                        const int32_t* __restrict__ num_edges_ptr, long long edge_capacity, const float* __restrict__ ori,
-                        const uint8_t* __restrict__ w1_img, const uint8_t* __restrict__ w_img, const float* __restrict__ b2,
-                        double radius, __half* __restrict__ kernels) {
-  using namespace edge3;
-  using edge::store_mono_part;
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
-  float* const s_b2 = reinterpret_cast<float*>(smem + kTilesBytes);                                   // [kD]
-  float* const s_geo = s_b2 + kD;                                                                      // [2][8 edges][kGeo]
-  Bars& bars = *reinterpret_cast<Bars*>(smem + kTilesBytes + (kD + 2 * kEdgesPerTile * kGeo) * sizeof(float));
-  uint32_t& tmem_base_s =
-      *reinterpret_cast<uint32_t*>(smem + kTilesBytes + (kD + 2 * kEdgesPerTile * kGeo) * sizeof(float) + sizeof(Bars));
-  if ((base - smem_u32(smem_raw)) + kTilesBytes + (kD + 2 * kEdgesPerTile * kGeo) * sizeof(float) + sizeof(Bars) + 16 > (uint32_t)kSmemBytes)
-    __trap();
-  uint8_t* const A2 = smem;                   // monomial tile A1, then the hidden layer
-  uint8_t* const S = A2 + kA2Bytes;           // two 16 KB halves (rows 0..63 / 64..127) of one layer's output tile
-  uint8_t* const W = S + kStageBytes;
-  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;   // warp-uniform
-  long long E = *num_edges_ptr;
-  if (E > edge_capacity) E = edge_capacity;
-  const long long tiles = (E + kEdgesPerTile - 1) / kEdgesPerTile;
-  const long long first = blockIdx.x, stride = gridDim.x;
-
-  for (int i = threadIdx.x; i < kD; i += kThreads3) s_b2[i] = b2[i];
+  for (int i = threadIdx.x; i < kD; i += kEdgeThreads) s_b2[i] = b2[i];
   if (threadIdx.x == 0) {
     for (int i = 0; i < kStages; ++i) { mbar_init(&bars.w_full[i], 1); mbar_init(&bars.w_empty[i], 1); }
     mbar_init(&bars.a1_full, kEpiWarps); mbar_init(&bars.a2_full, kEpiWarps);
@@ -999,7 +555,7 @@ edge_kernels_tc3_kernel(const double* __restrict__ dir, const double* __restrict
   const uint32_t tmem = tmem_base_s;
 
   if (warp == 3) {
-    // ---------------- geometry: the per-edge part of the invariants, up to two tiles ahead (as in version 1) --------
+    // ---------------- geometry: the per-edge part of the invariants, up to two tiles ahead ----------------
     uint32_t k = 0;
     for (long long tile = first; tile < tiles; tile += stride, ++k) {
       const int buf = k & 1;
@@ -1054,7 +610,7 @@ edge_kernels_tc3_kernel(const double* __restrict__ dir, const double* __restrict
       }
     }
   } else if (warp == 1) {
-    // ---------------- MMA issuer (warp-uniform, one elected lane; see version 1) ----------------
+    // ---------------- MMA issuer (warp-uniform, one elected lane; see the MLP kernel) ----------------
     if (first < tiles) {
       const uint32_t el = elect_one();
       const uint32_t a2_lo = umma_desc_lo(smem_u32(A2)), w_lo = umma_desc_lo(smem_u32(W));
@@ -1176,7 +732,7 @@ edge_kernels_tc3_kernel(const double* __restrict__ dir, const double* __restrict
       tmem_ld16_nowait(tmem + lane_addr + cgi * 32 + 16, r1);
       tmem_wait_ld();
     };
-    auto gen = [&](uint32_t k) {                     // monomials of tile ordinal k -> A2 (as A1), see version 1
+    auto gen = [&](uint32_t k) {                     // monomials of tile ordinal k -> A2 (GEMM1's A operand A1)
       const int buf = k & 1;
       mbar_wait(&bars.g_full[buf], (k >> 1) & 1);
       const float* gp = s_geo + (buf * kEdgesPerTile + (m >> 4)) * kGeo;
@@ -1362,8 +918,6 @@ edge_kernels_tc3_kernel(const double* __restrict__ dir, const double* __restrict
   }
 }
 
-int g_edge_variant = 3;      // 2: one epilogue group (16 warps); 3: two epilogue groups (G 16 + L 8 warps), the default
-
 int num_sms_tc() {
   static int sms = 0;
   if (!sms) {
@@ -1377,18 +931,7 @@ int num_sms_tc() {
 
 }  // namespace
 
-// debug only (not part of the public ABI): clock64 stamps of CTA 0 of the edge kernel, [6 tiles][2 roles][16]
-// debug only: select the edge-kernel implementation for same-process A/B timing (scratch/ab_edge.py)
-extern "C" int arreau_debug_set_edge_variant(int v) {
-  if (v < 2 || v > 3) return ARREAU_ERR_BAD_SHAPE;
-  g_edge_variant = v;
-  return ARREAU_OK;
-}
-
-extern "C" int arreau_debug_set_tc_profile_tile0(unsigned t0) {
-  return (int)cudaMemcpyToSymbol(g_tc_prof_tile0, &t0, sizeof(t0));
-}
-
+// debug only (not part of the public ABI): clock64 stamps of CTA 0 of the MLP and edge kernels (ARREAU_TC_PROFILE builds)
 extern "C" int arreau_debug_set_tc_profile(long long* buf) {
   return (int)cudaMemcpyToSymbol(g_tc_prof, &buf, sizeof(buf));
 }
@@ -1441,27 +984,15 @@ extern "C" int arreau_edge_kernels_f16(const double* dir, const double* dist, co
   if (edge_capacity < 0) return ARREAU_ERR_BAD_SHAPE;
   const long long tiles = (edge_capacity + edge::kEdgesPerTile - 1) / edge::kEdgesPerTile;
   const int grid = (int)(tiles < (long long)num_sms_tc() ? tiles : (long long)num_sms_tc());
-  if (g_edge_variant == 3) {
-    static bool attr3_set = false;
-    if (!attr3_set) {
-      cudaError_t e = cudaFuncSetAttribute(edge_kernels_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, edge3::kSmemBytes);
-      if (e != cudaSuccess) return (int)e;
-      attr3_set = true;
-    }
-    edge_kernels_tc3_kernel<<<grid, edge3::kThreads3, edge3::kSmemBytes, (cudaStream_t)stream>>>(
-        dir, dist, lattice, crystal_of_atom, src, num_edges_ptr, (long long)edge_capacity, ori, (const uint8_t*)w1_img,
-        (const uint8_t*)w_img, b2, radius, (__half*)kernels_f16);
-  } else {
-    static bool attr2_set = false;
-    if (!attr2_set) {
-      cudaError_t e = cudaFuncSetAttribute(edge_kernels_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, edge2::kSmemBytes);
-      if (e != cudaSuccess) return (int)e;
-      attr2_set = true;
-    }
-    edge_kernels_tc2_kernel<<<grid, kThreads, edge2::kSmemBytes, (cudaStream_t)stream>>>(
-        dir, dist, lattice, crystal_of_atom, src, num_edges_ptr, (long long)edge_capacity, ori, (const uint8_t*)w1_img,
-        (const uint8_t*)w_img, b2, radius, (__half*)kernels_f16);
+  static bool attr_set = false;
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(edge_kernels_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, edge::kSmemBytes);
+    if (e != cudaSuccess) return (int)e;
+    attr_set = true;
   }
+  edge_kernels_tc_kernel<<<grid, edge::kEdgeThreads, edge::kSmemBytes, (cudaStream_t)stream>>>(
+      dir, dist, lattice, crystal_of_atom, src, num_edges_ptr, (long long)edge_capacity, ori, (const uint8_t*)w1_img,
+      (const uint8_t*)w_img, b2, radius, (__half*)kernels_f16);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

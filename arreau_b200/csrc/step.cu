@@ -64,104 +64,30 @@ __global__ void step_noise_kernel(uint64_t seed, int step, long long n_normal, l
   }
 }
 
-// Per-crystal keyed draws of one evaluation batch (arreau_eval_noise).  Key = seed, counter = {crystal id (64 bits),
-// index within the crystal, stream tag}; tags 2..5 keep the counters apart from arreau_step_noise's tags 0 and 1.
-// Work items: [0, G) one per crystal (t, eps_l), [G, G + 2N) two per atom (eps_x), then ceil(Z/2) per atom (u).
-constexpr uint32_t kTagTimestep = 2, kTagLattice = 3, kTagFrac = 4, kTagType = 5;
-
-__global__ void eval_noise_kernel(uint64_t seed, int G, int N, int Z, int T, const int64_t* __restrict__ crystal_id,
-                                  const int32_t* __restrict__ atom_offset, const int32_t* __restrict__ crystal_of_atom,
-                                  int32_t* __restrict__ t_crystal, double* __restrict__ eps_x, double* __restrict__ u,
-                                  double* __restrict__ eps_l) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const int H = (Z + 1) / 2;
-  uint32_t r[4];
-  if (idx < G) {
-    const int g = (int)idx;
-    const uint64_t id = (uint64_t)crystal_id[g];
-    philox4x32_10(seed, id, 0u, kTagTimestep, r);
-    t_crystal[g] = min(1 + (int)(u01(r[0], r[1]) * (double)T), T);      // U{1..T}
-    double v[4];
-    philox4x32_10(seed, id, 0u, kTagLattice, r);
-    box_muller(r, v[0], v[1]);
-    philox4x32_10(seed, id, 1u, kTagLattice, r);
-    box_muller(r, v[2], v[3]);
-#pragma unroll
-    for (int d = 0; d < 3; ++d) eps_l[3 * (size_t)g + d] = v[d];
-    return;
-  }
-  long long j = idx - G;
-  if (j < 2LL * N) {
-    const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
-    const uint32_t a = (uint32_t)(b - atom_offset[g]);
-    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagFrac, r);
-    double v0, v1;
-    box_muller(r, v0, v1);
-    eps_x[3 * (size_t)b + 2 * k] = v0;
-    if (k == 0) eps_x[3 * (size_t)b + 1] = v1;
-    return;
-  }
-  j -= 2LL * N;
-  if (j < (long long)N * H) {
-    const int b = (int)(j / H), k = (int)(j % H), g = crystal_of_atom[b];
-    const uint32_t a = (uint32_t)(b - atom_offset[g]);
-    philox4x32_10(seed, (uint64_t)crystal_id[g], a * (uint32_t)H + k, kTagType, r);
-    u[(size_t)b * Z + 2 * k] = u01(r[0], r[1]);
-    if (2 * k + 1 < Z) u[(size_t)b * Z + 2 * k + 1] = u01(r[2], r[3]);
-  }
-}
-
-// Per-crystal keyed draws of the sampler (arreau_sample_init_keyed / arreau_sample_noise_keyed).  Same key and counter
-// words as eval_noise_kernel; the tag word of a step draw carries the step ordinal above its low 4 bits
-// (tag | step << 4, step < 2^28), so no draw of a trajectory meets another or arreau_step_noise's (0, 1) or
-// arreau_eval_noise's (2..5) tags.
-constexpr uint32_t kTagInitCell = 6, kTagInitFrac = 7, kTagStepLattice = 8, kTagStepFrac = 9, kTagStepType = 10;
+// Per-crystal keyed draws (arreau_eval_noise, arreau_sample_init_keyed, arreau_sample_noise_keyed).  Key = seed,
+// counter = {crystal id (64 bits), index within the crystal, tag word}.  A step's draws carry the step ordinal above the
+// tag's low 4 bits (tag | step << 4, step < 2^28), so no draw of a trajectory meets another, and the tags 2..10 keep
+// every keyed draw apart from arreau_step_noise's tags 0 and 1.
+struct KeyedTags {
+  uint32_t cell;              // per crystal, counter 0: one uniform (the timestep or the initial angle), if drawn
+  uint32_t len, len_ctr0;     // per crystal, counters len_ctr0, len_ctr0 + 1: three normals
+  uint32_t frac;              // per atom a, counters 2a, 2a + 1: three normals
+  uint32_t type;              // per atom a, counters a H .. a H + H - 1 with H = ceil(Z/2): Z uniforms
+};
+constexpr KeyedTags kEvalTags{2, 3, 0, 4, 5};        // t, eps_l, eps_x, u of an evaluation batch
+constexpr KeyedTags kInitTags{6, 6, 1, 7, 0};        // angle, lengths, frac of a sampler's initial state (no types)
+constexpr KeyedTags kStepTags{0, 8, 0, 9, 10};       // z_len, z_frac, u of one sampler step
 constexpr int kMaxKeyedStep = (1 << 28) - 1;
 
-// Work items: [0, G) one per crystal (beta, lengths), [G, G + 2N) two per atom (frac).
-__global__ void sample_init_keyed_kernel(uint64_t seed, int G, int N, const int64_t* __restrict__ crystal_id,
-                                         const int32_t* __restrict__ atom_offset,
-                                         const int32_t* __restrict__ crystal_of_atom, double pos_sigma_max,
-                                         double* __restrict__ angles, double* __restrict__ lengths,
-                                         double* __restrict__ frac) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  uint32_t r[4];
-  if (idx < G) {
-    const int g = (int)idx;
-    const uint64_t id = (uint64_t)crystal_id[g];
-    philox4x32_10(seed, id, 0u, kTagInitCell, r);
-    angles[3 * (size_t)g + 0] = 90.0;                          // monoclinic (90, U(90, 180), 90), degrees (quirk B5)
-    angles[3 * (size_t)g + 1] = 90.0 + 90.0 * u01(r[0], r[1]);
-    angles[3 * (size_t)g + 2] = 90.0;
-    double v[4];
-    philox4x32_10(seed, id, 1u, kTagInitCell, r);
-    box_muller(r, v[0], v[1]);
-    philox4x32_10(seed, id, 2u, kTagInitCell, r);
-    box_muller(r, v[2], v[3]);
-#pragma unroll
-    for (int d = 0; d < 3; ++d) lengths[3 * (size_t)g + d] = v[d];
-    return;
-  }
-  const long long j = idx - G;
-  if (j < 2LL * N) {
-    const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
-    const uint32_t a = (uint32_t)(b - atom_offset[g]);
-    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagInitFrac, r);
-    double v0, v1;
-    box_muller(r, v0, v1);
-    frac[3 * (size_t)b + 2 * k] = v0 * pos_sigma_max;
-    if (k == 0) frac[3 * (size_t)b + 1] = v1 * pos_sigma_max;
-  }
-}
-
-// Work items as eval_noise_kernel: [0, G) per crystal (z_len), [G, G + 2N) two per atom (z_frac), then ceil(Z/2) per
-// atom (u).  step_ptr (replay): the step ordinal is read from the device.
-__global__ void sample_noise_keyed_kernel(uint64_t seed, int step, int G, int N, int Z,
-                                          const int64_t* __restrict__ crystal_id,
-                                          const int32_t* __restrict__ atom_offset,
-                                          const int32_t* __restrict__ crystal_of_atom, double* __restrict__ z_len,
-                                          double* __restrict__ z_frac, double* __restrict__ u,
-                                          const int32_t* __restrict__ step_ptr) {
+// Work items: [0, G) one per crystal, [G, G + 2N) two per atom (the normals), then ceil(Z/2) per atom (the uniforms).
+// The per-crystal uniform goes to t_crystal as U{1..T} or to angles as the monoclinic (90, U(90, 180), 90) in degrees
+// (quirk B5), whichever is given.  step_ptr (replay): the step ordinal is read from the device.
+__global__ void keyed_noise_kernel(uint64_t seed, KeyedTags tags, int step, const int32_t* __restrict__ step_ptr, int G,
+                                   int N, int Z, const int64_t* __restrict__ crystal_id,
+                                   const int32_t* __restrict__ atom_offset, const int32_t* __restrict__ crystal_of_atom,
+                                   int T, int32_t* __restrict__ t_crystal, double* __restrict__ angles,
+                                   double* __restrict__ lengths, double frac_scale, double* __restrict__ frac,
+                                   double* __restrict__ u) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (step_ptr) step = *step_ptr;
   const uint32_t hi = (uint32_t)step << 4;
@@ -170,31 +96,41 @@ __global__ void sample_noise_keyed_kernel(uint64_t seed, int step, int G, int N,
   if (idx < G) {
     const int g = (int)idx;
     const uint64_t id = (uint64_t)crystal_id[g];
+    if (t_crystal || angles) {
+      philox4x32_10(seed, id, 0u, tags.cell | hi, r);
+      const double c = u01(r[0], r[1]);
+      if (t_crystal) t_crystal[g] = min(1 + (int)(c * (double)T), T);
+      if (angles) {
+        angles[3 * (size_t)g + 0] = 90.0;
+        angles[3 * (size_t)g + 1] = 90.0 + 90.0 * c;
+        angles[3 * (size_t)g + 2] = 90.0;
+      }
+    }
     double v[4];
-    philox4x32_10(seed, id, 0u, kTagStepLattice | hi, r);
+    philox4x32_10(seed, id, tags.len_ctr0, tags.len | hi, r);
     box_muller(r, v[0], v[1]);
-    philox4x32_10(seed, id, 1u, kTagStepLattice | hi, r);
+    philox4x32_10(seed, id, tags.len_ctr0 + 1, tags.len | hi, r);
     box_muller(r, v[2], v[3]);
 #pragma unroll
-    for (int d = 0; d < 3; ++d) z_len[3 * (size_t)g + d] = v[d];
+    for (int d = 0; d < 3; ++d) lengths[3 * (size_t)g + d] = v[d];
     return;
   }
   long long j = idx - G;
   if (j < 2LL * N) {
     const int b = (int)(j >> 1), k = (int)(j & 1), g = crystal_of_atom[b];
     const uint32_t a = (uint32_t)(b - atom_offset[g]);
-    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, kTagStepFrac | hi, r);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], 2u * a + k, tags.frac | hi, r);
     double v0, v1;
     box_muller(r, v0, v1);
-    z_frac[3 * (size_t)b + 2 * k] = v0;
-    if (k == 0) z_frac[3 * (size_t)b + 1] = v1;
+    frac[3 * (size_t)b + 2 * k] = v0 * frac_scale;
+    if (k == 0) frac[3 * (size_t)b + 1] = v1 * frac_scale;
     return;
   }
   j -= 2LL * N;
   if (j < (long long)N * H) {
     const int b = (int)(j / H), k = (int)(j % H), g = crystal_of_atom[b];
     const uint32_t a = (uint32_t)(b - atom_offset[g]);
-    philox4x32_10(seed, (uint64_t)crystal_id[g], a * (uint32_t)H + k, kTagStepType | hi, r);
+    philox4x32_10(seed, (uint64_t)crystal_id[g], a * (uint32_t)H + k, tags.type | hi, r);
     u[(size_t)b * Z + 2 * k] = u01(r[0], r[1]);
     if (2 * k + 1 < Z) u[(size_t)b * Z + 2 * k + 1] = u01(r[2], r[3]);
   }
@@ -257,17 +193,38 @@ extern "C" int arreau_workspace_bytes(int32_t N, int32_t G, int64_t edge_capacit
   return ARREAU_OK;
 }
 
+namespace {
+
+int launch_step_noise(uint64_t seed, int step, const int32_t* step_ptr, int G, int N, int Z, double* z_len,
+                      double* z_frac, double* u, cudaStream_t s) {
+  const long long n_len = 3LL * G, n_normal = n_len + 3LL * N, n_uniform = (long long)N * Z;
+  const long long work = ((n_normal > n_uniform ? n_normal : n_uniform) + 1) / 2;
+  step_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(seed, step, n_normal, n_uniform, z_len, n_len, z_frac,
+                                                                    u, step_ptr);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+int launch_keyed_noise(uint64_t seed, const KeyedTags& tags, int step, const int32_t* step_ptr, int G, int N, int Z,
+                       const int64_t* crystal_id, const int32_t* atom_offset, const int32_t* crystal_of_atom, int T,
+                       int32_t* t_crystal, double* angles, double* lengths, double frac_scale, double* frac, double* u,
+                       cudaStream_t s) {
+  const long long work = (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
+  keyed_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(seed, tags, step, step_ptr, G, N, Z, crystal_id,
+                                                                     atom_offset, crystal_of_atom, T, t_crystal, angles,
+                                                                     lengths, frac_scale, frac, u);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+}  // namespace
+
 extern "C" int arreau_step_noise(uint64_t seed, int32_t step, int32_t G, int32_t N, int32_t Z, double* z_len,
                                  double* z_frac, double* u, void* stream) {
   if (G < 0 || N < 0 || Z <= 0) return ARREAU_ERR_BAD_SHAPE;
-  const long long n_len = 3LL * G, n_normal = n_len + 3LL * N, n_uniform = (long long)N * Z;
-  const long long work = ((n_normal > n_uniform ? n_normal : n_uniform) + 1) / 2;
-  if (work == 0) return ARREAU_OK;          // an empty batch is a no-op (its buffers may be NULL)
+  if (G == 0 && N == 0) return ARREAU_OK;   // an empty batch is a no-op (its buffers may be NULL)
   if (!z_len || !z_frac || !u) return ARREAU_ERR_NULL;
-  step_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(seed, step, n_normal, n_uniform,
-                                                                                     z_len, n_len, z_frac, u, nullptr);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  return launch_step_noise(seed, step, nullptr, G, N, Z, z_len, z_frac, u, (cudaStream_t)stream);
 }
 
 extern "C" int arreau_eval_noise(uint64_t seed, int32_t G, int32_t N, int32_t Z, int32_t num_steps,
@@ -277,11 +234,8 @@ extern "C" int arreau_eval_noise(uint64_t seed, int32_t G, int32_t N, int32_t Z,
   if (G == 0) return ARREAU_OK;
   if (!crystal_id || !atom_offset || !t_crystal || !eps_l || (N > 0 && (!crystal_of_atom || !eps_x || !u)))
     return ARREAU_ERR_NULL;
-  const long long work = (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
-  eval_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      seed, G, N, Z, num_steps, crystal_id, atom_offset, crystal_of_atom, t_crystal, eps_x, u, eps_l);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  return launch_keyed_noise(seed, kEvalTags, 0, nullptr, G, N, Z, crystal_id, atom_offset, crystal_of_atom, num_steps,
+                            t_crystal, nullptr, eps_l, 1.0, eps_x, u, (cudaStream_t)stream);
 }
 
 extern "C" int arreau_sample_init_keyed(uint64_t seed, int32_t G, int32_t N, const int64_t* crystal_id,
@@ -292,15 +246,8 @@ extern "C" int arreau_sample_init_keyed(uint64_t seed, int32_t G, int32_t N, con
   if (G == 0) return ARREAU_OK;
   if (!crystal_id || !atom_offset || !angles || !lengths || (N > 0 && (!crystal_of_atom || !frac)))
     return ARREAU_ERR_NULL;
-  const long long work = (long long)G + 2LL * N;
-  sample_init_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      seed, G, N, crystal_id, atom_offset, crystal_of_atom, pos_sigma_max, angles, lengths, frac);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
-}
-
-static long long sample_noise_keyed_work(int G, int N, int Z) {
-  return (long long)G + 2LL * N + (long long)N * ((Z + 1) / 2);
+  return launch_keyed_noise(seed, kInitTags, 0, nullptr, G, N, 0, crystal_id, atom_offset, crystal_of_atom, 0, nullptr,
+                            angles, lengths, pos_sigma_max, frac, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t G, int32_t N, int32_t Z,
@@ -310,11 +257,8 @@ extern "C" int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t G,
   if (G < 0 || N < 0 || Z <= 0 || step < 0 || step > kMaxKeyedStep) return ARREAU_ERR_BAD_SHAPE;
   if (G == 0) return ARREAU_OK;
   if (!crystal_id || !atom_offset || !z_len || (N > 0 && (!crystal_of_atom || !z_frac || !u))) return ARREAU_ERR_NULL;
-  const long long work = sample_noise_keyed_work(G, N, Z);
-  sample_noise_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      seed, step, G, N, Z, crystal_id, atom_offset, crystal_of_atom, z_len, z_frac, u, nullptr);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  return launch_keyed_noise(seed, kStepTags, step, nullptr, G, N, Z, crystal_id, atom_offset, crystal_of_atom, 0, nullptr,
+                            nullptr, z_len, 1.0, z_frac, u, (cudaStream_t)stream);
 }
 
 #define ARREAU_TRY(call)        \
@@ -409,20 +353,23 @@ extern "C" int arreau_ponita_forward(const arreau_weights* w, const arreau_works
   return ARREAU_OK;
 }
 
-extern "C" int arreau_denoise_step(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
-                                   void* stream) {
-  if (!w || !ws || !a) return ARREAU_ERR_NULL;
+namespace {
+
+int lattice_from_angles(const arreau_step_args* a, int G, void* stream) {
+  if (a->angle_trig) return arreau_lattice_from_trig(a->lengths, a->angle_trig, G, a->lattice, stream);
+  return arreau_lattice_from_params(a->lengths, a->angles, G, a->lattice, stream);
+}
+
+// The launches of one denoise step after its noise is in place.  The timestep is a->t with the VP coefficients of `a`,
+// or, with t_of_atom, on the device: t_of_atom[N] and dyn = {t, VP coefficients} (arreau_denoise_step_replay).
+int denoise_step_body(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
+                      const int32_t* t_of_atom, const double* dyn, void* stream) {
   const int N = a->num_atoms_total, G = a->num_crystals, Z = w->num_states;
-  if (N < 0 || G < 0) return ARREAU_ERR_BAD_SHAPE;
-  if (N == 0 || G == 0) return ARREAU_OK;
-  if (w->num_scalar != Z + 2 * a->emb + 10 || w->num_vec != 4) return ARREAU_ERR_BAD_SHAPE;
+  const int t = t_of_atom ? 0 : a->t;
   // predict_scores: lattice, features, cartesian positions, graph, network   (diffusion_loss.py:112-197)
-  if (a->angle_trig)
-    ARREAU_TRY(arreau_lattice_from_trig(a->lengths, a->angle_trig, G, a->lattice, stream));
-  else
-    ARREAU_TRY(arreau_lattice_from_params(a->lengths, a->angles, G, a->lattice, stream));
+  ARREAU_TRY(lattice_from_angles(a, G, stream));
   ARREAU_TRY(arreau_assemble_features(a->frac, a->types, a->lengths, a->angles, a->lattice, a->atom_offset,
-                                      a->crystal_of_atom, nullptr, a->t, a->vp_betas, a->fourier_w, a->emb, N, G, Z,
+                                      a->crystal_of_atom, t_of_atom, t, a->vp_betas, a->fourier_w, a->emb, N, G, Z,
                                       a->x, a->vec, stream));
   ARREAU_TRY(arreau_frac_to_cart(a->frac, a->lattice, a->crystal_of_atom, N, a->pos, stream));
   const double r2 = a->radius * a->radius;
@@ -436,17 +383,29 @@ extern "C" int arreau_denoise_step(const arreau_weights* w, const arreau_workspa
                                    a->atom_offset, a->crystal_of_atom, N, G, a->radius, a->logits, a->score, a->len0,
                                    stream));
   // update: lengths, lattice, fractional coordinates, atom types   (diffusion_loss.py:338-349)
-  ARREAU_TRY(arreau_vp_lattice_reverse(a->lengths, a->len0, a->atom_offset, a->z_len, a->t, a->vp_cx0, a->vp_cxt,
-                                       a->vp_denom, a->vp_var, G, a->lengths, stream));
-  if (a->angle_trig)
-    ARREAU_TRY(arreau_lattice_from_trig(a->lengths, a->angle_trig, G, a->lattice, stream));
+  if (dyn)
+    ARREAU_TRY(arreau_vp_lattice_reverse_dyn(a->lengths, a->len0, a->atom_offset, a->z_len, dyn, G, a->lengths, stream));
   else
-    ARREAU_TRY(arreau_lattice_from_params(a->lengths, a->angles, G, a->lattice, stream));
-  ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, nullptr, a->t, a->ve_sigmas, N, a->frac, stream));
+    ARREAU_TRY(arreau_vp_lattice_reverse(a->lengths, a->len0, a->atom_offset, a->z_len, a->t, a->vp_cx0, a->vp_cxt,
+                                         a->vp_denom, a->vp_var, G, a->lengths, stream));
+  ARREAU_TRY(lattice_from_angles(a, G, stream));
+  ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, t_of_atom, t, a->ve_sigmas, N, a->frac, stream));
   if (a->update_types)
-    ARREAU_TRY(arreau_d3pm_reverse(a->types, a->logits, a->u_type, nullptr, a->t, a->q_keep, a->q_to_mask,
+    ARREAU_TRY(arreau_d3pm_reverse(a->types, a->logits, a->u_type, t_of_atom, t, a->q_keep, a->q_to_mask,
                                    a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->types, stream));
   return ARREAU_OK;
+}
+
+}  // namespace
+
+extern "C" int arreau_denoise_step(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
+                                   void* stream) {
+  if (!w || !ws || !a) return ARREAU_ERR_NULL;
+  const int N = a->num_atoms_total, G = a->num_crystals, Z = w->num_states;
+  if (N < 0 || G < 0) return ARREAU_ERR_BAD_SHAPE;
+  if (N == 0 || G == 0) return ARREAU_OK;
+  if (w->num_scalar != Z + 2 * a->emb + 10 || w->num_vec != 4) return ARREAU_ERR_BAD_SHAPE;
+  return denoise_step_body(w, ws, a, nullptr, nullptr, stream);
 }
 
 // The same step with every per-step scalar in device memory, so that ONE captured CUDA graph replays the whole
@@ -465,48 +424,14 @@ extern "C" int arreau_denoise_step_replay(const arreau_weights* w, const arreau_
   cudaStream_t s = (cudaStream_t)stream;
   step_advance_kernel<<<1, 1024, 0, s>>>(r->counter, r->t_first, r->vp_table, N, r->t_of_atom, r->dyn, r->step_out);
   CUDA_LAUNCH_CHECK();
-  if (r->crystal_id) {      // per-crystal keyed noise (arreau_sample_noise_keyed with the replay's step ordinal)
-    const long long work = sample_noise_keyed_work(G, N, Z);
-    sample_noise_keyed_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(
-        r->seed, 0, G, N, Z, r->crystal_id, a->atom_offset, a->crystal_of_atom, const_cast<double*>(a->z_len),
-        const_cast<double*>(a->z_frac), const_cast<double*>(a->u_type), r->step_out);
-    CUDA_LAUNCH_CHECK();
-  } else {
-    const long long n_len = 3LL * G, n_normal = n_len + 3LL * N, n_uniform = (long long)N * Z;
-    const long long work = ((n_normal > n_uniform ? n_normal : n_uniform) + 1) / 2;
-    // (the step's noise buffers are inputs of arreau_denoise_step; here the call itself fills them)
-    step_noise_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(r->seed, 0, n_normal, n_uniform,
-                                                                     const_cast<double*>(a->z_len), n_len,
-                                                                     const_cast<double*>(a->z_frac),
-                                                                     const_cast<double*>(a->u_type), r->step_out);
-    CUDA_LAUNCH_CHECK();
-  }
-  if (a->angle_trig)
-    ARREAU_TRY(arreau_lattice_from_trig(a->lengths, a->angle_trig, G, a->lattice, stream));
+  // (the step's noise buffers are inputs of arreau_denoise_step; here the call itself fills them)
+  double* const z_len = const_cast<double*>(a->z_len);
+  double* const z_frac = const_cast<double*>(a->z_frac);
+  double* const u = const_cast<double*>(a->u_type);
+  if (r->crystal_id)
+    ARREAU_TRY(launch_keyed_noise(r->seed, kStepTags, 0, r->step_out, G, N, Z, r->crystal_id, a->atom_offset,
+                                  a->crystal_of_atom, 0, nullptr, nullptr, z_len, 1.0, z_frac, u, s));
   else
-    ARREAU_TRY(arreau_lattice_from_params(a->lengths, a->angles, G, a->lattice, stream));
-  ARREAU_TRY(arreau_assemble_features(a->frac, a->types, a->lengths, a->angles, a->lattice, a->atom_offset,
-                                      a->crystal_of_atom, r->t_of_atom, 0, a->vp_betas, a->fourier_w, a->emb, N, G, Z,
-                                      a->x, a->vec, stream));
-  ARREAU_TRY(arreau_frac_to_cart(a->frac, a->lattice, a->crystal_of_atom, N, a->pos, stream));
-  const double r2 = a->radius * a->radius;
-  ARREAU_TRY(arreau_graph_count(a->pos, a->lattice, a->atom_offset, a->crystal_of_atom, N, G, r2, a->cap, 1,
-                                a->raw_count, a->deg, a->num_neighbors_image, stream));
-  ARREAU_TRY(arreau_graph_scan(a->deg, a->row_ptr, N, stream));
-  ARREAU_TRY(arreau_graph_fill(a->pos, a->lattice, a->atom_offset, a->crystal_of_atom, N, G, r2, a->cap, 1,
-                               a->raw_count, a->row_ptr, ws->edge_capacity, a->src, a->dst, a->cell, a->dist, a->dir,
-                               nullptr, nullptr, a->overflow_flag, stream));
-  ARREAU_TRY(arreau_ponita_forward(w, ws, a->precision, a->x, a->vec, a->row_ptr, a->src, a->dist, a->dir, a->lattice,
-                                   a->atom_offset, a->crystal_of_atom, N, G, a->radius, a->logits, a->score, a->len0,
-                                   stream));
-  ARREAU_TRY(arreau_vp_lattice_reverse_dyn(a->lengths, a->len0, a->atom_offset, a->z_len, r->dyn, G, a->lengths, stream));
-  if (a->angle_trig)
-    ARREAU_TRY(arreau_lattice_from_trig(a->lengths, a->angle_trig, G, a->lattice, stream));
-  else
-    ARREAU_TRY(arreau_lattice_from_params(a->lengths, a->angles, G, a->lattice, stream));
-  ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, r->t_of_atom, 0, a->ve_sigmas, N, a->frac, stream));
-  if (a->update_types)
-    ARREAU_TRY(arreau_d3pm_reverse(a->types, a->logits, a->u_type, r->t_of_atom, 0, a->q_keep, a->q_to_mask,
-                                   a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->types, stream));
-  return ARREAU_OK;
+    ARREAU_TRY(launch_step_noise(r->seed, 0, r->step_out, G, N, Z, z_len, z_frac, u, s));
+  return denoise_step_body(w, ws, a, r->t_of_atom, r->dyn, stream);
 }

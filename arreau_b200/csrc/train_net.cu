@@ -14,8 +14,9 @@
 //       sgemm_tma_kernel  ARREAU_PRECISION_TF32: persistent, warp-specialised tcgen05 kind::tf32 kernel fed by TMA tensor
 //                         maps, double-buffered TMEM accumulators, fused epilogues (bias, GELU, GELU', residual, column
 //                         sums) -- see the comment above it;
-//       sgemm_tc_kernel   the same product one tile per CTA with register-staged operands: fallback for operands a
-//                         tensor map cannot describe (K < 32, ragged contiguous extents);
+//       sgemm_tc_kernel   the same product one tile per CTA with register-staged operands: the TF32 path for operands a
+//                         tensor map cannot describe (K < 32, ragged contiguous extents); gemm() picks it from the
+//                         operands alone;
 //   * weight gradients reduce over the rows (edges x orientations, or atoms x orientations): split-K with
 //     per-split partial tiles and a fixed-order second stage -- no atomics, bit-reproducible run to run;
 //   * the message pass is transposed with a sender-side gather in edge order (deterministic) instead of
@@ -64,7 +65,6 @@ struct GemmArgs {
   const float* gz; long long gz_ld;
   const float* rowscale;
   const float* res_in; const float* res_scale;   // C2 = res_in[m][n] + res_scale[n] * v (pitch ldc) instead of the GELU
-  int mn_lbo, mn_sbo;
   int splits;                 // K splits (the persistent kernel's grid is not the tile grid)
   float* colsum_part;         // persistent kernel: per-CTA column sums of C, [grid / ntn * 4][N] (see GemmOpt::colsum_out), or null
   long long* prof;            // debug: per-CTA phase clocks of the persistent kernel ([grid][16]), or null
@@ -292,8 +292,6 @@ __device__ __forceinline__ void umma_tf32_e(uint32_t tmem_d, uint32_t a_lo, uint
 }
 }  // namespace tcg
 
-int g_tc_mn_lbo = 512, g_tc_mn_sbo = 2048;       // MN-major descriptor strides (bytes); debug-settable
-
 template <bool KCONTIG>
 __device__ __forceinline__ void tc_fetch(const float* __restrict__ X, long long ld, long long cblk, int x0, int xext,
                                          long long k0, long long kend, int tid, float4 (&r)[4]) {
@@ -355,7 +353,7 @@ sgemm_tc_kernel(const __grid_constant__ GemmArgs g) {
   const float* __restrict__ A = g.A;
   const float* __restrict__ B = g.B;
   const long long lda = g.lda, ldb = g.ldb, K = g.K, k_per_split = g.k_per_split;
-  const int M = g.M, N = g.N, mn_lbo = g.mn_lbo, mn_sbo = g.mn_sbo;
+  const int M = g.M, N = g.N;
   extern __shared__ __align__(1024) uint8_t gsm_raw[];
   const uint32_t base = (smem_u32(gsm_raw) + 1023u) & ~1023u;
   uint8_t* const sm = gsm_raw + (base - smem_u32(gsm_raw));
@@ -381,7 +379,8 @@ sgemm_tc_kernel(const __grid_constant__ GemmArgs g) {
   const uint32_t el = warp == 0 ? elect_one() : 0u;
   constexpr uint32_t kIdesc = tcg::idesc_tf32(!AK, !BK);
   // descriptor words: K-major: LBO unused (1), SBO = 1 KB (8-row groups), SWIZZLE_128B; MN-major: LBO = stride between the
-  // 32-element atoms along M/N, SBO = stride between the 4-k atoms, SWIZZLE_128B_BASE32B; version 1
+  // 32-element atoms along M/N, SBO = stride between the 4-k atoms (tc_stage's layout), SWIZZLE_128B_BASE32B; version 1
+  constexpr int mn_lbo = 512, mn_sbo = 2048;
   const uint32_t hi_k = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);
   const uint32_t hi_mn = (uint32_t)(mn_sbo >> 4) | (1u << 14) | (1u << 29);      // layout type 1 = SWIZZLE_128B_BASE32B
   const uint32_t a_hi = AK ? hi_k : hi_mn, b_hi = BK ? hi_k : hi_mn;
@@ -805,8 +804,6 @@ bool make_operand_map(CUtensorMap* m, const float* X, long long ld, long long cb
              CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-int g_tc_one_tile = 0;       // debug: 1 = sgemm_tc_kernel (one tile per CTA) instead of the persistent kernel (same-process A/B)
-
 // second stage of every split reduction: out[i] (=|+=) alpha * sum_s partial[s][i] in a FIXED order (deterministic):
 // a block covers 32 consecutive outputs with LANES split lanes; lane j adds the splits j, j + LANES, ... in order (coalesced
 // 128-byte reads), then the lane sums are added in lane order.  LANES = 32 for the long split lists of the column sums
@@ -873,7 +870,7 @@ int gemm(const Gemm& g, const float* A, long long lda, const float* B, long long
   const bool plain_out = !bias && !o.gelu_out && !o.gz && o.c_cblk == 128 && !o.colsum_out;   // what the split second stage can finish
   // tensor maps of the operands for the TMA-fed persistent kernel; an operand it cannot describe -> one tile per CTA
   alignas(64) CUtensorMap map_a, map_b;
-  const bool use_tma = g.tf32 && !g_tc_one_tile && make_operand_map<AK>(&map_a, A, lda, o.a_cblk, M, K) &&
+  const bool use_tma = g.tf32 && make_operand_map<AK>(&map_a, A, lda, o.a_cblk, M, K) &&
                        make_operand_map<BK>(&map_b, B, ldb, o.b_cblk, N, K);
   int splits = 1;
   if (K > 4096 && tiles < g.sms && plain_out) {      // reduction-dominated (weight gradients): split the rows
@@ -904,7 +901,7 @@ int gemm(const Gemm& g, const float* A, long long lda, const float* B, long long
   const bool fuse_colsum = o.colsum_out && use_tma && splits == 1 && ws_grid % ntn == 0 && o.c_cblk == 128 &&
                            (size_t)(ws_grid / ntn) * 4 * N <= g.partial_floats;
   GemmArgs a{A, lda, o.a_cblk, B, ldb, o.b_cblk, C, ldc, o.c_cblk, M, N, K, kps, alpha, bias, accumulate ? 1 : 0,
-             g.partial, o.gelu_out, o.gz, o.gz_ld, o.rowscale, o.res_in, o.res_scale, g_tc_mn_lbo, g_tc_mn_sbo, splits,
+             g.partial, o.gelu_out, o.gz, o.gz_ld, o.rowscale, o.res_in, o.res_scale, splits,
              fuse_colsum ? g.partial : nullptr, g_ws_prof};
   if (use_tma) {
     static bool attr_set = false;       // one flag per template instance
@@ -1494,18 +1491,6 @@ BwdBuffers carve(float* base, long long N, long long Ecap, int xl_pitch) {
 // ================================================================================================
 // C ABI
 // ================================================================================================
-// h[r][c] += ls[c] * m[r][c]   (convnext.py:31-32: layer_scale * x + input)
-__global__ void residual_add_kernel(const float* __restrict__ m, const float* __restrict__ ls, long long n4,
-                                    float* __restrict__ h) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n4) return;
-  const float4 mv = reinterpret_cast<const float4*>(m)[i];
-  const float4 sc = *reinterpret_cast<const float4*>(ls + (int)((i * 4) % kC));
-  float4 hv = reinterpret_cast<float4*>(h)[i];
-  hv.x = fmaf(sc.x, mv.x, hv.x); hv.y = fmaf(sc.y, mv.y, hv.y); hv.z = fmaf(sc.z, mv.z, hv.z); hv.w = fmaf(sc.w, mv.w, hv.w);
-  reinterpret_cast<float4*>(h)[i] = hv;
-}
-
 // Edge chain forward: monomials -> z1 -> a1 = gelu(z1) -> z2 -> kb = gelu(z2) * window, every matrix kept in the
 // workspace for the backward (geometry/invariants.py:10-31, embedding.py:10-14, ponita.py:65,94, windowing.py:21-29).
 // The activations leave the GEMMs' epilogues next to their pre-activations (no element-wise pass in between).
@@ -1599,16 +1584,9 @@ extern "C" int arreau_moments(const float* x, const float* sub_cols, int64_t n, 
   return ARREAU_OK;
 }
 
-// debug only (not part of the public ABI): TF32 GEMM implementation switch and MN-major descriptor strides
+// debug only (not part of the public ABI): per-CTA phase clocks of the persistent TF32 GEMM (GemmArgs::prof)
 extern "C" int arreau_debug_set_gemm_prof(long long* prof) {
   g_ws_prof = prof;
-  return ARREAU_OK;
-}
-
-extern "C" int arreau_debug_set_tf32_gemm(int legacy, int mn_lbo, int mn_sbo) {
-  g_tc_one_tile = legacy ? 1 : 0;        // 1 = the one-tile-per-CTA tcgen05 kernel instead of the persistent TMA-fed one
-  if (mn_lbo > 0) g_tc_mn_lbo = mn_lbo;
-  if (mn_sbo > 0) g_tc_mn_sbo = mn_sbo;
   return ARREAU_OK;
 }
 

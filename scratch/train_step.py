@@ -1,5 +1,4 @@
-"""A few C5 training steps (TF32 backward) for ncu launch lists: python scratch/train_step.py [steps] [legacy]"""
-import ctypes as C
+"""A few C5 training steps (TF32 backward) for ncu launch lists: python scratch/train_step.py [steps]"""
 import os
 import sys
 
@@ -7,18 +6,13 @@ import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from arreau_b200 import _lib  # noqa: E402
 from arreau_b200.diffusion.lattice_helpers import lattice_from_params  # noqa: E402
 from arreau_b200.synthetic import make_training_batch  # noqa: E402
 from arreau_b200.tables import build_tables  # noqa: E402
 from arreau_b200.training import FlatParams, FusedAdam, TrainEngine  # noqa: E402
 
 steps = int(sys.argv[1]) if len(sys.argv) > 1 else 3
-legacy = int(sys.argv[2]) if len(sys.argv) > 2 else 0
 dev = torch.device("cuda")
-lib = _lib.load()
-lib.arreau_debug_set_tf32_gemm.argtypes = [C.c_int, C.c_int, C.c_int]
-lib.arreau_debug_set_tf32_gemm(legacy, 0, 0)
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 w = np.load(os.path.join(ROOT, "tests", "golden", "weights_seed0.npz"))
 sd = {k: w[k] for k in w.files if k not in ("ori_grid", "fourier_w")}
@@ -45,4 +39,4 @@ for i in range(steps):
     e1.record()
     torch.cuda.synchronize()
     times.append(e0.elapsed_time(e1))
-print("G", G, "N", N, "E", te.eng.num_edges(), "legacy", legacy, "ms per step", np.round(times, 3).tolist(), "loss", te.loss.tolist()[0])
+print("G", G, "N", N, "E", te.eng.num_edges(), "ms per step", np.round(times, 3).tolist(), "loss", te.loss.tolist()[0])
