@@ -42,6 +42,11 @@ def sample_bravais_angles(lattice_type: str = "monoclinic"):
     return [90.0, np.random.uniform(90, 180), 90.0]
 
 
+def _fourier_w(t_emb_weights):
+    """The Gaussian Fourier frequencies of a GaussianFourierProjection, or the frequencies themselves."""
+    return getattr(t_emb_weights, "gaussian_fourier_proj_w", t_emb_weights)
+
+
 class _TrainStepLoss(torch.autograd.Function):
     """The scalar loss of one training step as an autograd node: the step's kernels have already produced the flat
     gradient buffer (TrainEngine.loss_and_grads), backward() hands its slices to the parameters."""
@@ -73,6 +78,7 @@ class DiffusionLoss(torch.nn.Module):
         self._engine = None
         self._engine_key = None
         self._train_engines = {}
+        self._eval_engines = {}
         self.backward_precision = "fp32"      # "tf32": tensor-core GEMMs in the backward pass (training.py)
         self.coord_loss_weight = self.atom_type_loss_weight = self.lattice_loss_weight = 1
 
@@ -107,62 +113,64 @@ class DiffusionLoss(torch.nn.Module):
         key = (id(net), na, str(device), debug, self.precision)
         packed = self.packed_weights(net, device)
         if self._engine is None or self._engine_key != key:
-            fw = t_emb_weights.gaussian_fourier_proj_w if hasattr(t_emb_weights, "gaussian_fourier_proj_w") else t_emb_weights
-            self._engine = DenoiseEngine(packed, self.tables, fw, na, self.cutoff, self.max_neighbors,
-                                         precision=self.precision, debug=debug, device=device)
+            self._engine = DenoiseEngine(packed, self.tables, _fourier_w(t_emb_weights), na, self.cutoff,
+                                         self.max_neighbors, precision=self.precision, debug=debug, device=device)
             self._engine_key = key
         elif self._engine.w is not packed:
             self._engine.w = packed
         return self._engine
 
+    @staticmethod
+    def _batch_engine(cache: dict, key, num_atoms, build, capacity=None, headroom: float = 1.25):
+        """The capacity-based engine cache[key], re-bound to the batch topology `num_atoms`.  It is rebuilt by
+        build(node_capacity, crystal_capacity) only when there is none or the batch exceeds its capacity: for
+        `capacity` (atoms, crystals), by default `headroom` x this batch, never below the old engine's."""
+        eng = cache.get(key)
+        if eng is not None and eng.fits(num_atoms):
+            if tuple(num_atoms) != eng.eng.topology:
+                eng.set_topology(num_atoms)
+            return eng
+        n_cap, g_cap = capacity or (int(sum(num_atoms) * headroom), int(len(num_atoms) * headroom))
+        if eng is not None:
+            n_cap, g_cap = max(n_cap, eng.eng.N_cap), max(g_cap, eng.eng.G_cap)
+        cache.pop(key, None)
+        eng = None                                          # free the old buffers before allocating the larger ones
+        cache[key] = eng = build(n_cap, g_cap)
+        return eng
+
     # -- training step (diffusion_loss.py:95-110,199-274) ---------------------------------------------
-    def train_engine_for(self, net, t_emb_weights, num_atoms, device, headroom: float = 1.25):
+    def train_engine_for(self, net, t_emb_weights, num_atoms, device):
         """ONE capacity-based TrainEngine per (parameters, backward precision): every batch topology (atoms per crystal)
-        is bound to its buffers in place; it is rebuilt -- with `headroom` -- only when a batch exceeds the capacity
+        is bound to its buffers in place; it is rebuilt -- with headroom -- only when a batch exceeds the capacity
         (the first batches of the first epoch), so a shuffled epoch does not reallocate (`self.train_engine_builds`
         counts the builds)."""
         from ..training import TrainEngine
         flat = net.flat if getattr(net, "flat", None) is not None and self._same_device(net.flat.device, device) \
             else net.flatten_parameters(device)
         na = [int(v) for v in torch.as_tensor(num_atoms).reshape(-1).tolist()]
-        key = (id(flat), self.backward_precision)
-        te = self._train_engines.get(key)
-        if te is None or not te.fits(na):
-            n_cap = max(int(sum(na) * headroom), te.eng.N_cap if te is not None else 0)
-            g_cap = max(int(len(na) * headroom), te.eng.G_cap if te is not None else 0)
-            fw = t_emb_weights.gaussian_fourier_proj_w if hasattr(t_emb_weights, "gaussian_fourier_proj_w") else t_emb_weights
-            self._train_engines.pop(key, None)
-            te = None                                           # free the old buffers before allocating the larger ones
-            te = TrainEngine(flat, self.tables, fw, net.ori_grid, na, self.cutoff, self.max_neighbors, device=device,
-                             backward_precision=self.backward_precision, node_capacity=n_cap, crystal_capacity=g_cap)
-            self._train_engines[key] = te
+
+        def build(n_cap, g_cap):
+            te = TrainEngine(flat, self.tables, _fourier_w(t_emb_weights), net.ori_grid, na, self.cutoff,
+                             self.max_neighbors, device=device, backward_precision=self.backward_precision,
+                             node_capacity=n_cap, crystal_capacity=g_cap)
             self.train_engine_builds = getattr(self, "train_engine_builds", 0) + 1
-        elif tuple(na) != te.eng.topology:
-            te.set_topology(na)
-        return te
+            return te
+        return self._batch_engine(self._train_engines, (id(flat), self.backward_precision), na, build)
 
     # -- evaluation (validation / test loss, arreau_b200/evaluation.py) --------------------------------
-    def eval_engine_for(self, net, t_emb_weights, num_atoms, device, capacity=None, headroom: float = 1.25):
+    def eval_engine_for(self, net, t_emb_weights, num_atoms, device, capacity=None):
         """ONE capacity-based EvalEngine (model precision, its own buffers: the training and sampling engines are not
-        touched), re-bound to every batch topology; rebuilt only when a batch exceeds the capacity.  capacity:
-        (atoms, crystals) to size it for up front."""
+        touched), re-bound to every batch topology; rebuilt only when a batch exceeds the capacity, and dropped when
+        the precision or the device changes.  capacity: (atoms, crystals) to size it for up front."""
         from ..evaluation import EvalEngine
         na = [int(v) for v in np.asarray(num_atoms).reshape(-1)]
-        ee = getattr(self, "_eval_engine", None)
-        if ee is not None and (ee.eng.precision != self.precision or not self._same_device(ee.device, device)):
-            ee = None
-        if ee is None or not ee.fits(na):
-            n_cap, g_cap = capacity if capacity is not None else (int(sum(na) * headroom), int(len(na) * headroom))
-            if ee is not None:
-                n_cap, g_cap = max(n_cap, ee.eng.N_cap), max(g_cap, ee.eng.G_cap)
-            fw = t_emb_weights.gaussian_fourier_proj_w if hasattr(t_emb_weights, "gaussian_fourier_proj_w") else t_emb_weights
-            self._eval_engine = ee = None                       # free the old buffers before allocating the larger ones
-            ee = EvalEngine(self.packed_weights(net, device), self.tables, fw, na, self.cutoff, self.max_neighbors,
-                            precision=self.precision, device=device, node_capacity=n_cap, crystal_capacity=g_cap)
-            self._eval_engine = ee
-        elif tuple(na) != ee.eng.topology:
-            ee.set_topology(na)
-        return ee
+        key = (self.precision, torch.device(device))
+        if key not in self._eval_engines:
+            self._eval_engines.clear()                      # one evaluation engine
+        build = lambda n_cap, g_cap: EvalEngine(  # noqa: E731
+            self.packed_weights(net, device), self.tables, _fourier_w(t_emb_weights), na, self.cutoff, self.max_neighbors,
+            precision=self.precision, device=device, node_capacity=n_cap, crystal_capacity=g_cap)
+        return self._batch_engine(self._eval_engines, key, na, build, capacity)
 
     @torch.no_grad()
     def evaluate(self, model, batch, t_emb_weights, crystal_ids, seed: int = 0, timestep=None, noise=None,

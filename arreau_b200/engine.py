@@ -374,12 +374,16 @@ class DenoiseEngine:
                   self.score.data_ptr(), self.len0.data_ptr(), self.stream)
         return self.logits, self.score, self.len0
 
-    def predict_scores(self, t) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-        """DiffusionLoss.predict_scores (diffusion_loss.py:112-197) on the engine state.
-        Returns (score[N,3], logits[N,Z], len0[G,3]) as fp32 device tensors (views of engine buffers)."""
-        self.prepare_inputs(t)
+    def prepare_batch(self, t, from_trig: bool = True) -> None:
+        """Inputs and graph of a forward on the engine state (prepare_inputs, then the radius graph)."""
+        self.prepare_inputs(t, from_trig)
         self._ensure_capacity()
         self.build_graph()
+
+    def predict_scores(self, t, from_trig: bool = True) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """DiffusionLoss.predict_scores (diffusion_loss.py:112-197) on the engine state; from_trig as in prepare_inputs.
+        Returns (score[N,3], logits[N,Z], len0[G,3]) as fp32 device tensors (views of engine buffers)."""
+        self.prepare_batch(t, from_trig)
         self.ws.onehot_types = self.types.data_ptr()      # x was assembled from self.types
         try:
             self.forward()

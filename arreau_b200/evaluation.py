@@ -1,8 +1,9 @@
 """Forward-only loss evaluation (validation / test loss) on the GPU.
 
-Per batch: upload -> per-crystal keyed noise (arreau_eval_noise) -> the training step's noising (`noise_into`) ->
-graph + forward (fp32 SIMT or fp16 tcgen05, the model's precision) -> per-crystal loss sums (arreau_eval_loss).  No
-backward, no gradient buffers, no torch RNG: evaluation leaves the training run exactly as it was.  Because every
+Per batch: per-crystal keyed noise (arreau_eval_noise) -> upload -> the training step's noising
+(`BatchEngine.noise_batch`) -> graph + forward (fp32 SIMT or fp16 tcgen05, the model's precision) -> per-crystal loss
+sums (arreau_eval_loss).  No backward, no gradient buffers, no torch RNG: evaluation leaves the training run exactly as
+it was.  Because every
 crystal's draws are keyed by (seed, crystal id) and its loss terms are summed over its own atoms only, the per-crystal
 numbers -- and every metric rebuilt from them -- do not depend on how the split is grouped into GPU batches or spread
 over ranks.
@@ -10,7 +11,7 @@ over ranks.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Sequence
+from typing import Dict, Optional
 
 import attr
 import numpy as np
@@ -19,10 +20,7 @@ import torch.distributed as dist
 
 from . import _lib
 from .distributed import all_gather_rows, shard_range
-from .engine import DenoiseEngine
-from .tables import DiffusionTables
-from .training import HYBRID_LOSS_COEFF, BatchEngine, noise_into, noising_buffers
-from .weights import PonitaWeights
+from .training import HYBRID_LOSS_COEFF, BatchEngine
 
 LOSS_PARTS = ("loss", "e_frac", "vb", "ce", "e_lat")
 
@@ -40,51 +38,23 @@ class EvalEngine(BatchEngine):
     """A capacity-sized DenoiseEngine (no debug buffers, no backward workspace) plus the noising buffers, re-bound per
     batch with `set_topology` like TrainEngine."""
 
-    def __init__(self, weights: PonitaWeights, tables: DiffusionTables, fourier_w, num_atoms: Sequence[int],
-                 radius: float, max_neighbors: int, precision: str = "fp32", device="cuda",
-                 node_capacity: Optional[int] = None, crystal_capacity: Optional[int] = None):
-        self.tabs = tables
-        self.device = dev = torch.device(device)
-        self.eng = DenoiseEngine(weights, tables, fourier_w, num_atoms, radius, max_neighbors, precision=precision,
-                                 debug=False, device=dev, node_capacity=node_capacity, crystal_capacity=crystal_capacity)
-        e = self.eng
-        self._bufs = noising_buffers(e.N_cap, e.G_cap, e.Z, dev)
-        self._bufs["crystal_ids"] = ("G", torch.zeros(e.G_cap, dtype=torch.int64, device=dev))
-        self._bufs["per_crystal"] = ("G", torch.zeros(e.G_cap, 4, dtype=torch.float64, device=dev))
-        self.d_alpha_bars = tables.vp_alpha_bars.to(torch.float32).to(dev)
-        self._bind()
+    def _own_bufs(self, N: int, G: int, Z: int) -> Dict[str, tuple]:
+        return {"crystal_ids": ("G", torch.zeros(G, dtype=torch.int64, device=self.device)),
+                "per_crystal": ("G", torch.zeros(G, 4, dtype=torch.float64, device=self.device))}
 
     def run(self, frac0, types0, lattice0, crystal_ids, seed: int = 0, timestep=None, noise=None):
         """Loss terms per crystal of the bound batch; returns (t_crystal[G], per_crystal[G,4]) as views of the engine's
         buffers.  timestep (scalar or [G]) / noise (eps_x[N,3], u[N,Z], eps_l[G,3]) replace the keyed draws."""
         e, tb = self.eng, self.tabs
-        self.frac0.copy_(torch.as_tensor(frac0).reshape(e.N, 3), non_blocking=True)
-        self.types0.copy_(torch.as_tensor(types0).reshape(e.N), non_blocking=True)
-        self.lattice0.copy_(torch.as_tensor(lattice0).reshape(e.G, 3, 3), non_blocking=True)
         ids = torch.as_tensor(crystal_ids, dtype=torch.int64).reshape(e.G)
         self.crystal_ids.copy_(ids.pin_memory() if ids.device.type == "cpu" else ids, non_blocking=True)
         if timestep is None or noise is None:
             _lib.call("arreau_eval_noise", C.c_uint64(int(seed)), e.G, e.N, e.Z, tb.T, self.crystal_ids.data_ptr(),
                       e.atom_offset.data_ptr(), e.crystal_of_atom.data_ptr(), self.t_crystal.data_ptr(),
                       self.eps_x.data_ptr(), self.u.data_ptr(), self.eps_l.data_ptr(), e.stream)
-        if timestep is not None:
-            t = torch.as_tensor(timestep).reshape(-1)
-            self.t_crystal.copy_((t.expand(e.G) if t.numel() == 1 else t).to(torch.int32), non_blocking=True)
-        if noise is not None:
-            eps_x, u, eps_l = noise
-            self.eps_x.copy_(torch.as_tensor(eps_x).reshape(e.N, 3), non_blocking=True)
-            self.u.copy_(torch.as_tensor(u).reshape(e.N, e.Z), non_blocking=True)
-            self.eps_l.copy_(torch.as_tensor(eps_l).reshape(e.G, 3), non_blocking=True)
-        torch.index_select(self.t_crystal, 0, e.crystal_of_atom[: e.N], out=self.t_atom)
-        noise_into(e, self)
-        e.prepare_inputs(self.t_atom, from_trig=False)
-        e._ensure_capacity()
-        e.build_graph()
-        e.ws.onehot_types = e.types.data_ptr()          # x[:, :Z] is one_hot(e.types)
-        try:
-            e.forward()
-        finally:
-            e.ws.onehot_types = None
+        self.upload_batch(frac0, types0, lattice0, timestep, noise)
+        self.noise_batch()
+        e.predict_scores(self.t_atom, from_trig=False)
         _lib.call("arreau_eval_loss", e.score.data_ptr(), e.logits.data_ptr(), e.len0.data_ptr(),
                   self.target_eps.data_ptr(), self.types0.data_ptr(), e.types.data_ptr(), self.t_atom.data_ptr(),
                   self.lengths0.data_ptr(), e.atom_offset.data_ptr(), e.d_q_keep.data_ptr(), e.d_q_to_mask.data_ptr(),

@@ -212,36 +212,29 @@ class FusedAdam:
             self.ema.version += 1
 
 
-def noising_buffers(N: int, G: int, Z: int, dev) -> Dict[str, tuple]:
-    """Capacity buffers of a clean batch, its random draws and the noising outputs: name -> (leading extent kind,
-    buffer), the layout `noise_into` reads."""
-    f64 = lambda *s: torch.zeros(*s, dtype=torch.float64, device=dev)  # noqa: E731
-    return {"frac0": ("N", f64(N, 3)), "types0": ("N", torch.zeros(N, dtype=torch.int64, device=dev)),
-            "lattice0": ("G", f64(G, 3, 3)), "lengths0": ("G", f64(G, 3)), "angles0": ("G", f64(G, 3)),
-            "target_eps": ("N", f64(N, 3)), "eps_x": ("N", f64(N, 3)), "u": ("N", f64(N, Z)), "eps_l": ("G", f64(G, 3)),
-            "t_crystal": ("G", torch.ones(G, dtype=torch.int32, device=dev)),
-            "t_atom": ("N", torch.ones(N, dtype=torch.int32, device=dev)), "terms": ("3N", f64(3 * N))}
-
-
-def noise_into(e: DenoiseEngine, b) -> None:
-    """VE_pbc.forward, D3PM.get_xt, matrix_to_params + VP_lattice.forward (diffusion_loss.py:218-237) of the clean
-    batch held by `b` (the `noising_buffers` of a training or evaluation engine, bound to e's topology) into the forward
-    engine's state."""
-    s = e.stream
-    _lib.call("arreau_matrix_to_params", b.lattice0.data_ptr(), e.G, b.lengths0.data_ptr(), b.angles0.data_ptr(), s)
-    _lib.call("arreau_ve_pbc_forward", b.frac0.data_ptr(), b.eps_x.data_ptr(), b.t_atom.data_ptr(),
-              e.d_ve_sigmas.data_ptr(), b.lattice0.data_ptr(), e.crystal_of_atom.data_ptr(), e.N,
-              e.frac.data_ptr(), b.target_eps.data_ptr(), s)
-    _lib.call("arreau_d3pm_q_sample", b.types0.data_ptr(), b.u.data_ptr(), b.t_atom.data_ptr(),
-              e.d_q_keep.data_ptr(), e.d_q_to_mask.data_ptr(), e.N, e.Z, e.types.data_ptr(), s)
-    _lib.call("arreau_vp_lattice_forward", b.lengths0.data_ptr(), b.eps_l.data_ptr(), b.t_crystal.data_ptr(),
-              b.d_alpha_bars.data_ptr(), e.G, e.lengths.data_ptr(), s)
-    e.angles.copy_(b.angles0)
-
-
 class BatchEngine:
     """A DenoiseEngine plus per-batch buffers (`_bufs`: name -> (leading extent kind, capacity buffer)) sized for a
-    CAPACITY and re-bound in place to every batch topology."""
+    CAPACITY and re-bound in place to every batch topology: the clean batch, its random draws and the noising outputs,
+    and a subclass's own buffers (`_own_bufs`)."""
+
+    def __init__(self, weights: PonitaWeights, tables: DiffusionTables, fourier_w, num_atoms: Sequence[int],
+                 radius: float, max_neighbors: int, precision: str = "fp32", device="cuda",
+                 node_capacity: Optional[int] = None, crystal_capacity: Optional[int] = None, debug: bool = False):
+        self.tabs = tables
+        self.device = dev = torch.device(device)
+        self.eng = e = DenoiseEngine(weights, tables, fourier_w, num_atoms, radius, max_neighbors, precision=precision,
+                                     debug=debug, device=dev, node_capacity=node_capacity,
+                                     crystal_capacity=crystal_capacity)
+        N, G, Z = e.N_cap, e.G_cap, e.Z
+        f64 = lambda *s: torch.zeros(*s, dtype=torch.float64, device=dev)  # noqa: E731
+        self._bufs = {"frac0": ("N", f64(N, 3)), "types0": ("N", torch.zeros(N, dtype=torch.int64, device=dev)),
+                      "lattice0": ("G", f64(G, 3, 3)), "lengths0": ("G", f64(G, 3)), "angles0": ("G", f64(G, 3)),
+                      "target_eps": ("N", f64(N, 3)), "eps_x": ("N", f64(N, 3)), "u": ("N", f64(N, Z)),
+                      "eps_l": ("G", f64(G, 3)), "t_crystal": ("G", torch.ones(G, dtype=torch.int32, device=dev)),
+                      "t_atom": ("N", torch.ones(N, dtype=torch.int32, device=dev)), "terms": ("3N", f64(3 * N))}
+        self._bufs.update(self._own_bufs(N, G, Z))
+        self.d_alpha_bars = tables.vp_alpha_bars.to(torch.float32).to(dev)
+        self._bind()
 
     def _bind(self) -> None:
         e = self.eng
@@ -258,6 +251,40 @@ class BatchEngine:
         self.eng.set_topology(num_atoms)
         self._bind()
 
+    def upload_batch(self, frac0, types0, lattice0, timestep=None, noise=None) -> None:
+        """Batch{X0, A0, L0}, and when given the timesteps (a scalar, [G] or [G,1]) and the noise (eps_x[N,3], u[N,Z],
+        eps_l[G,3]) in place of what the buffers hold; t_atom is gathered from the timesteps."""
+        e = self.eng
+        self.frac0.copy_(torch.as_tensor(frac0).reshape(e.N, 3), non_blocking=True)
+        self.types0.copy_(torch.as_tensor(types0).reshape(e.N), non_blocking=True)
+        self.lattice0.copy_(torch.as_tensor(lattice0).reshape(e.G, 3, 3), non_blocking=True)
+        if timestep is not None:
+            t = torch.as_tensor(timestep).reshape(-1)
+            self.t_crystal.copy_((t.expand(e.G) if t.numel() == 1 else t).to(torch.int32), non_blocking=True)
+        # one gather through the engine's atom -> crystal map (repeat_interleave would upload the counts and synchronise)
+        torch.index_select(self.t_crystal, 0, e.crystal_of_atom[: e.N], out=self.t_atom)
+        if noise is not None:
+            eps_x, u, eps_l = noise
+            self.eps_x.copy_(torch.as_tensor(eps_x).reshape(e.N, 3), non_blocking=True)
+            self.u.copy_(torch.as_tensor(u).reshape(e.N, e.Z), non_blocking=True)
+            self.eps_l.copy_(torch.as_tensor(eps_l).reshape(e.G, 3), non_blocking=True)
+
+    def noise_batch(self) -> None:
+        """VE_pbc.forward, D3PM.get_xt, matrix_to_params + VP_lattice.forward (diffusion_loss.py:218-237) of the clean
+        batch into the forward engine's state."""
+        e = self.eng
+        s = e.stream
+        _lib.call("arreau_matrix_to_params", self.lattice0.data_ptr(), e.G, self.lengths0.data_ptr(),
+                  self.angles0.data_ptr(), s)
+        _lib.call("arreau_ve_pbc_forward", self.frac0.data_ptr(), self.eps_x.data_ptr(), self.t_atom.data_ptr(),
+                  e.d_ve_sigmas.data_ptr(), self.lattice0.data_ptr(), e.crystal_of_atom.data_ptr(), e.N,
+                  e.frac.data_ptr(), self.target_eps.data_ptr(), s)
+        _lib.call("arreau_d3pm_q_sample", self.types0.data_ptr(), self.u.data_ptr(), self.t_atom.data_ptr(),
+                  e.d_q_keep.data_ptr(), e.d_q_to_mask.data_ptr(), e.N, e.Z, e.types.data_ptr(), s)
+        _lib.call("arreau_vp_lattice_forward", self.lengths0.data_ptr(), self.eps_l.data_ptr(), self.t_crystal.data_ptr(),
+                  self.d_alpha_bars.data_ptr(), e.G, e.lengths.data_ptr(), s)
+        e.angles.copy_(self.angles0)
+
 
 class TrainEngine(BatchEngine):
     """The training step's buffers on one GPU, sized for a CAPACITY (atoms, crystals) and re-bound in place to every
@@ -273,25 +300,22 @@ class TrainEngine(BatchEngine):
         if backward_precision not in ("fp32", "tf32"):
             raise ValueError("backward_precision must be 'fp32' or 'tf32'")
         self.backward_precision = _lib.PRECISION_TF32 if backward_precision == "tf32" else _lib.PRECISION_FP32
-        self.p, self.tabs = params, tables
-        self.device = dev = torch.device(device)
+        self.p = params
+        dev = torch.device(device)
         self.ori = (ori_grid.detach() if isinstance(ori_grid, torch.Tensor) else torch.as_tensor(np.asarray(ori_grid))) \
             .to(dev, torch.float32).contiguous()
         self.w = PonitaWeights.from_flat(params, self.ori)
-        self.eng = DenoiseEngine(self.w, tables, fourier_w, num_atoms, radius, max_neighbors, precision="fp32",
-                                 debug=True, device=dev, node_capacity=node_capacity, crystal_capacity=crystal_capacity)
-        e = self.eng
-        N, G, Z = e.N_cap, e.G_cap, e.Z
+        super().__init__(self.w, tables, fourier_w, num_atoms, radius, max_neighbors, device=dev,
+                         node_capacity=node_capacity, crystal_capacity=crystal_capacity, debug=True)
         f64 = lambda *s: torch.zeros(*s, dtype=torch.float64, device=dev)  # noqa: E731
-        f32 = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)  # noqa: E731
-        self._bufs = noising_buffers(N, G, Z, dev)
-        self._bufs.update({"dscore": ("N", f32(N, 3)), "dlogits": ("N", f32(N, Z)), "dlen0": ("G", f32(G, 3))})
         self.loss = f64(5)
-        self.d_alpha_bars = tables.vp_alpha_bars.to(torch.float32).to(dev)
         self.fold = torch.as_tensor(monomial_fold_table(), dtype=torch.int32).to(dev)
         self.mom_scratch, self.mom_out = f64(512), f64(2)
         self._bwd_ws = None
-        self._bind()
+
+    def _own_bufs(self, N: int, G: int, Z: int) -> Dict[str, tuple]:
+        f32 = lambda *s: torch.zeros(*s, dtype=torch.float32, device=self.device)  # noqa: E731
+        return {"dscore": ("N", f32(N, 3)), "dlogits": ("N", f32(N, Z)), "dlen0": ("G", f32(G, 3))}
 
     # ------------------------------------------------------------------ pieces (each = the mirrored reference call)
     def repack(self) -> None:
@@ -301,20 +325,7 @@ class TrainEngine(BatchEngine):
 
     def set_batch(self, frac0, types0, lattice0, timestep, eps_x, u, eps_l) -> None:
         """Batch{X0, A0, L0} and the step's random draws (diffusion_loss.py:205-237).  timestep: [G] or [G,1]."""
-        e = self.eng
-        self.frac0.copy_(torch.as_tensor(frac0).reshape(e.N, 3), non_blocking=True)
-        self.types0.copy_(torch.as_tensor(types0).reshape(e.N), non_blocking=True)
-        self.lattice0.copy_(torch.as_tensor(lattice0).reshape(e.G, 3, 3), non_blocking=True)
-        self.t_crystal.copy_(torch.as_tensor(timestep).reshape(e.G).to(torch.int32), non_blocking=True)
-        # one gather through the engine's atom -> crystal map (repeat_interleave would upload the counts and synchronise)
-        torch.index_select(self.t_crystal, 0, e.crystal_of_atom[: e.N], out=self.t_atom)
-        self.eps_x.copy_(torch.as_tensor(eps_x).reshape(e.N, 3), non_blocking=True)
-        self.u.copy_(torch.as_tensor(u).reshape(e.N, e.Z), non_blocking=True)
-        self.eps_l.copy_(torch.as_tensor(eps_l).reshape(e.G, 3), non_blocking=True)
-
-    def noise_batch(self) -> None:
-        """VE_pbc.forward, D3PM.get_xt, matrix_to_params + VP_lattice.forward into the forward engine's state."""
-        noise_into(self.eng, self)
+        self.upload_batch(frac0, types0, lattice0, timestep, (eps_x, u, eps_l))
 
     def _workspace(self) -> torch.Tensor:
         e = self.eng
@@ -332,9 +343,7 @@ class TrainEngine(BatchEngine):
         activations for the backward (arreau_ponita_forward_train); "fp32": the plain fp32 forward (the parity path),
         the backward recomputes what it needs."""
         e = self.eng
-        e.prepare_inputs(self.t_atom, from_trig=False)
-        e._ensure_capacity()
-        e.build_graph()
+        e.prepare_batch(self.t_atom, from_trig=False)
         self._forward_kept = 0
         if self.backward_precision == _lib.PRECISION_TF32:
             ws = self._workspace()

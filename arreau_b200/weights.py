@@ -8,6 +8,7 @@ and is passed explicitly.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Dict, Mapping
 
 import numpy as np
@@ -98,6 +99,8 @@ class PonitaWeights:
         w1 = sd["basis_fn.1.weight"]
         if w1.shape != (HIDDEN, 258) or sd["basis_fn.3.weight"].shape != (BASIS, HIDDEN):
             raise ValueError("unsupported model dims: kernels are specialised on hidden 128 / basis 256 / degree 3")
+        if sd["fiber_basis_fn.1.weight"].shape != (HIDDEN, 3):
+            raise ValueError("unsupported fiber basis input width")
         L = LAYERS
         for l in range(L):
             if f"interaction_layers.{l}.conv.kernel.weight" not in sd:
@@ -110,33 +113,11 @@ class PonitaWeights:
         w1m_t = np.zeros((MONO_PAD, HIDDEN))
         w1m_t[:NUM_MONO] = w1m.T
         w1m_t[NUM_MONO] = sd["basis_fn.1.bias"]            # constant-1 monomial carries the bias
-        lay = lambda name: np.stack([sd[f"interaction_layers.{l}.{name}"] for l in range(L)])  # noqa: E731
-        wk = lay("conv.kernel.weight")                     # [L,C,D]
-        wemb = sd["x_embedder.weight"]                     # [C, F+V]
-        wr = np.stack([sd[f"read_out_layers.{l}.weight"] for l in range(L)])   # [L,R,C]
-        br = np.stack([sd[f"read_out_layers.{l}.bias"] for l in range(L)])
-        self.num_readout = wr.shape[1]
-        self.num_states = self.num_readout - 4             # scalars | 1 vector | 0 global vec | 3 global scalars
-        self.num_vec = 4
-        self.num_scalar = wemb.shape[1] - self.num_vec
+        stack = lambda name: np.stack([sd[name.format(l=l)] for l in range(L)])  # noqa: E731
+        lay = lambda name: stack(f"interaction_layers.{{l}}.{name}")  # noqa: E731
         f32 = lambda a: torch.as_tensor(np.ascontiguousarray(a), dtype=torch.float32).to(self.device)  # noqa: E731
-        self.t: Dict[str, torch.Tensor] = dict(
-            ori=f32(ori), w_embed_t=f32(wemb.T), w1m_t=f32(w1m_t), w2_t=f32(sd["basis_fn.3.weight"].T),
-            b2=f32(sd["basis_fn.3.bias"]), wk_t=f32(wk.transpose(2, 0, 1).reshape(BASIS, L * HIDDEN)),
-            conv_bias=f32(lay("conv.bias")), ln_w=f32(lay("norm.weight")), ln_b=f32(lay("norm.bias")),
-            mlp_w1_t=f32(lay("linear_1.weight").transpose(0, 2, 1)), mlp_b1=f32(lay("linear_1.bias")),
-            mlp_w2_t=f32(lay("linear_2.weight").transpose(0, 2, 1)), mlp_b2=f32(lay("linear_2.bias")),
-            layer_scale=f32(lay("layer_scale")), wr_t=f32(wr.transpose(0, 2, 1)), br=f32(br),
-            fiber_kernel=torch.empty(L, NUM_ORI, NUM_ORI, HIDDEN, dtype=torch.float32, device=self.device))
-        # K3': input-independent fiber kernels, evaluated once on the device
-        fw1, fb1 = f32(sd["fiber_basis_fn.1.weight"]), f32(sd["fiber_basis_fn.1.bias"])
-        fw2, fb2 = f32(sd["fiber_basis_fn.3.weight"]), f32(sd["fiber_basis_fn.3.bias"])
-        fwf = f32(lay("conv.fiber_kernel.weight"))
-        if fw1.shape != (HIDDEN, 3):
-            raise ValueError("unsupported fiber basis input width")
+        self._fp32_layouts(lambda name: f32(stack(name) if "{l}" in name else sd[name]), f32(w1m_t), f32(ori))
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        _lib.call("arreau_fiber_kernel_precompute", self.t["ori"].data_ptr(), fw1.data_ptr(), fb1.data_ptr(),
-                  fw2.data_ptr(), fb2.data_ptr(), fwf.data_ptr(), self.t["fiber_kernel"].data_ptr(), stream)
         if with_f16:   # fp16 mma fragments of the fiber kernels for the tensor-core fiber conv
             self.t["fiber_frag"] = torch.empty(L * HIDDEN * 32 * 4, dtype=torch.int32, device=self.device)
             _lib.call("arreau_fiber_frag_pack", self.t["fiber_kernel"].data_ptr(), L, self.t["fiber_frag"].data_ptr(), stream)
@@ -150,6 +131,7 @@ class PonitaWeights:
             w2 = 0.5 * np.asarray(sd["basis_fn.3.weight"])                 # [D, C]
             chunks = [umma_tile_image(w2[nh * 128:(nh + 1) * 128, ks * 64:(ks + 1) * 64])
                       for nh in range(2) for ks in range(2)]
+            wk = lay("conv.kernel.weight")                                 # [L,C,D]
             chunks += [umma_tile_image(0.5 * wk[l][:, ks * 64:(ks + 1) * 64]) for l in range(L) for ks in range(4)]
             m1, m2 = lay("linear_1.weight"), 0.5 * lay("linear_2.weight")  # [L,4C,C], [L,C,4C]
             mlp = []
@@ -159,58 +141,9 @@ class PonitaWeights:
                 mlp += [g1[0], g1[1], g2[0], g1[2], g2[1], g1[3], g2[2], g2[3]]   # MMA issue order
             self.t.update(edge_w1_img=umma_tile_image(w1pad).to(self.device),
                           edge_w_img=torch.cat(chunks).to(self.device), mlp_w_img=torch.cat(mlp).to(self.device))
-            rv, rb = pooled_readout_weights(wr, br, ori)
+            rv, rb = pooled_readout_weights(stack("read_out_layers.{l}.weight"), stack("read_out_layers.{l}.bias"), ori)
             self.t.update(readout_v=f32(rv), readout_bias=f32(rb))
-        self.c = _lib.Weights()
-        for name, _ in _lib.Weights._fields_:
-            if name in self.t:
-                setattr(self.c, name, self.t[name].data_ptr())
-        self.c.num_scalar, self.c.num_vec, self.c.num_states = self.num_scalar, self.num_vec, self.num_states
-
-    @classmethod
-    def from_device_params(cls, sd: Mapping[str, torch.Tensor], ori_grid: torch.Tensor) -> "PonitaWeights":
-        """Kernel layouts of the fp32 path from fp32 DEVICE tensors keyed like the reference state_dict, with device
-        ops only (no host round trip): the training step re-packs its flat parameter buffer with this every step.
-        (Transposes / stacking are layout plumbing; the fiber kernels are evaluated by
-        arreau_fiber_kernel_precompute.)"""
-        self = cls.__new__(cls)
-        dev = sd["basis_fn.1.weight"].device
-        self.device = dev
-        L = LAYERS
-        f = lambda a: a.to(torch.float32).contiguous()  # noqa: E731
-        w1, b1 = f(sd["basis_fn.1.weight"]), f(sd["basis_fn.1.bias"])
-        fold = torch.as_tensor(monomial_fold_table(), dtype=torch.int32).to(dev)
-        w1m_t = torch.empty(MONO_PAD, HIDDEN, dtype=torch.float32, device=dev)
-        _lib.call("arreau_fold_basis_w1", w1.data_ptr(), b1.data_ptr(), fold.data_ptr(), w1m_t.data_ptr(),
-                  torch.cuda.current_stream(dev).cuda_stream)      # fixed summation order (no atomics)
-        lay = lambda name: torch.stack([sd[f"interaction_layers.{l}.{name}"] for l in range(L)])  # noqa: E731
-        wk = lay("conv.kernel.weight")
-        wemb = sd["x_embedder.weight"]
-        wr = torch.stack([sd[f"read_out_layers.{l}.weight"] for l in range(L)])
-        br = torch.stack([sd[f"read_out_layers.{l}.bias"] for l in range(L)])
-        self.num_readout = wr.shape[1]
-        self.num_states = self.num_readout - 4
-        self.num_vec = 4
-        self.num_scalar = wemb.shape[1] - self.num_vec
-        self.t = dict(
-            ori=f(ori_grid.to(dev)), w_embed_t=f(wemb.T), w1m_t=w1m_t, w2_t=f(sd["basis_fn.3.weight"].T),
-            b2=f(sd["basis_fn.3.bias"]), wk_t=f(wk.permute(2, 0, 1).reshape(BASIS, L * HIDDEN)),
-            conv_bias=f(lay("conv.bias")), ln_w=f(lay("norm.weight")), ln_b=f(lay("norm.bias")),
-            mlp_w1_t=f(lay("linear_1.weight").transpose(1, 2)), mlp_b1=f(lay("linear_1.bias")),
-            mlp_w2_t=f(lay("linear_2.weight").transpose(1, 2)), mlp_b2=f(lay("linear_2.bias")),
-            layer_scale=f(lay("layer_scale")), wr_t=f(wr.transpose(1, 2)), br=f(br),
-            fiber_kernel=torch.empty(L, NUM_ORI, NUM_ORI, HIDDEN, dtype=torch.float32, device=dev))
-        keep = [f(sd["fiber_basis_fn.1.weight"]), f(sd["fiber_basis_fn.1.bias"]), f(sd["fiber_basis_fn.3.weight"]),
-                f(sd["fiber_basis_fn.3.bias"]), f(lay("conv.fiber_kernel.weight"))]
-        _lib.call("arreau_fiber_kernel_precompute", self.t["ori"].data_ptr(), *[k.data_ptr() for k in keep],
-                  self.t["fiber_kernel"].data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
-        self._keep = keep + [w1, b1, fold]   # stay alive until the stream has consumed them
-        self.c = _lib.Weights()
-        for name, _ in _lib.Weights._fields_:
-            if name in self.t:
-                setattr(self.c, name, self.t[name].data_ptr())
-        self.c.num_scalar, self.c.num_vec, self.c.num_states = self.num_scalar, self.num_vec, self.num_states
-        return self
+        self._fill_struct()
 
     @classmethod
     def from_flat(cls, flat, ori_grid: torch.Tensor) -> "PonitaWeights":
@@ -218,47 +151,60 @@ class PonitaWeights:
         FlatParams, arreau_train_layout_t order): tensors whose kernel layout equals the reference's own layout are
         VIEWS of the flat buffer (no copy, so they are current after every optimizer step by construction), the six
         transposed matrices are one strided copy each, plus the monomial fold and the fiber-kernel precompute --
-        ~10 launches per step instead of the ~60 small stack / transpose kernels of from_device_params."""
+        ~10 launches per step."""
         self = cls.__new__(cls)
         dev = flat.data.device
         self.device = dev
-        L, lay, buf = LAYERS, flat.layout, flat.data
-        R, FV = flat.num_states + 4, flat.num_scalar + flat.num_vec
 
-        def view(off, *shape):
-            n = int(np.prod(shape))
-            return buf[off:off + n].view(*shape)
+        def get(name):
+            off, shape = flat.specs[name.format(l=0)]
+            if "{l}" in name:      # the flat layout keeps a tensor's layers consecutive: one [L, ...] view
+                shape = (LAYERS,) + shape
+            return flat.data[off:off + math.prod(shape)].view(*shape)
 
-        w1, b1 = view(lay.basis_w1, HIDDEN, 258), view(lay.basis_b1, HIDDEN)
         fold = getattr(flat, "_fold_table", None)
         if fold is None:
             fold = flat._fold_table = torch.as_tensor(monomial_fold_table(), dtype=torch.int32).to(dev)
         w1m_t = torch.empty(MONO_PAD, HIDDEN, dtype=torch.float32, device=dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.call("arreau_fold_basis_w1", w1.data_ptr(), b1.data_ptr(), fold.data_ptr(), w1m_t.data_ptr(), stream)
-        self.num_readout, self.num_states, self.num_vec, self.num_scalar = R, flat.num_states, flat.num_vec, flat.num_scalar
-        wk = view(lay.conv_kernel_w, L, HIDDEN, BASIS)
-        self.t = dict(
-            ori=ori_grid.to(dev, torch.float32).contiguous(), w_embed_t=view(lay.embed_w, HIDDEN, FV).t().contiguous(),
-            w1m_t=w1m_t, w2_t=view(lay.basis_w2, BASIS, HIDDEN).t().contiguous(), b2=view(lay.basis_b2, BASIS),
-            wk_t=wk.permute(2, 0, 1).reshape(BASIS, L * HIDDEN).contiguous(),
-            conv_bias=view(lay.conv_bias, L, HIDDEN), ln_w=view(lay.norm_w, L, HIDDEN), ln_b=view(lay.norm_b, L, HIDDEN),
-            mlp_w1_t=view(lay.lin1_w, L, WIDEN * HIDDEN, HIDDEN).transpose(1, 2).contiguous(),
-            mlp_b1=view(lay.lin1_b, L, WIDEN * HIDDEN),
-            mlp_w2_t=view(lay.lin2_w, L, HIDDEN, WIDEN * HIDDEN).transpose(1, 2).contiguous(),
-            mlp_b2=view(lay.lin2_b, L, HIDDEN), layer_scale=view(lay.layer_scale, L, HIDDEN),
-            wr_t=view(lay.readout_w, L, R, HIDDEN).transpose(1, 2).contiguous(), br=view(lay.readout_b, L, R),
-            fiber_kernel=torch.empty(L, NUM_ORI, NUM_ORI, HIDDEN, dtype=torch.float32, device=dev))
-        keep = [view(lay.fiber_w1, HIDDEN, 3), view(lay.fiber_b1, HIDDEN), view(lay.fiber_w2, BASIS, HIDDEN),
-                view(lay.fiber_b2, BASIS), view(lay.conv_fiber_w, L, HIDDEN, BASIS)]
-        _lib.call("arreau_fiber_kernel_precompute", self.t["ori"].data_ptr(), *[k.data_ptr() for k in keep],
-                  self.t["fiber_kernel"].data_ptr(), stream)
+        _lib.call("arreau_fold_basis_w1", get("basis_fn.1.weight").data_ptr(), get("basis_fn.1.bias").data_ptr(),
+                  fold.data_ptr(), w1m_t.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        self._fp32_layouts(get, w1m_t, ori_grid.to(dev, torch.float32).contiguous())
+        self._fill_struct()
+        return self
+
+    def _fp32_layouts(self, get, w1m_t: torch.Tensor, ori: torch.Tensor) -> None:
+        """`self.t`: the fp32 kernel layouts, and the fiber kernels evaluated on the device.  get(name) returns a
+        parameter under its reference name as an fp32 device tensor; a name with "{l}" stands for that tensor of every
+        interaction or read-out layer, stacked [L, ...].  w1m_t: basis_fn.1 folded onto the distinct monomials
+        [MONO_PAD, HIDDEN], the bias in row NUM_MONO."""
+        L = LAYERS
+        lay = lambda name: get(f"interaction_layers.{{l}}.{name}")  # noqa: E731
+        wemb, wr = get("x_embedder.weight"), get("read_out_layers.{l}.weight")   # [C, F+V], [L,R,C]
+        self.num_readout = wr.shape[1]
+        self.num_states = self.num_readout - 4             # scalars | 1 vector | 0 global vec | 3 global scalars
+        self.num_vec = 4
+        self.num_scalar = wemb.shape[1] - self.num_vec
+        self.t: Dict[str, torch.Tensor] = dict(
+            ori=ori, w_embed_t=wemb.t().contiguous(), w1m_t=w1m_t, w2_t=get("basis_fn.3.weight").t().contiguous(),
+            b2=get("basis_fn.3.bias"),
+            wk_t=lay("conv.kernel.weight").permute(2, 0, 1).reshape(BASIS, L * HIDDEN).contiguous(),
+            conv_bias=lay("conv.bias"), ln_w=lay("norm.weight"), ln_b=lay("norm.bias"),
+            mlp_w1_t=lay("linear_1.weight").transpose(1, 2).contiguous(), mlp_b1=lay("linear_1.bias"),
+            mlp_w2_t=lay("linear_2.weight").transpose(1, 2).contiguous(), mlp_b2=lay("linear_2.bias"),
+            layer_scale=lay("layer_scale"), wr_t=wr.transpose(1, 2).contiguous(), br=get("read_out_layers.{l}.bias"),
+            fiber_kernel=torch.empty(L, NUM_ORI, NUM_ORI, HIDDEN, dtype=torch.float32, device=self.device))
+        # K3': input-independent fiber kernels, evaluated once on the device
+        fiber = [get("fiber_basis_fn.1.weight"), get("fiber_basis_fn.1.bias"), get("fiber_basis_fn.3.weight"),
+                 get("fiber_basis_fn.3.bias"), lay("conv.fiber_kernel.weight")]
+        _lib.call("arreau_fiber_kernel_precompute", ori.data_ptr(), *[f.data_ptr() for f in fiber],
+                  self.t["fiber_kernel"].data_ptr(), torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _fill_struct(self) -> None:
         self.c = _lib.Weights()
         for name, _ in _lib.Weights._fields_:
             if name in self.t:
                 setattr(self.c, name, self.t[name].data_ptr())
         self.c.num_scalar, self.c.num_vec, self.c.num_states = self.num_scalar, self.num_vec, self.num_states
-        return self
 
     def ref(self):
         return C.byref(self.c)

@@ -106,7 +106,8 @@ def _eval_worker(rank, world, port, tmp_path, out):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
         from arreau_b200.evaluation import evaluate_dataset
-        res = evaluate_dataset(_fake_model(), _split(tmp_path), 4, "cpu", seed=1, gpu_batch=3)
+        # each rank writes its own copy of the dataset: a shared file could be read while the other rank rewrites it
+        res = evaluate_dataset(_fake_model(), _split(tmp_path / f"rank{rank}"), 4, "cpu", seed=1, gpu_batch=3)
         np.savez(os.path.join(out, f"e{rank}.npz"), terms=res["terms"], t=res["t"], loss=res["loss"], vb=res["vb"])
     finally:
         dist.destroy_process_group()

@@ -105,6 +105,31 @@ def test_sgemm_tf32_stays_in_bounds_and_is_deterministic(device, M, N, K, ak, bk
     assert rel_err(outs[0].cpu().numpy(), ref.cpu().numpy()) < 2e-3
 
 
+def test_flat_weight_layouts_match_state_dict_layouts(device, weights_npz):
+    """The training engine's kernel layouts (PonitaWeights.from_flat) against the sampling engine's (PonitaWeights of the
+    state_dict) for the same weights: bit-identical, except the folded first basis layer w1m_t, which the host folds in
+    fp64 and from_flat in fp32 on the device.  A monomial gathers at most 6 columns of basis_fn.1.weight, so the fp32
+    sum is within 5 * 2^-24 of the sum of the folded terms' magnitudes."""
+    from arreau_b200.training import FlatParams
+    from arreau_b200.weights import HIDDEN, MONO_PAD, NUM_MONO, PonitaWeights, monomial_fold_table
+    sd = {k: weights_npz[k] for k in weights_npz.files if k not in ("ori_grid", "fourier_w")}
+    p = FlatParams(164, 4, Z, device)
+    p.load_state_dict(sd)
+    host = PonitaWeights(sd, weights_npz["ori_grid"], device=device)
+    flat = PonitaWeights.from_flat(p, torch.as_tensor(weights_npz["ori_grid"]).to(device))
+    assert set(flat.t) <= set(host.t) and len(flat.t) == 17
+    assert (flat.num_scalar, flat.num_vec, flat.num_states) == (host.num_scalar, host.num_vec, host.num_states)
+    for k in flat.t:
+        if k != "w1m_t":
+            assert flat.t[k].dtype == host.t[k].dtype and torch.equal(flat.t[k], host.t[k]), k
+    mag = np.zeros((HIDDEN, NUM_MONO))
+    np.add.at(mag, (slice(None), monomial_fold_table()), np.abs(sd["basis_fn.1.weight"].astype(np.float64)))
+    bound = np.zeros((MONO_PAD, HIDDEN))
+    bound[:NUM_MONO] = 5 * 2.0 ** -24 * mag.T           # the bias row and the padding must be equal
+    err = np.abs(flat.t["w1m_t"].double().cpu().numpy() - host.t["w1m_t"].double().cpu().numpy())
+    assert np.all(err <= bound), float((err - bound).max())
+
+
 @pytest.mark.parametrize("case", [0, 1])
 def test_noising_matches_reference(device, gold, weights_npz, case):
     c = _case(gold("train_c5small.npz"), case)
