@@ -149,25 +149,52 @@ __global__ void ve_pbc_reverse_kernel(const double* frac, const float* __restric
 }
 
 // diffusion/d3pm.py:74-110,198-215 for the mask-absorbing chain; one warp per atom.
+//
+// kAllowed: the states an atom may take are restricted to its crystal's set A, bit d of allowed[4 g + d / 32] for
+// state d of crystal g = crystal_of_atom[b] (bits at d >= Z are ignored; a set with no bit below Z counts as every
+// state, so no input leaves an atom without a candidate).  For that atom:
+//   1. the x0 probabilities are the softmax of the logits over A: a state outside A has probability 0 (this is what
+//      sum_nomask, p_mask and f2 see);
+//   2. the argmax runs over A plus the mask state Z-1 at t >= 2 (the mask absorbs: a masked atom may stay masked), and
+//      over A alone at t == 1.  The exclusion is explicit: a state outside A still has the finite posterior
+//      log(f1 + eps) + log(0 + eps), which the Gumbel noise could lift above the others;
+//   3. with every state in A the result is bit-identical to the unconstrained kernel (the arithmetic is the same).
+// The unconstrained instantiation compiles to the code it had before the constraint existed.
+template <bool kAllowed>
 __global__ void __launch_bounds__(256)
 d3pm_reverse_kernel(const int64_t* types, const float* __restrict__ logits,
                     const double* __restrict__ u, const int32_t* __restrict__ t_of_atom, int t_scalar,
                     const double* __restrict__ q_keep, const double* __restrict__ q_to_mask,
                     double onestep_keep, double onestep_to_mask, int T, int N, int Z,
-                    int64_t* out) {   // out may alias types
+                    int64_t* out,   // out may alias types
+                    const int32_t* __restrict__ crystal_of_atom, const uint32_t* __restrict__ allowed) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= N) return;
   const int b = warp;
   const int t = t_of_atom ? t_of_atom[b] : t_scalar;
   const int xt = (int)types[b];
   const int mask = Z - 1;
-  constexpr int kPer = 4;   // Z <= 128
+  constexpr int kPer = 4;   // Z <= 128: lane's state d = lane + 32 r is bit `lane` of the crystal's mask word r
+  uint32_t in_set = 0xfu;   // bit r: state lane + 32 r is in A
+  if constexpr (kAllowed) {
+    const uint32_t* w = allowed + (size_t)kPer * crystal_of_atom[b];
+    uint32_t any = 0, mine = 0;
+#pragma unroll
+    for (int r = 0; r < kPer; ++r) {
+      const int lo = 32 * r;   // keep the bits of states d < Z only
+      const uint32_t valid = Z - lo >= 32 ? 0xffffffffu : (Z - lo <= 0 ? 0u : (1u << (Z - lo)) - 1u);
+      const uint32_t word = w[r];
+      any |= word & valid;
+      mine |= ((word >> lane) & 1u) << r;
+    }
+    if (any) in_set = mine;
+  }
   double lg[kPer], p[kPer];
   double mx = -INFINITY;
 #pragma unroll
   for (int r = 0; r < kPer; ++r) {
     const int d = lane + 32 * r;
-    lg[r] = d < Z ? (double)logits[(size_t)b * Z + d] : -INFINITY;
+    lg[r] = (d < Z && ((in_set >> r) & 1u)) ? (double)logits[(size_t)b * Z + d] : -INFINITY;
     mx = fmax(mx, lg[r]);
   }
   mx = warp_max(mx);
@@ -210,6 +237,7 @@ d3pm_reverse_kernel(const int64_t* types, const float* __restrict__ logits,
   for (int r = 0; r < kPer; ++r) {
     const int d = lane + 32 * r;
     if (d >= Z) continue;
+    if (kAllowed && !((in_set >> r) & 1u) && (t == 1 || d != mask)) continue;   // rule 2
     double lp;
     if (t == 1) {
       lp = lg[r];
@@ -326,17 +354,45 @@ extern "C" int arreau_ve_pbc_reverse(const double* frac, const float* score, con
   return ARREAU_OK;
 }
 
-extern "C" int arreau_d3pm_reverse(const int64_t* types, const float* logits, const double* u,
-                                   const int32_t* t_of_atom, int32_t t, const double* q_keep,
-                                   const double* q_to_mask, double onestep_keep, double onestep_to_mask,
-                                   int32_t num_steps, int32_t N, int32_t Z, int64_t* types_out, void* stream) {
+namespace {
+
+int launch_d3pm_reverse(const int64_t* types, const float* logits, const double* u, const int32_t* t_of_atom, int32_t t,
+                        const double* q_keep, const double* q_to_mask, double onestep_keep, double onestep_to_mask,
+                        int32_t num_steps, int32_t N, int32_t Z, const int32_t* crystal_of_atom, const uint32_t* allowed,
+                        int64_t* types_out, void* stream) {
   if (N == 0) return ARREAU_OK;
   if (!types || !logits || !u || !q_keep || !q_to_mask || !types_out) return ARREAU_ERR_NULL;
   if (N < 0 || Z <= 1 || Z > 128 || num_steps <= 0) return ARREAU_ERR_BAD_SHAPE;
   const long long threads = (long long)N * 32;
-  d3pm_reverse_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps, N, Z,
-      types_out);
+  const unsigned blocks = (unsigned)((threads + 255) / 256);
+  if (allowed)
+    d3pm_reverse_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+        types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps, N, Z, types_out,
+        crystal_of_atom, allowed);
+  else
+    d3pm_reverse_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+        types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps, N, Z, types_out,
+        nullptr, nullptr);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
+}
+
+}  // namespace
+
+extern "C" int arreau_d3pm_reverse(const int64_t* types, const float* logits, const double* u,
+                                   const int32_t* t_of_atom, int32_t t, const double* q_keep,
+                                   const double* q_to_mask, double onestep_keep, double onestep_to_mask,
+                                   int32_t num_steps, int32_t N, int32_t Z, int64_t* types_out, void* stream) {
+  return launch_d3pm_reverse(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask,
+                             num_steps, N, Z, nullptr, nullptr, types_out, stream);
+}
+
+extern "C" int arreau_d3pm_reverse_allowed(const int64_t* types, const float* logits, const double* u,
+                                           const int32_t* t_of_atom, int32_t t, const double* q_keep,
+                                           const double* q_to_mask, double onestep_keep, double onestep_to_mask,
+                                           int32_t num_steps, int32_t N, int32_t Z, const int32_t* crystal_of_atom,
+                                           const uint32_t* allowed, int64_t* types_out, void* stream) {
+  if (N != 0 && (!crystal_of_atom || !allowed)) return ARREAU_ERR_NULL;
+  return launch_d3pm_reverse(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask,
+                             num_steps, N, Z, crystal_of_atom, allowed, types_out, stream);
 }

@@ -390,7 +390,11 @@ int denoise_step_body(const arreau_weights* w, const arreau_workspace* ws, const
                                          a->vp_denom, a->vp_var, G, a->lengths, stream));
   ARREAU_TRY(lattice_from_angles(a, G, stream));
   ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, t_of_atom, t, a->ve_sigmas, N, a->frac, stream));
-  if (a->update_types)
+  if (a->update_types && a->allowed_states)
+    ARREAU_TRY(arreau_d3pm_reverse_allowed(a->types, a->logits, a->u_type, t_of_atom, t, a->q_keep, a->q_to_mask,
+                                           a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->crystal_of_atom,
+                                           a->allowed_states, a->types, stream));
+  else if (a->update_types)
     ARREAU_TRY(arreau_d3pm_reverse(a->types, a->logits, a->u_type, t_of_atom, t, a->q_keep, a->q_to_mask,
                                    a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->types, stream));
   return ARREAU_OK;

@@ -15,7 +15,7 @@ import torch
 import torch.nn.functional as F
 
 from .. import _lib
-from ..engine import DenoiseEngine
+from ..engine import DenoiseEngine, allowed_state_words
 from ..tables import POS_SIGMA_MAX, POS_SIGMA_MIN, build_tables
 from .d3pm import D3PM
 from .diffusion_helpers import VE_pbc, VP_lattice
@@ -255,7 +255,7 @@ class DiffusionLoss(torch.nn.Module):
                vis_name: str = "", visualization_setting=None, show_bonds: bool = False,
                constant_atoms: Optional[torch.Tensor] = None, num_atoms: Optional[torch.Tensor] = None,
                device="cuda", device_noise: bool = False, seed: int = 0, step_callback=None,
-               cuda_graph: bool = False, crystal_ids=None) -> SampleResult:
+               cuda_graph: bool = False, crystal_ids=None, allowed_states=None) -> SampleResult:
         """diffusion/diffusion_loss.py:277-377.  Extra keyword-only options (defaults reproduce the reference):
         `num_atoms` a per-crystal atom-count vector, `device_noise` Philox noise generated on the GPU,
         `step_callback(timestep, engine)` called after each step (e.g. to log E/N), `cuda_graph` (needs device_noise or
@@ -264,9 +264,16 @@ class DiffusionLoss(torch.nn.Module):
         `crystal_ids` (G integers): the initial state and every step's noise are drawn on the device per crystal, keyed
         by (seed, id) (arreau_sample_init_keyed / arreau_sample_noise_keyed), so a crystal's trajectory depends on the
         weights, the precision, the seed, its id and its atom count only -- not on the batch it is sampled in.  The
-        host generators (numpy, torch) are not touched; device_noise is implied."""
+        host generators (numpy, torch) are not touched; device_noise is implied.
+        `allowed_states` (bool [G,Z], or [Z] for every crystal): the states each crystal's atoms may take -- the type
+        update samples from the model's x0 prediction restricted to them (arreau_d3pm_reverse_allowed); leave the mask
+        state Z-1 out and every atom ends on an allowed element.  It cannot be combined with constant_atoms."""
         Z = len(z_table)
         G = num_samples_in_batch
+        if allowed_states is not None:         # checked before any device work
+            if constant_atoms is not None:
+                raise ValueError("allowed_states restricts the type update, which constant_atoms switches off")
+            allowed_state_words(allowed_states, G, Z)
         dd = torch.float64                                     # main_diffusion_generate.py:27
         keyed = crystal_ids is not None
         if keyed:
@@ -282,6 +289,7 @@ class DiffusionLoss(torch.nn.Module):
             frac_x = torch.randn([N, 3], dtype=dd) * pos_sigma_max
         atom_types = constant_atoms if constant_atoms is not None else torch.full((N,), Z - 1)
         eng = self.engine_for(model, t_emb_weights, na, torch.device(device))
+        eng.set_allowed_states(allowed_states)
         if keyed:
             eng.set_crystal_ids(crystal_ids)
             eng.init_state_keyed(seed, atom_types, pos_sigma_max)

@@ -33,6 +33,25 @@ def angle_factors(angles: torch.Tensor) -> torch.Tensor:
     return torch.stack([sin_b, cos_b, sin_a, torch.cos(gs), torch.sin(gs), cos_a], dim=1)
 
 
+def allowed_state_words(mask, G: int, Z: int) -> np.ndarray:
+    """A per-crystal allowed-state mask -- bool [G,Z], or [Z] for every crystal -- checked and packed into the [G,4]
+    uint32 words of arreau_d3pm_reverse_allowed (bit d of word d // 32 admits state d).  Raises ValueError on another
+    shape or dtype, or when a crystal admits no state other than the mask state Z-1 (it would end with no element)."""
+    m = np.asarray(mask.cpu() if isinstance(mask, torch.Tensor) else mask)
+    if m.dtype != np.bool_:
+        raise ValueError(f"allowed states must be a bool mask, got dtype {m.dtype}")
+    if m.ndim == 1 and m.shape[0] == Z:
+        m = np.broadcast_to(m, (G, Z))
+    if m.shape != (G, Z):
+        raise ValueError(f"allowed states must be a bool mask of shape [{Z}] or [{G}, {Z}], got {list(m.shape)}")
+    empty = np.flatnonzero(~m[:, :Z - 1].any(axis=1))
+    if empty.size:
+        raise ValueError(f"crystal {int(empty[0])} allows no element ({empty.size} such crystals)")
+    bits = np.zeros((G, 128), dtype=np.bool_)
+    bits[:, :Z] = m
+    return np.packbits(bits.reshape(G, 4, 32), axis=-1, bitorder="little").view("<u4").reshape(G, 4)
+
+
 def _i32(a, device):
     return torch.as_tensor(np.asarray(a), dtype=torch.int32).to(device)
 
@@ -52,7 +71,7 @@ class DenoiseEngine:
     _CRYSTAL_BUFS = {"lengths": ((3,), torch.float64), "angles": ((3,), torch.float64), "lattice": ((3, 3), torch.float64),
                      "angle_trig": ((6,), torch.float64), "num_neighbors_image": ((), torch.int64),
                      "len0": ((3,), torch.float32), "z_len": ((3,), torch.float64), "num_atoms": ((), torch.int64),
-                     "crystal_id": ((), torch.int64)}
+                     "crystal_id": ((), torch.int64), "allowed_states": ((4,), torch.int32)}
 
     def __init__(self, weights: PonitaWeights, tables: DiffusionTables, fourier_w, num_atoms: Sequence[int],
                  radius: float, max_neighbors: int, precision: str = "fp32", edge_capacity: Optional[int] = None,
@@ -109,6 +128,7 @@ class DenoiseEngine:
             raise ValueError(f"time embedding has {self.d_fourier_w.numel()} frequencies, the model expects {self.emb}")
         self.edge_capacity = -1
         self.G = self.N = 0
+        self.constrained = False        # args.allowed_states points at the allowed_states buffer
         self._debug_flat = None
         self._alloc_edges(int(edge_capacity) if edge_capacity is not None else
                           (Nc * self.cap if self.cap > 0 else max(1, 32 * Nc)))
@@ -157,6 +177,7 @@ class DenoiseEngine:
         self.args.num_atoms_total, self.args.num_crystals = N, G
         a, p = self.args, _lib.ptr
         a.z_len, a.z_frac, a.u_type = p(self.z_len), p(self.z_frac), p(self.u_type)
+        self.set_allowed_states(None)     # a constraint belongs to the batch it was set for
 
     # ------------------------------------------------------------------ buffers
     def _alloc_edges(self, capacity: int) -> None:
@@ -208,6 +229,7 @@ class DenoiseEngine:
         a.onestep_keep, a.onestep_to_mask = self.tabs.onestep_keep, self.tabs.onestep_to_mask
         a.emb, a.num_steps, a.cap, a.radius = self.emb, self.tabs.T, self.cap, self.radius
         a.precision, a.update_types = PRECISIONS[self.precision], 1
+        a.allowed_states = p("allowed_states") if self.constrained else None
         self.args = a
         if self.N:                      # re-allocation of a bound engine (uncapped graphs): keep the topology's views
             self.ws.pool = _lib.ptr(self.pool)
@@ -306,6 +328,22 @@ class DenoiseEngine:
         _lib.call("arreau_sample_noise_keyed", C.c_uint64(int(seed)), int(step), self.G, self.N, self.Z,
                   self.crystal_id.data_ptr(), self.atom_offset.data_ptr(), self.crystal_of_atom.data_ptr(),
                   self.z_len.data_ptr(), self.z_frac.data_ptr(), self.u_type.data_ptr(), self.stream)
+
+    # ------------------------------------------------------------------ chemical-system constraint
+    def set_allowed_states(self, mask) -> None:
+        """Restrict the states the type update may choose, per crystal of the bound batch: bool [G,Z], or [Z] for every
+        crystal (checked by allowed_state_words), or None for no constraint.  The mask is packed into the engine's
+        [G_cap,4] uint32 buffer, allocated once, and every later step -- arreau_denoise_step and the replayed trajectory
+        -- reads it there (arreau_d3pm_reverse_allowed); a trajectory graph bakes in whether the step is constrained, so
+        bind the mask before capture_trajectory_graph.  set_topology clears it."""
+        if mask is None:
+            self.constrained = False
+            self.args.allowed_states = None
+            return
+        words = torch.from_numpy(allowed_state_words(mask, self.G, self.Z).view(np.int32))
+        self.allowed_states.copy_(words.pin_memory() if self.device.type == "cuda" else words, non_blocking=True)
+        self.constrained = True
+        self.args.allowed_states = self.allowed_states.data_ptr()
 
     # ------------------------------------------------------------------ graph
     def _count(self) -> None:

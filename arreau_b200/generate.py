@@ -3,6 +3,8 @@
     python -m arreau_b200.generate --model_path model.ckpt --num_crystals 1024 --num_atoms 40 [--batch 1024]
     python -m arreau_b200.generate --model_path model.ckpt --num_crystals 1024 --num_atoms_from data/train.h5
     python -m arreau_b200.generate ... --keyed_noise      # the same crystals whatever --batch and the number of GPUs
+    python -m arreau_b200.generate ... --elements Li Fe P O     # only these elements (with --num_atoms[_from])
+    python -m arreau_b200.generate ... --compositions_from data/test.h5   # structures for the data's compositions
     torchrun --nproc-per-node 8 -m arreau_b200.generate ...      # crystals sharded over the GPUs, one gather at the end
 
 The reference samples 10 crystals per batch on the CPU; here a batch is as large as fits (1024 by default), every
@@ -30,20 +32,38 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
                         use_constant_atomic_symbols: Optional[list] = None, num_crystals_per_batch: int = 1024,
                         device="cuda", device_noise: bool = True, seed: int = 0, out_path: Optional[str] = None,
                         group=None, timings: Optional[dict] = None, num_atoms=None,
-                        keyed_noise: bool = False) -> SampleResult:
+                        keyed_noise: bool = False, elements=None, compositions=None) -> SampleResult:
     """main_diffusion_generate.py:52-94.  With torch.distributed initialised the crystals are sharded over the ranks;
     every rank returns the full gathered result and rank 0 writes `out_path`.  `timings` (optional dict) receives this
     rank's wall-clock seconds per phase: `sample` (list, one per batch), `gather`, `write`.  `num_atoms` (optional,
     length num_crystals) gives every crystal its own atom count instead of `num_atoms_per_sample`; each rank samples
     its shard of it (see `draw_num_atoms`).  `keyed_noise`: crystal i of the run gets id i and every draw of its
     trajectory is keyed by (seed, i) on the device (DiffusionLoss.sample's crystal_ids), so the result does not depend
-    on num_crystals_per_batch or on the number of ranks.  Without it, batch b0.. is sampled with seed + b0."""
-    if num_atoms is not None:
+    on num_crystals_per_batch or on the number of ranks.  Without it, batch b0.. is sampled with seed + b0.
+    `elements`: one chemical system (element symbols) for every crystal, or a list of num_crystals systems, sharded
+    like `num_atoms`; every atom of a crystal ends on an element of its system (PONITA_DIFFUSION.sample's `elements`).
+    `compositions`: num_crystals arrays of atomic numbers; each fixes its crystal's atom count and types (crystal
+    structure prediction), so it excludes num_atoms, use_constant_atomic_symbols and elements."""
+    if compositions is not None:
+        if num_atoms is not None or use_constant_atomic_symbols is not None or elements is not None:
+            raise ValueError("compositions fix atom counts and types: they cannot be combined with num_atoms, "
+                             "use_constant_atomic_symbols or elements")
+        compositions = [np.asarray(c, dtype=np.int64).reshape(-1) for c in compositions]
+        if len(compositions) != num_crystals:
+            raise ValueError(f"compositions must hold {num_crystals} crystals, got {len(compositions)}")
+        num_atoms = np.asarray([c.size for c in compositions], dtype=np.int64)
+    elif num_atoms is not None:
         num_atoms = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
         if num_atoms.shape[0] != num_crystals or np.any(num_atoms < 1):
             raise ValueError(f"num_atoms must hold {num_crystals} positive counts, got {num_atoms.shape[0]}")
         if use_constant_atomic_symbols is not None:
             raise ValueError("constant atomic symbols fix the atom count: they cannot be combined with num_atoms")
+    per_crystal_elements = elements is not None and not all(isinstance(e, str) for e in elements)
+    if elements is not None:
+        if use_constant_atomic_symbols is not None:
+            raise ValueError("constant atomic symbols fix the types: they cannot be combined with elements")
+        if per_crystal_elements and len(elements) != num_crystals:
+            raise ValueError(f"elements must hold one system or {num_crystals} systems, got {len(elements)}")
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     lo, hi = shard_range(num_crystals, rank, world)
@@ -51,7 +71,12 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
     t_batches = []
     for b0 in range(lo, hi, num_crystals_per_batch):
         nb = min(num_crystals_per_batch, hi - b0)
-        kw = {} if num_atoms is None else {"num_atoms": torch.from_numpy(num_atoms[b0:b0 + nb].copy())}
+        if compositions is not None:
+            kw = {"compositions": compositions[b0:b0 + nb]}
+        else:
+            kw = {} if num_atoms is None else {"num_atoms": torch.from_numpy(num_atoms[b0:b0 + nb].copy())}
+        if elements is not None:
+            kw["elements"] = elements[b0:b0 + nb] if per_crystal_elements else elements
         if keyed_noise:
             kw["crystal_ids"] = torch.arange(b0, b0 + nb, dtype=torch.int64)
         t0 = time.perf_counter()
@@ -89,6 +114,16 @@ def draw_num_atoms(dataset_counts, num_crystals: int, seed: int = 0) -> np.ndarr
     return np.random.default_rng(seed).choice(counts, size=num_crystals)
 
 
+def draw_compositions(dataset, num_crystals: int, seed: int = 0):
+    """(indices, compositions) of `num_crystals` crystals of a CrystalDataset drawn with replacement, seeded by `seed`:
+    their dataset indices (int64) and their atomic-number arrays.  Drawn before sharding, like draw_num_atoms, so it
+    does not depend on the number of ranks; the indices lead back to each composition's ground-truth structure."""
+    if len(dataset) == 0:
+        raise ValueError("the data set has no crystals to draw compositions from")
+    idx = np.random.default_rng(seed).choice(len(dataset), size=num_crystals).astype(np.int64)
+    return idx, [np.asarray(dataset.configs[i].atomic_numbers, dtype=np.int64).reshape(-1) for i in idx]
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--model_path", type=str, required=True)
@@ -103,13 +138,27 @@ def main(argv=None):
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--precision", default="fp16", choices=["fp32", "fp16"])
     ap.add_argument("--symbols", nargs="*", default=None, help="constant atomic symbols (use_constant_atomic_symbols)")
+    ap.add_argument("--elements", nargs="+", default=None, metavar="SYMBOL",
+                    help="chemical system: every atom of every crystal is one of these elements")
+    ap.add_argument("--compositions_from", nargs="+", default=None, metavar="DATA",
+                    help="sample structures for compositions drawn (seeded by --seed) from these dataset files' crystals; "
+                         "the output file also holds their dataset indices as source_index")
     ap.add_argument("--out", default=f"{OUT_DIR}/crystals.h5")
     ap.add_argument("--ori_grid", default=None, help=".npy [16,3] (or .npz with key ori_grid): the orientation grid the "
                     "model was trained with; a reference checkpoint does not carry it (quirk B2)")
     ap.add_argument("--no_strict", action="store_true", help="tolerate model tensors missing from the checkpoint")
     args = ap.parse_args(argv)
-    counts = None
-    if args.num_atoms_from is not None:
+    counts = compositions = source_index = None
+    if args.compositions_from is not None:
+        for opt in ("num_atoms", "num_atoms_from", "symbols", "elements"):
+            if getattr(args, opt) is not None:
+                ap.error(f"--compositions_from cannot be combined with --{opt} (the compositions fix counts and types)")
+        from .diffusion.lattice_dataset import CrystalDataset
+        source_index, compositions = draw_compositions(CrystalDataset(args.compositions_from), args.num_crystals,
+                                                       args.seed)
+    elif args.elements is not None and args.symbols is not None:
+        ap.error("--elements cannot be combined with --symbols (constant symbols fix the types)")
+    elif args.num_atoms_from is not None:
         if args.num_atoms is not None:
             ap.error("--num_atoms_from cannot be combined with --num_atoms")
         if args.symbols is not None:
@@ -131,9 +180,12 @@ def main(argv=None):
     model = PONITA_DIFFUSION.load_from_checkpoint(args.model_path, ori_grid=grid, strict=not args.no_strict,
                                                   precision=args.precision)
     res = generate_n_crystals(model, args.num_crystals, args.num_atoms, args.symbols, args.batch, device=dev,
-                              seed=args.seed, out_path=args.out, num_atoms=counts, keyed_noise=args.keyed_noise)
+                              seed=args.seed, num_atoms=counts, keyed_noise=args.keyed_noise, elements=args.elements,
+                              compositions=compositions)
     if not dist.is_initialized() or dist.get_rank() == 0:
-        print(f"wrote {res.num_atoms.shape[0]} crystals ({res.frac_x.shape[0]} atoms)")
+        extra = {} if source_index is None else {"source_index": source_index}
+        path = save_sample_results_to_hdf5(res, args.out, extra)
+        print(f"wrote {res.num_atoms.shape[0]} crystals ({res.frac_x.shape[0]} atoms) to {path}")
     if dist.is_initialized():
         dist.destroy_process_group()
 

@@ -9,7 +9,8 @@ conditions and the cell volume is at least 0.1 A^3 (CDVAE's `structure_validity`
 values into the valid fractions and the Wasserstein-1 distances of density, element count and atom count against a
 reference set (the data the model was trained on, or its test split).  `quality_record` is the compact subset that
 train.fit's sample-quality monitoring logs per pass (the per-crystal rows of all ranks are gathered with
-distributed.gather_crystal_metrics first).  Compositional validity (oxidation states),
+distributed.gather_crystal_metrics first).  `system_fractions` checks generated crystals against a chemical system
+(generate --elements) on the host.  Compositional validity (oxidation states),
 coverage, novelty and uniqueness need pymatgen / SMACT / CrystalNN and are not computed here."""
 from __future__ import annotations
 
@@ -23,7 +24,7 @@ import torch
 
 from .. import _lib
 from ..diffusion.diffusion_loss import SampleResult
-from ..tools.atomic_number_table import ATOMIC_MASS
+from ..tools.atomic_number_table import ATOMIC_MASS, ATOMIC_NUMBER
 from .process_generated_crystals import load_sample_results_from_hdf5
 
 # bits of CrystalMetrics.flags (ARREAU_METRICS_* in include/arreau_b200.h)
@@ -200,6 +201,29 @@ def summarize(generated: CrystalMetrics, reference: Optional[CrystalMetrics] = N
     return out
 
 
+def system_fractions(atomic_numbers, num_atoms, elements) -> dict:
+    """How well crystals stored back to back (atomic_numbers[N], num_atoms[G]) keep to the chemical system `elements`
+    (element symbols): frac_in_system, the share of crystals whose every atom is an element of the system, and
+    frac_full_system, the share in which every element of the system occurs (None for no crystals).  Host only."""
+    unknown = [e for e in elements if e not in ATOMIC_NUMBER]
+    if unknown or len(elements) == 0:
+        raise ValueError(f"not a chemical system: unknown element symbols {unknown}" if unknown else "empty chemical system")
+    system = np.unique([ATOMIC_NUMBER[e] for e in elements])
+    z = np.asarray(atomic_numbers, dtype=np.int64).reshape(-1)
+    na = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
+    if int(na.sum()) != z.shape[0] or np.any(na < 0):
+        raise ValueError(f"num_atoms (sum {int(na.sum())}) does not describe {z.shape[0]} atoms")
+    G = int(na.shape[0])
+    crystal = np.repeat(np.arange(G), na)
+    inside = np.isin(z, system)
+    outside = np.zeros(G, dtype=np.int64)
+    np.add.at(outside, crystal, ~inside)
+    present = np.zeros((G, system.size), dtype=np.bool_)
+    present[crystal[inside], np.searchsorted(system, z[inside])] = True
+    return dict(frac_in_system=_frac(int((outside == 0).sum()), G),
+                frac_full_system=_frac(int(present.all(axis=1).sum()), G))
+
+
 METRIC_FIELDS = ("num_atoms", "volume", "min_dist", "density", "num_elements", "flags")
 _FIELD_DTYPES = (np.int64, np.float64, np.float64, np.float64, np.int32, np.int32)
 # the compact record of one sample-quality pass of train.fit (its `sample_quality` history): the epoch and these keys
@@ -233,11 +257,16 @@ def main(argv=None):
     ap.add_argument("--reference", nargs="+", default=None, metavar="DATA",
                     help="dataset files (.h5 as written by prep_datasets.py, or .npz) to compare the distributions with")
     ap.add_argument("--json", default=None, metavar="PATH", help="also write the summary as JSON")
+    ap.add_argument("--elements", nargs="+", default=None, metavar="SYMBOL",
+                    help="chemical system the crystals were generated in: adds frac_in_system and frac_full_system")
     args = ap.parse_args(argv)
     from ..diffusion.lattice_dataset import CrystalDataset
-    generated = crystal_metrics(*sample_inputs(args.samples))
+    inputs = sample_inputs(args.samples)
+    generated = crystal_metrics(*inputs)
     reference = crystal_metrics(*dataset_inputs(CrystalDataset(args.reference))) if args.reference else None
     summary = summarize(generated, reference)
+    if args.elements:
+        summary.update(system_fractions(inputs[2], inputs[3], args.elements))
     for k, v in summary.items():
         print(f"{k}: {v}")
     if args.json:

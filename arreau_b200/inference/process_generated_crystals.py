@@ -6,6 +6,7 @@ part of this image -- the same five arrays under the same keys ("crystals/<name>
 from __future__ import annotations
 
 import os
+from typing import Optional
 
 import numpy as np
 
@@ -22,18 +23,21 @@ def _have_h5py() -> bool:
         return False
 
 
-def save_sample_results_to_hdf5(crystals: SampleResult, filename: str) -> str:
-    """process_generated_crystals.py:8-15.  Returns the path actually written (".npz" replaces ".h5" without h5py)."""
+def save_sample_results_to_hdf5(crystals: SampleResult, filename: str, extra: Optional[dict] = None) -> str:
+    """process_generated_crystals.py:8-15.  Returns the path actually written (".npz" replaces ".h5" without h5py).
+    `extra`: further arrays stored next to the five (e.g. `source_index` of generate --compositions_from); readers
+    that take the five keys are unaffected."""
     os.makedirs(os.path.dirname(os.path.abspath(filename)) or ".", exist_ok=True)
+    arrays = {**{k: getattr(crystals, k) for k in KEYS}, **(extra or {})}
     if _have_h5py() and not filename.endswith(".npz"):
         import h5py
         with h5py.File(filename, "w") as file:
             group = file.create_group("crystals")
-            for k in KEYS:
-                group.create_dataset(k, data=getattr(crystals, k))
+            for k, v in arrays.items():
+                group.create_dataset(k, data=v)
         return filename
     path = filename if filename.endswith(".npz") else os.path.splitext(filename)[0] + ".npz"
-    np.savez(path, **{f"crystals/{k}": np.asarray(getattr(crystals, k)) for k in KEYS})
+    np.savez(path, **{f"crystals/{k}": np.asarray(v) for k, v in arrays.items()})
     return path
 
 

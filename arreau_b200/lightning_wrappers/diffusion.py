@@ -17,7 +17,8 @@ import torch.nn as nn
 from ..diffusion.diffusion_helpers import GaussianFourierProjection
 from ..diffusion.diffusion_loss import DiffusionLoss, SampleResult
 from ..ponita.models.ponita import PonitaFiberBundle
-from ..tools.atomic_number_table import AtomicNumberTable, atomic_symbols_to_indices
+from ..tools.atomic_number_table import (AtomicNumberTable, allowed_states_of_elements, atomic_numbers_to_states,
+                                         atomic_symbols_to_indices)
 
 t_emb_dim = 64          # lightning_wrappers/diffusion.py:22-23
 fourier_scale = 16
@@ -77,12 +78,31 @@ class PONITA_DIFFUSION(nn.Module):
     # ---- sampling (:220-253) ------------------------------------------------------------------------------------------
     @torch.no_grad()
     def sample(self, num_atoms_per_sample: int, num_samples_in_batch: int, visualization_setting=None,
-               show_bonds: bool = False, use_constant_atomic_symbols: Optional[list] = None, **kw) -> SampleResult:
+               show_bonds: bool = False, use_constant_atomic_symbols: Optional[list] = None, elements=None,
+               compositions=None, **kw) -> SampleResult:
+        """:220-253, plus two ways to choose the chemistry (the model itself is unconditional):
+        `elements`: element symbols of one chemical system for every crystal, or a list of one system per crystal; the
+        type update chooses only among them (DiffusionLoss.sample's `allowed_states`).
+        `compositions`: one array of atomic numbers per crystal; it fixes that crystal's atom count and types, which
+        stay constant through the trajectory (crystal structure prediction; use_constant_atomic_symbols with one
+        composition per crystal).  Neither can be combined with use_constant_atomic_symbols or the other."""
         z_table = AtomicNumberTable(self.z_table_zs.tolist())
         constant_atoms = None
+        if sum(x is not None for x in (use_constant_atomic_symbols, elements, compositions)) > 1:
+            raise ValueError("use_constant_atomic_symbols, elements and compositions exclude each other")
         if use_constant_atomic_symbols is not None:
             constant_atoms = torch.as_tensor(np.repeat(atomic_symbols_to_indices(z_table, use_constant_atomic_symbols).numpy(),
                                                        num_samples_in_batch))
+        if compositions is not None:
+            comps = [np.asarray(c, dtype=np.int64).reshape(-1) for c in compositions]
+            if len(comps) != num_samples_in_batch or any(c.size == 0 for c in comps):
+                raise ValueError(f"compositions must hold {num_samples_in_batch} non-empty atomic-number arrays")
+            if kw.get("num_atoms") is not None:
+                raise ValueError("compositions fix the atom counts: they cannot be combined with num_atoms")
+            constant_atoms = torch.from_numpy(atomic_numbers_to_states(z_table, np.concatenate(comps)))
+            kw["num_atoms"] = torch.tensor([c.size for c in comps], dtype=torch.int64)
+        if elements is not None:
+            kw["allowed_states"] = allowed_states_of_elements(z_table, elements, num_samples_in_batch)
         return self.diffusion_loss.sample(model=self, z_table=z_table, t_emb_weights=self.t_emb,
                                           num_atoms_per_sample=num_atoms_per_sample,
                                           num_samples_in_batch=num_samples_in_batch, constant_atoms=constant_atoms, **kw)

@@ -56,3 +56,39 @@ def atomic_numbers_to_indices(z_table: AtomicNumberTable, atomic_numbers) -> tor
 def atomic_symbols_to_indices(z_table: AtomicNumberTable, atomic_symbols) -> torch.Tensor:
     """tools/atomic_number_table.py:84-89."""
     return atomic_numbers_to_indices(z_table, [ATOMIC_NUMBER[s] for s in atomic_symbols])
+
+
+def allowed_states_of_elements(z_table: AtomicNumberTable, elements, num_crystals: int) -> np.ndarray:
+    """The allowed-state mask of chemical-system-constrained sampling (DiffusionLoss.sample's `allowed_states`): bool
+    [Z] for one system -- a sequence of element symbols -- or [num_crystals, Z] for one system per crystal.  The mask
+    state (the table's last entry) is left out, so every atom ends on an element of its system.  ValueError names a
+    symbol that is not an element the model can emit, and refuses an empty system."""
+    def one(symbols) -> np.ndarray:
+        if isinstance(symbols, str) or not all(isinstance(e, str) for e in symbols):
+            raise ValueError(f"a chemical system is a list of element symbols, got {symbols!r}")
+        if len(symbols) == 0:
+            raise ValueError("empty chemical system")
+        index = {z: i for i, z in enumerate(z_table.zs[:-1])}
+        m = np.zeros(len(z_table), dtype=np.bool_)
+        for e in symbols:
+            if ATOMIC_NUMBER.get(e) not in index:
+                raise ValueError(f"element {e!r} is not one the model can generate (its z_table has "
+                                 f"{len(index)} elements)")
+            m[index[ATOMIC_NUMBER[e]]] = True
+        return m
+    elements = list(elements)
+    if all(isinstance(e, str) for e in elements):
+        return one(elements)
+    if len(elements) != num_crystals:
+        raise ValueError(f"{len(elements)} chemical systems for {num_crystals} crystals")
+    return np.stack([one(e if isinstance(e, str) else list(e)) for e in elements])
+
+
+def atomic_numbers_to_states(z_table: AtomicNumberTable, atomic_numbers) -> np.ndarray:
+    """Atom states (z_table indices, int64) of atomic numbers; ValueError names those the model cannot emit."""
+    a = np.asarray(atomic_numbers, dtype=np.int64).reshape(-1)
+    index = {z: i for i, z in enumerate(z_table.zs[:-1])}
+    missing = sorted({int(z) for z in a} - set(index))
+    if missing:
+        raise ValueError(f"atomic numbers {missing} are not elements the model can generate")
+    return np.asarray([index[int(z)] for z in a], dtype=np.int64)

@@ -341,6 +341,23 @@ int arreau_d3pm_reverse(const int64_t* types, const float* logits, const double*
                         double onestep_to_mask, int32_t num_steps, int32_t num_atoms_total, int32_t num_states,
                         int64_t* types_out, void* stream);
 
+/* The same step with the states restricted per crystal (chemical-system-constrained sampling).  allowed[G][4] u32:
+ * bit d of allowed[4 g + d / 32] admits state d for the atoms of crystal g = crystal_of_atom[b] (bits at d >= Z are
+ * ignored; a crystal with no bit below Z is unconstrained).  For an atom of crystal g with allowed set A:
+ *   1. the x0 probabilities are the softmax of the logits over A; states outside A have probability 0 (this feeds
+ *      sum_nomask, p_mask and f2);
+ *   2. the candidates of the argmax are A plus the mask state Z-1 at t >= 2 (the absorbing state: a masked atom may stay
+ *      masked) and A alone at t == 1.  States outside A are excluded explicitly: their posterior
+ *      log(f1 + eps) + log(0 + eps) is finite, so the Gumbel noise could still select them;
+ *   3. with every one of the Z bits set the output is bit-identical to arreau_d3pm_reverse.
+ * A set without the mask bit ends every atom on an element of A.  Same checks and error codes as arreau_d3pm_reverse,
+ * and ARREAU_ERR_NULL for a NULL crystal_of_atom or allowed (N > 0). */
+int arreau_d3pm_reverse_allowed(const int64_t* types, const float* logits, const double* u, const int32_t* t_of_atom,
+                                int32_t t, const double* q_keep, const double* q_to_mask, double onestep_keep,
+                                double onestep_to_mask, int32_t num_steps, int32_t num_atoms_total, int32_t num_states,
+                                const int32_t* crystal_of_atom, const uint32_t* allowed, int64_t* types_out,
+                                void* stream);
+
 /* Counter-based noise for throughput runs (the reference draws torch CPU noise, SURVEY 3.1): fills
  * z_len[G,3], z_frac[N,3] with N(0,1) and u[N,Z] with U[0,1) from Philox4x32-10 keyed by (seed, step). */
 int arreau_step_noise(uint64_t seed, int32_t step, int32_t num_crystals, int32_t num_atoms_total,
@@ -370,7 +387,9 @@ int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t num_crystals,
                               const int32_t* crystal_of_atom, double* z_len, double* z_frac, double* u, void* stream);
 
 /* One whole denoise step (the body of the sampler loop, diffusion_loss.py:319-349), every kernel
- * above on one stream with no host synchronisation.  State is updated in place. */
+ * above on one stream with no host synchronisation.  State is updated in place.
+ * ABI note: allowed_states was appended after update_types, so the fields before it keep their offsets; a caller must
+ * zero-initialise it (or set it) -- a struct of the earlier size is read past its end. */
 typedef struct arreau_step_args {
   /* state, fp64 / i64, updated in place */
   double* frac;            /* [N,3]   */
@@ -419,6 +438,8 @@ typedef struct arreau_step_args {
   double radius;
   int32_t precision;
   int32_t update_types;    /* 0: keep types (constant_atoms mode, diffusion_loss.py:348-349) */
+  const uint32_t* allowed_states; /* [G][4] device, or NULL (unconstrained): per-crystal allowed states of the type
+                                     update (see arreau_d3pm_reverse_allowed) */
 } arreau_step_args;
 
 int arreau_denoise_step(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
