@@ -48,7 +48,8 @@ class StepArgs(C.Structure):
         ("onestep_keep", f64), ("onestep_to_mask", f64),
         ("vp_cx0", f64), ("vp_cxt", f64), ("vp_denom", f64), ("vp_var", f64),
         ("emb", i32), ("num_steps", i32), ("t", i32), ("cap", i32), ("radius", f64),
-        ("precision", i32), ("update_types", i32), ("allowed_states", vp)]
+        ("precision", i32), ("update_types", i32), ("allowed_states", vp),
+        ("known_atom", vp), ("known_frac", vp), ("known_crystal", vp), ("known_lengths", vp), ("vp_alpha_bars", vp)]
 
 
 class StepReplay(C.Structure):
@@ -106,6 +107,9 @@ SIGNATURES = {
     "arreau_ve_pbc_reverse": [vp, vp, vp, vp, i32, vp, i32, vp, vp],
     "arreau_d3pm_reverse": [vp, vp, vp, vp, i32, vp, vp, f64, f64, i32, i32, i32, vp, vp],
     "arreau_d3pm_reverse_allowed": [vp, vp, vp, vp, i32, vp, vp, f64, f64, i32, i32, i32, vp, vp, vp, vp],
+    "arreau_vp_lattice_reverse_known": [vp, vp, vp, vp, i32, f64, f64, f64, f64, i32, vp, vp, vp, vp, vp],
+    "arreau_ve_pbc_reverse_known": [vp, vp, vp, vp, i32, vp, i32, vp, vp, vp, vp],
+    "arreau_d3pm_reverse_known": [vp, vp, vp, vp, i32, vp, vp, f64, f64, i32, i32, i32, vp, vp, vp, vp, vp],
     "arreau_step_noise": [C.c_uint64, i32, i32, i32, i32, vp, vp, vp, vp],
     "arreau_sample_init_keyed": [C.c_uint64, i32, i32, vp, vp, vp, f64, vp, vp, vp, vp],
     "arreau_sample_noise_keyed": [C.c_uint64, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp],

@@ -107,16 +107,39 @@ assemble_features_kernel(const double* __restrict__ frac, const int64_t* __restr
 }
 
 // diffusion/diffusion_helpers.py:185-199
+//
+// kKnown: a crystal g with known_crystal[g] != 0 has known lengths l0 = known_lengths[g] (structure-conditioned
+// sampling, RePaint replacement).  Its reverse update is discarded and replaced by a draw of the forward process at the
+// new level, q(x_{t-1} | l0) = sqrt(abar[t-1]) l0 + sqrt(1 - abar[t-1]) z with the step's own noise z and the fp32
+// abar table -- the arithmetic of vp_lattice_forward_kernel, so the two are bit-identical -- and l0 itself at t == 1.
+// The instance without it compiles to the code it had before the condition existed.
+template <bool kKnown>
 __global__ void vp_lattice_reverse_kernel(const double* lengths, const float* __restrict__ len0,
                                           const int32_t* __restrict__ atom_offset, const double* __restrict__ z,
                                           int t, double cx0, double cxt, double denom, double var, int G,
-                                          double* out, const double* __restrict__ dyn) {   // out may alias lengths
+                                          double* out, const double* __restrict__ dyn,   // out may alias lengths
+                                          const int32_t* __restrict__ known_crystal,
+                                          const double* __restrict__ known_lengths,
+                                          const float* __restrict__ alpha_bars) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= 3 * G) return;
   if (dyn) {      // replayable step: {t, cx0, cxt, denom, var} of the current replay live in device memory
     t = (int)dyn[0]; cx0 = dyn[1]; cxt = dyn[2]; denom = dyn[3]; var = dyn[4];
   }
   const int g = idx / 3;
+  if constexpr (kKnown) {
+    if (known_crystal[g]) {
+      const double l0 = known_lengths[idx];
+      if (t >= 2) {
+        const float ab = alpha_bars[t - 1];                           // fp32 table (quirk B1)
+        const double s1 = (double)sqrtf(ab), s2 = (double)sqrtf(1.0f - ab);
+        out[idx] = __dadd_rn(__dmul_rn(s1, l0), __dmul_rn(s2, z[idx]));
+      } else {
+        out[idx] = l0;
+      }
+      return;
+    }
+  }
   const double n = (double)(atom_offset[g + 1] - atom_offset[g]);
   const double pred = __dmul_rn((double)len0[idx], n);            // diffusion_loss.py:338
   const double mean = __ddiv_rn(__dadd_rn(__dmul_rn(cx0, pred), __dmul_rn(cxt, lengths[idx])), denom);
@@ -132,13 +155,26 @@ __device__ __forceinline__ double torch_remainder1(double a) {
 }
 
 // diffusion/diffusion_helpers.py:65-81
+//
+// kKnown: an atom b with known_atom[b] != 0 has a known position x0 = known_frac[b] in [0,1)^3.  Its reverse update is
+// replaced by q(x_{t-1} | x0) = (x0 + z sigma[t-1]) mod 1 with the step's own noise z -- the arithmetic of
+// ve_pbc_forward_kernel at level t-1, so the two are bit-identical -- and by x0 itself at t == 1.
+template <bool kKnown>
 __global__ void ve_pbc_reverse_kernel(const double* frac, const float* __restrict__ score,
                                       const double* __restrict__ z, const int32_t* __restrict__ t_of_atom,
                                       int t_scalar, const double* __restrict__ sigmas, int N,
-                                      double* out) {   // out may alias frac
+                                      double* out,   // out may alias frac
+                                      const int32_t* __restrict__ known_atom, const double* __restrict__ known_frac) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= 3 * N) return;
   const int t = t_of_atom ? t_of_atom[idx / 3] : t_scalar;
+  if constexpr (kKnown) {
+    if (known_atom[idx / 3]) {
+      const double x0 = known_frac[idx];
+      out[idx] = t >= 2 ? torch_remainder1(__dadd_rn(x0, __dmul_rn(z[idx], sigmas[t - 1]))) : x0;
+      return;
+    }
+  }
   const double s = sigmas[t];
   const double a = (t == 0) ? 0.0 : sigmas[t - 1];
   const double s2 = __dmul_rn(s, s), a2 = __dmul_rn(a, a);
@@ -160,17 +196,28 @@ __global__ void ve_pbc_reverse_kernel(const double* frac, const float* __restric
 //      log(f1 + eps) + log(0 + eps), which the Gumbel noise could lift above the others;
 //   3. with every state in A the result is bit-identical to the unconstrained kernel (the arithmetic is the same).
 // The unconstrained instantiation compiles to the code it had before the constraint existed.
-template <bool kAllowed>
+//
+// kKnown: an atom b with known_atom[b] != 0 keeps its state at every step, t == 1 included (structure-conditioned
+// sampling: its type is part of the known structure).  Without the override the t == 1 argmax would sample it from the
+// logits, and at t >= 2 the finite log(0 + eps) term would still let it flip.
+template <bool kAllowed, bool kKnown>
 __global__ void __launch_bounds__(256)
 d3pm_reverse_kernel(const int64_t* types, const float* __restrict__ logits,
                     const double* __restrict__ u, const int32_t* __restrict__ t_of_atom, int t_scalar,
                     const double* __restrict__ q_keep, const double* __restrict__ q_to_mask,
                     double onestep_keep, double onestep_to_mask, int T, int N, int Z,
                     int64_t* out,   // out may alias types
-                    const int32_t* __restrict__ crystal_of_atom, const uint32_t* __restrict__ allowed) {
+                    const int32_t* __restrict__ crystal_of_atom, const uint32_t* __restrict__ allowed,
+                    const int32_t* __restrict__ known_atom) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= N) return;
   const int b = warp;
+  if constexpr (kKnown) {
+    if (known_atom[b]) {
+      if (lane == 0) out[b] = types[b];
+      return;
+    }
+  }
   const int t = t_of_atom ? t_of_atom[b] : t_scalar;
   const int xt = (int)types[b];
   const int mask = Z - 1;
@@ -319,39 +366,91 @@ extern "C" int arreau_assemble_features(const double* frac, const int64_t* types
   return ARREAU_OK;
 }
 
+namespace {
+
+int launch_vp_lattice_reverse(const double* lengths, const float* len0, const int32_t* atom_offset, const double* z,
+                              int32_t t, double cx0, double cxt, double denom, double var, int32_t G, const double* dyn,
+                              const int32_t* known_crystal, const double* known_lengths, const float* alpha_bars,
+                              double* lengths_out, void* stream) {
+  const unsigned blocks = (unsigned)((3 * G + 127) / 128);
+  if (known_crystal)
+    vp_lattice_reverse_kernel<true><<<blocks, 128, 0, (cudaStream_t)stream>>>(
+        lengths, len0, atom_offset, z, t, cx0, cxt, denom, var, G, lengths_out, dyn, known_crystal, known_lengths,
+        alpha_bars);
+  else
+    vp_lattice_reverse_kernel<false><<<blocks, 128, 0, (cudaStream_t)stream>>>(
+        lengths, len0, atom_offset, z, t, cx0, cxt, denom, var, G, lengths_out, dyn, nullptr, nullptr, nullptr);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+int launch_ve_pbc_reverse(const double* frac, const float* score, const double* z, const int32_t* t_of_atom, int32_t t,
+                          const double* ve_sigmas, int32_t N, const int32_t* known_atom, const double* known_frac,
+                          double* frac_out, void* stream) {
+  if (N == 0) return ARREAU_OK;
+  if (!frac || !score || !z || !ve_sigmas || !frac_out) return ARREAU_ERR_NULL;
+  if (N < 0) return ARREAU_ERR_BAD_SHAPE;
+  const unsigned blocks = (unsigned)((3 * N + 255) / 256);
+  if (known_atom)
+    ve_pbc_reverse_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(frac, score, z, t_of_atom, t, ve_sigmas, N,
+                                                                         frac_out, known_atom, known_frac);
+  else
+    ve_pbc_reverse_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(frac, score, z, t_of_atom, t, ve_sigmas, N,
+                                                                          frac_out, nullptr, nullptr);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+}  // namespace
+
 extern "C" int arreau_vp_lattice_reverse(const double* lengths, const float* len0, const int32_t* atom_offset,
                                          const double* z, int32_t t, double cx0, double cxt, double denom,
                                          double var, int32_t G, double* lengths_out, void* stream) {
   if (G == 0) return ARREAU_OK;
   if (!lengths || !len0 || !atom_offset || !lengths_out || (t > 1 && !z)) return ARREAU_ERR_NULL;
   if (G < 0) return ARREAU_ERR_BAD_SHAPE;
-  vp_lattice_reverse_kernel<<<(3 * G + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-      lengths, len0, atom_offset, z, t, cx0, cxt, denom, var, G, lengths_out, nullptr);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  return launch_vp_lattice_reverse(lengths, len0, atom_offset, z, t, cx0, cxt, denom, var, G, nullptr, nullptr, nullptr,
+                                   nullptr, lengths_out, stream);
 }
 
-// the same with the timestep and the four posterior coefficients read from device memory (arreau_denoise_step_replay)
+extern "C" int arreau_vp_lattice_reverse_known(const double* lengths, const float* len0, const int32_t* atom_offset,
+                                               const double* z, int32_t t, double cx0, double cxt, double denom,
+                                               double var, int32_t G, const int32_t* known_crystal,
+                                               const double* known_lengths, const float* vp_alpha_bars,
+                                               double* lengths_out, void* stream) {
+  if (G == 0) return ARREAU_OK;
+  if (!lengths || !len0 || !atom_offset || !lengths_out || (t > 1 && !z)) return ARREAU_ERR_NULL;
+  if (!known_crystal || !known_lengths || !vp_alpha_bars) return ARREAU_ERR_NULL;
+  if (G < 0) return ARREAU_ERR_BAD_SHAPE;
+  return launch_vp_lattice_reverse(lengths, len0, atom_offset, z, t, cx0, cxt, denom, var, G, nullptr, known_crystal,
+                                   known_lengths, vp_alpha_bars, lengths_out, stream);
+}
+
+// the same with the timestep and the four posterior coefficients read from device memory (arreau_denoise_step_replay);
+// known_crystal NULL: no known lattice
 int arreau_vp_lattice_reverse_dyn(const double* lengths, const float* len0, const int32_t* atom_offset, const double* z,
-                                  const double* dyn, int32_t G, double* lengths_out, void* stream) {
+                                  const double* dyn, int32_t G, const int32_t* known_crystal,
+                                  const double* known_lengths, const float* vp_alpha_bars, double* lengths_out,
+                                  void* stream) {
   if (G == 0) return ARREAU_OK;
   if (!lengths || !len0 || !atom_offset || !lengths_out || !z || !dyn) return ARREAU_ERR_NULL;
-  vp_lattice_reverse_kernel<<<(3 * G + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-      lengths, len0, atom_offset, z, 0, 0.0, 0.0, 1.0, 0.0, G, lengths_out, dyn);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  if (known_crystal && (!known_lengths || !vp_alpha_bars)) return ARREAU_ERR_NULL;
+  return launch_vp_lattice_reverse(lengths, len0, atom_offset, z, 0, 0.0, 0.0, 1.0, 0.0, G, dyn, known_crystal,
+                                   known_lengths, vp_alpha_bars, lengths_out, stream);
 }
 
 extern "C" int arreau_ve_pbc_reverse(const double* frac, const float* score, const double* z,
                                      const int32_t* t_of_atom, int32_t t, const double* ve_sigmas, int32_t N,
                                      double* frac_out, void* stream) {
-  if (N == 0) return ARREAU_OK;
-  if (!frac || !score || !z || !ve_sigmas || !frac_out) return ARREAU_ERR_NULL;
-  if (N < 0) return ARREAU_ERR_BAD_SHAPE;
-  ve_pbc_reverse_kernel<<<(3 * N + 255) / 256, 256, 0, (cudaStream_t)stream>>>(frac, score, z, t_of_atom, t,
-                                                                                ve_sigmas, N, frac_out);
-  CUDA_LAUNCH_CHECK();
-  return ARREAU_OK;
+  return launch_ve_pbc_reverse(frac, score, z, t_of_atom, t, ve_sigmas, N, nullptr, nullptr, frac_out, stream);
+}
+
+extern "C" int arreau_ve_pbc_reverse_known(const double* frac, const float* score, const double* z,
+                                           const int32_t* t_of_atom, int32_t t, const double* ve_sigmas, int32_t N,
+                                           const int32_t* known_atom, const double* known_frac, double* frac_out,
+                                           void* stream) {
+  if (N != 0 && (!known_atom || !known_frac)) return ARREAU_ERR_NULL;
+  return launch_ve_pbc_reverse(frac, score, z, t_of_atom, t, ve_sigmas, N, known_atom, known_frac, frac_out, stream);
 }
 
 namespace {
@@ -359,20 +458,22 @@ namespace {
 int launch_d3pm_reverse(const int64_t* types, const float* logits, const double* u, const int32_t* t_of_atom, int32_t t,
                         const double* q_keep, const double* q_to_mask, double onestep_keep, double onestep_to_mask,
                         int32_t num_steps, int32_t N, int32_t Z, const int32_t* crystal_of_atom, const uint32_t* allowed,
-                        int64_t* types_out, void* stream) {
+                        const int32_t* known_atom, int64_t* types_out, void* stream) {
   if (N == 0) return ARREAU_OK;
   if (!types || !logits || !u || !q_keep || !q_to_mask || !types_out) return ARREAU_ERR_NULL;
   if (N < 0 || Z <= 1 || Z > 128 || num_steps <= 0) return ARREAU_ERR_BAD_SHAPE;
   const long long threads = (long long)N * 32;
   const unsigned blocks = (unsigned)((threads + 255) / 256);
-  if (allowed)
-    d3pm_reverse_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-        types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps, N, Z, types_out,
-        crystal_of_atom, allowed);
-  else
-    d3pm_reverse_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-        types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask, num_steps, N, Z, types_out,
-        nullptr, nullptr);
+  cudaStream_t s = (cudaStream_t)stream;
+#define ARREAU_D3PM_LAUNCH(A, K)                                                                                      \
+  d3pm_reverse_kernel<A, K><<<blocks, 256, 0, s>>>(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, \
+                                                   onestep_to_mask, num_steps, N, Z, types_out, crystal_of_atom,     \
+                                                   allowed, known_atom)
+  if (allowed && known_atom) ARREAU_D3PM_LAUNCH(true, true);
+  else if (allowed) ARREAU_D3PM_LAUNCH(true, false);
+  else if (known_atom) ARREAU_D3PM_LAUNCH(false, true);
+  else ARREAU_D3PM_LAUNCH(false, false);
+#undef ARREAU_D3PM_LAUNCH
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }
@@ -384,7 +485,7 @@ extern "C" int arreau_d3pm_reverse(const int64_t* types, const float* logits, co
                                    const double* q_to_mask, double onestep_keep, double onestep_to_mask,
                                    int32_t num_steps, int32_t N, int32_t Z, int64_t* types_out, void* stream) {
   return launch_d3pm_reverse(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask,
-                             num_steps, N, Z, nullptr, nullptr, types_out, stream);
+                             num_steps, N, Z, nullptr, nullptr, nullptr, types_out, stream);
 }
 
 extern "C" int arreau_d3pm_reverse_allowed(const int64_t* types, const float* logits, const double* u,
@@ -394,5 +495,16 @@ extern "C" int arreau_d3pm_reverse_allowed(const int64_t* types, const float* lo
                                            const uint32_t* allowed, int64_t* types_out, void* stream) {
   if (N != 0 && (!crystal_of_atom || !allowed)) return ARREAU_ERR_NULL;
   return launch_d3pm_reverse(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask,
-                             num_steps, N, Z, crystal_of_atom, allowed, types_out, stream);
+                             num_steps, N, Z, crystal_of_atom, allowed, nullptr, types_out, stream);
+}
+
+extern "C" int arreau_d3pm_reverse_known(const int64_t* types, const float* logits, const double* u,
+                                         const int32_t* t_of_atom, int32_t t, const double* q_keep,
+                                         const double* q_to_mask, double onestep_keep, double onestep_to_mask,
+                                         int32_t num_steps, int32_t N, int32_t Z, const int32_t* crystal_of_atom,
+                                         const uint32_t* allowed, const int32_t* known_atom, int64_t* types_out,
+                                         void* stream) {
+  if (N != 0 && (!known_atom || (allowed && !crystal_of_atom))) return ARREAU_ERR_NULL;
+  return launch_d3pm_reverse(types, logits, u, t_of_atom, t, q_keep, q_to_mask, onestep_keep, onestep_to_mask,
+                             num_steps, N, Z, crystal_of_atom, allowed, known_atom, types_out, stream);
 }

@@ -157,7 +157,9 @@ step_advance_kernel(int32_t* __restrict__ counter, int t_first, const double* __
 }  // namespace
 
 int arreau_vp_lattice_reverse_dyn(const double* lengths, const float* len0, const int32_t* atom_offset, const double* z,
-                                  const double* dyn, int32_t G, double* lengths_out, void* stream);   // csrc/state.cu
+                                  const double* dyn, int32_t G, const int32_t* known_crystal,
+                                  const double* known_lengths, const float* vp_alpha_bars, double* lengths_out,
+                                  void* stream);   // csrc/state.cu
 
 extern "C" int arreau_abi_version(void) { return 1; }
 
@@ -382,15 +384,29 @@ int denoise_step_body(const arreau_weights* w, const arreau_workspace* ws, const
   ARREAU_TRY(arreau_ponita_forward(w, ws, a->precision, a->x, a->vec, a->row_ptr, a->src, a->dist, a->dir, a->lattice,
                                    a->atom_offset, a->crystal_of_atom, N, G, a->radius, a->logits, a->score, a->len0,
                                    stream));
-  // update: lengths, lattice, fractional coordinates, atom types   (diffusion_loss.py:338-349)
+  // update: lengths, lattice, fractional coordinates, atom types   (diffusion_loss.py:338-349); the known part of the
+  // state, if any, is overwritten inside the same kernels, so the lattice below is formed from the known lengths
   if (dyn)
-    ARREAU_TRY(arreau_vp_lattice_reverse_dyn(a->lengths, a->len0, a->atom_offset, a->z_len, dyn, G, a->lengths, stream));
+    ARREAU_TRY(arreau_vp_lattice_reverse_dyn(a->lengths, a->len0, a->atom_offset, a->z_len, dyn, G, a->known_crystal,
+                                             a->known_lengths, a->vp_alpha_bars, a->lengths, stream));
+  else if (a->known_crystal)
+    ARREAU_TRY(arreau_vp_lattice_reverse_known(a->lengths, a->len0, a->atom_offset, a->z_len, a->t, a->vp_cx0,
+                                               a->vp_cxt, a->vp_denom, a->vp_var, G, a->known_crystal, a->known_lengths,
+                                               a->vp_alpha_bars, a->lengths, stream));
   else
     ARREAU_TRY(arreau_vp_lattice_reverse(a->lengths, a->len0, a->atom_offset, a->z_len, a->t, a->vp_cx0, a->vp_cxt,
                                          a->vp_denom, a->vp_var, G, a->lengths, stream));
   ARREAU_TRY(lattice_from_angles(a, G, stream));
-  ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, t_of_atom, t, a->ve_sigmas, N, a->frac, stream));
-  if (a->update_types && a->allowed_states)
+  if (a->known_atom)
+    ARREAU_TRY(arreau_ve_pbc_reverse_known(a->frac, a->score, a->z_frac, t_of_atom, t, a->ve_sigmas, N, a->known_atom,
+                                           a->known_frac, a->frac, stream));
+  else
+    ARREAU_TRY(arreau_ve_pbc_reverse(a->frac, a->score, a->z_frac, t_of_atom, t, a->ve_sigmas, N, a->frac, stream));
+  if (a->update_types && a->known_atom)
+    ARREAU_TRY(arreau_d3pm_reverse_known(a->types, a->logits, a->u_type, t_of_atom, t, a->q_keep, a->q_to_mask,
+                                         a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->crystal_of_atom,
+                                         a->allowed_states, a->known_atom, a->types, stream));
+  else if (a->update_types && a->allowed_states)
     ARREAU_TRY(arreau_d3pm_reverse_allowed(a->types, a->logits, a->u_type, t_of_atom, t, a->q_keep, a->q_to_mask,
                                            a->onestep_keep, a->onestep_to_mask, a->num_steps, N, Z, a->crystal_of_atom,
                                            a->allowed_states, a->types, stream));

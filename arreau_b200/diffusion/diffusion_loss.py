@@ -15,7 +15,7 @@ import torch
 import torch.nn.functional as F
 
 from .. import _lib
-from ..engine import DenoiseEngine, allowed_state_words
+from ..engine import DenoiseEngine, allowed_state_words, known_lattices, known_rows
 from ..tables import POS_SIGMA_MAX, POS_SIGMA_MIN, build_tables
 from .d3pm import D3PM
 from .diffusion_helpers import VE_pbc, VP_lattice
@@ -255,7 +255,8 @@ class DiffusionLoss(torch.nn.Module):
                vis_name: str = "", visualization_setting=None, show_bonds: bool = False,
                constant_atoms: Optional[torch.Tensor] = None, num_atoms: Optional[torch.Tensor] = None,
                device="cuda", device_noise: bool = False, seed: int = 0, step_callback=None,
-               cuda_graph: bool = False, crystal_ids=None, allowed_states=None) -> SampleResult:
+               cuda_graph: bool = False, crystal_ids=None, allowed_states=None, initial_types=None,
+               known_frac=None, known_lattice=None) -> SampleResult:
         """diffusion/diffusion_loss.py:277-377.  Extra keyword-only options (defaults reproduce the reference):
         `num_atoms` a per-crystal atom-count vector, `device_noise` Philox noise generated on the GPU,
         `step_callback(timestep, engine)` called after each step (e.g. to log E/N), `cuda_graph` (needs device_noise or
@@ -267,13 +268,37 @@ class DiffusionLoss(torch.nn.Module):
         host generators (numpy, torch) are not touched; device_noise is implied.
         `allowed_states` (bool [G,Z], or [Z] for every crystal): the states each crystal's atoms may take -- the type
         update samples from the model's x0 prediction restricted to them (arreau_d3pm_reverse_allowed); leave the mask
-        state Z-1 out and every atom ends on an allowed element.  It cannot be combined with constant_atoms."""
+        state Z-1 out and every atom ends on an allowed element.  It cannot be combined with constant_atoms.
+        `initial_types` (N states): the atoms' initial states instead of the mask state Z-1; unlike constant_atoms they
+        are then updated like any state.  Used for the types of known atoms.
+        `known_frac` ([N,3], NaN rows for free atoms) and `known_lattice` ([G,3,3], NaN matrices for free crystals):
+        structure-conditioned sampling (DenoiseEngine.set_known): the known positions, with the known atoms' initial
+        states as their types, and the known lattices are imposed on every step by replacement, and are the final
+        state's.  A known atom needs a type: its initial state may not be the mask state.  A known lattice needs
+        |det| >= 0.1 A^3."""
         Z = len(z_table)
         G = num_samples_in_batch
+        na = torch.full((G,), num_atoms_per_sample) if num_atoms is None else torch.as_tensor(num_atoms).reshape(-1)
+        N = int(na.sum())
         if allowed_states is not None:         # checked before any device work
             if constant_atoms is not None:
                 raise ValueError("allowed_states restricts the type update, which constant_atoms switches off")
             allowed_state_words(allowed_states, G, Z)
+        if initial_types is not None:
+            if constant_atoms is not None:
+                raise ValueError("initial_types and constant_atoms exclude each other")
+            initial_types = torch.as_tensor(initial_types).reshape(-1).to(torch.int64)
+            if initial_types.shape[0] != N or bool(((initial_types < 0) | (initial_types >= Z)).any()):
+                raise ValueError(f"initial_types must hold {N} states in 0..{Z - 1}")
+        atom_types = (constant_atoms if constant_atoms is not None else
+                      initial_types if initial_types is not None else torch.full((N,), Z - 1))
+        if known_frac is not None:
+            _, known = known_rows(known_frac, (N, 3), "known frac")
+            untyped = torch.nonzero(known & (torch.as_tensor(atom_types).reshape(-1) == Z - 1)).reshape(-1)
+            if untyped.numel():
+                raise ValueError(f"known atom {int(untyped[0])} has no type (its initial state is the mask state)")
+        if known_lattice is not None:
+            known_lattices(known_lattice, G)
         dd = torch.float64                                     # main_diffusion_generate.py:27
         keyed = crystal_ids is not None
         if keyed:
@@ -283,11 +308,8 @@ class DiffusionLoss(torch.nn.Module):
         else:
             angles = torch.tensor([sample_bravais_angles("monoclinic") for _ in range(G)], dtype=dd)
             lengths = torch.randn([G, 3], dtype=dd)
-        na = torch.full((G,), num_atoms_per_sample) if num_atoms is None else torch.as_tensor(num_atoms).reshape(-1)
-        N = int(na.sum())
         if not keyed:
             frac_x = torch.randn([N, 3], dtype=dd) * pos_sigma_max
-        atom_types = constant_atoms if constant_atoms is not None else torch.full((N,), Z - 1)
         eng = self.engine_for(model, t_emb_weights, na, torch.device(device))
         eng.set_allowed_states(allowed_states)
         if keyed:
@@ -295,6 +317,7 @@ class DiffusionLoss(torch.nn.Module):
             eng.init_state_keyed(seed, atom_types, pos_sigma_max)
         else:
             eng.set_state(frac_x, atom_types, lengths, angles)
+        eng.set_known(known_frac, known_lattice)      # after the state: it overrides the known lattices' drawn angles
         if cuda_graph and (not (device_noise or keyed) or self.max_neighbors <= 0):
             raise ValueError("cuda_graph=True needs device_noise=True (or crystal_ids) and max_neighbors > 0")
         if cuda_graph:

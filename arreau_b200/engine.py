@@ -52,6 +52,36 @@ def allowed_state_words(mask, G: int, Z: int) -> np.ndarray:
     return np.packbits(bits.reshape(G, 4, 32), axis=-1, bitorder="little").view("<u4").reshape(G, 4)
 
 
+def known_rows(x, shape, what: str) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(values, known) of a NaN-row encoding of a known part of the state: `x` of `shape`, where a row (everything
+    past the first dimension) that is NaN throughout is free.  Returns the values as fp64 on the host and the bool mask of
+    the known rows.  ValueError on another shape, a row that is only partly NaN, or an infinite value."""
+    v = torch.as_tensor(x).detach().to("cpu", torch.float64)
+    if tuple(v.shape) != tuple(shape):
+        raise ValueError(f"{what} must have shape {list(shape)}, got {list(v.shape)}")
+    nan = torch.isnan(v.reshape(v.shape[0], -1))
+    partial = torch.nonzero(nan.any(1) & ~nan.all(1)).reshape(-1)
+    if partial.numel():
+        raise ValueError(f"{what} row {int(partial[0])} is only partly NaN (a row is either known or NaN throughout)")
+    if bool(torch.isinf(v).any()):
+        raise ValueError(f"{what} holds an infinite value")
+    return v, ~nan.all(1)
+
+
+# a known lattice must span a cell: the volume floor below which crystal_metrics counts a cell as invalid
+MIN_CELL_VOLUME = 0.1
+
+
+def known_lattices(lattice, G: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """known_rows of a [G,3,3] lattice encoding (NaN matrices for free crystals), also refusing a known lattice with
+    |det| < MIN_CELL_VOLUME (cubic angstrom)."""
+    lat, known = known_rows(lattice, (G, 3, 3), "known lattice")
+    flat = torch.nonzero(known & (torch.linalg.det(torch.nan_to_num(lat)).abs() < MIN_CELL_VOLUME)).reshape(-1)
+    if flat.numel():
+        raise ValueError(f"known lattice {int(flat[0])} has |det| < {MIN_CELL_VOLUME} A^3: not a cell")
+    return lat, known
+
+
 def _i32(a, device):
     return torch.as_tensor(np.asarray(a), dtype=torch.int32).to(device)
 
@@ -67,11 +97,12 @@ class DenoiseEngine:
                   "raw_count": ((), torch.int32), "deg": ((), torch.int32), "crystal_of_atom": ((), torch.int32),
                   "t_of_atom": ((), torch.int32), "vec": ((4, 3), torch.float32), "score": ((3,), torch.float32),
                   "h": ((NUM_ORI, HIDDEN), torch.float32), "x1": ((NUM_ORI, HIDDEN), torch.float32),
-                  "z_frac": ((3,), torch.float64)}
+                  "z_frac": ((3,), torch.float64), "known_atom": ((), torch.int32), "known_frac": ((3,), torch.float64)}
     _CRYSTAL_BUFS = {"lengths": ((3,), torch.float64), "angles": ((3,), torch.float64), "lattice": ((3, 3), torch.float64),
                      "angle_trig": ((6,), torch.float64), "num_neighbors_image": ((), torch.int64),
                      "len0": ((3,), torch.float32), "z_len": ((3,), torch.float64), "num_atoms": ((), torch.int64),
-                     "crystal_id": ((), torch.int64), "allowed_states": ((4,), torch.int32)}
+                     "crystal_id": ((), torch.int64), "allowed_states": ((4,), torch.int32),
+                     "known_crystal": ((), torch.int32), "known_lengths": ((3,), torch.float64)}
 
     def __init__(self, weights: PonitaWeights, tables: DiffusionTables, fourier_w, num_atoms: Sequence[int],
                  radius: float, max_neighbors: int, precision: str = "fp32", edge_capacity: Optional[int] = None,
@@ -122,6 +153,7 @@ class DenoiseEngine:
         self.d_vp_betas = tables.vp_betas.to(torch.float64).to(dev)
         self.d_ve_sigmas = tables.ve_sigmas.to(torch.float64).to(dev)
         self.d_q_keep, self.d_q_to_mask = tables.q_keep.to(dev), tables.q_to_mask.to(dev)
+        self.d_vp_alpha_bars = tables.vp_alpha_bars.to(torch.float32).to(dev)
         self.d_fourier_w = torch.as_tensor(np.asarray(fourier_w.detach().cpu() if isinstance(fourier_w, torch.Tensor)
                                                       else fourier_w), dtype=torch.float64).to(dev)
         if self.d_fourier_w.numel() != self.emb:
@@ -129,6 +161,7 @@ class DenoiseEngine:
         self.edge_capacity = -1
         self.G = self.N = 0
         self.constrained = False        # args.allowed_states points at the allowed_states buffer
+        self.known_atoms = self.known_crystals = False   # args.known_atom / known_crystal point at their buffers
         self._debug_flat = None
         self._alloc_edges(int(edge_capacity) if edge_capacity is not None else
                           (Nc * self.cap if self.cap > 0 else max(1, 32 * Nc)))
@@ -178,6 +211,7 @@ class DenoiseEngine:
         a, p = self.args, _lib.ptr
         a.z_len, a.z_frac, a.u_type = p(self.z_len), p(self.z_frac), p(self.u_type)
         self.set_allowed_states(None)     # a constraint belongs to the batch it was set for
+        self.set_known()                  # and so does a known part of the state
 
     # ------------------------------------------------------------------ buffers
     def _alloc_edges(self, capacity: int) -> None:
@@ -230,6 +264,9 @@ class DenoiseEngine:
         a.emb, a.num_steps, a.cap, a.radius = self.emb, self.tabs.T, self.cap, self.radius
         a.precision, a.update_types = PRECISIONS[self.precision], 1
         a.allowed_states = p("allowed_states") if self.constrained else None
+        a.known_atom = p("known_atom") if self.known_atoms else None
+        a.known_crystal = p("known_crystal") if self.known_crystals else None
+        a.known_frac, a.known_lengths, a.vp_alpha_bars = p("known_frac"), p("known_lengths"), self.d_vp_alpha_bars.data_ptr()
         self.args = a
         if self.N:                      # re-allocation of a bound engine (uncapped graphs): keep the topology's views
             self.ws.pool = _lib.ptr(self.pool)
@@ -344,6 +381,52 @@ class DenoiseEngine:
         self.allowed_states.copy_(words.pin_memory() if self.device.type == "cuda" else words, non_blocking=True)
         self.constrained = True
         self.args.allowed_states = self.allowed_states.data_ptr()
+
+    # ------------------------------------------------------------------ structure conditioning
+    def set_known(self, frac=None, lattice=None) -> None:
+        """Fix part of the structure of the bound batch (RePaint replacement, arreau_ve_pbc_reverse_known and its two
+        siblings): after every step's reverse update a known row is overwritten with a draw of the forward process at
+        the new level, made from that row's own step noise, and with the known value itself at t = 1.
+        `frac` [N,3]: the known fractional positions, NaN rows for free atoms.  They are wrapped into [0,1) here
+        (remainder, and 0 where it gives 1).  A known atom also keeps its state: the engine's current `types` of that
+        row.
+        `lattice` [G,3,3]: the known lattices, NaN matrices for free crystals.  Their lengths are packed for the update,
+        and their angles (matrix_to_params) replace the crystal's `angles` / `angle_trig` now -- so call this after
+        set_state / init_state_keyed, which draw the angles.
+        None (the default) leaves that part unconditioned; an all-NaN array runs the conditioned kernels with nothing
+        known, which gives the unconditioned result bit for bit.  The values live in buffers allocated with the engine;
+        every later step -- arreau_denoise_step and the replayed trajectory -- reads them there.  A trajectory graph
+        bakes in whether the step is conditioned, so call this before capture_trajectory_graph.  set_topology clears
+        both.  Checked by known_rows / known_lattices."""
+        a = self.args
+        stage = (lambda t: t.pin_memory()) if self.device.type == "cuda" else (lambda t: t)  # noqa: E731
+        if frac is None:
+            self.known_atoms, a.known_atom = False, None
+        else:
+            f, known = known_rows(frac, (self.N, 3), "known frac")
+            f = torch.remainder(f, 1.0)
+            # remainder gives 1.0 for a tiny negative position (-1e-20 + 1 rounds up): the same point of the torus
+            f = torch.where(known[:, None] & (f != 1.0), f, torch.zeros_like(f))
+            self.known_frac.copy_(stage(f), non_blocking=True)
+            self.known_atom.copy_(stage(known.to(torch.int32)), non_blocking=True)
+            self.known_atoms, a.known_atom = True, self.known_atom.data_ptr()
+        if lattice is None:
+            self.known_crystals, a.known_crystal = False, None
+            return
+        lat, known = known_lattices(lattice, self.G)
+        idx = torch.nonzero(known).reshape(-1)
+        if idx.numel():
+            K, dev = int(idx.numel()), self.device
+            m = lat[idx].contiguous().to(dev)
+            lengths, angles = torch.empty(K, 3, dtype=torch.float64, device=dev), torch.empty(K, 3, dtype=torch.float64,
+                                                                                               device=dev)
+            _lib.call("arreau_matrix_to_params", m.data_ptr(), K, lengths.data_ptr(), angles.data_ptr(), self.stream)
+            di = idx.to(dev)
+            self.known_lengths.index_copy_(0, di, lengths)
+            self.angles.index_copy_(0, di, angles)
+            self.angle_trig.index_copy_(0, di, angle_factors(angles.to("cpu")).to(dev))
+        self.known_crystal.copy_(stage(known.to(torch.int32)), non_blocking=True)
+        self.known_crystals, a.known_crystal = True, self.known_crystal.data_ptr()
 
     # ------------------------------------------------------------------ graph
     def _count(self) -> None:

@@ -5,6 +5,8 @@
     python -m arreau_b200.generate ... --keyed_noise      # the same crystals whatever --batch and the number of GPUs
     python -m arreau_b200.generate ... --elements Li Fe P O     # only these elements (with --num_atoms[_from])
     python -m arreau_b200.generate ... --compositions_from data/test.h5   # structures for the data's compositions
+    python -m arreau_b200.generate ... --structures_from data/test.h5 --fix_lattice       # positions in the data's cells
+    python -m arreau_b200.generate ... --structures_from data/test.h5 --fix_lattice --free_elements Li   # where Li goes
     torchrun --nproc-per-node 8 -m arreau_b200.generate ...      # crystals sharded over the GPUs, one gather at the end
 
 The reference samples 10 crystals per batch on the CPU; here a batch is as large as fits (1024 by default), every
@@ -32,7 +34,8 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
                         use_constant_atomic_symbols: Optional[list] = None, num_crystals_per_batch: int = 1024,
                         device="cuda", device_noise: bool = True, seed: int = 0, out_path: Optional[str] = None,
                         group=None, timings: Optional[dict] = None, num_atoms=None,
-                        keyed_noise: bool = False, elements=None, compositions=None) -> SampleResult:
+                        keyed_noise: bool = False, elements=None, compositions=None, lattices=None,
+                        sites=None) -> SampleResult:
     """main_diffusion_generate.py:52-94.  With torch.distributed initialised the crystals are sharded over the ranks;
     every rank returns the full gathered result and rank 0 writes `out_path`.  `timings` (optional dict) receives this
     rank's wall-clock seconds per phase: `sample` (list, one per batch), `gather`, `write`.  `num_atoms` (optional,
@@ -43,7 +46,9 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
     `elements`: one chemical system (element symbols) for every crystal, or a list of num_crystals systems, sharded
     like `num_atoms`; every atom of a crystal ends on an element of its system (PONITA_DIFFUSION.sample's `elements`).
     `compositions`: num_crystals arrays of atomic numbers; each fixes its crystal's atom count and types (crystal
-    structure prediction), so it excludes num_atoms, use_constant_atomic_symbols and elements."""
+    structure prediction), so it excludes num_atoms, use_constant_atomic_symbols and elements.
+    `lattices` (num_crystals 3x3 lattices or None) and `sites` (num_crystals (atomic_numbers, frac) pairs or None) fix
+    part of each crystal's structure (PONITA_DIFFUSION.sample's `lattices` / `sites`), sharded like `compositions`."""
     if compositions is not None:
         if num_atoms is not None or use_constant_atomic_symbols is not None or elements is not None:
             raise ValueError("compositions fix atom counts and types: they cannot be combined with num_atoms, "
@@ -64,6 +69,9 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
             raise ValueError("constant atomic symbols fix the types: they cannot be combined with elements")
         if per_crystal_elements and len(elements) != num_crystals:
             raise ValueError(f"elements must hold one system or {num_crystals} systems, got {len(elements)}")
+    for name, per_crystal in (("lattices", lattices), ("sites", sites)):
+        if per_crystal is not None and len(per_crystal) != num_crystals:
+            raise ValueError(f"{name} must hold {num_crystals} crystals, got {len(per_crystal)}")
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     lo, hi = shard_range(num_crystals, rank, world)
@@ -77,6 +85,10 @@ def generate_n_crystals(model, num_crystals: int, num_atoms_per_sample: Optional
             kw = {} if num_atoms is None else {"num_atoms": torch.from_numpy(num_atoms[b0:b0 + nb].copy())}
         if elements is not None:
             kw["elements"] = elements[b0:b0 + nb] if per_crystal_elements else elements
+        if lattices is not None:
+            kw["lattices"] = lattices[b0:b0 + nb]
+        if sites is not None:
+            kw["sites"] = sites[b0:b0 + nb]
         if keyed_noise:
             kw["crystal_ids"] = torch.arange(b0, b0 + nb, dtype=torch.int64)
         t0 = time.perf_counter()
@@ -124,6 +136,33 @@ def draw_compositions(dataset, num_crystals: int, seed: int = 0):
     return idx, [np.asarray(dataset.configs[i].atomic_numbers, dtype=np.int64).reshape(-1) for i in idx]
 
 
+def known_structures(dataset, index, fix_lattice: bool, free_elements=None):
+    """(compositions, lattices, sites) of the CrystalDataset crystals `index` for structure-conditioned generation.
+    `fix_lattice`: each crystal keeps its lattice (else None).  `free_elements` (element symbols): every atom of
+    another element keeps its dataset position as a site, and the composition lists the sites first, then the free
+    atoms, in dataset order; None leaves every position free (sites None).  ValueError names an unknown symbol."""
+    from .tools.atomic_number_table import ATOMIC_NUMBER
+    free_z = None
+    if free_elements is not None:
+        unknown = [e for e in free_elements if e not in ATOMIC_NUMBER]
+        if unknown:
+            raise ValueError(f"unknown element symbols {unknown}")
+        free_z = [ATOMIC_NUMBER[e] for e in free_elements]
+    compositions, lattices, sites = [], [], []
+    for i in index:
+        cfg = dataset.configs[int(i)]
+        z = np.asarray(cfg.atomic_numbers, dtype=np.int64).reshape(-1)
+        lattices.append(np.asarray(cfg.L0, dtype=np.float64).reshape(3, 3) if fix_lattice else None)
+        if free_z is None:
+            compositions.append(z)
+            continue
+        free = np.isin(z, free_z)
+        compositions.append(np.concatenate([z[~free], z[free]]))
+        x = np.asarray(cfg.X0, dtype=np.float64).reshape(-1, 3)
+        sites.append((z[~free], x[~free]) if (~free).any() else None)
+    return compositions, (lattices if fix_lattice else None), (sites if free_z is not None else None)
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--model_path", type=str, required=True)
@@ -143,13 +182,38 @@ def main(argv=None):
     ap.add_argument("--compositions_from", nargs="+", default=None, metavar="DATA",
                     help="sample structures for compositions drawn (seeded by --seed) from these dataset files' crystals; "
                          "the output file also holds their dataset indices as source_index")
+    ap.add_argument("--structures_from", nargs="+", default=None, metavar="DATA",
+                    help="sample structures conditioned on crystals drawn (seeded by --seed) from these dataset files: "
+                         "their compositions, and with --fix_lattice / --free_elements part of their structure; the "
+                         "output file also holds their dataset indices as source_index")
+    ap.add_argument("--fix_lattice", action="store_true",
+                    help="with --structures_from: every crystal keeps its dataset lattice (structure prediction in a "
+                         "known cell)")
+    ap.add_argument("--free_elements", nargs="+", default=None, metavar="SYMBOL",
+                    help="with --structures_from: the atoms of these elements are generated, every other atom keeps its "
+                         "dataset position (structure completion)")
     ap.add_argument("--out", default=f"{OUT_DIR}/crystals.h5")
     ap.add_argument("--ori_grid", default=None, help=".npy [16,3] (or .npz with key ori_grid): the orientation grid the "
                     "model was trained with; a reference checkpoint does not carry it (quirk B2)")
     ap.add_argument("--no_strict", action="store_true", help="tolerate model tensors missing from the checkpoint")
     args = ap.parse_args(argv)
-    counts = compositions = source_index = None
-    if args.compositions_from is not None:
+    counts = compositions = source_index = lattices = sites = None
+    if args.structures_from is None and (args.fix_lattice or args.free_elements is not None):
+        ap.error("--fix_lattice and --free_elements need --structures_from")
+    if args.structures_from is not None:
+        for opt in ("num_atoms", "num_atoms_from", "symbols", "elements", "compositions_from"):
+            if getattr(args, opt) is not None:
+                ap.error(f"--structures_from cannot be combined with --{opt} (the structures fix counts and types)")
+        if not args.fix_lattice and args.free_elements is None:
+            ap.error("--structures_from needs --fix_lattice, --free_elements or both (what to keep of each structure)")
+        from .diffusion.lattice_dataset import CrystalDataset
+        data = CrystalDataset(args.structures_from)
+        source_index, _ = draw_compositions(data, args.num_crystals, args.seed)
+        try:
+            compositions, lattices, sites = known_structures(data, source_index, args.fix_lattice, args.free_elements)
+        except ValueError as e:
+            ap.error(str(e))
+    elif args.compositions_from is not None:
         for opt in ("num_atoms", "num_atoms_from", "symbols", "elements"):
             if getattr(args, opt) is not None:
                 ap.error(f"--compositions_from cannot be combined with --{opt} (the compositions fix counts and types)")
@@ -181,7 +245,7 @@ def main(argv=None):
                                                   precision=args.precision)
     res = generate_n_crystals(model, args.num_crystals, args.num_atoms, args.symbols, args.batch, device=dev,
                               seed=args.seed, num_atoms=counts, keyed_noise=args.keyed_noise, elements=args.elements,
-                              compositions=compositions)
+                              compositions=compositions, lattices=lattices, sites=sites)
     if not dist.is_initialized() or dist.get_rank() == 0:
         extra = {} if source_index is None else {"source_index": source_index}
         path = save_sample_results_to_hdf5(res, args.out, extra)

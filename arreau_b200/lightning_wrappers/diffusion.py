@@ -24,6 +24,50 @@ t_emb_dim = 64          # lightning_wrappers/diffusion.py:22-23
 fourier_scale = 16
 
 
+def known_lattice_array(lattices, num_crystals: int) -> np.ndarray:
+    """[G,3,3] fp64 known-lattice encoding of one 3x3 lattice or None per crystal (NaN matrices for None)."""
+    lattices = list(lattices)
+    if len(lattices) != num_crystals:
+        raise ValueError(f"lattices must hold {num_crystals} entries (a 3x3 lattice or None), got {len(lattices)}")
+    out = np.full((num_crystals, 3, 3), np.nan)
+    for g, lat in enumerate(lattices):
+        if lat is not None:
+            lat = np.asarray(lat, dtype=np.float64)
+            if lat.shape != (3, 3) or not np.isfinite(lat).all():
+                raise ValueError(f"lattice of crystal {g} must be a finite 3x3 matrix, got shape {list(lat.shape)}")
+            out[g] = lat
+    return out
+
+
+def known_site_arrays(sites, num_atoms, compositions=None):
+    """(frac [N,3] fp64 with NaN rows for free atoms, atomic numbers of the known atoms in row order) of one
+    (atomic_numbers[k], frac[k,3]) or None per crystal: the sites are the crystal's first k atoms.  ValueError when a
+    crystal has fewer than k atoms, a site position is not finite, or the crystal's composition does not begin with
+    the sites' atomic numbers."""
+    num_atoms = np.asarray(num_atoms, dtype=np.int64).reshape(-1)
+    sites = list(sites)
+    if len(sites) != num_atoms.shape[0]:
+        raise ValueError(f"sites must hold {num_atoms.shape[0]} entries ((atomic_numbers, frac) or None), got {len(sites)}")
+    off = np.concatenate([[0], np.cumsum(num_atoms)])
+    frac = np.full((int(off[-1]), 3), np.nan)
+    zs = []
+    for g, site in enumerate(sites):
+        if site is None:
+            continue
+        z = np.asarray(site[0], dtype=np.int64).reshape(-1)
+        x = np.asarray(site[1], dtype=np.float64)
+        k = z.shape[0]
+        if x.shape != (k, 3) or not np.isfinite(x).all():
+            raise ValueError(f"sites of crystal {g}: frac must be a finite [{k},3] array, got shape {list(x.shape)}")
+        if k > num_atoms[g]:
+            raise ValueError(f"crystal {g} has {k} sites but only {num_atoms[g]} atoms")
+        if compositions is not None and not np.array_equal(np.asarray(compositions[g])[:k], z):
+            raise ValueError(f"crystal {g}: its composition must begin with its {k} sites' atomic numbers")
+        frac[off[g]:off[g] + k] = x
+        zs.append(z)
+    return frac, (np.concatenate(zs) if zs else np.zeros(0, dtype=np.int64))
+
+
 class PONITA_DIFFUSION(nn.Module):
     """lightning_wrappers/diffusion.py:29-106,220-253."""
 
@@ -79,13 +123,20 @@ class PONITA_DIFFUSION(nn.Module):
     @torch.no_grad()
     def sample(self, num_atoms_per_sample: int, num_samples_in_batch: int, visualization_setting=None,
                show_bonds: bool = False, use_constant_atomic_symbols: Optional[list] = None, elements=None,
-               compositions=None, **kw) -> SampleResult:
+               compositions=None, lattices=None, sites=None, **kw) -> SampleResult:
         """:220-253, plus two ways to choose the chemistry (the model itself is unconditional):
         `elements`: element symbols of one chemical system for every crystal, or a list of one system per crystal; the
         type update chooses only among them (DiffusionLoss.sample's `allowed_states`).
         `compositions`: one array of atomic numbers per crystal; it fixes that crystal's atom count and types, which
         stay constant through the trajectory (crystal structure prediction; use_constant_atomic_symbols with one
-        composition per crystal).  Neither can be combined with use_constant_atomic_symbols or the other."""
+        composition per crystal).  Neither can be combined with use_constant_atomic_symbols or the other.
+        And two ways to fix part of the structure (DiffusionLoss.sample's `known_lattice` / `known_frac`):
+        `lattices`: one 3x3 lattice (angstrom, rows are the cell vectors) or None per crystal; a given lattice is the
+        crystal's at every step and in the result (structure prediction in a known cell).
+        `sites`: one (atomic_numbers[k], frac[k,3]) or None per crystal: the crystal's first k atoms sit at these
+        positions with these elements, and the rest is generated (structure completion).  The crystal's atom count
+        must be at least k; with `compositions` the composition's first k atomic numbers must be the sites'.  Without
+        `compositions` the other atoms start masked as usual.  It cannot be combined with use_constant_atomic_symbols."""
         z_table = AtomicNumberTable(self.z_table_zs.tolist())
         constant_atoms = None
         if sum(x is not None for x in (use_constant_atomic_symbols, elements, compositions)) > 1:
@@ -103,6 +154,20 @@ class PONITA_DIFFUSION(nn.Module):
             kw["num_atoms"] = torch.tensor([c.size for c in comps], dtype=torch.int64)
         if elements is not None:
             kw["allowed_states"] = allowed_states_of_elements(z_table, elements, num_samples_in_batch)
+        if lattices is not None:
+            kw["known_lattice"] = known_lattice_array(lattices, num_samples_in_batch)
+        if sites is not None:
+            if use_constant_atomic_symbols is not None:
+                raise ValueError("use_constant_atomic_symbols cannot be combined with sites")
+            counts = (torch.as_tensor(kw["num_atoms"]).reshape(-1).numpy() if kw.get("num_atoms") is not None else
+                      np.full(num_samples_in_batch, num_atoms_per_sample, dtype=np.int64))
+            frac, site_z = known_site_arrays(sites, counts, comps if compositions is not None else None)
+            known = ~np.isnan(frac[:, 0])
+            kw["known_frac"] = torch.from_numpy(frac)
+            if compositions is None:
+                types = np.full(frac.shape[0], len(z_table) - 1, dtype=np.int64)
+                types[known] = atomic_numbers_to_states(z_table, site_z)
+                kw["initial_types"] = torch.from_numpy(types)
         return self.diffusion_loss.sample(model=self, z_table=z_table, t_emb_weights=self.t_emb,
                                           num_atoms_per_sample=num_atoms_per_sample,
                                           num_samples_in_batch=num_samples_in_batch, constant_atoms=constant_atoms, **kw)

@@ -358,6 +358,33 @@ int arreau_d3pm_reverse_allowed(const int64_t* types, const float* logits, const
                                 const int32_t* crystal_of_atom, const uint32_t* allowed, int64_t* types_out,
                                 void* stream);
 
+/* Structure-conditioned sampling (RePaint replacement): the three reverse steps above with a known part of the state.
+ * After the reverse update of timestep t, a known row is overwritten with a draw of the forward process at the new
+ * level, q(x_{t-1} | x0), whose noise is the row's own step noise (its reverse draw is discarded, so no new draws):
+ *   arreau_vp_lattice_reverse_known: a crystal g with known_crystal[g] != 0 gets
+ *     lengths'[g] = sqrt(abar[t-1]) * known_lengths[g] + sqrt(1 - abar[t-1]) * z[g] at t >= 2 (vp_alpha_bars[T+1] f32,
+ *     the arithmetic of arreau_vp_lattice_forward at level t-1: bit-identical), and known_lengths[g] at t == 1;
+ *   arreau_ve_pbc_reverse_known: an atom b with known_atom[b] != 0 gets
+ *     frac'[b] = (known_frac[b] + z[b] * ve_sigmas[t-1]) mod 1 at t >= 2 (arreau_ve_pbc_forward's frac_noisy at level
+ *     t-1: bit-identical), and known_frac[b] (in [0,1)^3) at t == 1; t is the atom's t_of_atom[b] when given;
+ *   arreau_d3pm_reverse_known: an atom with known_atom[b] != 0 keeps its state types[b] at every t; the others take
+ *     arreau_d3pm_reverse's update, or arreau_d3pm_reverse_allowed's when allowed is given (crystal_of_atom then too;
+ *     both may be NULL).
+ * Every other row is bit-identical to the entry point without the suffix.  Same checks and error codes as those, and
+ * ARREAU_ERR_NULL for a NULL known buffer or vp_alpha_bars (G, N > 0). */
+int arreau_vp_lattice_reverse_known(const double* lengths, const float* len0, const int32_t* atom_offset,
+                                    const double* z, int32_t t, double cx0, double cxt, double denom, double var,
+                                    int32_t num_crystals, const int32_t* known_crystal, const double* known_lengths,
+                                    const float* vp_alpha_bars, double* lengths_out, void* stream);
+int arreau_ve_pbc_reverse_known(const double* frac, const float* score, const double* z, const int32_t* t_of_atom,
+                                int32_t t, const double* ve_sigmas, int32_t num_atoms_total, const int32_t* known_atom,
+                                const double* known_frac, double* frac_out, void* stream);
+int arreau_d3pm_reverse_known(const int64_t* types, const float* logits, const double* u, const int32_t* t_of_atom,
+                              int32_t t, const double* q_keep, const double* q_to_mask, double onestep_keep,
+                              double onestep_to_mask, int32_t num_steps, int32_t num_atoms_total, int32_t num_states,
+                              const int32_t* crystal_of_atom, const uint32_t* allowed, const int32_t* known_atom,
+                              int64_t* types_out, void* stream);
+
 /* Counter-based noise for throughput runs (the reference draws torch CPU noise, SURVEY 3.1): fills
  * z_len[G,3], z_frac[N,3] with N(0,1) and u[N,Z] with U[0,1) from Philox4x32-10 keyed by (seed, step). */
 int arreau_step_noise(uint64_t seed, int32_t step, int32_t num_crystals, int32_t num_atoms_total,
@@ -388,8 +415,9 @@ int arreau_sample_noise_keyed(uint64_t seed, int32_t step, int32_t num_crystals,
 
 /* One whole denoise step (the body of the sampler loop, diffusion_loss.py:319-349), every kernel
  * above on one stream with no host synchronisation.  State is updated in place.
- * ABI note: allowed_states was appended after update_types, so the fields before it keep their offsets; a caller must
- * zero-initialise it (or set it) -- a struct of the earlier size is read past its end. */
+ * ABI note: allowed_states was appended after update_types, and the five known-state fields after allowed_states, so
+ * the fields before them keep their offsets; a caller must zero-initialise them (or set them) -- a struct of an
+ * earlier size is read past its end. */
 typedef struct arreau_step_args {
   /* state, fp64 / i64, updated in place */
   double* frac;            /* [N,3]   */
@@ -440,6 +468,12 @@ typedef struct arreau_step_args {
   int32_t update_types;    /* 0: keep types (constant_atoms mode, diffusion_loss.py:348-349) */
   const uint32_t* allowed_states; /* [G][4] device, or NULL (unconstrained): per-crystal allowed states of the type
                                      update (see arreau_d3pm_reverse_allowed) */
+  /* structure conditioning (see arreau_ve_pbc_reverse_known): NULL known_atom / known_crystal = nothing known */
+  const int32_t* known_atom;      /* [N] device, nonzero: the atom's position and type are known */
+  const double* known_frac;       /* [N,3] its position in [0,1)^3 */
+  const int32_t* known_crystal;   /* [G] device, nonzero: the crystal's lengths are known (its angles are a->angles) */
+  const double* known_lengths;    /* [G,3] */
+  const float* vp_alpha_bars;     /* [T+1] f32 abar table, needed with known_crystal */
 } arreau_step_args;
 
 int arreau_denoise_step(const arreau_weights* w, const arreau_workspace* ws, const arreau_step_args* a,
