@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libarreau_b200.so")
 SOURCES = ["graph.cu", "state.cu", "model_simt.cu", "model_tc.cu", "step.cu", "train_ops.cu", "train_net.cu",
-           "metrics.cu"]
+           "metrics.cu", "match.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "tc_common.cuh"),
            os.path.join(ROOT, "include", "arreau_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -10,8 +10,9 @@ values into the valid fractions and the Wasserstein-1 distances of density, elem
 reference set (the data the model was trained on, or its test split).  `quality_record` is the compact subset that
 train.fit's sample-quality monitoring logs per pass (the per-crystal rows of all ranks are gathered with
 distributed.gather_crystal_metrics first).  `system_fractions` checks generated crystals against a chemical system
-(generate --elements) on the host.  Compositional validity (oxidation states),
-coverage, novelty and uniqueness need pymatgen / SMACT / CrystalNN and are not computed here."""
+(generate --elements) on the host.  With --match the crystals are also matched against their source structures
+(structure_match.py: CSP match rate and RMSE).  Compositional validity (oxidation states), coverage, novelty and
+uniqueness need pymatgen / SMACT / CrystalNN and are not computed here."""
 from __future__ import annotations
 
 import argparse
@@ -31,7 +32,6 @@ from .process_generated_crystals import load_sample_results_from_hdf5
 VALID, UNKNOWN_ELEMENT, DEGENERATE, EXTENDED_SEARCH = 1, 2, 4, 8
 # atoms per launch: bounds the device memory of a chunk (~24 bytes per atom of input) for data sets of any size
 MAX_CHUNK_ATOMS = 1 << 22
-_OUT_BYTES = 32   # per crystal: volume, min_dist, density (f64), num_elements, flags (i32)
 
 
 @dataclass
@@ -86,18 +86,15 @@ def _rows_on(x, lo: int, hi: int, dtype: torch.dtype, dev: torch.device) -> torc
     return torch.from_numpy(a).pin_memory().to(dev, non_blocking=True)
 
 
-def crystal_metrics(frac_x, lattice, atomic_numbers, num_atoms, device="cuda", min_dist: float = 0.5,
-                    min_volume: float = 0.1, max_chunk_atoms: int = MAX_CHUNK_ATOMS) -> CrystalMetrics:
-    """Metrics of G crystals stored back to back: frac_x[N,3], lattice[G,3,3] (rows a, b, c; pos = frac @ lattice),
-    atomic_numbers[N] (Z), num_atoms[G].  Each may be a numpy array or a tensor; tensors on `device` are read in
-    place.  The crystals are processed in chunks of at most `max_chunk_atoms` atoms (a larger crystal is a chunk of
-    its own), each with one device->host read; a crystal's results do not depend on the chunking.  `min_dist` (A) and
-    `min_volume` (A^3) are the validity thresholds."""
+def _cuda_device(device, what: str) -> torch.device:
     dev = torch.device(device)
     if dev.type != "cuda":
-        raise ValueError("crystal_metrics runs on a CUDA device")
-    if dev.index is None:
-        dev = torch.device("cuda", torch.cuda.current_device())
+        raise ValueError(f"{what} runs on a CUDA device")
+    return torch.device("cuda", torch.cuda.current_device()) if dev.index is None else dev
+
+
+def _check_inputs(frac_x, lattice, atomic_numbers, num_atoms):
+    """num_atoms as int64 and the atom offsets (G + 1 prefix sums), after checking the shapes of the four arrays."""
     na = np.asarray(num_atoms.cpu() if isinstance(num_atoms, torch.Tensor) else num_atoms, dtype=np.int64).reshape(-1)
     G, N = int(na.shape[0]), int(na.sum())
     if np.any(na < 0):
@@ -109,30 +106,55 @@ def crystal_metrics(frac_x, lattice, atomic_numbers, num_atoms, device="cuda", m
         raise ValueError("at most 2^31 - 1 atoms")
     off = np.zeros(G + 1, dtype=np.int64)
     np.cumsum(na, out=off[1:])
-    views = [np.empty(G), np.empty(G), np.empty(G), np.empty(G, dtype=np.int32), np.empty(G, dtype=np.int32)]
+    return na, off
+
+
+def _run_chunked(off, max_chunk_atoms: int, dtypes, launch, dev: torch.device):
+    """Per-crystal outputs of a kernel run over chunks of crystals of at most `max_chunk_atoms` atoms by the prefix
+    sums `off` (a larger crystal is a chunk of its own).  launch(g0, g1, ptrs, stream) enqueues crystals g0:g1 with
+    one output pointer per entry of `dtypes`; the outputs of a chunk share one device buffer and one device->host
+    read.  Returns one host array per dtype."""
+    G = len(off) - 1
+    items = [np.dtype(dt).itemsize for dt in dtypes]
+    ends = np.cumsum([0] + items)
+    views = [np.empty(G, dtype=dt) for dt in dtypes]
     with torch.cuda.device(dev):
-        mass = _mass_table(dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
         g0 = 0
         while g0 < G:
             g1 = int(np.searchsorted(off, off[g0] + max_chunk_atoms, side="right")) - 1
             g1 = min(max(g1, g0 + 1), G)
-            a0, a1, Gc = int(off[g0]), int(off[g1]), g1 - g0
-            f = _rows_on(frac_x, a0, a1, torch.float64, dev)
-            lat = _rows_on(lattice, g0, g1, torch.float64, dev)
-            z = _rows_on(atomic_numbers, a0, a1, torch.int64, dev)
-            o = _rows_on((off[g0:g1 + 1] - a0).astype(np.int32), 0, Gc + 1, torch.int32, dev)
-            out = torch.empty(Gc * _OUT_BYTES, dtype=torch.uint8, device=dev)
-            parts = [out[:Gc * 8].view(torch.float64), out[Gc * 8:Gc * 16].view(torch.float64),
-                     out[Gc * 16:Gc * 24].view(torch.float64), out[Gc * 24:Gc * 28].view(torch.int32),
-                     out[Gc * 28:].view(torch.int32)]
-            _lib.call("arreau_crystal_metrics", f.data_ptr(), lat.data_ptr(), z.data_ptr(), o.data_ptr(), a1 - a0, Gc,
-                      mass.data_ptr(), mass.shape[0] - 1, float(min_dist), float(min_volume),
-                      *[p.data_ptr() for p in parts], stream)
+            Gc = g1 - g0
+            out = torch.empty(Gc * int(ends[-1]), dtype=torch.uint8, device=dev)
+            launch(g0, g1, [out[Gc * int(lo):].data_ptr() for lo in ends[:-1]], stream)
             chunk = out.cpu().numpy()
-            for v, lo, hi, item in zip(views, (0, 8, 16, 24, 28), (8, 16, 24, 28, 32), (8, 8, 8, 4, 4)):
-                v[g0:g1] = chunk[Gc * lo:Gc * hi].view(np.float64 if item == 8 else np.int32)
+            for v, lo, hi, dt in zip(views, ends[:-1], ends[1:], dtypes):
+                v[g0:g1] = chunk[Gc * lo:Gc * hi].view(dt)
             g0 = g1
+    return views
+
+
+def crystal_metrics(frac_x, lattice, atomic_numbers, num_atoms, device="cuda", min_dist: float = 0.5,
+                    min_volume: float = 0.1, max_chunk_atoms: int = MAX_CHUNK_ATOMS) -> CrystalMetrics:
+    """Metrics of G crystals stored back to back: frac_x[N,3], lattice[G,3,3] (rows a, b, c; pos = frac @ lattice),
+    atomic_numbers[N] (Z), num_atoms[G].  Each may be a numpy array or a tensor; tensors on `device` are read in
+    place.  The crystals are processed in chunks of at most `max_chunk_atoms` atoms (a larger crystal is a chunk of
+    its own), each with one device->host read; a crystal's results do not depend on the chunking.  `min_dist` (A) and
+    `min_volume` (A^3) are the validity thresholds."""
+    dev = _cuda_device(device, "crystal_metrics")
+    na, off = _check_inputs(frac_x, lattice, atomic_numbers, num_atoms)
+
+    def launch(g0, g1, outs, stream):
+        a0, a1, Gc = int(off[g0]), int(off[g1]), g1 - g0
+        f = _rows_on(frac_x, a0, a1, torch.float64, dev)
+        lat = _rows_on(lattice, g0, g1, torch.float64, dev)
+        z = _rows_on(atomic_numbers, a0, a1, torch.int64, dev)
+        o = _rows_on((off[g0:g1 + 1] - a0).astype(np.int32), 0, Gc + 1, torch.int32, dev)
+        mass = _mass_table(dev)
+        _lib.call("arreau_crystal_metrics", f.data_ptr(), lat.data_ptr(), z.data_ptr(), o.data_ptr(), a1 - a0, Gc,
+                  mass.data_ptr(), mass.shape[0] - 1, float(min_dist), float(min_volume), *outs, stream)
+
+    views = _run_chunked(off, max_chunk_atoms, (np.float64, np.float64, np.float64, np.int32, np.int32), launch, dev)
     return CrystalMetrics(num_atoms=na, volume=views[0], min_dist=views[1], density=views[2], num_elements=views[3],
                           flags=views[4])
 
@@ -259,14 +281,31 @@ def main(argv=None):
     ap.add_argument("--json", default=None, metavar="PATH", help="also write the summary as JSON")
     ap.add_argument("--elements", nargs="+", default=None, metavar="SYMBOL",
                     help="chemical system the crystals were generated in: adds frac_in_system and frac_full_system")
+    ap.add_argument("--match", action="store_true",
+                    help="match every generated crystal against its source structure (the samples' source_index into "
+                         "--reference, which must be the files generate drew from): adds match_rate and mean_rms")
     args = ap.parse_args(argv)
+    if args.match and not args.reference:
+        ap.error("--match needs --reference (the data files generate drew the compositions or structures from)")
     from ..diffusion.lattice_dataset import CrystalDataset
+    from .process_generated_crystals import load_extra_arrays
+    from .structure_match import check_source_index, match_summary, select_crystals, structure_match
     inputs = sample_inputs(args.samples)
+    ref_inputs = dataset_inputs(CrystalDataset(args.reference)) if args.reference else None
+    source_index = None
+    if args.match:
+        try:
+            source_index = check_source_index(load_extra_arrays(args.samples, ("source_index",)).get("source_index"),
+                                              len(inputs[3]), len(ref_inputs[3]))
+        except ValueError as e:
+            ap.error(str(e))
     generated = crystal_metrics(*inputs)
-    reference = crystal_metrics(*dataset_inputs(CrystalDataset(args.reference))) if args.reference else None
+    reference = crystal_metrics(*ref_inputs) if ref_inputs is not None else None
     summary = summarize(generated, reference)
     if args.elements:
         summary.update(system_fractions(inputs[2], inputs[3], args.elements))
+    if args.match:
+        summary.update(match_summary(structure_match(inputs, select_crystals(ref_inputs, source_index)), generated))
     for k, v in summary.items():
         print(f"{k}: {v}")
     if args.json:

@@ -52,6 +52,18 @@ def load_sample_results_from_hdf5(filename: str) -> SampleResult:
         return SampleResult(**{k: file["crystals"][k][:] for k in KEYS})
 
 
+def load_extra_arrays(filename: str, keys) -> dict:
+    """The arrays among `keys` stored next to the five by save_sample_results_to_hdf5(extra=...) (e.g. source_index),
+    by key; a key the file lacks is left out."""
+    if filename.endswith(".npz") or not _have_h5py():
+        path = filename if filename.endswith(".npz") else os.path.splitext(filename)[0] + ".npz"
+        z = np.load(path)
+        return {k: z[f"crystals/{k}"] for k in keys if f"crystals/{k}" in z.files}
+    import h5py
+    with h5py.File(filename, "r") as file:
+        return {k: file["crystals"][k][:] for k in keys if k in file["crystals"]}
+
+
 def get_crystal_indexes(sample_result: SampleResult, sample_idx: int):
     """process_generated_crystals.py:34-38."""
     start = sample_result.idx_start[sample_idx]

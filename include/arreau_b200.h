@@ -676,6 +676,36 @@ int arreau_crystal_metrics(const double* frac, const double* lattice, const int6
                            double* volume, double* min_dist, double* density, int32_t* num_elements, int32_t* flags,
                            void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Beyond the reference: a paired structure matcher for crystal structure prediction (match rate and
+ * RMSE, as CDVAE and DiffCSP report them with pymatgen's StructureMatcher).  No reference lines to cite.
+ * ------------------------------------------------------------------------------------------- */
+
+#define ARREAU_MATCH_MATCHED 1       /* a candidate with rms < stol exists                                   */
+#define ARREAU_MATCH_COMPOSITION 2   /* the multisets of Z differ (atom counts included); not searched       */
+#define ARREAU_MATCH_DEGENERATE 4    /* non-finite input, |det| < 0.1 A^3, an empty crystal, atoms not sorted */
+                                     /* by Z, bad offsets, or a reduction that did not converge              */
+#define ARREAU_MATCH_SEARCH_LIMIT 8  /* a length band held more than 128 lattice points, or the search box   */
+                                     /* more than 255 steps along a basis vector; not scored                 */
+#define ARREAU_MATCH_TOO_LARGE 16    /* more than 256 atoms; not searched                                    */
+
+/* Crystal g of set 1 (generated) against crystal g of set 2 (source), for g < num_pairs, as pymatgen's
+ * StructureMatcher(stol, ltol, angle_tol, scale=True, attempt_supercell=False, primitive_cell=False)
+ * .get_rms_dist(crystal1, crystal2) computes it (DiffCSP: stol 0.5, ltol 0.3, angle_tol 10 degrees); csrc/match.cu
+ * states the steps and the pymatgen function each mirrors.  Per set: frac[N,3] f64, lattice[G,3,3] f64 rows a, b, c,
+ * z[N] i64 and offset[G+1] i32 (prefix sums of the atom counts); within each crystal the atoms must be sorted by Z.
+ * Outputs per pair: rms[G] and max_dist[G], the normalised (by (n / V_avg)^(1/3)) rms and largest displacement of
+ * the candidate with the smallest rms over every lattice mapping and translation (NaN when no candidate exists or
+ * the pair was not searched); num_mappings[G], the lattice mappings found; flags[G], ARREAU_MATCH_* bits (at most
+ * one of COMPOSITION, DEGENERATE, SEARCH_LIMIT, TOO_LARGE).  Up to 256 atoms per crystal, fp64, one warp per pair;
+ * a pair's outputs depend only on that pair, bit for bit, whatever batch it is in.  stol, ltol and angle_tol must be
+ * finite and positive (ARREAU_ERR_BAD_SHAPE). */
+int arreau_structure_match(const double* frac1, const double* lattice1, const int64_t* z1, const int32_t* offset1,
+                           const double* frac2, const double* lattice2, const int64_t* z2, const int32_t* offset2,
+                           int32_t num_atoms1, int32_t num_atoms2, int32_t num_pairs, double stol, double ltol,
+                           double angle_tol, double* rms, double* max_dist, int32_t* num_mappings, int32_t* flags,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif
