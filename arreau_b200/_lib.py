@@ -138,6 +138,8 @@ SIGNATURES = {
     "arreau_crystal_metrics": [vp, vp, vp, vp, i32, i32, vp, i32, f64, f64, vp, vp, vp, vp, vp, vp],
     # structure matcher
     "arreau_structure_match": [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, f64, f64, f64, vp, vp, vp, vp, vp],
+    "arreau_structure_fit_pairs": [vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, i32, i32, vp, vp, i32, f64, f64, f64,
+                                   vp, vp, vp, vp],
 }
 RESTYPES = {"arreau_launch_count": i64, "arreau_ponita_backward_workspace_bytes": i64}
 

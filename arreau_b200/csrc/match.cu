@@ -19,6 +19,18 @@
 //                   matching is rejected here);
 //   result          the smallest rms = |dist| / sqrt(n) over every mapping and translation (first one on ties).
 //
+// Fit (arreau_structure_fit_pairs, structure_match_kernel<true>): StructureMatcher(stol, ltol, angle_tol, scale=True,
+// attempt_supercell=False, primitive_cell=False).fit(a, b), i.e. _match(..., use_rms=False, break_on_match=True), on
+// pair p = crystal index1[p] of set 1 (a, whose lattice is mapped, as struct1) and crystal index2[p] of set 2 (b).  The
+// pipeline above is unchanged; a candidate's value is max(dist) instead of the rms, the pair is matched iff some
+// candidate has max(dist) < stol, and the search stops at the first such candidate in the fixed enumeration order
+// (mappings by band index ia, ib, ic, then translations), leaving every loop warp-uniformly.  Outputs: max_dist (the
+// first value below stol, else the smallest found, NaN without a candidate), num_mappings (the mappings visited: all
+// of them when not matched) and flags.  Fit-matched implies rms-matched (rms <= max on the same candidate), not the
+// converse.  The uniqueness / novelty bookkeeping on top of it (inference/structure_match.py) is pymatgen's
+// group_structures on crystals with the same multiset of Z: with primitive_cell=False and no supercells, fit never
+// holds between different atom counts.  The kFit = false instance compiles to the same SASS as before the template.
+//
 // Layout.  Atoms are sorted by Z within each crystal (the host sorts, stably), so the element blocks of the two
 // crystals coincide when their compositions do, and atom k of either crystal has the same element.  A warp holds its
 // pair's coordinates in shared memory; per-pair and per-mapping lattice work (LLL, Niggli, the average lattice) is
@@ -446,18 +458,32 @@ __device__ __forceinline__ int block_end(const int64_t* z, int n, int b0) {
   return b1;
 }
 
+// kFit = false: pair g is crystal g of both sets, the objective is the rms (get_rms_dist).  kFit = true: pair g is
+// crystal index1[g] of set 1 (C1 crystals) against crystal index2[g] of set 2 (C2 crystals), the objective is the
+// largest distance (fit), and the search stops at the first candidate below stol; rms_out is not written.
+template <bool kFit>
 __global__ void __launch_bounds__(32) structure_match_kernel(
     const double* __restrict__ frac1, const double* __restrict__ lattice1, const int64_t* __restrict__ z1,
     const int32_t* __restrict__ offset1, const double* __restrict__ frac2, const double* __restrict__ lattice2,
     const int64_t* __restrict__ z2, const int32_t* __restrict__ offset2, int32_t N1, int32_t N2, int32_t G,
     double stol, double ltol, double angle_tol, double* __restrict__ rms_out, double* __restrict__ max_dist_out,
-    int32_t* __restrict__ num_mappings_out, int32_t* __restrict__ flags_out) {
+    int32_t* __restrict__ num_mappings_out, int32_t* __restrict__ flags_out, const int32_t* __restrict__ index1,
+    const int32_t* __restrict__ index2, int32_t C1, int32_t C2) {
   __shared__ PairSmem s;
   const int lane = threadIdx.x;
   const int g = blockIdx.x;
   if (g >= G) return;
-  const int a0 = offset1[g], a1 = offset1[g + 1], c0 = offset2[g], c1 = offset2[g + 1];
-  const bool bad_offsets = !(a0 >= 0 && a1 >= a0 && a1 <= N1 && c0 >= 0 && c1 >= c0 && c1 <= N2);
+  int x1 = g, x2 = g;                 // the crystals of the pair in set 1 and set 2
+  bool bad_index = false;
+  if constexpr (kFit) {
+    x1 = index1[g];
+    x2 = index2[g];
+    bad_index = !(x1 >= 0 && x1 < C1 && x2 >= 0 && x2 < C2);
+    if (bad_index) x1 = x2 = 0;
+  }
+  const int a0 = bad_index ? 0 : offset1[x1], a1 = bad_index ? 0 : offset1[x1 + 1];
+  const int c0 = bad_index ? 0 : offset2[x2], c1 = bad_index ? 0 : offset2[x2 + 1];
+  const bool bad_offsets = bad_index || !(a0 >= 0 && a1 >= a0 && a1 <= N1 && c0 >= 0 && c1 >= c0 && c1 <= N2);
   int flags = 0, num_mappings = 0;
   double best_rms = NAN, best_max = NAN;
   const int n = bad_offsets ? 0 : a1 - a0;
@@ -492,8 +518,8 @@ __global__ void __launch_bounds__(32) structure_match_kernel(
     for (int r = 0; r < 3; ++r)
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
-        L1[r][c] = lattice1[(int64_t)g * 9 + r * 3 + c];
-        L2[r][c] = lattice2[(int64_t)g * 9 + r * 3 + c];
+        L1[r][c] = lattice1[(int64_t)x1 * 9 + r * 3 + c];
+        L2[r][c] = lattice2[(int64_t)x2 * 9 + r * 3 + c];
         finite = finite && isfinite(L1[r][c]) && isfinite(L2[r][c]);
       }
     if (!finite || !(fabs(det3(L1)) >= kMinVolume) || !(fabs(det3(L2)) >= kMinVolume)) {
@@ -612,12 +638,13 @@ __global__ void __launch_bounds__(32) structure_match_kernel(
     }
     __syncwarp();
     double best = INFINITY, best_md = NAN;
-    for (int ia = 0; ia < cnt[0]; ++ia) {
-      for (int ib = 0; ib < cnt[1]; ++ib) {
+    bool found = false;       // kFit: a candidate below stol was found (warp-uniform); every loop ends
+    for (int ia = 0; ia < cnt[0] && !(kFit && found); ++ia) {
+      for (int ib = 0; ib < cnt[1] && !(kFit && found); ++ib) {
         if (!((s.mask[2][ia][ib >> 5] >> (ib & 31)) & 1u)) continue;
-        for (int w = 0; w < kBandCap / 32; ++w) {
+        for (int w = 0; w < kBandCap / 32 && !(kFit && found); ++w) {
           unsigned bits = s.mask[0][ib][w] & s.mask[1][ia][w];
-          while (bits) {
+          while (bits && !(kFit && found)) {
             const int ic = w * 32 + __ffs(bits) - 1;
             bits &= bits - 1;
             if (ic >= cnt[2]) break;
@@ -737,11 +764,20 @@ __global__ void __launch_bounds__(32) structure_match_kernel(
                 sq = fma(dist, dist, sq);
                 mx = fmax(mx, dist);
               }
-              const double rms = sqrt(warp_sum(sq)) / sqrt((double)n);
-              mx = warp_max(mx);
-              if (rms < best) {
-                best = rms;
-                best_md = mx;
+              if constexpr (kFit) {
+                mx = warp_max(mx);
+                if (mx < best) best = mx;
+                if (mx < stol) {
+                  found = true;
+                  break;
+                }
+              } else {
+                const double rms = sqrt(warp_sum(sq)) / sqrt((double)n);
+                mx = warp_max(mx);
+                if (rms < best) {
+                  best = rms;
+                  best_md = mx;
+                }
               }
             }
             __syncwarp();
@@ -751,13 +787,13 @@ __global__ void __launch_bounds__(32) structure_match_kernel(
     }
     if (best < INFINITY) {
       best_rms = best;
-      best_max = best_md;
+      best_max = kFit ? best : best_md;
       if (best < stol) flags = ARREAU_MATCH_MATCHED;
     }
   }
 
   if (lane == 0) {
-    rms_out[g] = best_rms;
+    if constexpr (!kFit) rms_out[g] = best_rms;
     max_dist_out[g] = best_max;
     num_mappings_out[g] = num_mappings;
     flags_out[g] = flags;
@@ -779,9 +815,30 @@ extern "C" int arreau_structure_match(const double* frac1, const double* lattice
   if (num_pairs < 0 || num_atoms1 < 0 || num_atoms2 < 0 || !(stol > 0.0) || !(ltol > 0.0) || !(angle_tol > 0.0) ||
       !isfinite(stol) || !isfinite(ltol) || !isfinite(angle_tol))
     return ARREAU_ERR_BAD_SHAPE;
-  structure_match_kernel<<<(unsigned)num_pairs, 32, 0, (cudaStream_t)stream>>>(
+  structure_match_kernel<false><<<(unsigned)num_pairs, 32, 0, (cudaStream_t)stream>>>(
       frac1, lattice1, z1, offset1, frac2, lattice2, z2, offset2, num_atoms1, num_atoms2, num_pairs, stol, ltol,
-      angle_tol, rms, max_dist, num_mappings, flags);
+      angle_tol, rms, max_dist, num_mappings, flags, nullptr, nullptr, num_pairs, num_pairs);
+  CUDA_LAUNCH_CHECK();
+  return ARREAU_OK;
+}
+
+extern "C" int arreau_structure_fit_pairs(const double* frac1, const double* lattice1, const int64_t* z1,
+                                          const int32_t* offset1, int32_t num_atoms1, int32_t num_crystals1,
+                                          const double* frac2, const double* lattice2, const int64_t* z2,
+                                          const int32_t* offset2, int32_t num_atoms2, int32_t num_crystals2,
+                                          const int32_t* index1, const int32_t* index2, int32_t num_pairs,
+                                          double stol, double ltol, double angle_tol, double* max_dist,
+                                          int32_t* num_mappings, int32_t* flags, void* stream) {
+  if (num_pairs == 0) return ARREAU_OK;
+  if (!lattice1 || !offset1 || !lattice2 || !offset2 || !index1 || !index2 || !max_dist || !num_mappings || !flags)
+    return ARREAU_ERR_NULL;
+  if ((num_atoms1 > 0 && (!frac1 || !z1)) || (num_atoms2 > 0 && (!frac2 || !z2))) return ARREAU_ERR_NULL;
+  if (num_pairs < 0 || num_atoms1 < 0 || num_atoms2 < 0 || num_crystals1 < 0 || num_crystals2 < 0 || !(stol > 0.0) ||
+      !(ltol > 0.0) || !(angle_tol > 0.0) || !isfinite(stol) || !isfinite(ltol) || !isfinite(angle_tol))
+    return ARREAU_ERR_BAD_SHAPE;
+  structure_match_kernel<true><<<(unsigned)num_pairs, 32, 0, (cudaStream_t)stream>>>(
+      frac1, lattice1, z1, offset1, frac2, lattice2, z2, offset2, num_atoms1, num_atoms2, num_pairs, stol, ltol,
+      angle_tol, nullptr, max_dist, num_mappings, flags, index1, index2, num_crystals1, num_crystals2);
   CUDA_LAUNCH_CHECK();
   return ARREAU_OK;
 }

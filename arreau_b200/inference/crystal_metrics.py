@@ -11,8 +11,10 @@ reference set (the data the model was trained on, or its test split).  `quality_
 train.fit's sample-quality monitoring logs per pass (the per-crystal rows of all ranks are gathered with
 distributed.gather_crystal_metrics first).  `system_fractions` checks generated crystals against a chemical system
 (generate --elements) on the host.  With --match the crystals are also matched against their source structures
-(structure_match.py: CSP match rate and RMSE).  Compositional validity (oxidation states), coverage, novelty and
-uniqueness need pymatgen / SMACT / CrystalNN and are not computed here."""
+(structure_match.py: CSP match rate and RMSE).  With --unique_novel they are grouped by pymatgen's
+StructureMatcher.fit (group_structures: uniqueness) and matched against the --reference crystals of the same
+composition (novelty), on the GPU matcher (structure_match.py).  Compositional validity (oxidation states) and
+coverage need SMACT / CrystalNN and are not computed here."""
 from __future__ import annotations
 
 import argparse
@@ -284,12 +286,20 @@ def main(argv=None):
     ap.add_argument("--match", action="store_true",
                     help="match every generated crystal against its source structure (the samples' source_index into "
                          "--reference, which must be the files generate drew from): adds match_rate and mean_rms")
+    ap.add_argument("--unique_novel", action="store_true",
+                    help="group the crystals with pymatgen's StructureMatcher.fit (default tolerances) and match them "
+                         "against --reference, normally the training files: adds frac_unique, frac_novel, "
+                         "frac_unique_novel and num_new_formula")
     args = ap.parse_args(argv)
     if args.match and not args.reference:
         ap.error("--match needs --reference (the data files generate drew the compositions or structures from)")
+    if args.unique_novel and not args.reference:
+        ap.error("--unique_novel needs --reference (the data files novelty is measured against, normally the "
+                 "training files)")
     from ..diffusion.lattice_dataset import CrystalDataset
     from .process_generated_crystals import load_extra_arrays
-    from .structure_match import check_source_index, match_summary, select_crystals, structure_match
+    from .structure_match import (check_source_index, match_summary, select_crystals, structure_match, unique_novel,
+                                  unique_novel_summary)
     inputs = sample_inputs(args.samples)
     ref_inputs = dataset_inputs(CrystalDataset(args.reference)) if args.reference else None
     source_index = None
@@ -306,6 +316,8 @@ def main(argv=None):
         summary.update(system_fractions(inputs[2], inputs[3], args.elements))
     if args.match:
         summary.update(match_summary(structure_match(inputs, select_crystals(ref_inputs, source_index)), generated))
+    if args.unique_novel:
+        summary.update(unique_novel_summary(unique_novel(inputs, generated, ref_inputs)))
     for k, v in summary.items():
         print(f"{k}: {v}")
     if args.json:

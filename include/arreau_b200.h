@@ -706,6 +706,23 @@ int arreau_structure_match(const double* frac1, const double* lattice1, const in
                            double angle_tol, double* rms, double* max_dist, int32_t* num_mappings, int32_t* flags,
                            void* stream);
 
+/* Pair p is crystal index1[p] of set 1 against crystal index2[p] of set 2, for p < num_pairs, as pymatgen's
+ * StructureMatcher(stol, ltol, angle_tol, scale=True, attempt_supercell=False, primitive_cell=False)
+ * .fit(crystal1, crystal2) decides it (pymatgen's defaults: stol 0.3, ltol 0.2, angle_tol 5 degrees): the steps of
+ * arreau_structure_match, with a candidate's value its largest normalised distance instead of its rms, and the search
+ * stopped at the first candidate below stol in the enumeration order; crystal1's lattice is the one mapped.  Per set:
+ * frac, lattice, z and offset as above for num_crystals crystals and num_atoms atoms; index1[P], index2[P] i32.
+ * Outputs per pair: max_dist[P], the first value below stol, else the smallest found (NaN when no candidate exists or
+ * the pair was not searched); num_mappings[P], the lattice mappings visited (all of them when not matched); flags[P],
+ * ARREAU_MATCH_* bits, MATCHED when fit holds, DEGENERATE also for an index outside its set.  The argument checks,
+ * limits and determinism are those of arreau_structure_match. */
+int arreau_structure_fit_pairs(const double* frac1, const double* lattice1, const int64_t* z1, const int32_t* offset1,
+                               int32_t num_atoms1, int32_t num_crystals1, const double* frac2, const double* lattice2,
+                               const int64_t* z2, const int32_t* offset2, int32_t num_atoms2, int32_t num_crystals2,
+                               const int32_t* index1, const int32_t* index2, int32_t num_pairs, double stol,
+                               double ltol, double angle_tol, double* max_dist, int32_t* num_mappings, int32_t* flags,
+                               void* stream);
+
 #ifdef __cplusplus
 }
 #endif
