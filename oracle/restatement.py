@@ -327,10 +327,14 @@ class DiffusionTables:
 
 def predict_scores(w: PonitaWeights, tabs: DiffusionTables, fourier_w: torch.Tensor, frac: torch.Tensor,
                    types_onehot: torch.Tensor, t: torch.Tensor, num_atoms: torch.Tensor, lengths: torch.Tensor,
-                   angles: torch.Tensor, radius: float, max_neighbors: int, return_graph: bool = False):
-    """diffusion/diffusion_loss.py:112-197."""
+                   angles: torch.Tensor, radius: float, max_neighbors: int, return_graph: bool = False,
+                   lattice: Optional[torch.Tensor] = None):
+    """diffusion/diffusion_loss.py:112-197.  `lattice` [G,3,3], when given, replaces lattice_from_params(lengths,
+    angles): a caller comparing with another implementation passes that implementation's lattice, because its sin/cos
+    may differ in the last bit, and the mirror images of an atom are exactly as far away as each other, so which of
+    such a pair the neighbour cap keeps is decided by that bit."""
     G = num_atoms.shape[0]
-    lat = lattice_from_params(lengths, angles)
+    lat = lattice_from_params(lengths, angles) if lattice is None else lattice
     tt = tabs.vp_betas[t].view(-1, 1)
     t_emb = fourier_time_embedding(tt, fourier_w)
     rep = lambda a: torch.repeat_interleave(a, num_atoms, dim=0)

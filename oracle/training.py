@@ -6,13 +6,16 @@ the random draws INJECTED (timestep per crystal, eps_x, u_type, eps_len -- in th
 `draw_training_noise`), and obtains the parameter gradients with torch autograd on the restated forward
 (oracle/restatement.py: ponita_forward), like the reference's `loss.backward()`.
 
+`ponita_vjp` gives the network's parameter gradients for arbitrary output cotangents, computed crystal slice by
+crystal slice, so that each output's share of the backward can be checked on its own and at full batch size.
+
 Pinning: oracle/gen_golden.py::gen_training runs the LIVE reference's DiffusionLoss.__call__ + backward on the
 same seeded batch, asserts this restatement equal (loss <= 1e-12, grads <= 1e-9 relative) and writes
 tests/golden/train_c5small.npz.
 """
 from __future__ import annotations
 
-from typing import Dict, Tuple
+from typing import Dict, List, Mapping, Optional, Sequence, Tuple
 
 import torch
 
@@ -149,6 +152,83 @@ def training_grads(w: R.PonitaWeights, *args, **kw) -> Tuple[torch.Tensor, Dict[
     grads = torch.autograd.grad(loss, [leaves[k] for k in names], allow_unused=True)
     g = {k: (torch.zeros_like(leaves[k]) if gv is None else gv) for k, gv in zip(names, grads)}
     return loss.detach(), g, {k: (v.detach() if isinstance(v, torch.Tensor) else v) for k, v in parts.items()}
+
+
+def ponita_vjp(w: R.PonitaWeights, tabs: R.DiffusionTables, fourier_w, frac, types, t_atom, num_atoms, lengths, angles,
+               radius: float, max_neighbors: int, cotangents: Sequence[Tuple[Optional[torch.Tensor], ...]],
+               slice_crystals: Optional[int] = None, lattice: Optional[torch.Tensor] = None):
+    """Vector-Jacobian products of R.predict_scores at one noised state: for every cotangent set (dscore[N,3],
+    dlogits[N,Z], dlen0[G,3]; None = zero) the parameter gradients of <dscore, score> + <dlogits, logits> +
+    <dlen0, len0>, i.e. autograd with those grad_outputs.  frac[N,3], types[N] (states, one-hot encoded here),
+    t_atom[N], num_atoms[G], lengths / angles [G,3]; lattice [G,3,3] as in R.predict_scores.
+
+    Computed as a sum over slices of `slice_crystals` whole crystals (default: the whole batch in one slice), one
+    forward per slice and one backward per cotangent set.  This is exact, not an approximation: no edge crosses a
+    crystal and every pooling is per crystal, so each slice is a batch of its own and the gradient of the batch is the
+    sum of the slices' gradients.
+
+    Returns (outputs {score, logits, len0} of the whole batch, [{param name: gradient}] per cotangent set, the graph:
+    edge_index [2,E] with global atom indices (row 0 sender, row 1 receiver) and cell_offsets [E,3])."""
+    num_atoms = torch.as_tensor(num_atoms, dtype=torch.long)
+    G = int(num_atoms.shape[0])
+    off = [0] + torch.cumsum(num_atoms, 0).tolist()
+    step = G if slice_crystals is None else max(1, int(slice_crystals))
+    onehot = torch.nn.functional.one_hot(torch.as_tensor(types, dtype=torch.long), tabs.Z).to(frac.dtype)
+    t_atom = torch.as_tensor(t_atom, dtype=torch.long)
+    leaves = {k: v.detach().clone().requires_grad_(True) for k, v in w.sd.items()}
+    w2 = R.PonitaWeights(leaves, w.ori_grid, w.radius, w.num_layers)
+    names = list(leaves)
+    grads = [{k: torch.zeros_like(leaves[k]) for k in names} for _ in cotangents]
+    outs: Dict[str, list] = {"score": [], "logits": [], "len0": []}
+    edges = []
+    for g0 in range(0, G, step):
+        g1 = min(G, g0 + step)
+        a0, a1 = off[g0], off[g1]
+        score, logits, len0, graph = R.predict_scores(w2, tabs, fourier_w, frac[a0:a1], onehot[a0:a1], t_atom[a0:a1],
+                                                      num_atoms[g0:g1], lengths[g0:g1], angles[g0:g1], radius,
+                                                      max_neighbors, return_graph=True,
+                                                      lattice=None if lattice is None else lattice[g0:g1])
+        edges.append((graph[0] + a0, graph[1]))
+        for name, v in (("score", score), ("logits", logits), ("len0", len0)):
+            outs[name].append(v.detach())
+        for i, cot in enumerate(cotangents):
+            pairs = [(y, c[rows]) for y, c, rows in zip((score, logits, len0), cot,
+                                                        (slice(a0, a1), slice(a0, a1), slice(g0, g1))) if c is not None]
+            if not pairs:
+                continue
+            gs = torch.autograd.grad([y for y, _ in pairs], [leaves[k] for k in names], [c.to(y.dtype) for y, c in pairs],
+                                     retain_graph=i + 1 < len(cotangents), allow_unused=True)
+            for k, gv in zip(names, gs):
+                if gv is not None:
+                    grads[i][k] += gv
+    graph = ((torch.cat([e for e, _ in edges], 1), torch.cat([c for _, c in edges])) if edges else
+             (torch.zeros(2, 0, dtype=torch.long), torch.zeros(0, 3, dtype=frac.dtype)))
+    return {k: torch.cat(v) for k, v in outs.items()}, grads, graph
+
+
+def gradient_blocks(shapes: Mapping[str, Sequence[int]], num_states: int, num_scalar: int
+                    ) -> List[Tuple[str, List[Tuple[str, tuple]]]]:
+    """A partition of every parameter element into the blocks a gradient is compared by: (block name, [(parameter
+    name, index into that tensor)]).  Each read-out layer's weight and bias rows are split by the output they produce
+    (logits rows [0, Z), the score row Z, the len0 rows Z+1..Z+3), a row's weight and bias in one block: the lattice
+    term otherwise dominates the tensor and hides the others, and the score bias alone nearly cancels over the
+    orientation grid.  x_embedder.weight is split into its scalar and its vector columns.  Every other tensor is one
+    block."""
+    Z, F = num_states, num_scalar
+    blocks = []
+    for k in shapes:
+        if k.startswith("read_out_layers.") and k.endswith(".bias"):
+            continue
+        if k.startswith("read_out_layers.") and k.endswith(".weight"):
+            kb = k[: -len("weight")] + "bias"
+            for out, rows in (("logits", slice(0, Z)), ("score", slice(Z, Z + 1)), ("len0", slice(Z + 1, Z + 4))):
+                blocks.append((f"{k[: -len('.weight')]}[{out}]", [(k, (rows, slice(None))), (kb, (rows,))]))
+        elif k == "x_embedder.weight":
+            blocks.append((k + "[scalar]", [(k, (slice(None), slice(0, F)))]))
+            blocks.append((k + "[vector]", [(k, (slice(None), slice(F, None)))]))
+        else:
+            blocks.append((k, [(k, (Ellipsis,))]))
+    return blocks
 
 
 def calibrate(w: R.PonitaWeights, x, vec, edge_index, dists, direction, lattice, batch, num_graphs) -> Dict[str, torch.Tensor]:
